@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — PHOENIX NeuralODE hot path on B200: gene-steps/s (forward solve + adjoint) at the genome-scale shape.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3], the configuration the metric "at ~11k genes" is quoted on; SURVEY.md 8d C4):
 ODENet(ndim=11165, neurons=200); one step = one training-step batch of the hot path = 17 independent samples, each
@@ -18,6 +18,10 @@ e2e     the same step through the public Python API from pinned HOST buffers, H2
         identical solves) + backward; the literal per-sample loop over phoenix_b200.odeint_adjoint is timed beside it
         (e2e.per_sample_api_value).
 N > 1   weak scaling: every rank runs its own 17 samples, then ONE NCCL sum-allreduce of the flat gradient.
+
+--dump-outputs DIR writes what the last timed step of `value` computed as float32 DIR/<name>.npy (38 MB): y [17, 2, 1, G]
+(the solution at both output times), adj_y0 [17, 1, G] (d loss / d y0) and grad_<parameter> (the six parameter gradients,
+summed over the ranks).  The inputs are seeded, so two builds can be compared output for output.
 """
 import argparse
 import ctypes
@@ -28,6 +32,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 REPO = os.path.dirname(os.path.abspath(__file__))
@@ -342,6 +347,12 @@ def run_ours(args):
     sampler = ClockSampler(local, rank)
     sampler.start()
     ms_res = timed(lambda: step_resident(True), args.steps)
+    outputs = None
+    if args.dump_outputs:   # copied now: the dense-weight leg below reuses these buffers
+        outputs = {"y": yout, "adj_y0": adj_y0}
+        for (name, _), g in zip(net.named_parameters(), engine.split_flat_grads(gsum, G, H)):
+            outputs["grad_" + name.replace(".", "_")] = g
+        outputs = {k: v.cpu().numpy() for k, v in outputs.items()}
     evals = 0
     for i in range(BATCH):
         evals += int(st_f[i, 3]) + int(st_a[i, 3])
@@ -535,6 +546,10 @@ def run_ours(args):
                                            peak_source=("MEASURED_PEAKS.json bf16_tflops / 2" if peaks
                                                         else "fallback 1590 / 2"))
         print(json.dumps(line), flush=True)
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -546,7 +561,11 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)

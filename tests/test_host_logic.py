@@ -102,9 +102,12 @@ def test_flat_grad_layout_matches_reference_parameter_order():
     assert torch.equal(torch.cat([v.reshape(-1) for v in views]), flat)
 
 
-def test_checkpoint_round_trip(tmp_path):
+def test_checkpoint_round_trip(tmp_path, monkeypatch):
+    # save() inserts the suffixes at the first '.' of the whole path, as the reference does (odenet.py:100-111), so a
+    # '.' in a directory name would misplace the files: work with a bare file name inside tmp_path
+    monkeypatch.chdir(tmp_path)
     net = small_net()
-    fp = os.path.join(str(tmp_path), "model.pt")
+    fp = "model.pt"
     net.save(fp)
     for suffix in ("_prods", "_sums", "_alpha_comb", "_gene_multipliers"):
         assert os.path.exists(os.path.join(str(tmp_path), "model" + suffix + ".pt"))

@@ -1,17 +1,10 @@
-"""CPU: the input pipeline (phoenix_b200/io.py, SURVEY 8 f4) against the reference's own readers on the SHIPPED files
-(build container only: /root/reference is not on the GPU box) and on synthetic files (everywhere)."""
+"""CPU: the input pipeline (phoenix_b200/io.py, SURVEY 8 f4) on synthetic files."""
 import os
-import sys
-import types
 
 import numpy as np
-import pytest
 import torch
 
 from phoenix_b200 import io as pio
-
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference checkout (build container only)")
 
 
 def _write_expression_csv(path, dim, lengths, rng):
@@ -48,34 +41,3 @@ def test_read_prior_matrix_dense_and_triplets(tmp_path):
     np.savetxt(t, np.array([[2, 4, 1.0], [5, 1, -0.5]]), delimiter=",")
     assert torch.equal(pio.read_prior_matrix(t, sparse=True, num_genes=5), torch.from_numpy(m).float())
 
-
-@needs_ref
-@pytest.mark.parametrize("rel", ["pramila_yeast_data/clean_data/pramila_500genes_1sample_24T.csv",
-                                 "breast_cancer_data/clean_data/desmedt_500genes_1TESTsample_8middleT.csv"])
-def test_readcsv_identical_to_the_reference(rel):
-    sys.path.insert(0, REF + "/ode_net/code")
-    try:
-        saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "csvreader" or k.startswith("torchdiffeq")}
-        import csvreader as ref
-    finally:
-        sys.path.remove(REF + "/ode_net/code")
-    a = ref.readcsv(os.path.join(REF, rel), "cpu", noise_to_add=0, scale_expression=1)
-    b = pio.readcsv(os.path.join(REF, rel), "cpu", 0, 1)
-    for k in list(sys.modules):
-        if k == "csvreader" or k.startswith("torchdiffeq"):
-            sys.modules.pop(k)
-    sys.modules.update(saved)
-    assert a[4:6] == b[4:6]
-    for i in (0, 2, 6):
-        for x, y in zip(a[i], b[i]):
-            assert x.dtype == y.dtype and np.array_equal(x, y, equal_nan=True)
-    for i in (1, 3, 7):
-        for x, y in zip(a[i], b[i]):
-            assert x.dtype == y.dtype and torch.equal(x, y)
-
-
-@needs_ref
-def test_read_prior_matrix_identical_to_the_reference_on_the_shipped_prior():
-    fp = REF + "/ground_truth_simulator/clean_data/edge_prior_matrix_G350_noise_0.0.csv"
-    ref = torch.from_numpy(np.genfromtxt(fp, delimiter=",")).float()      # train_insilico.py:66-68
-    assert torch.equal(pio.read_prior_matrix(fp), ref)

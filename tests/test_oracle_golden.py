@@ -10,8 +10,19 @@ RHS = [m["name"] for m in manifest("rhs")]
 SOLVE = [m for m in manifest("solve")]
 
 
+@pytest.fixture
+def golden_threads():
+    """Sets the number of torch CPU threads for one test.  MKL splits the reductions of a matmul by thread count, so the
+    bit-exact comparisons run with the counts the goldens were generated with (tests/golden/make_golden.py): 8 for the
+    RHS cases, 1 for the stored solves."""
+    saved = torch.get_num_threads()
+    yield torch.set_num_threads
+    torch.set_num_threads(saved)
+
+
 @pytest.mark.parametrize("name", RHS)
-def test_rhs_and_vjp_match_reference_autograd(name):
+def test_rhs_and_vjp_match_reference_autograd(name, golden_threads):
+    golden_threads(8)
     d = load(name)
     w = weights_of(d)
     y, g = torch.from_numpy(d["y"]), torch.from_numpy(d["g"])
@@ -28,7 +39,8 @@ def test_rhs_and_vjp_match_reference_autograd(name):
 
 
 @pytest.mark.parametrize("m", SOLVE, ids=[m["name"] for m in SOLVE])
-def test_solve_and_adjoint_match_reference(m):
+def test_solve_and_adjoint_match_reference(m, golden_threads):
+    golden_threads(1)
     d = load(m["name"])
     w = weights_of(d)
     y0, t = torch.from_numpy(d["y0"]), torch.from_numpy(d["t"])
