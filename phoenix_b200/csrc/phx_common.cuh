@@ -301,8 +301,11 @@ static inline size_t phx_rows_smem_layout(int nCTA, int K2, int gpc, int adjoint
     t.sp = take(sizeof(float) * RMx * K2);
     t.xv = adjoint ? take(sizeof(float) * 2 * RMx * K2) : none;
     // cross-group fold buffer [ngg/2][RM][K2] followed by the J partials [nqw][gpc][RM]: together they are the scratch
-    // of the theta passes (per-gene activation tables rebuilt from the stored stage inputs)
-    t.red = take(sizeof(float) * (ngg / 2) * RMx * K2);
+    // of the theta passes (per-gene activation tables rebuilt from the stored stage inputs).  The adjoint's state-cotangent
+    // pass keeps its v partials [nqw][gpc][RM] in the fold buffer (the u partials sit in the J partials): it must hold
+    // them too, or a CTA with more than (ngg/2) K2 / nqw genes overwrites its own u partials.
+    const size_t fold = (size_t)(ngg / 2) * K2, vpart = adjoint ? (size_t)nqw * gpc : 0;
+    t.red = take(sizeof(float) * RMx * (fold > vpart ? fold : vpart));
     t.jred = take(sizeof(float) * nqw * RMx * gpc);
     if (adjoint) {
         const size_t have = off - t.red, need = 2 * sizeof(float) * PHX_ROWS_NFS * RMx * gpc;

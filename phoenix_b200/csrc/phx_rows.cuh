@@ -127,8 +127,10 @@ struct RowsView {
     __device__ __forceinline__ float* fgj() const { return s.at<float>(p.so.FGJ); }
     __device__ __forceinline__ float* fm() const { return s.at<float>(p.so.FM); }
     __device__ __forceinline__ const float4* w1() const { return s.at<float4>(p.so.w1r); }
-    __device__ __forceinline__ uint32_t col_fsp(int fs, int b) const { return tq + (uint32_t)(p.tm_fac + (fs * RM + b) * 4); }
-    __device__ __forceinline__ uint32_t col_fg(int fs, int b) const { return tq + (uint32_t)(p.tm_fac + ((NFS + fs) * RM + b) * 4); }
+    // K2-long factor tables in tensor memory, row by row: row b (b < p.rows) owns 2 x NFS slots of 4 columns, so the
+    // rows of a pass take the 2 * NFS * 4 * rows columns phx_rows_plan budgets beside the WA slice
+    __device__ __forceinline__ uint32_t col_fsp(int fs, int b) const { return tq + (uint32_t)(p.tm_fac + (b * 2 * NFS + fs) * 4); }
+    __device__ __forceinline__ uint32_t col_fg(int fs, int b) const { return tq + (uint32_t)(p.tm_fac + (b * 2 * NFS + NFS + fs) * 4); }
 };
 
 // one-time staging: constants, the W1 slice (rows padded to w1_stride float4), the WA slice (shared or tensor memory)
@@ -864,7 +866,7 @@ __device__ __forceinline__ void rows_adj_eval(const ResParams& __restrict__ p, S
 #pragma unroll
             for (int b = 0; b < RM; ++b) {
                 const int fs = rc->r[b].fslot[sid];
-                if (fs >= 0) {   // uniform over the warp
+                if (b < p.rows && fs >= 0) {   // uniform over the warp
                     tm_st4(v.col_fsp(fs, b), fok ? stage4[b * K2q + fq] : zero4());
                     tm_st4(v.col_fg(fs, b), fok ? xv4[b * K2q + fq] : zero4());
                 }
@@ -1235,12 +1237,13 @@ __device__ __noinline__ double rows_theta_zero_norm(const ResParams& __restrict_
         const RowCtl& c = rc->r[v.gg];
         const int f1 = c.fslot[sid1], f0 = sid0 >= 0 ? c.fslot[sid0] : c.fslot[sid1];
         float4 sp1, sp0, g1, g0;
-        tm_ld4(v.col_fsp(f1, v.gg), sp1);
-        tm_ld4(v.col_fsp(f0, v.gg), sp0);
-        tm_ld4(v.col_fg(f1, v.gg), g1);
-        tm_ld4(v.col_fg(f0, v.gg), g0);
+        const int bt = v.gg < p.rows ? v.gg : 0;   // the rows a pass does not hold have no factor columns (val stays 0)
+        tm_ld4(v.col_fsp(f1, bt), sp1);
+        tm_ld4(v.col_fsp(f0, bt), sp0);
+        tm_ld4(v.col_fg(f1, bt), g1);
+        tm_ld4(v.col_fg(f0, bt), g0);
         double val[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};   // sp11 sp10 sp00 | gs11 gs10 gs00 | gp11 gp10 gp00
-        if (v.qok) {
+        if (v.qok && v.gg < p.rows) {
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const double a1 = comp4(sp1, e), a0 = comp4(sp0, e), b1 = comp4(g1, e), b0 = comp4(g0, e);
@@ -1330,7 +1333,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
         v.fm()[i] = 0.f;
     }
     if (v.warp < 4) {
-        for (int c = 0; c < 2 * NFS * RM; ++c) tm_st4(v.tq + (uint32_t)(p.tm_fac + 4 * c), zero4());
+        for (int c = 0; c < 2 * NFS * p.rows; ++c) tm_st4(v.tq + (uint32_t)(p.tm_fac + 4 * c), zero4());
         tm_wait_st();
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
