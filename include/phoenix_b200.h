@@ -177,6 +177,19 @@ int phx_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, co
                       const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                       void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                       int steplog_cap, void* stream);
+/* ---- adjoint parameters (adjoint.py:185-193: the members of adjoint_params that require grad) -------------------------
+ * The *_masked variants of the adjoint entry points take param_mask, a 6-bit set of parameters in reference order: bit
+ * i = the i-th of (gene_multipliers, Wp, bp, Ws, bs, Wa), PHX_PARAMS_ALL = all six (what the unmasked entry points
+ * pass).  Only the cotangents of the parameters in the mask are integrated, and only they make up the parameter block of
+ * the error norm (count = their total size; with an empty mask the block is absent).  The blocks of grads_flat outside
+ * the mask are written as zeros (phx_unpack_grads_masked with accumulate != 0 leaves them as they are).  A mask outside
+ * 0 .. 0x3F returns PHX_ERR_INVALID. */
+#define PHX_PARAMS_ALL 0x3F
+int phx_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                             int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                             const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                             void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                             int steplog_cap, int param_mask, void* stream);
 
 /* ---- N independent problems per launch (the per-sample loop of training_step, train_insilico.py:128-130) -------- */
 /* Problem i: initial state y0 + i*B*G, its own T increasing times t_host[i*T .. i*T+T), outputs y_out + i*T*B*G, its own
@@ -192,6 +205,11 @@ int phx_solve_adjoint_many(phx_ctx* ctx, int G, int H, int B, int N, const float
                            int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                            void* workspace, size_t workspace_bytes, phx_status* status, void* stream);
+int phx_solve_adjoint_many_masked(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host,
+                                  int T, int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                  void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
+                                  void* stream);
 
 /* ---- the same two solves for ANY number of rows B (streaming engine) ---------------------------------------- */
 /* phx_solve_forward / phx_solve_adjoint keep the whole solve in one persistent cooperative launch and need the rows
@@ -219,6 +237,11 @@ int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* pac
                              const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                              void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                              int steplog_cap, void* stream);
+int phx_stream_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                                    int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                    const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                    void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                    int steplog_cap, int param_mask, void* stream);
 
 /* ---- the sample loop of training_step as rows of ONE launch (train_insilico.py:128-130) ------------------------------- */
 /* N independent ONE-ROW problems (y0 [N][G], each with its own T increasing times t_host[i*T .. i*T+T), its own dopri5 step
@@ -248,10 +271,17 @@ int phx_solve_adjoint_rows(phx_ctx* ctx, int G, int H, int N, const float* packe
                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
                            void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                            int steplog_cap, void* stream);
+int phx_solve_adjoint_rows_masked(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
+                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
+                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                  int steplog_cap, int param_mask, void* stream);
 size_t phx_packed_grad_bytes(int G, int H);
 int phx_rows_grad_parts(const phx_ctx* ctx, int G, int H, int N);
 int phx_unpack_grads(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
                      int accumulate, void* stream);
+int phx_unpack_grads_masked(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
+                            int accumulate, int param_mask, void* stream);
 /* Cotangent of the data loss of training_step, loss = torch.mean((predictions - targets)**2) (train_insilico.py:132):
  * grad[r][g] = scale * (pred[r][g] - target[r][g]) for `rows` samples of G genes, scale = 2 / (rows * G); pred and grad
  * rows are pred_stride / grad_stride floats apart (the t1 slices of the [N][T][G] solver output and of grad_y), target is

@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(_HERE, "libphoenix_b200.so")
 
 PHX_OK = 0
 METHOD_IDS = {"euler": 0, "midpoint": 1, "rk4": 2, "dopri5": 3}
+PARAMS_ALL = 0x3F   # adjoint parameter mask: bit i = the i-th ODENet parameter in reference order
 PREC_FP32, PREC_TF32, PREC_3XTF32 = 0, 1, 3
 ST_OK, ST_DT_UNDERFLOW, ST_NONFINITE, ST_MAX_STEPS, ST_RUNNING = 0, 1, 2, 3, 99
 
@@ -25,6 +26,8 @@ EXPORTS = [
     "phx_stream_workspace_bytes", "phx_stream_solve_forward", "phx_stream_solve_adjoint",
     "phx_rows_supported", "phx_rows_plan_describe", "phx_rows_workspace_bytes", "phx_solve_forward_rows",
     "phx_solve_adjoint_rows", "phx_unpack_grads", "phx_packed_grad_bytes", "phx_rows_grad_parts",
+    "phx_solve_adjoint_masked", "phx_solve_adjoint_many_masked", "phx_stream_solve_adjoint_masked",
+    "phx_solve_adjoint_rows_masked", "phx_unpack_grads_masked",
     "phx_prior_loss", "phx_prior_setup", "phx_tc_set_pair", "phx_tc_prof_dump", "phx_ctx_set_global_norm", "phx_peer_allreduce", "phx_peer_allreduce_nvls", "phx_mse_grad", "phx_hill_planes", "phx_hill_cache_set",
 ]
 
@@ -132,6 +135,12 @@ def _declare(lib):
     lib.phx_rows_grad_parts.argtypes = [c_void_p, c_int, c_int, c_int]
     lib.phx_rows_grad_parts.restype = c_int
     lib.phx_unpack_grads.restype = c_int
+    # the *_masked variants: one int param_mask before the stream argument
+    for name in ("phx_solve_adjoint", "phx_solve_adjoint_many", "phx_stream_solve_adjoint", "phx_solve_adjoint_rows",
+                 "phx_unpack_grads"):
+        fn = getattr(lib, name + "_masked")
+        fn.argtypes = getattr(lib, name).argtypes[:-1] + [c_int, c_void_p]
+        fn.restype = c_int
     lib.phx_prior_loss.argtypes = [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, ctypes.c_float, c_void_p,
                                    c_void_p, c_void_p, c_size_t, c_void_p]
     lib.phx_prior_loss.restype = c_int

@@ -65,14 +65,15 @@ __global__ void pack_kernel(int G, int H, int Hp, int K2, const float* __restric
 // packed-layout cotangents (phx_packed_grad_offsets) -> the reference's flat order (phx_grad_offsets).  The two branch
 // matrices are transposed ([G][K2] gene-major -> [H][G]) through a 32 x 33 shared-memory tile so that both the reads
 // (along k) and the writes (along g) are coalesced.
+// Blocks outside `mask` (PHX_P_*) are not read: they are written as zeros, or left as they are when accumulating.
 __global__ void unpack_w1_kernel(int G, int H, int Hp, int K2, const float* __restrict__ w1bar, int nparts, size_t pstride,
-                                 float* __restrict__ Ws, float* __restrict__ Wp, int accumulate) {
+                                 float* __restrict__ Ws, float* __restrict__ Wp, int accumulate, int mask) {
     __shared__ float tile[32][33];
     const int g0 = blockIdx.x * 32, k0 = blockIdx.y * 32;
     for (int r = threadIdx.y; r < 32; r += blockDim.y) {
         const int g = g0 + r, k = k0 + threadIdx.x;
         float t = 0.f;
-        if (g < G && k < K2)
+        if (g < G && k < K2 && (mask & (k >= Hp ? PHX_P_WP : PHX_P_WS)))
             for (int q = 0; q < nparts; ++q) t += w1bar[q * pstride + (size_t)g * K2 + k];   // fixed order over the parts
         tile[r][threadIdx.x] = t;
     }
@@ -84,6 +85,10 @@ __global__ void unpack_w1_kernel(int G, int H, int Hp, int K2, const float* __re
         if (h >= H) continue;
         float* dst = (half ? Wp : Ws) + (size_t)h * G + g;
         const float v = tile[threadIdx.x][r];
+        if (!(mask & (half ? PHX_P_WP : PHX_P_WS))) {
+            if (!accumulate) *dst = 0.f;
+            continue;
+        }
         *dst = accumulate ? *dst + v : v;
     }
 }
@@ -101,29 +106,41 @@ __global__ void mse_grad_kernel(int rows, int G, const float* __restrict__ pred,
 __global__ void unpack_rest_kernel(int G, int H, int Hp, int K2, const float* __restrict__ wabar,
                                    const float* __restrict__ biasbar, const float* __restrict__ mbar, int nparts,
                                    size_t pstride, float* __restrict__ Wa, float* __restrict__ bs,
-                                   float* __restrict__ bp, float* __restrict__ m, int accumulate) {
+                                   float* __restrict__ bp, float* __restrict__ m, int accumulate, int mask) {
     auto psum = [&](const float* base, size_t i) {
         float t = 0.f;
         for (int q = 0; q < nparts; ++q) t += base[q * pstride + i];
         return t;
+    };
+    // a block outside `mask` is not read: zeros, or left as it is when accumulating
+    auto put = [&](float* dst, int bit, const float* base, size_t i) {
+        if (mask & bit) {
+            const float v = psum(base, i);
+            *dst = accumulate ? *dst + v : v;
+        } else if (!accumulate) {
+            *dst = 0.f;
+        }
     };
     const size_t stride = (size_t)gridDim.x * blockDim.x;
     const size_t n = (size_t)G * 2 * H;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const size_t g = i / (2 * H);
         const int kk = (int)(i - g * 2 * H);
-        const float v = psum(wabar, g * K2 + (kk < H ? kk : Hp + kk - H));
-        Wa[i] = accumulate ? Wa[i] + v : v;
+        put(Wa + i, PHX_P_WA, wabar, g * K2 + (kk < H ? kk : Hp + kk - H));
     }
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)H; i += stride) {
-        const float vs = psum(biasbar, i), vp = psum(biasbar, Hp + i);
-        bs[i] = accumulate ? bs[i] + vs : vs;
-        bp[i] = accumulate ? bp[i] + vp : vp;
+        put(bs + i, PHX_P_BS, biasbar, i);
+        put(bp + i, PHX_P_BP, biasbar, Hp + i);
     }
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)G; i += stride) {
-        const float vm = psum(mbar, i);
-        m[i] = accumulate ? m[i] + vm : vm;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)G; i += stride) put(m + i, PHX_P_M, mbar, i);
+}
+
+bool check_mask(int mask) {
+    if (mask < 0 || mask > PHX_P_ALL) {
+        phx_set_error("param_mask must be a 6-bit mask (0 .. 0x3F), got %d", mask);
+        return false;
     }
+    return true;
 }
 
 bool check_dims(int G, int H, int B) {
@@ -442,8 +459,19 @@ int phx_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, co
                       int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                       const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat, void* workspace,
                       size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap, void* stream) {
+    return phx_solve_adjoint_masked(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, y_saved,
+                                    grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status, steplog, steplog_cap,
+                                    PHX_P_ALL, stream);
+}
+
+int phx_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                             int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                             const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat, void* workspace,
+                             size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
+                             int param_mask, void* stream) {
     PhxDevGuard dev_guard(ctx);
     g_err[0] = 0;
+    if (!check_mask(param_mask)) return PHX_ERR_INVALID;
     if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
         return PHX_ERR_INVALID;
@@ -457,6 +485,7 @@ int phx_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, co
     p.grad_y = grad_y;
     p.adj_y0 = adj_y0;
     p.theta0 = grads_flat;  // written once by the kernel (never read while still zero): no memset needed
+    p.pmask = param_mask;
     return phx_resident_launch(p, plan, (cudaStream_t)stream);
 }
 
@@ -487,8 +516,19 @@ int phx_solve_adjoint_many(phx_ctx* ctx, int G, int H, int B, int N, const float
                            int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                            void* workspace, size_t workspace_bytes, phx_status* status, void* stream) {
+    return phx_solve_adjoint_many_masked(ctx, G, H, B, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
+                                         y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status, PHX_P_ALL,
+                                         stream);
+}
+
+int phx_solve_adjoint_many_masked(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host,
+                                  int T, int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                  void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
+                                  void* stream) {
     PhxDevGuard dev_guard(ctx);
     g_err[0] = 0;
+    if (!check_mask(param_mask)) return PHX_ERR_INVALID;
     if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
         return PHX_ERR_INVALID;
@@ -505,6 +545,7 @@ int phx_solve_adjoint_many(phx_ctx* ctx, int G, int H, int B, int N, const float
     p.yout_stride = (long long)T * B * G;
     p.adj_stride = (long long)B * G;
     p.theta_stride = (long long)phx_grad_offsets(G, H).total;
+    p.pmask = param_mask;
     return phx_resident_launch(p, plan, (cudaStream_t)stream);
 }
 
@@ -630,17 +671,24 @@ int phx_rows_grad_parts(const phx_ctx* ctx, int G, int H, int N) {
 
 int phx_unpack_grads(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
                      int accumulate, void* stream) {
+    return phx_unpack_grads_masked(ctx, G, H, packed_grads, nparts, grads_flat, accumulate, PHX_P_ALL, stream);
+}
+
+int phx_unpack_grads_masked(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
+                            int accumulate, int param_mask, void* stream) {
     PhxDevGuard dev_guard(ctx);
-    if (!ctx || !check_dims(G, H, 1) || !packed_grads || !grads_flat || nparts < 1) return PHX_ERR_INVALID;
+    if (!ctx || !check_dims(G, H, 1) || !packed_grads || !grads_flat || nparts < 1 || !check_mask(param_mask))
+        return PHX_ERR_INVALID;
     const int Hp = phx_Hp(H), K2 = 2 * Hp;
     const PhxPackedGradOff po = phx_packed_grad_offsets(G, H);
     const PhxGradOff fo = phx_grad_offsets(G, H);
     dim3 grid((G + 31) / 32, (K2 + 31) / 32), block(32, 8);
     unpack_w1_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(G, H, Hp, K2, packed_grads + po.W1, nparts, po.total,
-                                                               grads_flat + fo.Ws, grads_flat + fo.Wp, accumulate);
+                                                               grads_flat + fo.Ws, grads_flat + fo.Wp, accumulate,
+                                                               param_mask);
     unpack_rest_kernel<<<ctx->num_sms * 4, 256, 0, (cudaStream_t)stream>>>(
         G, H, Hp, K2, packed_grads + po.WA, packed_grads + po.bias, packed_grads + po.m, nparts, po.total,
-        grads_flat + fo.Wa, grads_flat + fo.bs, grads_flat + fo.bp, grads_flat + fo.m, accumulate);
+        grads_flat + fo.Wa, grads_flat + fo.bs, grads_flat + fo.bp, grads_flat + fo.m, accumulate, param_mask);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
         phx_set_error("unpack_grads launch: %s", cudaGetErrorString(e));
@@ -675,8 +723,19 @@ int phx_solve_adjoint_rows(phx_ctx* ctx, int G, int H, int N, const float* packe
                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
                            void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                            int steplog_cap, void* stream) {
+    return phx_solve_adjoint_rows_masked(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
+                                         y_saved, grad_y, adj_y0, grads_packed_parts, workspace, workspace_bytes, status,
+                                         steplog, steplog_cap, PHX_P_ALL, stream);
+}
+
+int phx_solve_adjoint_rows_masked(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
+                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
+                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                  int steplog_cap, int param_mask, void* stream) {
     PhxDevGuard dev_guard(ctx);
     g_err[0] = 0;
+    if (!check_mask(param_mask)) return PHX_ERR_INVALID;
     if (!y_saved || !grad_y || !adj_y0 || !grads_packed_parts) {
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_packed_parts");
         return PHX_ERR_INVALID;
@@ -697,6 +756,7 @@ int phx_solve_adjoint_rows(phx_ctx* ctx, int G, int H, int N, const float* packe
     p.theta_ws = (float*)workspace + o_th;
     p.gsum = grads_packed_parts;
     p.gsum_acc = 0;
+    p.pmask = param_mask;
     return phx_rows_launch(p, plan, (cudaStream_t)stream);
 }
 

@@ -82,6 +82,32 @@ static inline __host__ __device__ PhxGradOff phx_grad_offsets(int G, int H) {
     return o;
 }
 
+// Adjoint parameter mask: bit i = the i-th parameter in reference order (m, Wp, bp, Ws, bs, Wa).  The adjoint solvers
+// integrate, put in the error norm and return only the cotangents of the parameters in the mask; the others come back
+// as zeros.
+enum { PHX_P_M = 1, PHX_P_WP = 2, PHX_P_BP = 4, PHX_P_WS = 8, PHX_P_BS = 16, PHX_P_WA = 32, PHX_P_ALL = 63 };
+// number of cotangent elements in the mask
+static inline __host__ __device__ size_t phx_mask_count(int G, int H, int mask) {
+    const size_t HG = (size_t)H * G;
+    return ((mask & PHX_P_M) ? (size_t)G : 0) + ((mask & PHX_P_WP) ? HG : 0) + ((mask & PHX_P_BP) ? (size_t)H : 0) +
+           ((mask & PHX_P_WS) ? HG : 0) + ((mask & PHX_P_BS) ? (size_t)H : 0) + ((mask & PHX_P_WA) ? 2 * HG : 0);
+}
+// offsets of the masked-in blocks when only they are stored, back to back in reference order (masked-out blocks get the
+// offset of the next kept one and are never addressed); phx_compact_grad_offsets(G, H, PHX_P_ALL) == phx_grad_offsets
+static inline __host__ __device__ PhxGradOff phx_compact_grad_offsets(int G, int H, int mask) {
+    PhxGradOff o;
+    const size_t HG = (size_t)H * G;
+    size_t at = 0;
+    o.m = at;  at += (mask & PHX_P_M) ? (size_t)G : 0;
+    o.Wp = at; at += (mask & PHX_P_WP) ? HG : 0;
+    o.bp = at; at += (mask & PHX_P_BP) ? (size_t)H : 0;
+    o.Ws = at; at += (mask & PHX_P_WS) ? HG : 0;
+    o.bs = at; at += (mask & PHX_P_BS) ? (size_t)H : 0;
+    o.Wa = at; at += (mask & PHX_P_WA) ? 2 * HG : 0;
+    o.total = at;
+    return o;
+}
+
 // Parameter cotangents in the PACKED layout = the layout of the packed weights themselves: W1bar[G][K2] (row g =
 // [Wsbar[:, g] | Wpbar[:, g]]), WAbar[G][K2], biasbar[K2] ([bs | bp]), mbar[G]; every row 16-byte aligned, the rows of one
 // CTA's gene slice contiguous.  phx_unpack_grads converts to the reference's flat order.
@@ -249,6 +275,7 @@ struct ResParams {
     float* gsum;           // [ppk] packed cotangents summed over all problems of the launch
     int gsum_acc;          // != 0: add to gsum instead of overwriting it
     long long ppk;
+    int pmask;             // adjoint: parameters whose cotangents are integrated (PHX_P_*)
 };
 #define PHX_PROF_SLOTS 32
 #define PHX_T_INLINE 64
@@ -377,7 +404,7 @@ int phx_rhs_forward_launch(int G, int H, int B, const PhxPacked& w, const float*
 bool phx_rhs_post_supported(const PhxPacked& w, int H, int B);
 int phx_rhs_vjp_launch(int G, int H, int B, const PhxPacked& w, const float* y, const float* g, int decay,
                        float* ybar, float* grads_flat, int accumulate, float* f_out, float fscale, float* ws,
-                       cudaStream_t stream);
+                       cudaStream_t stream, int pmask = PHX_P_ALL, const PhxGradOff* goff = nullptr);
 size_t phx_rhs_workspace_floats(int G, int H, int B);
 int phx_prior_loss_launch(int G, int H, int B, const PhxPacked& w, const float* x, const float* prior_grad, float scale,
                           float* gcot, float* loss, float* ws, cudaStream_t stream);
@@ -401,7 +428,8 @@ int phx_tc_joint_launch(int G, int H, int B, const PhxPacked& w, const float* y,
 int phx_tc_prior_loss_launch(int G, int H, int B, const PhxPacked& w, const float* x, const float* prior_grad, float scale,
                              float* gcot, float* loss, float* SP, double* part, float* tcws, cudaStream_t stream);
 int phx_tc_vjp_params_launch(int G, int H, int B, const PhxPacked& w, const float* y, const float* g, int decay,
-                             float* grads_flat, int accumulate, float* tcws, cudaStream_t stream);
+                             float* grads_flat, int accumulate, float* tcws, cudaStream_t stream,
+                             int pmask = PHX_P_ALL, const PhxGradOff* goff = nullptr);
 
 void phx_set_error(const char* fmt, ...);
 int phx_ctx_device(const phx_ctx* ctx);

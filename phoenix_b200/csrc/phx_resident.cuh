@@ -1830,24 +1830,29 @@ __device__ __noinline__ PPSums ppass(const ResParams& __restrict__ p, int g_lo, 
     const PhxGradOff off = phx_grad_offsets(p.G, p.H);
     const int Hp = p.Hp, H = p.H, G = p.G;
     const float atol_f = p.atol_f, rtol_f = p.rtol_f;
+    // only the blocks of the adjoint parameters are read or written (p.pmask); the others are zeroed once at the end
+    const int pm = p.pmask;
     if (MODE == PP_COPY) {
         float k[7] = {0, 0, 0, 0, 0, 0, 0};
-        for (int j = threadIdx.x; j < n_loc; j += THREADS) theta_elem<MODE>(atol_f, rtol_f, a, off.m + g_lo + j, k, acc0, acc1);
+        if (pm & PHX_P_M)
+            for (int j = threadIdx.x; j < n_loc; j += THREADS) theta_elem<MODE>(atol_f, rtol_f, a, off.m + g_lo + j, k, acc0, acc1);
         for (int h = 0; h < H; ++h)
             for (int j = threadIdx.x; j < n_loc; j += THREADS) {
-                theta_elem<MODE>(atol_f, rtol_f, a, off.Wp + (size_t)h * G + g_lo + j, k, acc0, acc1);
-                theta_elem<MODE>(atol_f, rtol_f, a, off.Ws + (size_t)h * G + g_lo + j, k, acc0, acc1);
+                if (pm & PHX_P_WP) theta_elem<MODE>(atol_f, rtol_f, a, off.Wp + (size_t)h * G + g_lo + j, k, acc0, acc1);
+                if (pm & PHX_P_WS) theta_elem<MODE>(atol_f, rtol_f, a, off.Ws + (size_t)h * G + g_lo + j, k, acc0, acc1);
             }
-        for (size_t e = threadIdx.x; e < (size_t)n_loc * 2 * H; e += THREADS)
-            theta_elem<MODE>(atol_f, rtol_f, a, off.Wa + (size_t)g_lo * 2 * H + e, k, acc0, acc1);
+        if (pm & PHX_P_WA)
+            for (size_t e = threadIdx.x; e < (size_t)n_loc * 2 * H; e += THREADS)
+                theta_elem<MODE>(atol_f, rtol_f, a, off.Wa + (size_t)g_lo * 2 * H + e, k, acc0, acc1);
         if (blockIdx.x == 0)
             for (int h = threadIdx.x; h < H; h += THREADS) {
-                theta_elem<MODE>(atol_f, rtol_f, a, off.bp + h, k, acc0, acc1);
-                theta_elem<MODE>(atol_f, rtol_f, a, off.bs + h, k, acc0, acc1);
+                if (pm & PHX_P_BP) theta_elem<MODE>(atol_f, rtol_f, a, off.bp + h, k, acc0, acc1);
+                if (pm & PHX_P_BS) theta_elem<MODE>(atol_f, rtol_f, a, off.bs + h, k, acc0, acc1);
             }
         return PPSums{acc0, acc1};
     }
     // m
+    if (pm & PHX_P_M)
     for (int j = threadIdx.x; j < n_loc; j += THREADS) {
         if constexpr (MODE == PP_STEP) {
             theta_step(atol_f, rtol_f, a, off.m + g_lo + j, [&](int q) { return s.FM()[j * 8 + q]; }, acc0, acc1);
@@ -1860,15 +1865,19 @@ __device__ __noinline__ PPSums ppass(const ResParams& __restrict__ p, int g_lo, 
     }
     auto ident = [](int c) { return c; };
     // Wp, Ws : rows h (factors FG), this CTA's gene columns (factors FL / FS)
-    pp_block<MODE, BT>(atol_f, rtol_f, a, H, n_loc, s.FG() + (size_t)Hp * QB, s.FL(), ident, off.Wp + g_lo, (size_t)G, acc0, acc1);
-    pp_block<MODE, BT>(atol_f, rtol_f, a, H, n_loc, s.FG(), s.FS(), ident, off.Ws + g_lo, (size_t)G, acc0, acc1);
+    if (pm & PHX_P_WP)
+        pp_block<MODE, BT>(atol_f, rtol_f, a, H, n_loc, s.FG() + (size_t)Hp * QB, s.FL(), ident, off.Wp + g_lo, (size_t)G, acc0, acc1);
+    if (pm & PHX_P_WS)
+        pp_block<MODE, BT>(atol_f, rtol_f, a, H, n_loc, s.FG(), s.FS(), ident, off.Ws + g_lo, (size_t)G, acc0, acc1);
     // Wa : this CTA's gene rows (factors FGJ), 2H columns (factors FSP, skipping the padded columns)
-    pp_block<MODE, BT>(atol_f, rtol_f, a, n_loc, 2 * H, s.FGJ(), s.FSP(), [&](int kk) { return kk < H ? kk : Hp + kk - H; },
-                       off.Wa + (size_t)g_lo * 2 * H, (size_t)2 * H, acc0, acc1);
+    if (pm & PHX_P_WA)
+        pp_block<MODE, BT>(atol_f, rtol_f, a, n_loc, 2 * H, s.FGJ(), s.FSP(), [&](int kk) { return kk < H ? kk : Hp + kk - H; },
+                           off.Wa + (size_t)g_lo * 2 * H, (size_t)2 * H, acc0, acc1);
     // biases : CTA 0
     if (blockIdx.x == 0) {
         for (int h = threadIdx.x; h < 2 * H; h += THREADS) {
             const bool prod = h >= H;
+            if (!(pm & (prod ? PHX_P_BP : PHX_P_BS))) continue;
             const float* up = s.FG() + (size_t)(prod ? Hp + h - H : h) * QB;
             if constexpr (MODE == PP_STEP) {
                 theta_step(atol_f, rtol_f, a, (prod ? off.bp + (h - H) : off.bs + h),
@@ -1932,20 +1941,22 @@ __device__ __noinline__ double theta_zero_norm(const ResParams& p, int n_loc, in
     for (int b = 0; b < BT; ++b) { idx[M] = s1 * BT + b; sgn[M] = 1.f; ++M; }
     if (s0 >= 0)
         for (int b = 0; b < BT; ++b) { idx[M] = s0 * BT + b; sgn[M] = -1.f; ++M; }
-    const int Hp = p.Hp;
+    const int Hp = p.Hp, pm = p.pmask;
     double tot = 0;
-    // Wp, Ws (padded branch columns hold zeros), Wa
-    tot += gram_sq(s, s.FG() + (size_t)Hp * QB, Hp, s.FL(), n_loc, QB, idx, sgn, M);
-    tot += gram_sq(s, s.FG(), Hp, s.FS(), n_loc, QB, idx, sgn, M);
-    tot += gram_sq(s, s.FGJ(), n_loc, s.FSP(), p.K2, QB, idx, sgn, M);
+    // Wp, Ws (padded branch columns hold zeros), Wa -- the adjoint parameters only (every thread takes the same branches)
+    if (pm & PHX_P_WP) tot += gram_sq(s, s.FG() + (size_t)Hp * QB, Hp, s.FL(), n_loc, QB, idx, sgn, M);
+    if (pm & PHX_P_WS) tot += gram_sq(s, s.FG(), Hp, s.FS(), n_loc, QB, idx, sgn, M);
+    if (pm & PHX_P_WA) tot += gram_sq(s, s.FGJ(), n_loc, s.FSP(), p.K2, QB, idx, sgn, M);
     // m (per gene) and, on CTA 0, the biases: direct
     double loc = 0;
+    if (pm & PHX_P_M)
     for (int j = threadIdx.x; j < n_loc; j += THREADS) {
         float k = s.FM()[j * 8 + s1] - (s0 >= 0 ? s.FM()[j * 8 + s0] : 0.f);
         loc += (double)k * (double)k;
     }
     if (blockIdx.x == 0) {
         for (int h = threadIdx.x; h < p.K2; h += THREADS) {
+            if (!(pm & (h < Hp ? PHX_P_BS : PHX_P_BP))) continue;
             float k1 = 0.f, k0 = 0.f;
             for (int b = 0; b < BT; ++b) {
                 k1 += s.FG()[(size_t)h * QB + s1 * BT + b];
@@ -2014,7 +2025,10 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
     const int BL = p.B * p.gpc;
     const double Nel = (double)p.B * (double)p.G;
     const PhxGradOff goff = phx_grad_offsets(p.G, p.H);
-    const double Pel = (double)goff.total;
+    // theta block of the norm: the adjoint parameters only; with none the block is absent (th_rms == 0 never wins the
+    // max over the other, non-negative blocks)
+    const double Pel = (double)phx_mask_count(p.G, p.H, p.pmask);
+    auto th_rms = [&](double sum) { return Pel > 0 ? sqrtf((float)(sum / Pel)) : 0.f; };
     float* Y = s.st();
     float* A = s.st() + BL;
     float* Y1 = s.st() + 2 * BL;
@@ -2178,9 +2192,9 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                     pf.tick(PT_NORMS);
                     if (threadIdx.x == 0) {
                         float d0 = fmaxf(fmaxf(sqrtf((float)(c->dsum[0] / Nel)), sqrtf((float)(c->dsum[1] / Nel))),
-                                         sqrtf((float)(c->dsum[2] / Pel)));
+                                         th_rms(c->dsum[2]));
                         float d1 = fmaxf(fmaxf(sqrtf((float)(c->dsum[3] / Nel)), sqrtf((float)(c->dsum[4] / Nel))),
-                                         sqrtf((float)(c->dsum[5] / Pel)));
+                                         th_rms(c->dsum[5]));
                         c->d1 = d1;
                         c->h0 = init_h0(d0, d1);
                         c->nonfinite_prev = c->dsum[6] > 0.0;
@@ -2201,7 +2215,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                     pf.tick(PT_NORMS);
                     if (threadIdx.x == 0) {
                         float d2 = fmaxf(fmaxf(sqrtf((float)(c->dsum[0] / Nel)), sqrtf((float)(c->dsum[1] / Nel))),
-                                         sqrtf((float)(c->dsum[2] / Pel))) / c->h0;
+                                         th_rms(c->dsum[2])) / c->h0;
                         c->dt = init_dt(c->h0, c->d1, d2);
                         c->n_rhs += 2;
                     }
@@ -2307,7 +2321,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 pf.tick(PT_NORMS);
                 if (threadIdx.x == 0) {
                     float ratio = fmaxf(fmaxf(sqrtf((float)(c->dsum[0] / Nel)), sqrtf((float)(c->dsum[1] / Nel))),
-                                        sqrtf((float)(c->dsum[2] / Pel)));
+                                        th_rms(c->dsum[2]));
                     // torch's max() over 0-dim tensors is Python max: a NaN in a later block does not propagate the
                     // same way; treat any NaN as NaN (step rejected, dt -> NaN -> underflow assertion)
                     if (isnan(c->dsum[0]) || isnan(c->dsum[1]) || isnan(c->dsum[2])) ratio = nanf("");
@@ -2378,6 +2392,18 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
         }
         __syncthreads();
         ppass<PP_COPY, BT>(p, g_lo, n_loc);
+    }
+    if (!theta_zero && p.pmask != PHX_P_ALL) {
+        // the blocks of parameters outside the adjoint set were never touched: report zeros
+        const int pm = p.pmask;
+        const size_t HG = (size_t)p.H * p.G;
+        const size_t lo[6] = {goff.m, goff.Wp, goff.bp, goff.Ws, goff.bs, goff.Wa};
+        const size_t n[6] = {(size_t)p.G, HG, (size_t)p.H, HG, (size_t)p.H, 2 * HG};
+        for (int q = 0; q < 6; ++q) {
+            if (pm & (1 << q)) continue;
+            for (size_t i = (size_t)blockIdx.x * THREADS + threadIdx.x; i < n[q]; i += (size_t)gridDim.x * THREADS)
+                theta0p[lo[q] + i] = 0.f;
+        }
     }
     pf.tick(PT_PP_COPY);
     __syncthreads();

@@ -224,8 +224,9 @@ __global__ void colsum_bias_kernel(const float* GS, int B, int K2, int Hp, int H
     if (ok)
         for (int b = threadIdx.y; b < B; b += CS) t += GS[(size_t)b * K2 + col];
     t = colsum_fold(t, sh);
-    if (ok && threadIdx.y == 0) {
-        float* dst = (k < H) ? (bs_bar + k) : (bp_bar + (k - H));
+    float* const base = (k < H) ? bs_bar : bp_bar;   // nullptr: that bias is not wanted
+    if (ok && threadIdx.y == 0 && base) {
+        float* dst = base + ((k < H) ? k : k - H);
         *dst = accumulate ? *dst + t : t;
     }
 }
@@ -310,7 +311,7 @@ int phx_rhs_forward_launch(int G, int H, int B, const PhxPacked& w, const float*
 
 int phx_rhs_vjp_launch(int G, int H, int B, const PhxPacked& w, const float* y, const float* g, int decay,
                        float* ybar, float* grads, int accumulate_flags, float* f_out, float fscale, float* ws,
-                       cudaStream_t st) {
+                       cudaStream_t st, int pmask, const PhxGradOff* goff) {
     const int Hp = phx_Hp(H), K2 = 2 * Hp;
     const int accumulate = accumulate_flags & 1;
     float* SP = ws;
@@ -319,7 +320,7 @@ int phx_rhs_vjp_launch(int G, int H, int B, const PhxPacked& w, const float* y, 
     const float* W1 = reinterpret_cast<const float*>(w.W1);
     const float* WA = reinterpret_cast<const float*>(w.WA);
     const bool tc = w.tc && phx_tc_shape_ok(H, B);
-    const bool needJ = (f_out != nullptr) || (grads && decay);
+    const bool needJ = (f_out != nullptr) || (grads && decay && (pmask & PHX_P_M));
     bool direct_f = false;
     if (tc) {
         // tensor cores: [S|P], gSP, the state cotangent and the un-decayed joint (phx_tc.cu); the K = B parameter
@@ -374,37 +375,41 @@ int phx_rhs_vjp_launch(int G, int H, int B, const PhxPacked& w, const float* y, 
         if (decay) decay_kernel<<<blocks, 256, 0, st>>>(J, y, w.relum, G, n, fscale, f_out);
         else cudaMemcpyAsync(f_out, J, n * sizeof(float), cudaMemcpyDeviceToDevice, st);
     }
-    if (grads) {
-        const PhxGradOff off = phx_grad_offsets(G, H);
+    // parameter cotangents: only the blocks in pmask, at the offsets `goff` (default: the flat reference layout)
+    if (grads && pmask) {
+        const PhxGradOff off = goff ? *goff : phx_grad_offsets(G, H);
         if (tc) {
             int rc = phx_tc_vjp_params_launch(G, H, B, w, y, g, decay, grads, accumulate,
-                                              ws + rhs_base_floats(G, H, B), st);
+                                              ws + rhs_base_floats(G, H, B), st, pmask, &off);
             if (rc != PHX_OK) return rc;
         } else {
-            {   // Wa_bar[g][k] = sum_b gJ[b][g] SP[b][k]
+            if (pmask & PHX_P_WA) {   // Wa_bar[g][k] = sum_b gJ[b][g] SP[b][k]
                 LoadGJT la{g, w.relum, G, decay};
                 LoadRowMajorB lb{SP, K2, 0};
                 EpiGradWa ep{grads + off.Wa, H, Hp, accumulate};
                 sgemm(G, K2, B, la, lb, ep, st);
             }
-            {   // Ws_bar[h][g] = sum_b GS[b][h] s[b][g]
+            if (pmask & PHX_P_WS) {   // Ws_bar[h][g] = sum_b GS[b][h] s[b][g]
                 LoadTransA la{GS, K2, 0};
                 LoadActB lb{y, G, 0};
                 EpiGrad ep{grads + off.Ws, G, accumulate};
                 sgemm(H, G, B, la, lb, ep, st);
             }
-            {   // Wp_bar[h][g] = sum_b GS[b][Hp+h] l[b][g]
+            if (pmask & PHX_P_WP) {   // Wp_bar[h][g] = sum_b GS[b][Hp+h] l[b][g]
                 LoadTransA la{GS, K2, Hp};
                 LoadActB lb{y, G, 1};
                 EpiGrad ep{grads + off.Wp, G, accumulate};
                 sgemm(H, G, B, la, lb, ep, st);
             }
         }
-        colsum_bias_kernel<<<(2 * H + CS - 1) / CS, dim3(CS, CS), 0, st>>>(GS, B, K2, Hp, H, grads + off.bs,
-                                                                           grads + off.bp, accumulate);
-        colsum_mult_kernel<<<(G + CS - 1) / CS, dim3(CS, CS), 0, st>>>(g, direct_f ? f_out : J, y, w.maskm, B, G,
-                                                                       grads + off.m, accumulate, decay, direct_f,
-                                                                       w.relum, fscale);
+        if (pmask & (PHX_P_BS | PHX_P_BP))
+            colsum_bias_kernel<<<(2 * H + CS - 1) / CS, dim3(CS, CS), 0, st>>>(
+                GS, B, K2, Hp, H, (pmask & PHX_P_BS) ? grads + off.bs : nullptr,
+                (pmask & PHX_P_BP) ? grads + off.bp : nullptr, accumulate);
+        if (pmask & PHX_P_M)
+            colsum_mult_kernel<<<(G + CS - 1) / CS, dim3(CS, CS), 0, st>>>(g, direct_f ? f_out : J, y, w.maskm, B, G,
+                                                                           grads + off.m, accumulate, decay, direct_f,
+                                                                           w.relum, fscale);
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {

@@ -1000,8 +1000,11 @@ __device__ __forceinline__ float2 bc2(float x) { return make_float2(x, x); }
 // The step / fixed passes are instruction-bound (8.9 M elements x rows at the headline shape): the three 6-term
 // combinations of an element pair run as packed fp32x2 FMAs (FFMA2), the tolerance division is MUFU.RCP + FMUL (the error
 // ratio only feeds the accept test and the step-size law), a non-finite theta is caught by a NaN-propagating FMA.
-template <int MODE>
-__device__ __noinline__ void rows_theta_pass(const ResParams& __restrict__ p, int g_lo, int n_loc, uint32_t tmem, double* out) {
+// ALL: every parameter is an adjoint parameter (p.pmask == PHX_P_ALL), so the mask tests fold away and the pass is the
+// code it was before masks existed -- it is the instruction-bound part of the kernel (see rows_theta_pass)
+template <int MODE, bool ALL>
+__device__ __noinline__ void rows_theta_pass_impl(const ResParams& __restrict__ p, int g_lo, int n_loc, uint32_t tmem,
+                                                  double* out) {
     Smem s(p);
     s.tmem = tmem;
     RowsView v(p, s);
@@ -1027,6 +1030,11 @@ __device__ __noinline__ void rows_theta_pass(const ResParams& __restrict__ p, in
     if (threadIdx.x < WARPS * 8) dred[threadIdx.x] = 0.0;
     __syncthreads();
     const int j0 = v.gg * p.gpg, jend = min(j0 + p.gpg, n_loc);
+    // only the adjoint parameters' parts of the packed slice are read or written (p.pmask): WAbar, the Ws (q < Hq) or Wp
+    // half of a W1bar row and of the bias, mbar
+    const int pm = ALL ? (int)PHX_P_ALL : p.pmask;
+    const bool keep_wa = pm & PHX_P_WA, keep_w1 = pm & (v.q >= Hq ? PHX_P_WP : PHX_P_WS);
+    const bool keep_b = pm & (v.q >= Hq ? PHX_P_BP : PHX_P_BS), keep_m = pm & PHX_P_M;
 #pragma unroll 1
     for (int b = 0; b < RM; ++b) {
         if (!pp[b].active) continue;
@@ -1117,7 +1125,7 @@ __device__ __noinline__ void rows_theta_pass(const ResParams& __restrict__ p, in
             const float* U = (blk == 0 ? v.fgj() : (v.q >= Hq ? UL : US)) + b * NFS;
             const size_t base = (blk == 0 ? off.WA : off.W1) + (size_t)g_lo * p.K2 + 4 * (size_t)v.q;
 #pragma unroll 1
-            for (int j = j0; j < jend; ++j) {
+            for (int j = j0; (blk == 0 ? keep_wa : keep_w1) && j < jend; ++j) {
                 float u[NV];
                 if (NV == NFS) {
                     const float2* u2 = reinterpret_cast<const float2*>(U + j * (RM * NFS));
@@ -1133,7 +1141,7 @@ __device__ __noinline__ void rows_theta_pass(const ResParams& __restrict__ p, in
                 }
                 quad(u, V, base + (size_t)j * p.K2);
             }
-            if (blk == 1 && blockIdx.x == 0 && v.gg == 0) {   // biases: stage derivative = gS | gLP itself
+            if (blk == 1 && blockIdx.x == 0 && v.gg == 0 && keep_b) {   // biases: stage derivative = gS | gLP itself
                 float u[NV];
 #pragma unroll
                 for (int f = 0; f < NV; ++f) u[f] = 1.f;
@@ -1142,7 +1150,7 @@ __device__ __noinline__ void rows_theta_pass(const ResParams& __restrict__ p, in
         }
         // gene multipliers: two genes per thread (elements e = (gene, row b)); an odd tail pairs with an all-zero element,
         // which adds exactly 0 to every sum
-        for (int jp = 2 * (int)threadIdx.x; jp < n_loc; jp += 2 * THREADS) {
+        for (int jp = 2 * (int)threadIdx.x; keep_m && jp < n_loc; jp += 2 * THREADS) {
             const bool two = jp + 1 < n_loc;
             const int e0 = jp * RM + b, e1 = (two ? jp + 1 : jp) * RM + b;
             float u[NV];
@@ -1175,6 +1183,12 @@ __device__ __noinline__ void rows_theta_pass(const ResParams& __restrict__ p, in
     __syncthreads();
 }
 
+template <int MODE>
+__device__ __forceinline__ void rows_theta_pass(const ResParams& __restrict__ p, int g_lo, int n_loc, uint32_t tmem, double* out) {
+    if (p.pmask == PHX_P_ALL) rows_theta_pass_impl<MODE, true>(p, g_lo, n_loc, tmem, out);
+    else rows_theta_pass_impl<MODE, false>(p, g_lo, n_loc, tmem, out);
+}
+
 // gsum (+)= sum over the valid rows of their final packed cotangents; every element is read by the thread that wrote it
 __device__ __noinline__ void rows_theta_sum(const ResParams& __restrict__ p, int g_lo, int n_loc, float* gsum,
                                             bool accumulate) {
@@ -1199,17 +1213,19 @@ __device__ __noinline__ void rows_theta_sum(const ResParams& __restrict__ p, int
         *reinterpret_cast<float4*>(gsum + idx) = t;
     };
     const int j0 = v.gg * p.gpg, jend = min(j0 + p.gpg, n_loc);
+    const int pm = p.pmask, Hq = p.Hp >> 2;   // the adjoint parameters' parts only (rows_theta_pass)
     if (v.qok) {
         for (int blk = 0; blk < 2; ++blk) {
+            if (!(pm & (blk == 0 ? PHX_P_WA : (v.q >= Hq ? PHX_P_WP : PHX_P_WS)))) continue;
             const size_t base = (blk == 0 ? off.WA : off.W1) + (size_t)g_lo * p.K2 + 4 * (size_t)v.q;
             for (int j = j0; j < jend; ++j) quad(base + (size_t)j * p.K2);
         }
-        if (blockIdx.x == 0 && v.gg == 0) quad(off.bias + 4 * (size_t)v.q);
+        if (blockIdx.x == 0 && v.gg == 0 && (pm & (v.q >= Hq ? PHX_P_BP : PHX_P_BS))) quad(off.bias + 4 * (size_t)v.q);
     }
     // multipliers: thread (gene j, row b) of the passes wrote element j of row b; lane b == 0 of every gene sums the rows
     // after the warp's writes are visible to it (same warp: the four row-threads of a gene are adjacent lanes)
     __syncwarp();
-    for (int e = threadIdx.x; e < n_loc * RM; e += THREADS) {
+    for (int e = threadIdx.x; (pm & PHX_P_M) && e < n_loc * RM; e += THREADS) {
         if ((e & 3) != 0) continue;
         const size_t idx = off.m + g_lo + (e >> 2);
         float t = accumulate ? gsum[idx] : 0.f;
@@ -1293,12 +1309,16 @@ __device__ __noinline__ double rows_theta_zero_norm(const ResParams& __restrict_
         auto comb = [&](double u11, double u10, double u00, double v11, double v10, double v00) {
             return sid0 >= 0 ? (u11 * v11 - 2.0 * u10 * v10 + u00 * v00) : u11 * v11;
         };
-        res += comb(keep[0], keep[1], keep[2], V9[0], V9[1], V9[2]);   // WAbar: gJ x S|Pr
-        res += comb(keep[3], keep[4], keep[5], V9[3], V9[4], V9[5]);   // Wsbar: s x gS
-        res += comb(L[0], L[1], L[2], V9[6], V9[7], V9[8]);             // Wpbar: l x gLP
-        res += L[3];                                                     // mbar
-        if (blockIdx.x == 0)
-            res += sid0 >= 0 ? (V9[3] - 2.0 * V9[4] + V9[5]) + (V9[6] - 2.0 * V9[7] + V9[8]) : V9[3] + V9[6];
+        const int pm = p.pmask;   // the adjoint parameters only
+        if (pm & PHX_P_WA) res += comb(keep[0], keep[1], keep[2], V9[0], V9[1], V9[2]);   // WAbar: gJ x S|Pr
+        if (pm & PHX_P_WS) res += comb(keep[3], keep[4], keep[5], V9[3], V9[4], V9[5]);   // Wsbar: s x gS
+        if (pm & PHX_P_WP) res += comb(L[0], L[1], L[2], V9[6], V9[7], V9[8]);             // Wpbar: l x gLP
+        if (pm & PHX_P_M) res += L[3];                                                     // mbar
+        if (blockIdx.x == 0) {   // (x + 0.0 == x: with both biases the sum is formed as before)
+            const double bs2 = sid0 >= 0 ? (V9[3] - 2.0 * V9[4] + V9[5]) : V9[3];
+            const double bp2 = sid0 >= 0 ? (V9[6] - 2.0 * V9[7] + V9[8]) : V9[6];
+            if (pm & (PHX_P_BS | PHX_P_BP)) res += ((pm & PHX_P_BS) ? bs2 : 0.0) + ((pm & PHX_P_BP) ? bp2 : 0.0);
+        }
         res /= (double)p.atol_f * (double)p.atol_f;
     }
     __syncthreads();
@@ -1314,7 +1334,10 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
     const int g_lo = s.g_lo, n_loc = s.n_loc;
     const int tot = n_loc * RM, BL = RM * p.gpc;
     const double Nel = (double)p.G;
-    const double Pel = (double)phx_grad_offsets(p.G, p.H).total;
+    // theta block of the norm: the adjoint parameters only; with none the block is absent (th_rms == 0 never wins the
+    // max over the other, non-negative blocks)
+    const double Pel = (double)phx_mask_count(p.G, p.H, p.pmask);
+    auto th_rms = [&](double sum) { return Pel > 0 ? sqrtf((float)(sum / Pel)) : 0.f; };
     float* Y = v.st(0);
     float* A = v.st(1);
     float* Y1 = v.st(2);
@@ -1548,15 +1571,15 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         const double* d = dsum + threadIdx.x * 7;
                         if (which == 0) {
                             const float d0 = fmaxf(fmaxf(sqrtf((float)(d[0] / Nel)), sqrtf((float)(d[1] / Nel))),
-                                                   sqrtf((float)(d[2] / Pel)));
+                                                   th_rms(d[2]));
                             const float d1 = fmaxf(fmaxf(sqrtf((float)(d[3] / Nel)), sqrtf((float)(d[4] / Nel))),
-                                                   sqrtf((float)(d[5] / Pel)));
+                                                   th_rms(d[5]));
                             c.d1 = d1;
                             c.h0 = init_h0(d0, d1);
                             c.nonfinite_prev = d[6] > 0.0;
                         } else {
                             const float d2 = fmaxf(fmaxf(sqrtf((float)(d[0] / Nel)), sqrtf((float)(d[1] / Nel))),
-                                                   sqrtf((float)(d[2] / Pel))) / c.h0;
+                                                   th_rms(d[2])) / c.h0;
                             c.dt = init_dt(c.h0, c.d1, d2);
                             if (!c.done) c.n_rhs += 2;
                         }
@@ -1674,7 +1697,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         if (!c.done) {
                             const double* d = dsum + threadIdx.x * 4;
                             float ratio = fmaxf(fmaxf(sqrtf((float)(d[0] / Nel)), sqrtf((float)(d[1] / Nel))),
-                                                sqrtf((float)(d[2] / Pel)));
+                                                th_rms(d[2]));
                             // torch's max() over 0-dim tensors is Python max: a NaN in a later block does not propagate
                             // the same way; treat any NaN as NaN (step rejected, dt -> NaN -> underflow assertion)
                             if (isnan(d[0]) || isnan(d[1]) || isnan(d[2])) ratio = nanf("");

@@ -273,6 +273,8 @@ struct Stream {
     void* sum_user = nullptr;
     int sum_world = 1;
     bool fuse = false;                 // stage algebra in the RHS epilogue (forward solves on the tensor-core path)
+    int pmask = PHX_P_ALL;             // adjoint: parameters whose cotangents make up the theta segment
+    PhxGradOff goff{};                 // adjoint: their offsets in the theta segment (back to back, reference order)
 
     // stage derivative `slot` of every segment at the current stage inputs (at_x0: at the step's start values themselves,
     // read in place -- no copy into the stage-input buffers)
@@ -282,8 +284,10 @@ struct Stream {
         if (!adjoint)
             return phx_rhs_forward_launch(G, H, B, w, in(segs[0]), segs[0].k[slot], 1, fsign, rhs_ws, st, post);
         // reverse time: ky = -f, ka = VJP_y(cotangent a), ktheta = VJP_theta(cotangent a)
-        return phx_rhs_vjp_launch(G, H, B, w, in(segs[0]), in(segs[1]), 1, segs[1].k[slot], segs[2].k[slot], 0,
-                                  segs[0].k[slot], -1.f, rhs_ws, st);
+        // (no theta segment when no parameter is integrated)
+        return phx_rhs_vjp_launch(G, H, B, w, in(segs[0]), in(segs[1]), 1, segs[1].k[slot],
+                                  segs.size() > 2 ? segs[2].k[slot] : nullptr, 0, segs[0].k[slot], -1.f, rhs_ws, st,
+                                  pmask, &goff);
     }
     // reduce a 3-value kernel result for segment si into sums_dev[si]
     // reduce the per-block partials of the LAST 3-value kernel launched for segment si (`blocks` = its grid size)
@@ -714,10 +718,24 @@ int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* pac
                              const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                              void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                              int steplog_cap, void* stream) {
+    return phx_stream_solve_adjoint_masked(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
+                                           y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status,
+                                           steplog, steplog_cap, PHX_P_ALL, stream);
+}
+
+int phx_stream_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                                    int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                    const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                    void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                    int steplog_cap, int param_mask, void* stream) {
     PhxDevGuard dev_guard(ctx);
     Stream S;
     float* base;
     cudaStream_t st = (cudaStream_t)stream;
+    if (param_mask < 0 || param_mask > PHX_P_ALL) {
+        phx_set_error("param_mask must be a 6-bit mask (0 .. 0x3F), got %d", param_mask);
+        return PHX_ERR_INVALID;
+    }
     if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
         return PHX_ERR_INVALID;
@@ -726,6 +744,11 @@ int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* pac
                    workspace_bytes, steplog, steplog_cap, st, &base);
     if (rc != PHX_OK) return rc;
     const size_t BG = (size_t)B * G, P = phx_grad_offsets(G, H).total;
+    // the theta segment holds the adjoint parameters' cotangents only, back to back in reference order (all six: the
+    // flat layout itself), at the start of grads_flat; it is absent when there are none
+    const size_t PS = phx_mask_count(G, H, param_mask);
+    S.pmask = param_mask;
+    S.goff = phx_compact_grad_offsets(G, H, param_mask);
     Seg y, a, th;
     y.n = a.n = BG; y.count = a.count = (double)BG;
     y.x0 = base; y.x1 = base + BG; y.xs = base + 2 * BG;
@@ -735,12 +758,12 @@ int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* pac
     for (int i = 0; i < 7; ++i) a.k[i] = ab + (3 + i) * BG;
     float* tb = ab + 10 * BG;
     tb += (4 - ((size_t)(tb - (float*)workspace) & 3)) & 3;
-    th.n = P; th.count = (double)P;
+    th.n = PS; th.count = (double)PS;
     th.x0 = grads_flat; th.x1 = tb; th.xs = nullptr;
-    for (int i = 0; i < 7; ++i) th.k[i] = tb + (size_t)(1 + i) * P;
+    for (int i = 0; i < 7; ++i) th.k[i] = tb + (size_t)(1 + i) * PS;
     S.segs.push_back(y);
     S.segs.push_back(a);
-    S.segs.push_back(th);
+    if (PS > 0) S.segs.push_back(th);
     cudaMemsetAsync(grads_flat, 0, P * sizeof(float), st);
     cudaMemcpyAsync(S.segs[1].x0, grad_y + (size_t)(T - 1) * BG, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
     for (int iv = T - 1; iv >= 1 && rc == PHX_OK && S.status.code == PHX_ST_OK; --iv) {
@@ -755,7 +778,7 @@ int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* pac
                               // after the step leaves it in x0; y is replaced by the saved state anyway
                               // (in place: every element is read before it is overwritten)
                               S.interp_seg(1, S.segs[1].x1, xs, sl, dtf, cmid);
-                              S.interp_seg(2, S.segs[2].x1, xs, sl, dtf, cmid);
+                              if (PS > 0) S.interp_seg(2, S.segs[2].x1, xs, sl, dtf, cmid);
                           });
         }
         if (rc != PHX_OK) break;
@@ -764,8 +787,28 @@ int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* pac
     }
     if (rc != PHX_OK) return rc;
     cudaMemcpyAsync(adj_y0, S.segs[1].x0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
-    if (S.segs[2].x0 != grads_flat)
-        cudaMemcpyAsync(grads_flat, S.segs[2].x0, P * sizeof(float), cudaMemcpyDeviceToDevice, st);
+    if (param_mask == PHX_P_ALL) {
+        if (S.segs[2].x0 != grads_flat)
+            cudaMemcpyAsync(grads_flat, S.segs[2].x0, P * sizeof(float), cudaMemcpyDeviceToDevice, st);
+    } else {
+        // back to the flat layout: the kept blocks from the segment (moved out of grads_flat first), zeros elsewhere
+        const float* src = nullptr;
+        if (PS > 0) {
+            src = S.segs[2].x0;
+            if (src == grads_flat) {
+                cudaMemcpyAsync(S.segs[2].x1, grads_flat, PS * sizeof(float), cudaMemcpyDeviceToDevice, st);
+                src = S.segs[2].x1;
+            }
+        }
+        cudaMemsetAsync(grads_flat, 0, P * sizeof(float), st);
+        const PhxGradOff fo = phx_grad_offsets(G, H), co = S.goff;
+        const size_t HG = (size_t)H * G;
+        const size_t flo[6] = {fo.m, fo.Wp, fo.bp, fo.Ws, fo.bs, fo.Wa}, clo[6] = {co.m, co.Wp, co.bp, co.Ws, co.bs, co.Wa};
+        const size_t n[6] = {(size_t)G, HG, (size_t)H, HG, (size_t)H, 2 * HG};
+        for (int q = 0; q < 6; ++q)
+            if (param_mask & (1 << q))
+                cudaMemcpyAsync(grads_flat + flo[q], src + clo[q], n[q] * sizeof(float), cudaMemcpyDeviceToDevice, st);
+    }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
         phx_set_error("stream adjoint: %s", cudaGetErrorString(e));

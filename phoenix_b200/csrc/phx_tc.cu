@@ -1068,6 +1068,7 @@ __global__ void tc_gradfinish_kernel(int which, int G, int Gpad, int H, int Hn, 
             br = c / H; n = c % H;
         }
         const int nslots = br ? ks_p : ks_s;
+        if (which == 0 && !(br ? d1 : d0)) continue;   // that half is not wanted
         float v = 0.f;
         for (int s = 0; s < nslots; ++s) v += part[((size_t)s * Gpad + g) * (2 * Hn) + br * Hn + n];
         float* dst = which == 0 ? (br ? d1 : d0) + (size_t)n * G + g : d0 + (size_t)g * 2 * H + br * H + n;
@@ -1740,22 +1741,32 @@ int phx_tc_joint_launch(int G, int H, int B, const PhxPacked& w, const float* y,
 //   Wa_bar[g][k] = sum_b (g relu(m))[b][g] [S|P][b][k],  Ws_bar[h][g] = sum_b gS[b][h] s[b][g],  Wp_bar likewise with l
 // (Linear backward, odenet.py:86-89), written / accumulated into the flat gradient vector.
 int phx_tc_vjp_params_launch(int G, int H, int B, const PhxPacked& w, const float* y, const float* g, int decay,
-                             float* grads, int accumulate, float* tcws, cudaStream_t st) {
+                             float* grads, int accumulate, float* tcws, cudaStream_t st, int pmask,
+                             const PhxGradOff* goff) {
     const TcScratch sc = carve(G, H, B, tcws);
     const int nterms = (w.tc == 1) ? 1 : 3, Hn = phx_tc_Hn(H);
-    const PhxGradOff off = phx_grad_offsets(G, H);
+    const PhxGradOff off = goff ? *goff : phx_grad_offsets(G, H);
     const size_t total = (size_t)G * 2 * H;
     int blocks = (int)((total + 255) / 256);
     if (blocks > PHX_TC_SMS * 16) blocks = PHX_TC_SMS * 16;
     PhxTcBranchPlan pl;
-    int rc = launch_branch_mma(1, 1, G, H, B, nterms, g, decay ? w.relum : nullptr, sc.sptimg, sc.gslots, &pl, st);
-    if (rc != PHX_OK) return rc;
-    tc_gradfinish_kernel<<<blocks, 256, 0, st>>>(1, G, phx_round_up(pl.mtiles, 2) * 128, H, Hn, pl.ks_s, pl.ks_p, sc.gslots,
-                                                 grads + off.Wa, nullptr, accumulate);
-    rc = launch_branch_mma(0, 1, G, H, B, nterms, y, nullptr, sc.gstimg, sc.gslots, &pl, st);
-    if (rc != PHX_OK) return rc;
-    tc_gradfinish_kernel<<<blocks, 256, 0, st>>>(0, G, phx_round_up(pl.mtiles, 2) * 128, H, Hn, pl.ks_s, pl.ks_p, sc.gslots,
-                                                 grads + off.Ws, grads + off.Wp, accumulate);
+    int rc;
+    if (pmask & PHX_P_WA) {
+        rc = launch_branch_mma(1, 1, G, H, B, nterms, g, decay ? w.relum : nullptr, sc.sptimg, sc.gslots, &pl, st);
+        if (rc != PHX_OK) return rc;
+        tc_gradfinish_kernel<<<blocks, 256, 0, st>>>(1, G, phx_round_up(pl.mtiles, 2) * 128, H, Hn, pl.ks_s, pl.ks_p,
+                                                     sc.gslots, grads + off.Wa, nullptr, accumulate);
+    }
+    // Ws and Wp come out of one launch with one K split (phx_tc_branch_plan): with one of them frozen the launch and
+    // its split stay as they are and only the kept half is written, so the kept half is bit-identical to the
+    // all-parameter call
+    if (pmask & (PHX_P_WS | PHX_P_WP)) {
+        rc = launch_branch_mma(0, 1, G, H, B, nterms, y, nullptr, sc.gstimg, sc.gslots, &pl, st);
+        if (rc != PHX_OK) return rc;
+        tc_gradfinish_kernel<<<blocks, 256, 0, st>>>(0, G, phx_round_up(pl.mtiles, 2) * 128, H, Hn, pl.ks_s, pl.ks_p,
+                                                     sc.gslots, (pmask & PHX_P_WS) ? grads + off.Ws : nullptr,
+                                                     (pmask & PHX_P_WP) ? grads + off.Wp : nullptr, accumulate);
+    }
     return check_launch("tc vjp_params");
 }
 

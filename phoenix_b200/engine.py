@@ -532,9 +532,10 @@ def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_t
     return yout
 
 
-def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy, adj_shape):
+def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy, adj_shape,
+                  param_mask=_lib.PARAMS_ALL):
     """Backward sweeps of N one-row problems (ys, gy: [N, T, ..., G] memory order): adj_y0 and the SUM over the problems of
-    the six parameter cotangents (flat, reference order)."""
+    the six parameter cotangents (flat, reference order; zeros for the parameters outside ``param_mask``)."""
     N, T = len(t_rows), len(t_rows[0])
     nb = lib.phx_rows_workspace_bytes(_lib.ctx(dev), G, H, N, T, 1)
     ws = _workspace(dev, nb, "solve")
@@ -548,11 +549,15 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
     log, cap = _steplog_rows(N)
     flat_t = (ctypes.c_double * (N * T))(*[x for r in t_rows for x in r])
     sp = _stream_ptr(dev)
-    rc = lib.phx_solve_adjoint_rows(ctx, G, H, N, _ptr(packed), flat_t, T, int(t_is_f32), _lib.METHOD_IDS[method],
-                                    float(rtol), float(atol), int(max_num_steps), _ptr(ys), _ptr(gy), _ptr(adj_y0),
-                                    _ptr(gpk), _ptr(ws), ws.numel(), _ptr(stn), _ptr(log), cap, sp)
-    _lib.check(rc, "solve_adjoint_rows")
-    _lib.check(lib.phx_unpack_grads(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, sp), "unpack_grads")
+    args = (ctx, G, H, N, _ptr(packed), flat_t, T, int(t_is_f32), _lib.METHOD_IDS[method], float(rtol), float(atol),
+            int(max_num_steps), _ptr(ys), _ptr(gy), _ptr(adj_y0), _ptr(gpk), _ptr(ws), ws.numel(), _ptr(stn), _ptr(log), cap)
+    if param_mask == _lib.PARAMS_ALL:
+        _lib.check(lib.phx_solve_adjoint_rows(*args, sp), "solve_adjoint_rows")
+        _lib.check(lib.phx_unpack_grads(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, sp), "unpack_grads")
+    else:
+        _lib.check(lib.phx_solve_adjoint_rows_masked(*args, param_mask, sp), "solve_adjoint_rows")
+        _lib.check(lib.phx_unpack_grads_masked(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, param_mask, sp),
+                   "unpack_grads")
     _tls().last_status_block = stn
     for i in range(N):
         _finish(stn[i], "adjoint solve %d" % i if N > 1 else "adjoint solve", dev)
@@ -590,7 +595,11 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
 
 
 @_on_model_device
-def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y):
+def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
+                  param_mask=_lib.PARAMS_ALL):
+    """adj_y0 and the six parameter cotangents of one backward sweep.  ``param_mask`` (bit i = the i-th parameter in
+    reference order): the adjoint parameters, the only ones integrated and put in the error norm; the cotangents of the
+    others come back as zeros."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -601,7 +610,7 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     lib = _lib.load()
     if _use_rows(lib, dev, G, H, B, True, single=True, T=T):
         return _adjoint_rows(lib, net, packed, G, H, dev, [t_list], t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[0].shape))
+                             tuple(ys[0].shape), param_mask)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
     ws = _workspace(dev, nb, "solve" if engine == "resident" else "stream")
     adj_y0 = torch.empty_like(ys[0])
@@ -610,9 +619,14 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     st = _new_status()
     log, cap = _steplog()
     fn = lib.phx_solve_adjoint if engine == "resident" else lib.phx_stream_solve_adjoint
-    rc = fn(_lib.ctx(dev), G, H, B, _ptr(packed), _t_array(t_list), T, int(t_is_f32), _lib.METHOD_IDS[method],
+    args = (_lib.ctx(dev), G, H, B, _ptr(packed), _t_array(t_list), T, int(t_is_f32), _lib.METHOD_IDS[method],
             float(rtol), float(atol), int(max_num_steps), _ptr(ys), _ptr(gy), _ptr(adj_y0), _ptr(grads), _ptr(ws),
-            ws.numel(), _ptr(st), _ptr(log), cap, _stream_ptr(dev))
+            ws.numel(), _ptr(st), _ptr(log), cap)
+    if param_mask == _lib.PARAMS_ALL:
+        rc = fn(*args, _stream_ptr(dev))
+    else:
+        fn = lib.phx_solve_adjoint_masked if engine == "resident" else lib.phx_stream_solve_adjoint_masked
+        rc = fn(*args, param_mask, _stream_ptr(dev))
     _lib.check(rc, "solve_adjoint")
     _finish(st, "adjoint solve", dev)
     return adj_y0, split_flat_grads(grads, G, H)
@@ -751,9 +765,11 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
 
 
 @_on_model_device
-def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y):
+def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
+                       param_mask=_lib.PARAMS_ALL):
     """Backward sweeps of N independent problems (``y_saved``, ``grad_y``: ``[N, T, *S, G]``): adj_y0 ``[N, *S, G]`` and
-    the six parameter cotangents summed over the problems (what autograd accumulates into ``.grad``)."""
+    the six parameter cotangents summed over the problems (what autograd accumulates into ``.grad``); zeros for the
+    parameters outside ``param_mask`` (see solve_adjoint)."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -764,7 +780,7 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     lib = _lib.load()
     if _use_rows(lib, dev, G, H, B, True):
         return _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[:, 0].shape))
+                             tuple(ys[:, 0].shape), param_mask)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
     ws = _workspace(dev, nb, "solve" if engine == "resident" else "stream")
     adj_y0 = torch.empty_like(ys[:, 0])
@@ -772,7 +788,14 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     chunk = min(N, _MANY_CHUNK)
     grads = torch.empty(chunk, P, dtype=torch.float32, device=ys.device)
     total = None
-    fn = lib.phx_solve_adjoint if engine == "resident" else lib.phx_stream_solve_adjoint
+    full = param_mask == _lib.PARAMS_ALL
+    if full:
+        fn = lib.phx_solve_adjoint if engine == "resident" else lib.phx_stream_solve_adjoint
+        many = lib.phx_solve_adjoint_many
+    else:   # the masked entry points take param_mask right before the stream
+        fn0 = lib.phx_solve_adjoint_masked if engine == "resident" else lib.phx_stream_solve_adjoint_masked
+        fn = lambda *a: fn0(*a[:-1], param_mask, a[-1])  # noqa: E731
+        many = lambda *a: lib.phx_solve_adjoint_many_masked(*a[:-1], param_mask, a[-1])  # noqa: E731
     ctx, sp, mid = _lib.ctx(dev), _stream_ptr(dev), _lib.METHOD_IDS[method]
     pk, wsp, wsn = _ptr(packed), _ptr(ws), ws.numel()
     stride = ys[0].numel() * 4
@@ -787,7 +810,7 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
                 n = min(per, hi - l2)
                 stn = _new_status_block(n)
                 flat_t = (ctypes.c_double * (n * T))(*[x for r in t_rows[l2:l2 + n] for x in r])
-                rc = lib.phx_solve_adjoint_many(
+                rc = many(
                     ctx, G, H, B, n, pk, flat_t, T, int(t_is_f32), mid, float(rtol), float(atol), int(max_num_steps),
                     ctypes.c_void_p(ys.data_ptr() + l2 * stride), ctypes.c_void_p(gy.data_ptr() + l2 * stride),
                     ctypes.c_void_p(adj_y0.data_ptr() + l2 * astride),

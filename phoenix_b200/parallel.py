@@ -43,12 +43,14 @@ def flat_grad_view(net):
     return torch.empty(0, dtype=g0.dtype, device=g0.device).set_(st, g0.storage_offset(), (off - g0.storage_offset(),))
 
 
-def adopt_flat_grads_(net, flat):
-    """Make the six ``.grad`` tensors views of ``flat`` (no copy)."""
+def adopt_flat_grads_(net, flat, keep=None):
+    """Make the six ``.grad`` tensors views of ``flat`` (no copy).  ``keep``: six flags; a parameter whose flag is False
+    keeps ``.grad`` None (a parameter outside the adjoint set got no gradient, and an optimiser must not move it)."""
     o = 0
-    for p in engine.net_params(net):
+    for i, p in enumerate(engine.net_params(net)):
         n = p.numel()
-        p.grad = flat[o:o + n].view_as(p)
+        if keep is None or keep[i]:
+            p.grad = flat[o:o + n].view_as(p)
         o += n
 
 
@@ -75,7 +77,9 @@ def allreduce_grads(net, group=None, average=True, extra=None):
     One collective over the flat ``[P]`` gradient, IN PLACE when the six gradients are views of one buffer
     (``flat_grad_view``: the normal case after a backward through this package -- no gather / scatter passes over the
     35.8 MB vector); otherwise they are gathered once and ``.grad`` becomes views of the reduced buffer (no copy back).
-    ``extra`` rides in a second, tiny collective in the first case and at the tail of the vector in the second."""
+    ``extra`` rides in a second, tiny collective in the first case and at the tail of the vector in the second.
+    A parameter without a gradient (frozen, or left out of ``adjoint_params``; the same on every rank) enters the sum as
+    zeros and keeps ``.grad`` None."""
     if not dist.is_available() or not dist.is_initialized() or dist.get_world_size(group) == 1:
         return extra
     world = dist.get_world_size(group)
@@ -96,6 +100,7 @@ def allreduce_grads(net, group=None, average=True, extra=None):
             if out is not None:
                 out /= world
         return out
+    had = [p.grad is not None for p in engine.net_params(net)]
     flat = flatten_grads(net)
     n = flat.numel()
     if extra is not None:
@@ -103,7 +108,7 @@ def allreduce_grads(net, group=None, average=True, extra=None):
     dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
     if average:
         flat /= world
-    adopt_flat_grads_(net, flat[:n])
+    adopt_flat_grads_(net, flat[:n], had)
     return flat[n:].view_as(extra) if extra is not None else None
 
 
@@ -234,6 +239,7 @@ def _peer_allreduce_grads(net, pr, average, extra):
     params = engine.net_params(net)
     P = sum(p.numel() for p in params)
     flat = flat_grad_view(net)
+    had = [p.grad is not None for p in params]
     buf = pr.buffer
     in_place = flat is not None and flat.data_ptr() == buf.data_ptr()
     if not in_place:
@@ -256,7 +262,7 @@ def _peer_allreduce_grads(net, pr, average, extra):
         n = P + extra.numel()
     pr.reduce(scale=(1.0 / pr.world) if average else 1.0, numel=n)
     if not in_place:
-        adopt_flat_grads_(net, buf[:P])
+        adopt_flat_grads_(net, buf[:P], had)
     return buf[P:n].clone().view_as(extra) if extra is not None else None
 
 

@@ -105,12 +105,13 @@ def _register_node(ctx, func, y0, tl, t_is_f32, adj):
     """Forward side: note the node if its backward may be batched with its siblings' (a one-row state that needs no
     gradient itself -- the training loop's case)."""
     ctx.group = None
-    if (not DEFER_ADJOINT or ctx.needs_input_grad[8] or not any(ctx.needs_input_grad[9:])
+    if (not DEFER_ADJOINT or ctx.needs_input_grad[8] or not any(ctx.needs_input_grad[9:]) or not adj[4]
             or y0.numel() != y0.shape[-1]):
         return   # (nothing to differentiate -- e.g. a validation pass under no_grad -- is not a node at all)
     with _defer_lock:
         _node_seq[0] += 1
         ctx.seq = _node_seq[0]
+        # adj[4], the adjoint parameter mask, is part of the key: only nodes with the same adjoint set share a sweep
         ctx.group = (len(tl), t_is_f32, adj, tuple(y0.shape), y0.device, tuple(ctx.needs_input_grad[9:]))
         nodes = _live_nodes.get(func)
         if nodes is None:
@@ -179,22 +180,59 @@ class OdeintAdjointMethod(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
-        a_method, a_rtol, a_atol, a_max = ctx.adj
+        a_method, a_rtol, a_atol, a_max, mask = ctx.adj
+        if not mask and not ctx.needs_input_grad[8]:
+            return (None,) * (9 + len(ctx.needs_input_grad[9:]))   # only parameters outside adjoint_params want one
         batch = _defer(ctx, y, grad_y) if (ctx.group is not None and DEFER_ADJOINT) else _NOT_DEFERRED
         if batch is None:
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))
         with torch.no_grad():
             if batch is _NOT_DEFERRED:
                 adj_y0, grads = engine.solve_adjoint(ctx.func, ctx.tl, ctx.t_is_f32, a_method, a_rtol, a_atol, a_max,
-                                                     y, grad_y)
+                                                     y, grad_y, **_masked(mask))
             else:
                 t_rows, ys, gys = batch
                 adj_y0, grads = engine.solve_adjoint_many(ctx.func, t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
-                                                          a_max, ys, gys)
-        out = [None] * 8 + [adj_y0 if ctx.needs_input_grad[8] else None]
-        for i, need in enumerate(ctx.needs_input_grad[9:]):
-            out.append(grads[i] if need else None)
-        return tuple(out)
+                                                          a_max, ys, gys, **_masked(mask))
+        return _grads_out(ctx, adj_y0, grads, mask)
+
+
+def _masked(mask):
+    """The engine's keyword for a proper subset of the parameters; with all six the engine is called as it always was."""
+    return {} if mask == 0x3F else {"param_mask": mask}
+
+
+def _grads_out(ctx, adj_y0, grads, mask):
+    """backward's result: adj_y0 for y0, and a cotangent only for the parameters in the adjoint set (None for the others
+    even when they require grad: the reference's adjoint node does not take them as inputs)."""
+    out = [None] * 8 + [adj_y0 if ctx.needs_input_grad[8] else None]
+    for i, need in enumerate(ctx.needs_input_grad[9:]):
+        out.append(grads[i] if (need and mask >> i & 1) else None)
+    return tuple(out)
+
+
+def _adjoint_mask(func, adjoint_params):
+    """The six ODENet parameters and the mask (bit i = the i-th in reference order) of the adjoint set S: the members of
+    ``adjoint_params`` -- all six when None -- that require grad (adjoint.py:185-193)."""
+    params = engine.net_params(func)
+    if adjoint_params is None:
+        chosen = params
+    else:
+        chosen = list(adjoint_params)
+        ids = [id(p) for p in params]
+        seen = set()
+        for p in chosen:
+            if not torch.is_tensor(p) or id(p) not in ids:
+                raise NotImplementedError("adjoint_params may only hold parameters of the ODENet being integrated "
+                                          "(gene_multipliers and the weights / biases of its three linear layers)")
+            if id(p) in seen:
+                raise NotImplementedError("adjoint_params holds the same parameter twice")
+            seen.add(id(p))
+    mask = 0
+    for i, p in enumerate(params):
+        if p.requires_grad and any(p is c for c in chosen):
+            mask |= 1 << i
+    return params, mask
 
 
 def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None, adjoint_rtol=None,
@@ -205,9 +243,6 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
         raise ValueError('func must be an instance of nn.Module to specify the adjoint parameters; alternatively they '
                          'can be specified explicitly via the `adjoint_params` argument. If there are no parameters '
                          'then it is allowable to set `adjoint_params=()`.')
-    if adjoint_params is not None:
-        raise NotImplementedError("explicit adjoint_params are not supported: the adjoint kernel always produces the "
-                                  "six ODENet parameter cotangents")
     if adjoint_rtol is None:
         adjoint_rtol = rtol
     if adjoint_atol is None:
@@ -226,9 +261,9 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
                                                               adjoint_options)
     if rev:
         raise NotImplementedError("odeint_adjoint with decreasing t is not part of the PHOENIX path")
-    params = engine.net_params(func)
+    params, mask = _adjoint_mask(func, adjoint_params)
     return OdeintAdjointMethod.apply(func, tl, t_is_f32, method, rtol, atol, max_steps,
-                                     (a_method, a_rtol, a_atol, a_max), y0, *params)
+                                     (a_method, a_rtol, a_atol, a_max, mask), y0, *params)
 
 
 class OdeintAdjointManyMethod(torch.autograd.Function):
@@ -245,23 +280,23 @@ class OdeintAdjointManyMethod(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
-        a_method, a_rtol, a_atol, a_max = ctx.adj
+        a_method, a_rtol, a_atol, a_max, mask = ctx.adj
+        if not mask and not ctx.needs_input_grad[8]:
+            return (None,) * (9 + len(ctx.needs_input_grad[9:]))
         with torch.no_grad():
             adj_y0, grads = engine.solve_adjoint_many(ctx.func, ctx.t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
-                                                      a_max, y, grad_y)
-        out = [None] * 8 + [adj_y0 if ctx.needs_input_grad[8] else None]
-        for i, need in enumerate(ctx.needs_input_grad[9:]):
-            out.append(grads[i] if need else None)
-        return tuple(out)
+                                                      a_max, y, grad_y, **_masked(mask))
+        return _grads_out(ctx, adj_y0, grads, mask)
 
 
-def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None):
+def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None, adjoint_params=None):
     """The per-sample loop of the reference's ``training_step`` (train_insilico.py:128-130,
     ``[odeint(odenet, batch_point, time_points, method=method)[1] for ...]``) as ONE call: ``y0`` is ``[N, *S, G]``
     (N independent initial states), ``t`` is ``[N, T]`` (each sample's own times, increasing) and the result is
     ``[N, T, *S, G]`` with ``result[i] == odeint_adjoint(func, y0[i], t[i], ...)`` bit for bit: every sample is still
     its own solve with its own step controller (NOT the global-norm batched call).  Gradients flow to ``y0`` and to the
-    six ODENet parameters (summed over the samples) through one autograd node.  No reference counterpart: opt-in."""
+    ODENet parameters of ``adjoint_params`` that require grad (default: all six; summed over the samples) through one
+    autograd node.  No reference counterpart: opt-in."""
     assert torch.is_tensor(t) and t.ndimension() == 2, "t must be a [N, T] tensor of per-sample times"
     assert torch.is_tensor(y0) and y0.shape[0] == t.shape[0], "y0 and t must hold the same number of samples"
     if y0.shape[0] == 0:
@@ -273,6 +308,6 @@ def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=
         assert all(b > a for a, b in zip(r, r[1:])), 't must be strictly increasing for every sample'
     if rev:
         raise NotImplementedError("odeint_adjoint_many with decreasing t is not part of the PHOENIX path")
-    params = engine.net_params(func)
+    params, mask = _adjoint_mask(func, adjoint_params)
     return OdeintAdjointManyMethod.apply(func, rows, t_is_f32, method, rtol_f, atol_f, max_steps,
-                                         (method, rtol_f, atol_f, max_steps), y0, *params)
+                                         (method, rtol_f, atol_f, max_steps, mask), y0, *params)
