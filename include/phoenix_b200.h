@@ -183,8 +183,13 @@ int phx_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, co
  * pass).  Only the cotangents of the parameters in the mask are integrated, and only they make up the parameter block of
  * the error norm (count = their total size; with an empty mask the block is absent).  The blocks of grads_flat outside
  * the mask are written as zeros (phx_unpack_grads_masked with accumulate != 0 leaves them as they are).  A mask outside
- * 0 .. 0x3F returns PHX_ERR_INVALID. */
+ * 0 .. 0x3F returns PHX_ERR_INVALID.
+ * PHX_NORM_SEMINORM may be OR-ed into the param_mask of the four adjoint solves (not phx_unpack_grads_masked): dopri5 then
+ * measures the error with the seminorm of Kidger, Chen & Lyons (2021), the mixed norm without the parameter block, in
+ * Hairer's initial step and in every error ratio, while the low six bits still choose the integrated cotangents.
+ * Fixed grids use no norm and are unaffected.  With it the accepted range is 0 .. 0x7F. */
 #define PHX_PARAMS_ALL 0x3F
+#define PHX_NORM_SEMINORM 0x40
 int phx_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
                              int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                              const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,

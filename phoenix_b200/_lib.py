@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_HERE, "libphoenix_b200.so")
 PHX_OK = 0
 METHOD_IDS = {"euler": 0, "midpoint": 1, "rk4": 2, "dopri5": 3}
 PARAMS_ALL = 0x3F   # adjoint parameter mask: bit i = the i-th ODENet parameter in reference order
+NORM_SEMINORM = 0x40   # OR-ed into an adjoint solve's mask: the dopri5 error norm leaves out the parameter block
 PREC_FP32, PREC_TF32, PREC_3XTF32 = 0, 1, 3
 ST_OK, ST_DT_UNDERFLOW, ST_NONFINITE, ST_MAX_STEPS, ST_RUNNING = 0, 1, 2, 3, 99
 

@@ -143,6 +143,15 @@ bool check_mask(int mask) {
     return true;
 }
 
+// the adjoint solves also take PHX_NORM_SEMINORM
+bool check_adjoint_mask(int mask) {
+    if (mask < 0 || mask > (PHX_P_ALL | PHX_NORM_SEMINORM)) {
+        phx_set_error("param_mask must be a 6-bit mask, optionally with PHX_NORM_SEMINORM (0 .. 0x7F), got %d", mask);
+        return false;
+    }
+    return true;
+}
+
 bool check_dims(int G, int H, int B) {
     if (G < 1 || H < 1 || B < 1) {
         phx_set_error("invalid dims G=%d H=%d B=%d", G, H, B);
@@ -471,7 +480,7 @@ int phx_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* pac
                              int param_mask, void* stream) {
     PhxDevGuard dev_guard(ctx);
     g_err[0] = 0;
-    if (!check_mask(param_mask)) return PHX_ERR_INVALID;
+    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
     if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
         return PHX_ERR_INVALID;
@@ -528,7 +537,7 @@ int phx_solve_adjoint_many_masked(phx_ctx* ctx, int G, int H, int B, int N, cons
                                   void* stream) {
     PhxDevGuard dev_guard(ctx);
     g_err[0] = 0;
-    if (!check_mask(param_mask)) return PHX_ERR_INVALID;
+    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
     if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
         return PHX_ERR_INVALID;
@@ -735,7 +744,7 @@ int phx_solve_adjoint_rows_masked(phx_ctx* ctx, int G, int H, int N, const float
                                   int steplog_cap, int param_mask, void* stream) {
     PhxDevGuard dev_guard(ctx);
     g_err[0] = 0;
-    if (!check_mask(param_mask)) return PHX_ERR_INVALID;
+    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
     if (!y_saved || !grad_y || !adj_y0 || !grads_packed_parts) {
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_packed_parts");
         return PHX_ERR_INVALID;

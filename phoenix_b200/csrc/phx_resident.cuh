@@ -1611,7 +1611,8 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_fwd_kernel(const __grid_co
 //   Wp[h][g]  : sum_b gLP[q][b][h] * l[q][b][g]        bp[h] : sum_b gLP[q][b][h]
 //   Ws[h][g]  : sum_b gS [q][b][h] * s[q][b][g]        bs[h] : sum_b gS [q][b][h]
 //   Wa[g][k]  : sum_b gJ [q][b][g] * SP[q][b][k]
-enum { PP_D01 = 0, PP_D2 = 1, PP_STEP = 2, PP_FIXED = 3, PP_COPY = 4 };
+// PP_SOL: PP_STEP without the error estimate and its norm sums -- the seminorm's pass, run after the accept decision
+enum { PP_D01 = 0, PP_D2 = 1, PP_STEP = 2, PP_FIXED = 3, PP_COPY = 4, PP_SOL = 5 };
 
 struct PPArgs {
     const float* src;   // theta at step start; nullptr while theta is known to be identically zero
@@ -1681,7 +1682,8 @@ __device__ __forceinline__ void theta_elem(const float atol_f, const float rtol_
 // PP_STEP for one theta element with the seven stage derivatives produced on the fly by kq(q) (q = physical slot):
 // no k[] array exists, so nothing can be demoted to local memory (a select chain over an array is turned into a
 // dynamically indexed load by the optimiser).  Same operation order as the reference's k.matmul(dt * c).
-template <typename KQ>
+// ERR == false (PP_SOL): the written value only -- no error combination, no norm sums.
+template <bool ERR = true, typename KQ>
 __device__ __forceinline__ float theta_step_val(const float atol_f, const float rtol_f, const PPArgs& a, const float th0, KQ kq,
                                                 double& acc0, double& acc1) {
     float inc = 0.f, e = 0.f, md = 0.f, kf = 0.f, kl = 0.f;
@@ -1690,34 +1692,37 @@ __device__ __forceinline__ float theta_step_val(const float atol_f, const float 
         const float t = kq(q);
         if (q == 0) {
             inc = t * a.coef_sol[0];
-            e = t * a.coef_err[0];
+            if (ERR) e = t * a.coef_err[0];
             md = t * a.coef_mid[0];
         } else {
             inc = fmaf(t, a.coef_sol[q], inc);
-            e = fmaf(t, a.coef_err[q], e);
+            if (ERR) e = fmaf(t, a.coef_err[q], e);
             md = fmaf(t, a.coef_mid[q], md);
         }
         kf = (q == a.slot_first) ? t : kf;
         kl = (q == a.slot_last) ? t : kl;
     }
     const float th1 = th0 + inc;
-    const float tol = atol_f + rtol_f * fmaxf(fabsf(th0), fabsf(th1));
-    const float r = e / tol;
-    acc0 += (double)(r * r);
-    if (!isfinite(th1)) acc1 += 1.0;
+    if (ERR) {
+        const float tol = atol_f + rtol_f * fmaxf(fabsf(th0), fabsf(th1));
+        const float r = e / tol;
+        acc0 += (double)(r * r);
+        if (!isfinite(th1)) acc1 += 1.0;
+    }
     return a.last ? interp_eval(th0, th1, th0 + md, kf, kl, a.dtf, a.xs) : th1;
 }
-template <typename KQ>
+template <bool ERR = true, typename KQ>
 __device__ __forceinline__ void theta_step(const float atol_f, const float rtol_f, const PPArgs& a, size_t idx, KQ kq,
                                            double& acc0, double& acc1) {
     const float th0 = a.src ? a.src[idx] : 0.f;
-    a.dst[idx] = theta_step_val(atol_f, rtol_f, a, th0, kq, acc0, acc1);
+    a.dst[idx] = theta_step_val<ERR>(atol_f, rtol_f, a, th0, kq, acc0, acc1);
 }
 
-// which factor slots a mode needs, as k[0..NK): D01 {s0}, D2 {s0, s1}, STEP all seven physical slots, FIXED 0..3
+// which factor slots a mode needs, as k[0..NK): D01 {s0}, D2 {s0, s1}, STEP / SOL all seven physical slots, FIXED 0..3
 template <int MODE>
 struct PPSlots {
-    static constexpr int NK = (MODE == PP_D01) ? 1 : (MODE == PP_D2 ? 2 : (MODE == PP_STEP ? 7 : (MODE == PP_FIXED ? 4 : 0)));
+    static constexpr int NK = (MODE == PP_D01) ? 1
+                            : (MODE == PP_D2 ? 2 : ((MODE == PP_STEP || MODE == PP_SOL) ? 7 : (MODE == PP_FIXED ? 4 : 0)));
 };
 template <int MODE>
 __device__ __forceinline__ int pp_slot(const PPArgs& a, int i) {
@@ -1750,7 +1755,7 @@ __device__ __forceinline__ void pp_block(const float atol_f, const float rtol_f,
 #pragma unroll
             for (int b = 0; b < BT; ++b) v[i][b] = vp[uo[i] + b];
         }
-        if constexpr (MODE == PP_STEP) {
+        if constexpr (MODE == PP_STEP || MODE == PP_SOL) {
             // two rows per iteration: the per-element chain (7-term combinations, a division, the quartic) is long
             // and the rows are independent, so interleaving them doubles the instruction-level parallelism
             for (int r = ry; r < R; r += 2 * RG) {
@@ -1769,7 +1774,7 @@ __device__ __forceinline__ void pp_block(const float atol_f, const float rtol_f,
                 const size_t iA = gbase + (size_t)r * ld + c0 + cx, iB = gbase + (size_t)(two ? r2 : r) * ld + c0 + cx;
                 const float thA = a.src ? a.src[iA] : 0.f, thB = a.src ? a.src[iB] : 0.f;
                 double b0 = 0, b1 = 0;
-                const float oA = theta_step_val(atol_f, rtol_f, a, thA,
+                const float oA = theta_step_val<MODE == PP_STEP>(atol_f, rtol_f, a, thA,
                                                 [&](int q) {
                                                     float t = 0.f;
 #pragma unroll
@@ -1777,7 +1782,7 @@ __device__ __forceinline__ void pp_block(const float atol_f, const float rtol_f,
                                                     return t;
                                                 },
                                                 acc0, acc1);
-                const float oB = theta_step_val(atol_f, rtol_f, a, thB,
+                const float oB = theta_step_val<MODE == PP_STEP>(atol_f, rtol_f, a, thB,
                                                 [&](int q) {
                                                     float t = 0.f;
 #pragma unroll
@@ -1854,8 +1859,9 @@ __device__ __noinline__ PPSums ppass(const ResParams& __restrict__ p, int g_lo, 
     // m
     if (pm & PHX_P_M)
     for (int j = threadIdx.x; j < n_loc; j += THREADS) {
-        if constexpr (MODE == PP_STEP) {
-            theta_step(atol_f, rtol_f, a, off.m + g_lo + j, [&](int q) { return s.FM()[j * 8 + q]; }, acc0, acc1);
+        if constexpr (MODE == PP_STEP || MODE == PP_SOL) {
+            theta_step<MODE == PP_STEP>(atol_f, rtol_f, a, off.m + g_lo + j, [&](int q) { return s.FM()[j * 8 + q]; },
+                                        acc0, acc1);
         } else {
             float k[7];
 #pragma unroll
@@ -1879,8 +1885,8 @@ __device__ __noinline__ PPSums ppass(const ResParams& __restrict__ p, int g_lo, 
             const bool prod = h >= H;
             if (!(pm & (prod ? PHX_P_BP : PHX_P_BS))) continue;
             const float* up = s.FG() + (size_t)(prod ? Hp + h - H : h) * QB;
-            if constexpr (MODE == PP_STEP) {
-                theta_step(atol_f, rtol_f, a, (prod ? off.bp + (h - H) : off.bs + h),
+            if constexpr (MODE == PP_STEP || MODE == PP_SOL) {
+                theta_step<MODE == PP_STEP>(atol_f, rtol_f, a, (prod ? off.bp + (h - H) : off.bs + h),
                            [&](int q) {
                                float t = 0.f;
                                for (int b = 0; b < BT; ++b) t += up[q * BT + b];
@@ -2012,7 +2018,8 @@ __device__ __forceinline__ void adj_eval(const ResParams& __restrict__ p, Smem& 
     pf.tick(PT_PHASE_C);
 }
 
-template <int NV, int BT>
+// SEMI: the seminorm (p.pmask & PHX_NORM_SEMINORM), an instantiation of its own so that the default norm keeps its code
+template <int NV, int BT, bool SEMI>
 __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_constant__ ResParams p) {
     constexpr int QB = (7 * BT + 3) & ~3;
     Smem s(p);
@@ -2026,8 +2033,9 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
     const double Nel = (double)p.B * (double)p.G;
     const PhxGradOff goff = phx_grad_offsets(p.G, p.H);
     // theta block of the norm: the adjoint parameters only; with none the block is absent (th_rms == 0 never wins the
-    // max over the other, non-negative blocks)
-    const double Pel = (double)phx_mask_count(p.G, p.H, p.pmask);
+    // max over the other, non-negative blocks).  The seminorm drops it too: no theta norm pass runs, and the theta step
+    // pass moves after the accept decision (accepted attempts only, solution combination only, in place)
+    const double Pel = SEMI ? 0.0 : (double)phx_mask_count(p.G, p.H, p.pmask);
     auto th_rms = [&](double sum) { return Pel > 0 ? sqrtf((float)(sum / Pel)) : 0.f; };
     float* Y = s.st();
     float* A = s.st() + BL;
@@ -2180,11 +2188,14 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 __syncthreads();
                 pf.tick(PT_COMBINE);
                 if (which == 0) {
-                    if (theta_zero) acc[5] += theta_zero_norm<BT>(p, n_loc, 0, -1);
-                    else {
-                        PPSums ps = ppass<PP_D01, BT>(p, g_lo, n_loc);
-                        acc[2] += ps.a0;
-                        acc[5] += ps.a1;
+                    if (!SEMI) {   // (the seminorm has no theta block)
+                        if (theta_zero) {
+                            acc[5] += theta_zero_norm<BT>(p, n_loc, 0, -1);
+                        } else {
+                            PPSums ps = ppass<PP_D01, BT>(p, g_lo, n_loc);
+                            acc[2] += ps.a0;
+                            acc[5] += ps.a1;
+                        }
                     }
                     pf.tick(PT_PP_D01);
                     block_sum_d<7>(acc, s.dred(), c->dsum);
@@ -2207,8 +2218,10 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                     });
                     __syncthreads();
                 } else {
-                    if (theta_zero) acc[2] += theta_zero_norm<BT>(p, n_loc, 1, 0);
-                    else acc[2] += ppass<PP_D2, BT>(p, g_lo, n_loc).a0;
+                    if (!SEMI) {
+                        if (theta_zero) acc[2] += theta_zero_norm<BT>(p, n_loc, 1, 0);
+                        else acc[2] += ppass<PP_D2, BT>(p, g_lo, n_loc).a0;
+                    }
                     pf.tick(PT_PP_D2);
                     block_sum_d<7>(acc, s.dred(), c->dsum);
                     grid_sum_d(p, s, c->dsum, 3);
@@ -2296,7 +2309,8 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 if (threadIdx.x == 0) {
                     PPArgs& pa = *s.at<PPArgs>(p.so.ppa);
                     pa.src = theta_zero ? nullptr : (cur ? p.theta1 : theta0p);
-                    pa.dst = theta_zero ? theta0p : (cur ? theta0p : p.theta1);
+                    // (seminorm: cur stays 0, the pass writes in place)
+                    pa.dst = (theta_zero || SEMI) ? theta0p : (cur ? theta0p : p.theta1);
                     pa.dtf = c->dtf;
                     pa.last = c->last;
                     for (int q = 0; q < 7; ++q) {
@@ -2310,7 +2324,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 }
                 __syncthreads();
                 pf.tick(PT_COMBINE);
-                {
+                if (!SEMI) {
                     PPSums ps = ppass<PP_STEP, BT>(p, g_lo, n_loc);
                     acc[2] += ps.a0;
                     acc[3] += ps.a1;
@@ -2342,7 +2356,17 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 }
                 __syncthreads();
                 if (c->accept) {
-                    if (theta_zero) { cur = 0; theta_zero = false; } else cur ^= 1;
+                    if (SEMI) {
+                        // the seminorm's theta step: accepted attempts only, in place (cur stays 0)
+                        ppass<PP_SOL, BT>(p, g_lo, n_loc);
+                        pf.tick(PT_PP_STEP);
+                        theta_zero = false;
+                    } else if (theta_zero) {
+                        cur = 0;
+                        theta_zero = false;
+                    } else {
+                        cur ^= 1;
+                    }
                     if (c->last) {
                         // last step of the interval: dense output at t_end for adj_y (adj_params: done in the pass)
                         const float dtf = c->dtf;
@@ -2393,7 +2417,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
         __syncthreads();
         ppass<PP_COPY, BT>(p, g_lo, n_loc);
     }
-    if (!theta_zero && p.pmask != PHX_P_ALL) {
+    if (!theta_zero && (SEMI ? p.pmask & PHX_P_ALL : p.pmask) != PHX_P_ALL) {
         // the blocks of parameters outside the adjoint set were never touched: report zeros
         const int pm = p.pmask;
         const size_t HG = (size_t)p.H * p.G;

@@ -34,7 +34,18 @@ int launch_coop(KernelT kernel, const ResParams& p, const ResLaunchPlan& plan, c
 #define PHX_FN PHX_CAT(phx_launch_fwd_nv, PHX_NV)
 #endif
 
+#if PHX_KIND_ADJ
+int PHX_FN(const ResParams& p, const ResLaunchPlan& plan, cudaStream_t stream) {
+    if (p.pmask & PHX_NORM_SEMINORM) {
+        if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4, true>, p, plan, stream);
+        return launch_coop(PHX_KERNEL<PHX_NV, 1, true>, p, plan, stream);
+    }
+    if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4, false>, p, plan, stream);
+    return launch_coop(PHX_KERNEL<PHX_NV, 1, false>, p, plan, stream);
+}
+#else
 int PHX_FN(const ResParams& p, const ResLaunchPlan& plan, cudaStream_t stream) {
     if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4>, p, plan, stream);
     return launch_coop(PHX_KERNEL<PHX_NV, 1>, p, plan, stream);
 }
+#endif

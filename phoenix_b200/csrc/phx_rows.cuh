@@ -1183,9 +1183,10 @@ __device__ __noinline__ void rows_theta_pass_impl(const ResParams& __restrict__ 
     __syncthreads();
 }
 
-template <int MODE>
+// SEMI: p.pmask may carry PHX_NORM_SEMINORM above the six parameter bits
+template <int MODE, bool SEMI>
 __device__ __forceinline__ void rows_theta_pass(const ResParams& __restrict__ p, int g_lo, int n_loc, uint32_t tmem, double* out) {
-    if (p.pmask == PHX_P_ALL) rows_theta_pass_impl<MODE, true>(p, g_lo, n_loc, tmem, out);
+    if ((SEMI ? (p.pmask & PHX_P_ALL) : p.pmask) == PHX_P_ALL) rows_theta_pass_impl<MODE, true>(p, g_lo, n_loc, tmem, out);
     else rows_theta_pass_impl<MODE, false>(p, g_lo, n_loc, tmem, out);
 }
 
@@ -1325,6 +1326,8 @@ __device__ __noinline__ double rows_theta_zero_norm(const ResParams& __restrict_
     return res;
 }
 
+// SEMI: the seminorm (p.pmask & PHX_NORM_SEMINORM), an instantiation of its own so that the default norm keeps its code
+template <bool SEMI>
 __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __grid_constant__ ResParams p) {
     Smem s(p);
     RowsView v(p, s);
@@ -1335,8 +1338,10 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
     const int tot = n_loc * RM, BL = RM * p.gpc;
     const double Nel = (double)p.G;
     // theta block of the norm: the adjoint parameters only; with none the block is absent (th_rms == 0 never wins the
-    // max over the other, non-negative blocks)
-    const double Pel = (double)phx_mask_count(p.G, p.H, p.pmask);
+    // max over the other, non-negative blocks).  The seminorm drops it too: no theta norm pass or Gram sum runs, and the
+    // theta step pass moves after the accept decision (accepted rows only, solution combination only)
+    constexpr bool semi = SEMI;
+    const double Pel = semi ? 0.0 : (double)phx_mask_count(p.G, p.H, p.pmask);
     auto th_rms = [&](double sum) { return Pel > 0 ? sqrtf((float)(sum / Pel)) : 0.f; };
     float* Y = v.st(0);
     float* A = v.st(1);
@@ -1486,7 +1491,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         });
                 }
                 __syncthreads();
-                rows_theta_pass<TP_FIXED>(p, g_lo, n_loc, s.tmem, tsum);
+                rows_theta_pass<TP_FIXED, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
                 pf.tick(PT_PP_STEP);
                 if (threadIdx.x < RM) {
                     RowCtl& c = rc->r[threadIdx.x];
@@ -1531,7 +1536,8 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         }
                         return 0.f;
                     });
-                    // theta norms: Gram sums while a row's accumulator is still zero, a pass over memory otherwise
+                    // theta norms: Gram sums while a row's accumulator is still zero, a pass over memory otherwise (none
+                    // under the seminorm)
                     bool any_nz = false;
                     for (int b = 0; b < RM; ++b) any_nz |= (!rc->r[b].done && !rc->r[b].theta_zero);
                     if (threadIdx.x < RM) {
@@ -1544,17 +1550,20 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         a.active = !c.done && !c.theta_zero;
                     }
                     __syncthreads();
-                    const double zn = rows_theta_zero_norm(p, n_loc, s.tmem, which == 0 ? 0 : 6, which == 0 ? -1 : 0);
-                    if (any_nz) {
-                        if (which == 0) rows_theta_pass<TP_D01>(p, g_lo, n_loc, s.tmem, tsum);
-                        else rows_theta_pass<TP_D2>(p, g_lo, n_loc, s.tmem, tsum);
+                    const double zn =
+                        semi ? 0.0 : rows_theta_zero_norm(p, n_loc, s.tmem, which == 0 ? 0 : 6, which == 0 ? -1 : 0);
+                    if (any_nz && !semi) {
+                        if (which == 0) rows_theta_pass<TP_D01, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
+                        else rows_theta_pass<TP_D2, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
                     }
                     pf.tick(which == 0 ? PT_PP_D01 : PT_PP_D2);
                     block_sum_rows<7>(v, acc, dsum);
                     if (threadIdx.x < RM) {
                         const RowCtl& c = rc->r[threadIdx.x];
                         double* d = dsum + threadIdx.x * 7;
-                        if (c.theta_zero) {
+                        if (semi) {
+                            // (the seminorm has no theta block)
+                        } else if (c.theta_zero) {
                             d[which == 0 ? 5 : 2] += zn;
                         } else if (which == 0) {
                             d[2] += tsum[2 * threadIdx.x];
@@ -1678,13 +1687,13 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         if (c.last) rows_interp_weights(c, a);
                     }
                     __syncthreads();
-                    if (threadIdx.x == 0) plan_spec(iv == 1);
+                    if (threadIdx.x == 0 && !semi) plan_spec(iv == 1);
                     __syncthreads();
                     pf.tick(PT_COMBINE);
-                    rows_theta_pass<TP_STEP>(p, g_lo, n_loc, s.tmem, tsum);
+                    if (!semi) rows_theta_pass<TP_STEP, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
                     pf.tick(PT_PP_STEP);
                     block_sum_rows<4>(v, acc, dsum);
-                    if (threadIdx.x < RM) {
+                    if (threadIdx.x < RM && !semi) {
                         dsum[threadIdx.x * 4 + 2] += tsum[2 * threadIdx.x];
                         dsum[threadIdx.x * 4 + 3] += tsum[2 * threadIdx.x + 1];
                     }
@@ -1718,7 +1727,19 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         }
                     }
                     __syncthreads();
-                    if (rc->spec_pass) {
+                    if (semi) {
+                        // the accepted rows' theta step, as a fixed-grid pass with the solution (or dense-output)
+                        // weights wo: acceptance is known, so a speculative final step goes straight into the group sum
+                        if (threadIdx.x < RM) pp[threadIdx.x].active = rc->r[threadIdx.x].accept;
+                        __syncthreads();
+                        if (threadIdx.x == 0) plan_spec(iv == 1);
+                        __syncthreads();
+                        rows_theta_pass<TP_FIXED, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
+                        pf.tick(PT_PP_STEP);
+                        if (threadIdx.x < RM && pp[threadIdx.x].spec) rc->r[threadIdx.x].spec_done = 1;
+                        if (threadIdx.x == 0 && rc->spec_pass) rc->spec_valid = 1;
+                        __syncthreads();
+                    } else if (rc->spec_pass) {
                         // did every speculating row accept?  otherwise materialise the accepted ones
                         if (threadIdx.x == 0) {
                             bool ok = true;
@@ -1734,7 +1755,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                             }
                         }
                         __syncthreads();
-                        if (rc->redo) rows_theta_pass<TP_STEP>(p, g_lo, n_loc, s.tmem, tsum);
+                        if (rc->redo) rows_theta_pass<TP_STEP, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
                     }
                     for (int e = threadIdx.x; e < tot; e += THREADS) {
                         const RowCtl& c = rc->r[e & 3];

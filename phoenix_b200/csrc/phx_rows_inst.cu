@@ -23,7 +23,8 @@ int launch_rows(KernelT kernel, const ResParams& p, const RowsPlan& plan, cudaSt
 
 #if PHX_KIND_ADJ
 int phx_launch_rows_adj(const ResParams& p, const RowsPlan& plan, cudaStream_t stream) {
-    return launch_rows(phx_rows_adj_kernel, p, plan, stream);
+    if (p.pmask & PHX_NORM_SEMINORM) return launch_rows(phx_rows_adj_kernel<true>, p, plan, stream);
+    return launch_rows(phx_rows_adj_kernel<false>, p, plan, stream);
 }
 #else
 int phx_launch_rows_fwd(const ResParams& p, const RowsPlan& plan, cudaStream_t stream) {

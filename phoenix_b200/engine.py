@@ -556,7 +556,8 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
         _lib.check(lib.phx_unpack_grads(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, sp), "unpack_grads")
     else:
         _lib.check(lib.phx_solve_adjoint_rows_masked(*args, param_mask, sp), "solve_adjoint_rows")
-        _lib.check(lib.phx_unpack_grads_masked(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, param_mask, sp),
+        _lib.check(lib.phx_unpack_grads_masked(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0,
+                                               param_mask & _lib.PARAMS_ALL, sp),
                    "unpack_grads")
     _tls().last_status_block = stn
     for i in range(N):
@@ -599,7 +600,8 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
                   param_mask=_lib.PARAMS_ALL):
     """adj_y0 and the six parameter cotangents of one backward sweep.  ``param_mask`` (bit i = the i-th parameter in
     reference order): the adjoint parameters, the only ones integrated and put in the error norm; the cotangents of the
-    others come back as zeros."""
+    others come back as zeros.  With ``_lib.NORM_SEMINORM`` also set, the dopri5 error norm leaves the parameter block
+    out altogether (the seminorm)."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()

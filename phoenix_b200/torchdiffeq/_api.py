@@ -8,6 +8,7 @@ import torch
 import torch.nn as nn
 
 from .. import engine
+from .._lib import NORM_SEMINORM, PARAMS_ALL
 from ..odenet import ODENet
 
 # every method string the vendored package registers (odeint.py:9-22); only the four PHOENIX uses are accelerated
@@ -105,13 +106,14 @@ def _register_node(ctx, func, y0, tl, t_is_f32, adj):
     """Forward side: note the node if its backward may be batched with its siblings' (a one-row state that needs no
     gradient itself -- the training loop's case)."""
     ctx.group = None
-    if (not DEFER_ADJOINT or ctx.needs_input_grad[8] or not any(ctx.needs_input_grad[9:]) or not adj[4]
+    if (not DEFER_ADJOINT or ctx.needs_input_grad[8] or not any(ctx.needs_input_grad[9:]) or not adj[4] & PARAMS_ALL
             or y0.numel() != y0.shape[-1]):
         return   # (nothing to differentiate -- e.g. a validation pass under no_grad -- is not a node at all)
     with _defer_lock:
         _node_seq[0] += 1
         ctx.seq = _node_seq[0]
-        # adj[4], the adjoint parameter mask, is part of the key: only nodes with the same adjoint set share a sweep
+        # adj[4], the adjoint parameter mask with the norm bit, is part of the key: only nodes with the same adjoint set
+        # and the same error norm share a sweep
         ctx.group = (len(tl), t_is_f32, adj, tuple(y0.shape), y0.device, tuple(ctx.needs_input_grad[9:]))
         nodes = _live_nodes.get(func)
         if nodes is None:
@@ -181,7 +183,7 @@ class OdeintAdjointMethod(torch.autograd.Function):
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
         a_method, a_rtol, a_atol, a_max, mask = ctx.adj
-        if not mask and not ctx.needs_input_grad[8]:
+        if not mask & PARAMS_ALL and not ctx.needs_input_grad[8]:
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))   # only parameters outside adjoint_params want one
         batch = _defer(ctx, y, grad_y) if (ctx.group is not None and DEFER_ADJOINT) else _NOT_DEFERRED
         if batch is None:
@@ -198,13 +200,15 @@ class OdeintAdjointMethod(torch.autograd.Function):
 
 
 def _masked(mask):
-    """The engine's keyword for a proper subset of the parameters; with all six the engine is called as it always was."""
-    return {} if mask == 0x3F else {"param_mask": mask}
+    """The engine's keyword for a proper subset of the parameters or the seminorm; with all six parameters and the
+    default norm the engine is called as it always was."""
+    return {} if mask == PARAMS_ALL else {"param_mask": mask}
 
 
 def _grads_out(ctx, adj_y0, grads, mask):
     """backward's result: adj_y0 for y0, and a cotangent only for the parameters in the adjoint set (None for the others
-    even when they require grad: the reference's adjoint node does not take them as inputs)."""
+    even when they require grad: the reference's adjoint node does not take them as inputs).  Only the six parameter bits
+    of ``mask`` are read, never the norm bit."""
     out = [None] * 8 + [adj_y0 if ctx.needs_input_grad[8] else None]
     for i, need in enumerate(ctx.needs_input_grad[9:]):
         out.append(grads[i] if (need and mask >> i & 1) else None)
@@ -235,10 +239,26 @@ def _adjoint_mask(func, adjoint_params):
     return params, mask
 
 
+def _adjoint_norm(adjoint_options):
+    """Take ``norm`` out of the adjoint options: the remaining options and the norm's bit of the adjoint mask
+    (NORM_SEMINORM for ``"seminorm"``, 0 when no norm is given)."""
+    if adjoint_options is None or "norm" not in adjoint_options:
+        return adjoint_options, 0
+    opts = dict(adjoint_options)
+    norm = opts.pop("norm")
+    if not (isinstance(norm, str) and norm == "seminorm"):
+        raise NotImplementedError('adjoint_options["norm"] = {!r} is not supported: the error norm is evaluated on the '
+                                  'device, and only "seminorm" (the mixed norm without the parameter block) is '
+                                  'implemented there'.format(norm))
+    return opts, NORM_SEMINORM
+
+
 def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None, adjoint_rtol=None,
                    adjoint_atol=None, adjoint_method=None, adjoint_options=None, adjoint_params=None):
     """adjoint.py:165-204: same as ``odeint`` but differentiable w.r.t. y0 and the ODENet parameters through the
-    continuous adjoint, solved backwards with the forward method / tolerances unless overridden."""
+    continuous adjoint, solved backwards with the forward method / tolerances unless overridden.
+    ``adjoint_options=dict(norm="seminorm")`` measures the dopri5 backward's error without the parameter cotangents
+    (Kidger, Chen & Lyons, 2021), in the initial step and in every error ratio."""
     if adjoint_params is None and not isinstance(func, nn.Module):
         raise ValueError('func must be an instance of nn.Module to specify the adjoint parameters; alternatively they '
                          'can be specified explicitly via the `adjoint_params` argument. If there are no parameters '
@@ -249,6 +269,7 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
         adjoint_atol = atol
     if adjoint_method is None:
         adjoint_method = method
+    adjoint_options, norm_bit = _adjoint_norm(adjoint_options)
     if adjoint_options is None:
         adjoint_options = {k: v for k, v in options.items() if k != "norm"} if options is not None else {}
     same = (adjoint_rtol is rtol and adjoint_atol is atol and adjoint_method is method and not adjoint_options
@@ -263,7 +284,7 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
         raise NotImplementedError("odeint_adjoint with decreasing t is not part of the PHOENIX path")
     params, mask = _adjoint_mask(func, adjoint_params)
     return OdeintAdjointMethod.apply(func, tl, t_is_f32, method, rtol, atol, max_steps,
-                                     (a_method, a_rtol, a_atol, a_max, mask), y0, *params)
+                                     (a_method, a_rtol, a_atol, a_max, mask | norm_bit), y0, *params)
 
 
 class OdeintAdjointManyMethod(torch.autograd.Function):
@@ -281,7 +302,7 @@ class OdeintAdjointManyMethod(torch.autograd.Function):
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
         a_method, a_rtol, a_atol, a_max, mask = ctx.adj
-        if not mask and not ctx.needs_input_grad[8]:
+        if not mask & PARAMS_ALL and not ctx.needs_input_grad[8]:
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))
         with torch.no_grad():
             adj_y0, grads = engine.solve_adjoint_many(ctx.func, ctx.t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
@@ -289,14 +310,16 @@ class OdeintAdjointManyMethod(torch.autograd.Function):
         return _grads_out(ctx, adj_y0, grads, mask)
 
 
-def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None, adjoint_params=None):
+def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None, adjoint_params=None,
+                        adjoint_options=None):
     """The per-sample loop of the reference's ``training_step`` (train_insilico.py:128-130,
     ``[odeint(odenet, batch_point, time_points, method=method)[1] for ...]``) as ONE call: ``y0`` is ``[N, *S, G]``
     (N independent initial states), ``t`` is ``[N, T]`` (each sample's own times, increasing) and the result is
     ``[N, T, *S, G]`` with ``result[i] == odeint_adjoint(func, y0[i], t[i], ...)`` bit for bit: every sample is still
     its own solve with its own step controller (NOT the global-norm batched call).  Gradients flow to ``y0`` and to the
     ODENet parameters of ``adjoint_params`` that require grad (default: all six; summed over the samples) through one
-    autograd node.  No reference counterpart: opt-in."""
+    autograd node.  ``adjoint_options`` as in ``odeint_adjoint`` (default: the forward options without ``norm``).  No
+    reference counterpart: opt-in."""
     assert torch.is_tensor(t) and t.ndimension() == 2, "t must be a [N, T] tensor of per-sample times"
     assert torch.is_tensor(y0) and y0.shape[0] == t.shape[0], "y0 and t must hold the same number of samples"
     if y0.shape[0] == 0:
@@ -308,6 +331,10 @@ def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=
         assert all(b > a for a, b in zip(r, r[1:])), 't must be strictly increasing for every sample'
     if rev:
         raise NotImplementedError("odeint_adjoint_many with decreasing t is not part of the PHOENIX path")
+    adjoint_options, norm_bit = _adjoint_norm(adjoint_options)
+    a_max = max_steps
+    if adjoint_options is not None:
+        a_max = _normalise(func, y0[0], t[0], rtol, atol, method, adjoint_options)[6]
     params, mask = _adjoint_mask(func, adjoint_params)
     return OdeintAdjointManyMethod.apply(func, rows, t_is_f32, method, rtol_f, atol_f, max_steps,
-                                         (method, rtol_f, atol_f, max_steps, mask), y0, *params)
+                                         (method, rtol_f, atol_f, a_max, mask | norm_bit), y0, *params)
