@@ -283,6 +283,69 @@ int phx_solve_adjoint_rows_masked(phx_ctx* ctx, int G, int H, int N, const float
                                   int steplog_cap, int param_mask, void* stream);
 size_t phx_packed_grad_bytes(int G, int H);
 int phx_rows_grad_parts(const phx_ctx* ctx, int G, int H, int N);
+
+/* ---- fixed-grid solves on a step grid (odeint options=dict(step_size=h), torchdiffeq solvers.py:48-50, 77-103) ----------
+ * The *_grid variants take the same arguments as the entry point they are named after (the adjoint ones: as its *_masked
+ * variant, param_mask included; PHX_NORM_SEMINORM is accepted and has no effect) plus the grid, host arrays, right before
+ * the stream.  The method must be euler, midpoint or rk4; the caller builds the grid (the Python layer does it with the
+ * reference's own tensor ops) and no kernel computes one:
+ *   grid_steps[q] >= 1 steps per segment and their float32 dt back to back in grid_dt (in segment order).  A forward
+ *     segment is a problem (N of them; 1 for the one-problem calls); an adjoint segment is an output interval of a problem,
+ *     [N][T-1] with the interval [t[i], t[i+1]] at index i, its steps in the order the backward takes them (from t[i+1]).
+ *   forward only, [N][T-1]: grid_out_step[j-1] = the step (counted from 0 within the problem, non-decreasing in j) whose
+ *     end is the first grid point >= t[j], and grid_out_slope[j-1] = (t[j] - t0) / (t1 - t0) of that step, rounded to
+ *     float32; output j is then y0 + slope * (y1 - y0), or y1 itself when the slope is negative (t[j] == t1).
+ * Between the steps the state is not restarted at the output times.  status.n_rhs = stages x steps.  The grid is copied
+ * into the workspace (not for the streaming engine), which must then hold phx_grid_workspace_bytes(N, T, total steps)
+ * more bytes than the entry point's own size function asks for.  An invalid grid (a step count < 1, a dt that is negative
+ * or not finite, an output step out of range or decreasing, a NaN slope) returns PHX_ERR_INVALID. */
+size_t phx_grid_workspace_bytes(int N, int T, int64_t total_steps);
+int phx_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
+                           const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
+                           double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
+                           phx_status* status, double* steplog, int steplog_cap, const float* grid_dt,
+                           const int32_t* grid_steps, const int32_t* grid_out_step, const float* grid_out_slope,
+                           void* stream);
+int phx_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                           int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                           const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                           void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                           int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
+                           void* stream);
+int phx_solve_forward_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const float* y0,
+                                const double* t_host, int T, int t_is_f32, int method, double rtol, double atol,
+                                int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
+                                phx_status* status, const float* grid_dt, const int32_t* grid_steps,
+                                const int32_t* grid_out_step, const float* grid_out_slope, void* stream);
+int phx_solve_adjoint_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host,
+                                int T, int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
+                                const float* grid_dt, const int32_t* grid_steps, void* stream);
+int phx_solve_forward_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const float* y0,
+                                const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
+                                double atol, int64_t max_num_steps, float* y_out, void* workspace,
+                                size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
+                                const float* grid_dt, const int32_t* grid_steps, const int32_t* grid_out_step,
+                                const float* grid_out_slope, void* stream);
+int phx_solve_adjoint_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
+                                int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
+                                void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
+                                void* stream);
+int phx_stream_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
+                                  const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
+                                  double atol, int64_t max_num_steps, float* y_out, void* workspace,
+                                  size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
+                                  const float* grid_dt, const int32_t* grid_steps, const int32_t* grid_out_step,
+                                  const float* grid_out_slope, void* stream);
+int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                  int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
+                                  void* stream);
 int phx_unpack_grads(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
                      int accumulate, void* stream);
 int phx_unpack_grads_masked(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,

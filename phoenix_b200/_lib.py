@@ -29,6 +29,9 @@ EXPORTS = [
     "phx_solve_adjoint_rows", "phx_unpack_grads", "phx_packed_grad_bytes", "phx_rows_grad_parts",
     "phx_solve_adjoint_masked", "phx_solve_adjoint_many_masked", "phx_stream_solve_adjoint_masked",
     "phx_solve_adjoint_rows_masked", "phx_unpack_grads_masked",
+    "phx_grid_workspace_bytes", "phx_solve_forward_grid", "phx_solve_adjoint_grid", "phx_solve_forward_many_grid",
+    "phx_solve_adjoint_many_grid", "phx_solve_forward_rows_grid", "phx_solve_adjoint_rows_grid",
+    "phx_stream_solve_forward_grid", "phx_stream_solve_adjoint_grid",
     "phx_prior_loss", "phx_prior_setup", "phx_tc_set_pair", "phx_tc_prof_dump", "phx_ctx_set_global_norm", "phx_peer_allreduce", "phx_peer_allreduce_nvls", "phx_mse_grad", "phx_hill_planes", "phx_hill_cache_set",
 ]
 
@@ -141,6 +144,18 @@ def _declare(lib):
                  "phx_unpack_grads"):
         fn = getattr(lib, name + "_masked")
         fn.argtypes = getattr(lib, name).argtypes[:-1] + [c_int, c_void_p]
+        fn.restype = c_int
+    # the *_grid variants (fixed-grid solves on a step grid): the forward ones take (grid_dt, grid_steps, grid_out_step,
+    # grid_out_slope), the adjoint ones -- which follow the *_masked argument lists -- (grid_dt, grid_steps) before the stream
+    lib.phx_grid_workspace_bytes.argtypes = [c_int, c_int, c_int64]
+    lib.phx_grid_workspace_bytes.restype = c_size_t
+    for name in ("phx_solve_forward", "phx_solve_forward_many", "phx_solve_forward_rows", "phx_stream_solve_forward"):
+        fn = getattr(lib, name + "_grid")
+        fn.argtypes = getattr(lib, name).argtypes[:-1] + [c_void_p] * 4 + [c_void_p]
+        fn.restype = c_int
+    for name in ("phx_solve_adjoint", "phx_solve_adjoint_many", "phx_solve_adjoint_rows", "phx_stream_solve_adjoint"):
+        fn = getattr(lib, name + "_grid")
+        fn.argtypes = getattr(lib, name + "_masked").argtypes[:-1] + [c_void_p] * 2 + [c_void_p]
         fn.restype = c_int
     lib.phx_prior_loss.argtypes = [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, ctypes.c_float, c_void_p,
                                    c_void_p, c_void_p, c_size_t, c_void_p]

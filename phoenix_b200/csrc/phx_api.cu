@@ -1,4 +1,5 @@
 // extern "C" entry points of libphoenix_b200.so (declared in include/phoenix_b200.h).
+#include <math.h>
 #include <stdarg.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -160,7 +161,81 @@ bool check_dims(int G, int H, int B) {
     return true;
 }
 
+// ---- fixed-grid step grids (the *_grid entry points) -----------------------------------------------------------------
+// the grid goes to the workspace right after the solver's own part, 16-byte aligned
+size_t grid_room(size_t need) { return (need + 15) & ~(size_t)15; }
+
+// total steps of a grid (for the workspace check; a negative count is refused by phx_grid_stage afterwards)
+long long grid_steps(const PhxGridHost& g, int N, int T, int adjoint) {
+    const long long nseg = adjoint ? (long long)N * (T - 1) : N;
+    long long tot = 0;
+    if (g.steps)
+        for (long long q = 0; q < nseg; ++q) tot += g.steps[q] > 0 ? g.steps[q] : 0;
+    return tot;
+}
+
 }  // namespace
+
+int phx_grid_stage(const PhxGridHost& g, int N, int T, int method, int forward, void* room, cudaStream_t stream,
+                   ResParams* p, std::vector<int>* off) {
+    if (method == PHX_DOPRI5 || method < PHX_EULER || method > PHX_DOPRI5) {
+        phx_set_error("a step grid is for the fixed-grid methods (euler, midpoint, rk4), got method id %d", method);
+        return PHX_ERR_INVALID;
+    }
+    if (!g.dt || !g.steps || (forward && (!g.out_step || !g.out_slope))) {
+        phx_set_error("null grid array");
+        return PHX_ERR_INVALID;
+    }
+    const int nseg = forward ? N : N * (T - 1), nout = forward ? N * (T - 1) : 0;
+    std::vector<int> o(nseg + 1, 0);
+    for (int q = 0; q < nseg; ++q) {
+        if (g.steps[q] < 1 || (long long)o[q] + g.steps[q] > (1LL << 30)) {
+            phx_set_error("grid segment %d: step count %d out of range", q, g.steps[q]);
+            return PHX_ERR_INVALID;
+        }
+        o[q + 1] = o[q] + g.steps[q];
+    }
+    for (int k = 0; k < o[nseg]; ++k)
+        if (!(g.dt[k] >= 0.f) || isinf(g.dt[k])) {
+            phx_set_error("grid step %d: dt %g is not a finite non-negative number", k, (double)g.dt[k]);
+            return PHX_ERR_INVALID;
+        }
+    for (int q = 0; q < N && forward; ++q)
+        for (int j = 0; j + 1 < T; ++j) {
+            const int k = g.out_step[q * (T - 1) + j];
+            if (k < 0 || k >= g.steps[q] || (j > 0 && k < g.out_step[q * (T - 1) + j - 1])) {
+                phx_set_error("problem %d, output %d: step %d is out of range or the output map decreases", q, j + 1, k);
+                return PHX_ERR_INVALID;
+            }
+            if (isnan(g.out_slope[q * (T - 1) + j])) {
+                phx_set_error("problem %d, output %d: the slope is NaN", q, j + 1);
+                return PHX_ERR_INVALID;
+            }
+        }
+    if (off) *off = o;
+    if (!room) return PHX_OK;
+    // one copy: dt | goff | gout | gsl, each part padded to 16 bytes
+    auto pad = [](size_t n) { return (n + 3) & ~(size_t)3; };
+    const size_t n_dt = pad(o[nseg]), n_off = pad(nseg + 1), n_out = pad(nout);
+    std::vector<uint32_t> buf(n_dt + n_off + 2 * n_out, 0);
+    memcpy(buf.data(), g.dt, sizeof(float) * o[nseg]);
+    memcpy(buf.data() + n_dt, o.data(), sizeof(int) * (nseg + 1));
+    if (nout) {
+        memcpy(buf.data() + n_dt + n_off, g.out_step, sizeof(int) * nout);
+        memcpy(buf.data() + n_dt + n_off + n_out, g.out_slope, sizeof(float) * nout);
+    }
+    cudaError_t e = cudaMemcpyAsync(room, buf.data(), sizeof(uint32_t) * buf.size(), cudaMemcpyHostToDevice, stream);
+    if (e != cudaSuccess) {
+        phx_set_error("cudaMemcpyAsync(grid): %s", cudaGetErrorString(e));
+        return PHX_ERR_CUDA;
+    }
+    const uint32_t* d = (const uint32_t*)room;
+    p->gdt = (const float*)d;
+    p->goff = (const int*)(d + n_dt);
+    p->gout = nout ? (const int*)(d + n_dt + n_off) : nullptr;
+    p->gsl = nout ? (const float*)(d + n_dt + n_off + n_out) : nullptr;
+    return PHX_OK;
+}
 
 int phx_tc_prepare(phx_ctx* ctx, int G, int H, int B, const float* packed, PhxPacked* view, cudaStream_t stream) {
     *view = phx_packed_view(packed, G, H);
@@ -379,7 +454,8 @@ int phx_solve_workspace_init(void* workspace, size_t workspace_bytes, void* stre
 static int solve_common(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
                         int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps, int adjoint,
                         void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                        int steplog_cap, cudaStream_t stream, ResParams* p, ResLaunchPlan* plan, int nprob = 1) {
+                        int steplog_cap, cudaStream_t stream, ResParams* p, ResLaunchPlan* plan, int nprob = 1,
+                        const PhxGridHost* grid = nullptr) {
     if (!ctx || !check_dims(G, H, B) || !packed || !t_host || !workspace) {
         if (g_err[0] == 0) phx_set_error("null argument");
         return PHX_ERR_INVALID;
@@ -412,8 +488,9 @@ static int solve_common(phx_ctx* ctx, int G, int H, int B, const float* packed, 
     if (rc != PHX_OK) return rc;
     size_t o_t, o_th;
     size_t need = phx_resident_workspace_floats(G, H, B, T, adjoint, &o_t, &o_th) * sizeof(float);
-    if (workspace_bytes < need) {
-        phx_set_error("solve workspace too small: %zu < %zu", workspace_bytes, need);
+    const size_t need_grid = grid ? grid_room(need) + phx_grid_workspace_bytes(nprob, T, grid_steps(*grid, nprob, T, adjoint)) : need;
+    if (workspace_bytes < need_grid) {
+        phx_set_error("solve workspace too small: %zu < %zu", workspace_bytes, need_grid);
         return PHX_ERR_WORKSPACE;
     }
     float* ws = (float*)workspace;
@@ -431,6 +508,9 @@ static int solve_common(phx_ctx* ctx, int G, int H, int B, const float* packed, 
     p->status = status; p->steplog = steplog; p->steplog_cap = steplog ? steplog_cap : 0;
     p->prof = ctx->prof;
     p->nprob = nprob;
+    if (grid && (rc = phx_grid_stage(*grid, nprob, T, method, !adjoint, (char*)workspace + grid_room(need), stream, p,
+                                     nullptr)) != PHX_OK)
+        return rc;
     if (T * nprob <= PHX_T_INLINE) {
         for (int i = 0; i < T * nprob; ++i) p->t_small[i] = t_host[i];  // travels with the kernel parameters
         return PHX_OK;
@@ -563,7 +643,7 @@ int phx_solve_adjoint_many_masked(phx_ctx* ctx, int G, int H, int B, int N, cons
 static int rows_common(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T, int t_is_f32,
                        int method, double rtol, double atol, int64_t max_num_steps, int adjoint, void* workspace,
                        size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap, cudaStream_t stream,
-                       ResParams* p, RowsPlan* plan, size_t* off_theta) {
+                       ResParams* p, RowsPlan* plan, size_t* off_theta, const PhxGridHost* grid = nullptr) {
     if (!ctx || !check_dims(G, H, 1) || !packed || !t_host || !workspace || N < 1) {
         if (g_err[0] == 0) phx_set_error("null argument");
         return PHX_ERR_INVALID;
@@ -590,8 +670,9 @@ static int rows_common(phx_ctx* ctx, int G, int H, int N, const float* packed, c
     if (rc != PHX_OK) return rc;
     size_t o_t;
     const size_t need = phx_rows_workspace_floats(G, H, N, T, plan->rows, adjoint, &o_t, off_theta) * sizeof(float);
-    if (workspace_bytes < need) {
-        phx_set_error("rows workspace too small: %zu < %zu", workspace_bytes, need);
+    const size_t need_grid = grid ? grid_room(need) + phx_grid_workspace_bytes(N, T, grid_steps(*grid, N, T, adjoint)) : need;
+    if (workspace_bytes < need_grid) {
+        phx_set_error("rows workspace too small: %zu < %zu", workspace_bytes, need_grid);
         return PHX_ERR_WORKSPACE;
     }
     float* ws = (float*)workspace;
@@ -613,6 +694,9 @@ static int rows_common(phx_ctx* ctx, int G, int H, int N, const float* packed, c
     p->tm_wa = plan->tm_wa; p->tm_fac = plan->tm_fac;
     p->y0_stride = G; p->yout_stride = (long long)T * G; p->adj_stride = G;
     p->ppk = (long long)phx_packed_grad_offsets(G, H).total;
+    if (grid && (rc = phx_grid_stage(*grid, N, T, method, !adjoint, (char*)workspace + grid_room(need), stream, p,
+                                     nullptr)) != PHX_OK)
+        return rc;
     if ((size_t)T * N <= PHX_T_INLINE) {
         for (int i = 0; i < T * N; ++i) p->t_small[i] = t_host[i];
         return PHX_OK;
@@ -758,6 +842,174 @@ int phx_solve_adjoint_rows_masked(phx_ctx* ctx, int G, int H, int N, const float
     size_t o_th = 0;
     int rc = rows_common(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
                          workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, &o_th);
+    if (rc != PHX_OK) return rc;
+    p.ysaved = y_saved;
+    p.grad_y = grad_y;
+    p.adj_y0 = adj_y0;
+    p.theta_ws = (float*)workspace + o_th;
+    p.gsum = grads_packed_parts;
+    p.gsum_acc = 0;
+    p.pmask = param_mask;
+    return phx_rows_launch(p, plan, (cudaStream_t)stream);
+}
+
+
+/* ---- fixed-grid solves on the caller's step grid (options=dict(step_size=...), solvers.py:48-50, 77-103) ---------------- */
+size_t phx_grid_workspace_bytes(int N, int T, int64_t total_steps) {
+    if (N < 1 || T < 2 || total_steps < 0) return 0;
+    const size_t nseg = (size_t)N * (T - 1);
+    return 4 * (((size_t)total_steps + 3) / 4 * 4 + (nseg + 4) / 4 * 4 + 2 * ((nseg + 3) / 4 * 4)) + 16;
+}
+
+int phx_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0, const double* t_host,
+                           int T, int t_is_f32, int reversed, int method, double rtol, double atol, int64_t max_num_steps,
+                           float* y_out, void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                           int steplog_cap, const float* grid_dt, const int32_t* grid_steps_, const int32_t* grid_out_step,
+                           const float* grid_out_slope, void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    g_err[0] = 0;
+    if (!y0 || !y_out) {
+        phx_set_error("null y0 / y_out");
+        return PHX_ERR_INVALID;
+    }
+    const PhxGridHost grid{grid_dt, grid_steps_, grid_out_step, grid_out_slope};
+    ResParams p;
+    ResLaunchPlan plan;
+    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
+                          workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, 1, &grid);
+    if (rc != PHX_OK) return rc;
+    p.y0 = y0;
+    p.yout = y_out;
+    p.fsign = reversed ? -1.f : 1.f;
+    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+}
+
+int phx_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                           int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                           const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat, void* workspace,
+                           size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap, int param_mask,
+                           const float* grid_dt, const int32_t* grid_steps_, void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    g_err[0] = 0;
+    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
+    if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
+        phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
+        return PHX_ERR_INVALID;
+    }
+    const PhxGridHost grid{grid_dt, grid_steps_, nullptr, nullptr};
+    ResParams p;
+    ResLaunchPlan plan;
+    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
+                          workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, 1, &grid);
+    if (rc != PHX_OK) return rc;
+    p.ysaved = y_saved;
+    p.grad_y = grad_y;
+    p.adj_y0 = adj_y0;
+    p.theta0 = grads_flat;
+    p.pmask = param_mask & PHX_P_ALL;   // (a fixed grid uses no norm)
+    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+}
+
+int phx_solve_forward_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const float* y0,
+                                const double* t_host, int T, int t_is_f32, int method, double rtol, double atol,
+                                int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
+                                phx_status* status, const float* grid_dt, const int32_t* grid_steps_,
+                                const int32_t* grid_out_step, const float* grid_out_slope, void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    g_err[0] = 0;
+    if (!y0 || !y_out) {
+        phx_set_error("null y0 / y_out");
+        return PHX_ERR_INVALID;
+    }
+    const PhxGridHost grid{grid_dt, grid_steps_, grid_out_step, grid_out_slope};
+    ResParams p;
+    ResLaunchPlan plan;
+    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
+                          workspace_bytes, status, nullptr, 0, (cudaStream_t)stream, &p, &plan, N, &grid);
+    if (rc != PHX_OK) return rc;
+    p.y0 = y0;
+    p.yout = y_out;
+    p.y0_stride = (long long)B * G;
+    p.yout_stride = (long long)T * B * G;
+    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+}
+
+int phx_solve_adjoint_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host, int T,
+                                int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
+                                const float* grid_dt, const int32_t* grid_steps_, void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    g_err[0] = 0;
+    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
+    if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
+        phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
+        return PHX_ERR_INVALID;
+    }
+    const PhxGridHost grid{grid_dt, grid_steps_, nullptr, nullptr};
+    ResParams p;
+    ResLaunchPlan plan;
+    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
+                          workspace_bytes, status, nullptr, 0, (cudaStream_t)stream, &p, &plan, N, &grid);
+    if (rc != PHX_OK) return rc;
+    p.ysaved = y_saved;
+    p.grad_y = grad_y;
+    p.adj_y0 = adj_y0;
+    p.theta0 = grads_flat;
+    p.yout_stride = (long long)T * B * G;
+    p.adj_stride = (long long)B * G;
+    p.theta_stride = (long long)phx_grad_offsets(G, H).total;
+    p.pmask = param_mask & PHX_P_ALL;   // (a fixed grid uses no norm)
+    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+}
+
+int phx_solve_forward_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const float* y0,
+                                const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
+                                double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
+                                phx_status* status, double* steplog, int steplog_cap, const float* grid_dt,
+                                const int32_t* grid_steps_, const int32_t* grid_out_step, const float* grid_out_slope,
+                                void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    g_err[0] = 0;
+    if (!y0 || !y_out) {
+        phx_set_error("null y0 / y_out");
+        return PHX_ERR_INVALID;
+    }
+    const PhxGridHost grid{grid_dt, grid_steps_, grid_out_step, grid_out_slope};
+    ResParams p;
+    RowsPlan plan;
+    int rc = rows_common(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
+                         workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, nullptr, &grid);
+    if (rc != PHX_OK) return rc;
+    p.y0 = y0;
+    p.yout = y_out;
+    p.fsign = reversed ? -1.f : 1.f;
+    return phx_rows_launch(p, plan, (cudaStream_t)stream);
+}
+
+int phx_solve_adjoint_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
+                                int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
+                                void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps_,
+                                void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    g_err[0] = 0;
+    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
+    if (!y_saved || !grad_y || !adj_y0 || !grads_packed_parts) {
+        phx_set_error("null y_saved / grad_y / adj_y0 / grads_packed_parts");
+        return PHX_ERR_INVALID;
+    }
+    if ((uintptr_t)grads_packed_parts & 15) {
+        phx_set_error("grads_packed_parts must be 16-byte aligned");
+        return PHX_ERR_INVALID;
+    }
+    const PhxGridHost grid{grid_dt, grid_steps_, nullptr, nullptr};
+    ResParams p;
+    RowsPlan plan;
+    size_t o_th = 0;
+    int rc = rows_common(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
+                         workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, &o_th, &grid);
     if (rc != PHX_OK) return rc;
     p.ysaved = y_saved;
     p.grad_y = grad_y;

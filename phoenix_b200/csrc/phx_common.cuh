@@ -13,6 +13,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <vector>
 #include "../../include/phoenix_b200.h"
 
 #define PHX_THREADS 512
@@ -276,6 +277,14 @@ struct ResParams {
     int gsum_acc;          // != 0: add to gsum instead of overwriting it
     long long ppk;
     int pmask;             // adjoint: parameters whose cotangents are integrated (PHX_P_*)
+    // fixed-grid solves on the caller's step grid (the *_grid entry points, options=dict(step_size=...)); gdt == nullptr:
+    // one step per output interval.  Segment q (forward: problem q; adjoint: interval iv of problem pi, q = pi*(T-1)+iv-1)
+    // takes the steps gdt[goff[q] .. goff[q+1]).  Forward output j >= 1 of problem pi is written in step
+    // gout[pi*(T-1)+j-1] of its problem, as y + gsl[...] * (y1 - y), or as y1 itself when gsl[...] < 0
+    const float* gdt;
+    const int* goff;
+    const int* gout;
+    const float* gsl;
 };
 #define PHX_PROF_SLOTS 32
 #define PHX_T_INLINE 64
@@ -361,6 +370,21 @@ int phx_rows_launch(const ResParams& p, const RowsPlan& plan, cudaStream_t strea
 int phx_resident_plan(int num_sms, int G, int H, int B, int adjoint, ResLaunchPlan* plan);
 size_t phx_resident_workspace_floats(int G, int H, int B, int T, int adjoint, size_t* off_t, size_t* off_theta1);
 int phx_resident_launch(const ResParams& p, const ResLaunchPlan& plan, cudaStream_t stream);
+
+// A fixed-grid solve's step grid as the *_grid entry points take it (include/phoenix_b200.h): nseg segments (forward: the
+// N problems; adjoint: the N * (T-1) intervals, problem-major), steps[q] >= 1 steps each, their dt back to back; forward
+// only: out_step / out_slope [N][T-1], the step of each output time j >= 1 and its slope (< 0: exact hit, take y1).
+struct PhxGridHost {
+    const float* dt;
+    const int32_t* steps;
+    const int32_t* out_step;
+    const float* out_slope;
+};
+// Validates the grid (phx_set_error + PHX_ERR_INVALID otherwise); with `room` (device, >= phx_grid_workspace_bytes) set,
+// copies it there on `stream` and points p->gdt / goff / gout / gsl at it.  `off` (may be null) receives the segment
+// offsets into dt (nseg + 1 entries).
+int phx_grid_stage(const PhxGridHost& g, int N, int T, int method, int forward, void* room, cudaStream_t stream,
+                   ResParams* p, std::vector<int>* off);
 
 // ---- RK stage algebra fused into the RHS (streaming solvers, forward solves on the tensor-core path) ------------------
 // With k = the stage derivative a forward RHS launch produces, the epilogue of the joint contraction also writes

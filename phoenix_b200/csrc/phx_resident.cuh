@@ -1348,7 +1348,9 @@ __device__ __forceinline__ void eval_B(const ResParams& __restrict__ p, Smem& __
 // =====================================================================================================================
 // Forward solve
 // =====================================================================================================================
-template <int NV, int BT>
+// GRID: the fixed grid is the caller's step grid (p.gdt != nullptr), an instantiation of its own so that the default
+// (one step per output interval) and dopri5 keep their code
+template <int NV, int BT, bool GRID>
 __global__ void __launch_bounds__(PHX_THREADS, 1) phx_fwd_kernel(const __grid_constant__ ResParams p) {
     Smem s(p);
     const int g_lo = s.g_lo, n_loc = s.n_loc;
@@ -1390,13 +1392,20 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_fwd_kernel(const __grid_co
     __syncthreads();
 
     if (p.method != PHX_DOPRI5) {
-        // ---- fixed grid: one step per output interval (solvers.py:48-50, 77-95) ----
+        // ---- fixed grid (solvers.py:48-50, 77-103): one step per output interval, or the steps of the caller's grid
+        // (p.gdt), whose output times are written from the step that reaches them: y1 on an exact hit, else y + s (y1 - y)
         const float third = (float)(1.0 / 3.0);
+        const int nk = GRID ? p.goff[pi + 1] - p.goff[pi] : p.T - 1;
+        int jn = 1;   // first output time not written yet (grid)
         eval_A<NV, BT>(p, s);
-        for (int i = 0; i + 1 < p.T; ++i) {
-            const float dtf = p.t_is_f32 ? ((float)tget(p, pi, i + 1) - (float)tget(p, pi, i)) : (float)(tget(p, pi, i + 1) - tget(p, pi, i));
+        for (int i = 0; i < nk; ++i) {
+            const float dtf = GRID ? p.gdt[p.goff[pi] + i]
+                                    : (p.t_is_f32 ? ((float)tget(p, pi, i + 1) - (float)tget(p, pi, i)) : (float)(tget(p, pi, i + 1) - tget(p, pi, i)));
             float* yo = youtp + (size_t)(i + 1) * BG;
-            const bool more = i + 2 < p.T;   // another interval follows: its first pass A is fused into the last stage
+            int je = jn;   // grid: outputs [jn, je) are written by this step
+            if (GRID)
+                while (je < p.T && p.gout[pi * (p.T - 1) + je - 1] == i) ++je;
+            const bool more = i + 1 < nk;   // another step follows: its first pass A is fused into the last stage
             // one call site for every stage of every fixed-grid method (the stage algebra switches at run time)
             const int nst = (p.method == PHX_EULER) ? 1 : (p.method == PHX_MIDPOINT ? 2 : 4);
             const float half = 0.5f * dtf;
@@ -1416,16 +1425,25 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_fwd_kernel(const __grid_co
                         if (lead && !last) K(st)[li] = f;
                     }
                     if (last && lead) {
+                        if (GRID) {
+                            // (op by op, solvers.py:97-103; the build does not contract to fma)
+                            for (int jj = jn; jj < je; ++jj) {
+                                const float sl = p.gsl[pi * (p.T - 1) + jj - 1];
+                                youtp[(size_t)jj * BG + (size_t)b * p.G + g_lo + j] = sl < 0.f ? yn : Y[li] + sl * (yn - Y[li]);
+                            }
+                        } else {
+                            yo[(size_t)b * p.G + g_lo + j] = yn;
+                        }
                         Y[li] = yn;
-                        yo[(size_t)b * p.G + g_lo + j] = yn;
                     }
                     return yn;
                 });
             }
+            jn = je;
         }
         if (threadIdx.x == 0) {
             int per = (p.method == PHX_EULER) ? 1 : (p.method == PHX_MIDPOINT ? 2 : 4);
-            c->n_rhs = per * (p.T - 1);
+            c->n_rhs = per * nk;
             c->tcur = tget(p, pi, p.T - 1);
         }
         __syncthreads();
@@ -2019,7 +2037,8 @@ __device__ __forceinline__ void adj_eval(const ResParams& __restrict__ p, Smem& 
 }
 
 // SEMI: the seminorm (p.pmask & PHX_NORM_SEMINORM), an instantiation of its own so that the default norm keeps its code
-template <int NV, int BT, bool SEMI>
+// GRID: as in phx_fwd_kernel (fixed grids use no norm: the grid instantiations are the default-norm ones)
+template <int NV, int BT, bool SEMI, bool GRID>
 __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_constant__ ResParams p) {
     constexpr int QB = (7 * BT + 3) & ~3;
     Smem s(p);
@@ -2097,8 +2116,22 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
         const double t_start = -tget(p, pi, iv), t_end = -tget(p, pi, iv - 1);
 
         if (p.method != PHX_DOPRI5) {
-            const float dtf = p.t_is_f32 ? ((float)tget(p, pi, iv) - (float)tget(p, pi, iv - 1)) : (float)(tget(p, pi, iv) - tget(p, pi, iv - 1));
+            // one step per interval, or the steps of the interval's own grid (p.gdt): y and adj_y advance together, and
+            // every step runs its own theta pass
+            const int seg = pi * (p.T - 1) + iv - 1;
+            const int nk = GRID ? p.goff[seg + 1] - p.goff[seg] : 1;
+            for (int k = 0; k < nk; ++k) {
+            const float dtf = GRID ? p.gdt[p.goff[seg] + k]
+                                    : (p.t_is_f32 ? ((float)tget(p, pi, iv) - (float)tget(p, pi, iv - 1)) : (float)(tget(p, pi, iv) - tget(p, pi, iv - 1)));
+            const bool more = k + 1 < nk;
             const float third = (float)(1.0 / 3.0);
+            if (k > 0) {   // the next step starts from the state the last one left in Y / A
+                for_local(p, g_lo, n_loc, [&](int b, int j, int g, size_t gi, int li) {
+                    set_y_input(s.ysb(), s.acts(), s.actl(), li, Y[li]);
+                    set_a_input(li, j, A[li]);
+                });
+                __syncthreads();
+            }
             if (threadIdx.x == 0) {
                 PPArgs& pa = *s.at<PPArgs>(p.so.ppa);
                 pa.src = theta_zero ? nullptr : theta0p;
@@ -2131,7 +2164,14 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                             else if (st == 2) an = A[li] + dtf * (KA(0)[li] - KA(1)[li] + ka);
                             else an = A[li] + (KA(0)[li] + 3.f * (KA(1)[li] + KA(2)[li]) + ka) * dtf * 0.125f;
                         }
-                        if (last && lead) A[li] = an;
+                        if (last && lead) {
+                            A[li] = an;
+                            if (more) {   // y at the step's end (KY of every stage is in place after pass 1)
+                                const float ky = KY(nst - 1)[li];
+                                if (p.method != PHX_RK4) Y[li] = Y[li] + dtf * ky;
+                                else Y[li] = Y[li] + (KY(0)[li] + 3.f * (KY(1)[li] + KY(2)[li]) + ky) * dtf * 0.125f;
+                            }
+                        }
                         return an;
                     });
             }
@@ -2146,6 +2186,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 c->tcur = t_end;
             }
             __syncthreads();
+            }
         } else {
             // ------------------------------ dopri5 on the augmented state ------------------------------
             if (threadIdx.x == 0) {

@@ -36,16 +36,24 @@ int launch_coop(KernelT kernel, const ResParams& p, const ResLaunchPlan& plan, c
 
 #if PHX_KIND_ADJ
 int PHX_FN(const ResParams& p, const ResLaunchPlan& plan, cudaStream_t stream) {
+    if (p.gdt) {   // a fixed grid uses no norm: the seminorm bit changes nothing there
+        if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4, false, true>, p, plan, stream);
+        return launch_coop(PHX_KERNEL<PHX_NV, 1, false, true>, p, plan, stream);
+    }
     if (p.pmask & PHX_NORM_SEMINORM) {
+        if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4, true, false>, p, plan, stream);
+        return launch_coop(PHX_KERNEL<PHX_NV, 1, true, false>, p, plan, stream);
+    }
+    if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4, false, false>, p, plan, stream);
+    return launch_coop(PHX_KERNEL<PHX_NV, 1, false, false>, p, plan, stream);
+}
+#else
+int PHX_FN(const ResParams& p, const ResLaunchPlan& plan, cudaStream_t stream) {
+    if (p.gdt) {
         if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4, true>, p, plan, stream);
         return launch_coop(PHX_KERNEL<PHX_NV, 1, true>, p, plan, stream);
     }
     if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4, false>, p, plan, stream);
     return launch_coop(PHX_KERNEL<PHX_NV, 1, false>, p, plan, stream);
-}
-#else
-int PHX_FN(const ResParams& p, const ResLaunchPlan& plan, cudaStream_t stream) {
-    if (p.B > 1) return launch_coop(PHX_KERNEL<PHX_NV, 4>, p, plan, stream);
-    return launch_coop(PHX_KERNEL<PHX_NV, 1>, p, plan, stream);
 }
 #endif

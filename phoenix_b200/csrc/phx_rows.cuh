@@ -39,6 +39,8 @@ struct RowCtl {
     int slot[7];    // physical state slot (K / KY / KA) of logical stage q; FSAL swaps 0 <-> 6
     int fslot[7];   // physical factor slot of logical stage q (-1: the stage keeps no factors)
     int cur, theta_zero, pend, spec_done;
+    int stepping;   // fixed grid: the row takes the current step (0: past its last step -- or its interval's last)
+    int gj0, gj1;   // fixed grid, forward: the output times [gj0, gj1) the current step writes
 };
 struct RowsCtl {
     RowCtl r[RM];
@@ -531,26 +533,47 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_fwd_kernel(const __gr
         __syncthreads();
 
         if (p.method != PHX_DOPRI5) {
-            // ---- fixed grid: one step per output interval (solvers.py:48-50, 77-95) ----
+            // ---- fixed grid (solvers.py:48-50, 77-103): one step per output interval, or the steps of each row's own
+            // grid (p.gdt); a row past its last step is left as it is while the others go on ----
             const float third = (float)(1.0 / 3.0);
             const int nst = (p.method == PHX_EULER) ? 1 : (p.method == PHX_MIDPOINT ? 2 : 4);
+            int nk = p.T - 1;
+            if (p.gdt) {
+                nk = 0;
+                for (int b = 0; b < nr; ++b) nk = max(nk, p.goff[q0 + b + 1] - p.goff[q0 + b]);
+            }
+            if (threadIdx.x < RM) {
+                RowCtl& c = rc->r[threadIdx.x];
+                c.gj0 = c.gj1 = 1;
+                c.stepping = 1;
+            }
             rows_eval_A(p, s, v);
-            for (int i = 0; i + 1 < p.T; ++i) {
+            for (int i = 0; i < nk; ++i) {
                 if (threadIdx.x < RM) {
                     RowCtl& c = rc->r[threadIdx.x];
-                    if (c.valid) {
-                        const double ta = tget_rows(p, q0 + threadIdx.x, i), tb = tget_rows(p, q0 + threadIdx.x, i + 1);
-                        c.dtf = p.t_is_f32 ? ((float)tb - (float)ta) : (float)(tb - ta);
-                    } else {
+                    const int q = q0 + threadIdx.x;
+                    if (!c.valid) {
                         c.dtf = 0.f;
+                    } else if (p.gdt) {
+                        c.stepping = i < p.goff[q + 1] - p.goff[q];
+                        c.dtf = c.stepping ? p.gdt[p.goff[q] + i] : 0.f;
+                        int je = c.gj1;
+                        while (je < p.T && p.gout[q * (p.T - 1) + je - 1] == i) ++je;
+                        c.gj0 = c.gj1;
+                        c.gj1 = je;
+                    } else {
+                        const double ta = tget_rows(p, q, i), tb = tget_rows(p, q, i + 1);
+                        c.dtf = p.t_is_f32 ? ((float)tb - (float)ta) : (float)(tb - ta);
                     }
                 }
                 __syncthreads();
-                const bool more = i + 2 < p.T;
+                const bool more = i + 1 < nk;
                 for (int st = 0; st < nst; ++st) {
                     const bool last = st + 1 == nst;
                     rows_fwd_eval(p, s, v, !last || more, [&](int b, int j, int li, float f) {
-                        const float dtf = rc->r[b].dtf;
+                        const RowCtl& c = rc->r[b];
+                        if (!c.stepping) return Y[li];   // (its stage input stays its state)
+                        const float dtf = c.dtf;
                         float yn;
                         if (p.method == PHX_EULER) {
                             yn = Y[li] + dtf * f;
@@ -564,8 +587,18 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_fwd_kernel(const __gr
                             if (!last) K(st)[li] = f;
                         }
                         if (last) {
+                            if (b < nr) {
+                                float* yo = p.yout + (size_t)(q0 + b) * p.yout_stride + g_lo + j;
+                                if (p.gdt) {
+                                    for (int jj = c.gj0; jj < c.gj1; ++jj) {
+                                        const float sl = p.gsl[(q0 + b) * (p.T - 1) + jj - 1];
+                                        yo[(size_t)jj * p.G] = sl < 0.f ? yn : Y[li] + sl * (yn - Y[li]);
+                                    }
+                                } else {
+                                    yo[(size_t)(i + 1) * p.G] = yn;
+                                }
+                            }
                             Y[li] = yn;
-                            if (b < nr) p.yout[(size_t)(q0 + b) * p.yout_stride + (size_t)(i + 1) * p.G + g_lo + j] = yn;
                         }
                         return yn;
                     });
@@ -573,7 +606,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_fwd_kernel(const __gr
             }
             if (threadIdx.x < nr) {
                 RowCtl& c = rc->r[threadIdx.x];
-                c.n_rhs = nst * (p.T - 1);
+                c.n_rhs = nst * (p.gdt ? p.goff[q0 + threadIdx.x + 1] - p.goff[q0 + threadIdx.x] : p.T - 1);
                 c.tcur = tget_rows(p, q0 + threadIdx.x, p.T - 1);
                 row_write_status(p, q0 + threadIdx.x, c);
             }
@@ -1442,9 +1475,31 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
             if (!dop) {
                 const float third = (float)(1.0 / 3.0);
                 const int nst = (p.method == PHX_EULER) ? 1 : (p.method == PHX_MIDPOINT ? 2 : 4);
+                // one step per interval, or the steps of each row's own grid of this interval (p.gdt): a row that has
+                // taken all of its steps sits out (RowPP.active = 0) until every row has
+                int nk = 1;
+                if (p.gdt) {
+                    nk = 0;
+                    for (int b = 0; b < nr; ++b) {
+                        const int sg = (q0 + b) * (p.T - 1) + iv - 1;
+                        nk = max(nk, p.goff[sg + 1] - p.goff[sg]);
+                    }
+                }
+                for (int k = 0; k < nk; ++k) {
+                if (k > 0) {   // the next step starts from the state the last one left in Y / A
+                    for (int e = threadIdx.x; e < p.gpc * RM; e += THREADS)
+                        set_input(e, e >> 2, Y[e], A[e], rc->r[e & 3].fslot[0]);
+                }
                 if (threadIdx.x < RM) {
-                    const RowCtl& c = rc->r[threadIdx.x];
+                    RowCtl& c = rc->r[threadIdx.x];
                     RowPP& a = pp[threadIdx.x];
+                    int rk = 1;
+                    if (p.gdt && c.valid) {
+                        const int sg = (q0 + threadIdx.x) * (p.T - 1) + iv - 1;
+                        rk = p.goff[sg + 1] - p.goff[sg];
+                        c.dtf = k < rk ? p.gdt[p.goff[sg] + k] : 0.f;
+                    }
+                    c.stepping = !c.done && k < rk;
                     float* th = p.theta_ws + (size_t)(2 * threadIdx.x) * p.ppk;
                     a.src = c.theta_zero ? nullptr : th;
                     a.dst = th;
@@ -1457,11 +1512,12 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         a.wo[0] = a.wo[3] = c.dtf * 0.125f;
                         a.wo[1] = a.wo[2] = 3.f * c.dtf * 0.125f;
                     }
-                    a.last = 1;
-                    a.active = !c.done;
+                    a.last = k + 1 == rk;
+                    a.active = c.stepping;
                 }
                 __syncthreads();
                 if (threadIdx.x == 0) plan_spec(iv == 1);
+                const bool more = k + 1 < nk;
                 for (int st = 0; st < nst; ++st) {
                     const bool last = st + 1 == nst;
                     rows_adj_eval(
@@ -1486,7 +1542,14 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                                 else if (st == 2) an = A[li] + dtf * (KA(0)[li] - KA(1)[li] + ka);
                                 else an = A[li] + (KA(0)[li] + 3.f * (KA(1)[li] + KA(2)[li]) + ka) * dtf * 0.125f;
                             }
-                            if (last) A[li] = an;
+                            if (last && rc->r[b].stepping) {
+                                A[li] = an;
+                                if (more) {   // y at the step's end (KY of every stage is in place after pass 1)
+                                    const float ky = KY(nst - 1)[li];
+                                    if (p.method != PHX_RK4) Y[li] = Y[li] + dtf * ky;
+                                    else Y[li] = Y[li] + (KY(0)[li] + 3.f * (KY(1)[li] + KY(2)[li]) + ky) * dtf * 0.125f;
+                                }
+                            }
                             return an;
                         });
                 }
@@ -1495,7 +1558,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                 pf.tick(PT_PP_STEP);
                 if (threadIdx.x < RM) {
                     RowCtl& c = rc->r[threadIdx.x];
-                    if (!c.done) {
+                    if (c.stepping) {
                         if (pp[threadIdx.x].spec) c.spec_done = 1;
                         else { c.theta_zero = 0; c.cur = 0; }
                         c.n_rhs += nst;
@@ -1504,6 +1567,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                 }
                 if (threadIdx.x == 0 && rc->spec_pass) rc->spec_valid = 1;
                 __syncthreads();
+                }
             } else {
                 // ------------------------------ dopri5 on the augmented state, one controller per row -----------------
                 if (threadIdx.x < RM) {

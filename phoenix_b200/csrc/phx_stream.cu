@@ -220,6 +220,11 @@ __global__ void add_kernel(float* x, const float* y, size_t n) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
         x[i] = x[i] + y[i];
 }
+// an output time inside a fixed-grid step (solvers.py:97-103): y0 + slope * (y1 - y0), op by op
+__global__ void lerp_kernel(float* out, const float* y0, const float* y1, float slope, size_t n) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+        out[i] = y0[i] + slope * (y1[i] - y0[i]);
+}
 
 inline bool al16(const void* p) { return p == nullptr || ((uintptr_t)p & 15) == 0; }
 inline bool kset_al16(const KSet& a) {
@@ -663,10 +668,14 @@ size_t phx_stream_workspace_bytes(const phx_ctx* ctx, int G, int H, int B, int T
     return stream_ws_floats(G, H, B, T, adjoint, nullptr, nullptr, nullptr, nullptr) * sizeof(float);
 }
 
-int phx_stream_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
-                             const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
-                             double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
-                             phx_status* status, double* steplog, int steplog_cap, void* stream) {
+}  // extern "C"
+
+namespace {
+
+int stream_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0, const double* t_host, int T,
+                   int t_is_f32, int reversed, int method, double rtol, double atol, int64_t max_num_steps, float* y_out,
+                   void* workspace, size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
+                   const PhxGridHost* grid, void* stream) {
     PhxDevGuard dev_guard(ctx);
     Stream S;
     float* base;
@@ -675,6 +684,7 @@ int phx_stream_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* pac
         phx_set_error("null y0 / y_out");
         return PHX_ERR_INVALID;
     }
+    if (grid && phx_grid_stage(*grid, 1, T, method, 1, nullptr, st, nullptr, nullptr) != PHX_OK) return PHX_ERR_INVALID;
     int rc = setup(S, ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
                    workspace_bytes, steplog, steplog_cap, st, &base);
     if (rc != PHX_OK) return rc;
@@ -697,7 +707,25 @@ int phx_stream_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* pac
     for (int i = 0; i < 7; ++i) y.k[i] = base + (3 + i) * BG;
     S.segs.push_back(y);
     cudaMemcpyAsync(y_out, y0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
-    if (method != PHX_DOPRI5) {
+    if (method != PHX_DOPRI5 && grid) {
+        // the caller's grid: a step that ends on an output time writes that output slice, the others a scratch slot
+        // (x0 / x1, never the step's own input); output times inside the step are interpolated between the two
+        S.segs[0].x0 = y_out;
+        float* cur = y_out;
+        int jn = 1;
+        for (int k = 0; k < grid->steps[0] && rc == PHX_OK; ++k) {
+            int je = jn;
+            while (je < T && grid->out_step[je - 1] == k) ++je;
+            const bool hit = je > jn && grid->out_slope[je - 2] < 0.f;   // an exact hit is the step's last output
+            float* dst = hit ? y_out + (size_t)(je - 1) * BG : (cur == base ? base + BG : base);
+            rc = S.fixed_step(grid->dt[k], dst);
+            for (int j = jn; j < je && rc == PHX_OK; ++j)
+                if (!(grid->out_slope[j - 1] < 0.f))
+                    lerp_kernel<<<nblk(BG), EB, 0, st>>>(y_out + (size_t)j * BG, cur, dst, grid->out_slope[j - 1], BG);
+            cur = dst;
+            jn = je;
+        }
+    } else if (method != PHX_DOPRI5) {
         // fixed grid: the state of interval i is read from the output slice i and written to slice i + 1
         S.segs[0].x0 = y_out;
         for (int i = 0; i + 1 < T && rc == PHX_OK; ++i) rc = S.fixed_step(fixed_dt(t_host, i, t_is_f32), y_out + (size_t)(i + 1) * BG);
@@ -718,6 +746,29 @@ int phx_stream_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* pac
     return PHX_OK;
 }
 
+}  // namespace
+
+extern "C" {
+
+int phx_stream_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
+                             const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
+                             double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
+                             phx_status* status, double* steplog, int steplog_cap, void* stream) {
+    return stream_forward(ctx, G, H, B, packed, y0, t_host, T, t_is_f32, reversed, method, rtol, atol, max_num_steps,
+                          y_out, workspace, workspace_bytes, status, steplog, steplog_cap, nullptr, stream);
+}
+
+int phx_stream_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
+                                  const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
+                                  double atol, int64_t max_num_steps, float* y_out, void* workspace,
+                                  size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
+                                  const float* grid_dt, const int32_t* grid_steps, const int32_t* grid_out_step,
+                                  const float* grid_out_slope, void* stream) {
+    const PhxGridHost grid{grid_dt, grid_steps, grid_out_step, grid_out_slope};
+    return stream_forward(ctx, G, H, B, packed, y0, t_host, T, t_is_f32, reversed, method, rtol, atol, max_num_steps,
+                          y_out, workspace, workspace_bytes, status, steplog, steplog_cap, &grid, stream);
+}
+
 int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
                              int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                              const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
@@ -733,6 +784,18 @@ int phx_stream_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const flo
                                     const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                                     void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                                     int steplog_cap, int param_mask, void* stream) {
+    return phx_stream_solve_adjoint_grid(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
+                                         y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status, steplog,
+                                         steplog_cap, param_mask, nullptr, nullptr, stream);
+}
+
+// grid_dt == nullptr: one step per interval (the entry points above)
+int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                                  int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
+                                  void* stream) {
     PhxDevGuard dev_guard(ctx);
     Stream S;
     float* base;
@@ -746,6 +809,9 @@ int phx_stream_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const flo
         phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
         return PHX_ERR_INVALID;
     }
+    std::vector<int> goff;   // the grid's interval offsets into grid_dt
+    const PhxGridHost grid{grid_dt, grid_steps, nullptr, nullptr};
+    if (grid_dt && phx_grid_stage(grid, 1, T, method, 0, nullptr, st, nullptr, &goff) != PHX_OK) return PHX_ERR_INVALID;
     int rc = setup(S, ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
                    workspace_bytes, steplog, steplog_cap, st, &base);
     if (rc != PHX_OK) return rc;
@@ -777,7 +843,9 @@ int phx_stream_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const flo
     cudaMemcpyAsync(S.segs[1].x0, grad_y + (size_t)(T - 1) * BG, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
     for (int iv = T - 1; iv >= 1 && rc == PHX_OK && S.status.code == PHX_ST_OK; --iv) {
         cudaMemcpyAsync(S.segs[0].x0, y_saved + (size_t)iv * BG, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
-        if (method != PHX_DOPRI5) {
+        if (method != PHX_DOPRI5 && grid_dt) {
+            for (int k = goff[iv - 1]; k < goff[iv] && rc == PHX_OK; ++k) rc = S.fixed_step(grid_dt[k]);
+        } else if (method != PHX_DOPRI5) {
             rc = S.fixed_step(fixed_dt(t_host, iv - 1, t_is_f32));
         } else {
             double t_end = -t_host[iv - 1];

@@ -464,6 +464,76 @@ def _t_array(t_list):
     return arr
 
 
+# ---- fixed-grid step grids (options=dict(step_size=h); solvers.py:48-50, 77-103) -----------------------------------------
+# Built here, once per call, with the reference's own tensor ops in the dtype of t (float32 or float64), so the steps and
+# the interpolation slopes are the reference's bit for bit; the kernels only consume them (include/phoenix_b200.h, the
+# *_grid entry points).
+def fixed_grid(t, step_size):
+    """The grid of ``FixedGridODESolver`` over the increasing 1-D tensor ``t`` (the solver's t, after the negation of a
+    decreasing t), in t's dtype; raises the reference's AssertionError when it misses t[-1].  ``step_size``: a float or a
+    0-dim CPU tensor, which takes part in the arithmetic with its own dtype, as in the reference."""
+    niters = torch.ceil((t[-1] - t[0]) / step_size + 1).item()
+    grid = torch.arange(0, niters, dtype=t.dtype) * step_size + t[0]
+    if grid[-1] > t[-1]:
+        grid[-1] = t[-1]
+    assert grid[0] == t[0] and grid[-1] == t[-1]
+    return grid
+
+
+def forward_grid(t_list, t_is_f32, step_size):
+    """One problem's forward grid: the float32 dt of every step, and for every output time t[j], j >= 1, the step whose
+    end is the first grid point >= t[j] and the float32 slope (t[j] - t0) / (t1 - t0) of that step (-1: t[j] == t1)."""
+    t = torch.tensor(t_list, dtype=torch.float32 if t_is_f32 else torch.float64)
+    grid = fixed_grid(t, step_size)
+    k = torch.searchsorted(grid[1:], t[1:])
+    t0, t1 = grid[k], grid[k + 1]
+    slope = torch.where(t[1:] == t1, -1.0, ((t[1:] - t0) / (t1 - t0)).float())
+    return (grid[1:] - grid[:-1]).float(), k.to(torch.int32), slope.float()
+
+
+def adjoint_grid(t_list, t_is_f32, step_size):
+    """One problem's backward grids: the float32 dt of the steps of every interval [t[i], t[i+1]], each integrated on
+    its own grid over the negated times [-t[i+1], -t[i]] (adjoint.py: odeint over t[i:i+2].flip(0)), and their counts."""
+    dtype = torch.float32 if t_is_f32 else torch.float64
+    dts = []
+    for i in range(len(t_list) - 1):
+        g = fixed_grid(torch.tensor([-t_list[i + 1], -t_list[i]], dtype=dtype), step_size)
+        dts.append((g[1:] - g[:-1]).float())
+    return torch.cat(dts), [int(d.numel()) for d in dts]
+
+
+class _Grid:
+    """Step grids of consecutive problems as the *_grid entry points take them (host arrays, kept alive here)."""
+
+    def __init__(self, parts, forward):
+        self.forward = forward
+        self.dt = torch.cat([q[0] for q in parts]).contiguous()
+        if forward:
+            self.steps = torch.tensor([int(q[0].numel()) for q in parts], dtype=torch.int32)
+            self.out_step = torch.cat([q[1] for q in parts]).contiguous()
+            self.out_slope = torch.cat([q[2] for q in parts]).contiguous()
+        else:
+            self.steps = torch.tensor([n for q in parts for n in q[1]], dtype=torch.int32)
+
+    def args(self):
+        a = [ctypes.c_void_p(self.dt.data_ptr()), ctypes.c_void_p(self.steps.data_ptr())]
+        if self.forward:
+            a += [ctypes.c_void_p(self.out_step.data_ptr()), ctypes.c_void_p(self.out_slope.data_ptr())]
+        return a
+
+    def nbytes(self, lib, N, T):
+        """Workspace room for the grid behind the solver's own part (16-byte alignment included)."""
+        return 16 + lib.phx_grid_workspace_bytes(N, T, self.dt.numel())
+
+
+def _grids(t_rows, t_is_f32, step_size, forward):
+    """Per-problem grids (None without a step size: the calls stay the one-step-per-interval entry points)."""
+    if step_size is None:
+        return None
+    build = forward_grid if forward else adjoint_grid
+    return [build(r, t_is_f32, step_size) for r in t_rows]
+
+
 def _pick_engine(lib, dev, G, H, B, T, adjoint):
     """Resident (one persistent cooperative launch) when the rows fit on chip, else the streaming engine."""
     if FORCE_ENGINE != "stream" and B <= lib.phx_resident_max_rows(int(adjoint)):
@@ -512,19 +582,26 @@ def _steplog_rows(n):
 
 
 def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_time, method, rtol, atol, max_num_steps,
-                  out_shape):
-    """N one-row problems (y0c [N, G]) in lock-step; returns yout of shape out_shape (= [N, T, ..., G] memory order)."""
+                  out_shape, grids=None):
+    """N one-row problems (y0c [N, G]) in lock-step; returns yout of shape out_shape (= [N, T, ..., G] memory order).
+    ``grids``: the problems' forward step grids (forward_grid), or None."""
     N, T = len(t_rows), len(t_rows[0])
     nb = lib.phx_rows_workspace_bytes(_lib.ctx(dev), G, H, N, T, 0)
+    grid = _Grid(grids, True) if grids is not None else None
+    if grid is not None:
+        nb += grid.nbytes(lib, N, T)
     ws = _workspace(dev, nb, "solve")
     yout = torch.empty(out_shape, dtype=torch.float32, device=y0c.device)
     stn = _new_status_block(N)
     log, cap = _steplog_rows(N)
     flat_t = (ctypes.c_double * (N * T))(*[x for r in t_rows for x in r])
-    rc = lib.phx_solve_forward_rows(_lib.ctx(dev), G, H, N, _ptr(packed), _ptr(y0c), flat_t, T, int(t_is_f32),
-                                    int(reversed_time), _lib.METHOD_IDS[method], float(rtol), float(atol),
-                                    int(max_num_steps), _ptr(yout), _ptr(ws), ws.numel(), _ptr(stn), _ptr(log), cap,
-                                    _stream_ptr(dev))
+    args = (_lib.ctx(dev), G, H, N, _ptr(packed), _ptr(y0c), flat_t, T, int(t_is_f32), int(reversed_time),
+            _lib.METHOD_IDS[method], float(rtol), float(atol), int(max_num_steps), _ptr(yout), _ptr(ws), ws.numel(),
+            _ptr(stn), _ptr(log), cap)
+    if grid is None:
+        rc = lib.phx_solve_forward_rows(*args, _stream_ptr(dev))
+    else:
+        rc = lib.phx_solve_forward_rows_grid(*args, *grid.args(), _stream_ptr(dev))
     _lib.check(rc, "solve_forward_rows")
     _tls().last_status_block = stn
     for i in range(N):
@@ -533,11 +610,15 @@ def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_t
 
 
 def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy, adj_shape,
-                  param_mask=_lib.PARAMS_ALL):
+                  param_mask=_lib.PARAMS_ALL, grids=None):
     """Backward sweeps of N one-row problems (ys, gy: [N, T, ..., G] memory order): adj_y0 and the SUM over the problems of
-    the six parameter cotangents (flat, reference order; zeros for the parameters outside ``param_mask``)."""
+    the six parameter cotangents (flat, reference order; zeros for the parameters outside ``param_mask``).  ``grids``:
+    the problems' backward step grids (adjoint_grid), or None."""
     N, T = len(t_rows), len(t_rows[0])
     nb = lib.phx_rows_workspace_bytes(_lib.ctx(dev), G, H, N, T, 1)
+    grid = _Grid(grids, False) if grids is not None else None
+    if grid is not None:
+        nb += grid.nbytes(lib, N, T)
     ws = _workspace(dev, nb, "solve")
     adj_y0 = torch.empty(adj_shape, dtype=torch.float32, device=ys.device)
     ctx = _lib.ctx(dev)
@@ -551,7 +632,12 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
     sp = _stream_ptr(dev)
     args = (ctx, G, H, N, _ptr(packed), flat_t, T, int(t_is_f32), _lib.METHOD_IDS[method], float(rtol), float(atol),
             int(max_num_steps), _ptr(ys), _ptr(gy), _ptr(adj_y0), _ptr(gpk), _ptr(ws), ws.numel(), _ptr(stn), _ptr(log), cap)
-    if param_mask == _lib.PARAMS_ALL:
+    if grid is not None:
+        _lib.check(lib.phx_solve_adjoint_rows_grid(*args, param_mask, *grid.args(), sp), "solve_adjoint_rows")
+        _lib.check(lib.phx_unpack_grads_masked(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0,
+                                               param_mask & _lib.PARAMS_ALL, sp),
+                   "unpack_grads")
+    elif param_mask == _lib.PARAMS_ALL:
         _lib.check(lib.phx_solve_adjoint_rows(*args, sp), "solve_adjoint_rows")
         _lib.check(lib.phx_unpack_grads(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, sp), "unpack_grads")
     else:
@@ -566,7 +652,9 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
 
 
 @_on_model_device
-def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, max_num_steps):
+def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, max_num_steps, step_size=None):
+    """``step_size`` (fixed-grid methods): integrate on the reference's grid of that spacing and interpolate the output
+    times inside a step (solvers.py:48-50, 77-103); None: one step per output interval."""
     packed, G, H, dev = packed_weights(net)
     if y0.shape[-1] != G:
         raise RuntimeError("last dimension of y0 (%d) must equal ndim (%d)" % (y0.shape[-1], G))
@@ -578,18 +666,27 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
     if T == 1:
         return y0c.unsqueeze(0).clone()
     lib = _lib.load()
+    grids = _grids([t_list], t_is_f32, step_size, True)
     if _use_rows(lib, dev, G, H, B, False, single=True, T=T):
         return _forward_rows(lib, net, packed, G, H, dev, y0c, [t_list], t_is_f32, reversed_time, method, rtol, atol,
-                             max_num_steps, (T,) + tuple(y0c.shape))
+                             max_num_steps, (T,) + tuple(y0c.shape), grids)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, False)
+    grid = _Grid(grids, True) if grids is not None else None
+    if grid is not None and engine == "resident":
+        nb += grid.nbytes(lib, 1, T)
     ws = _workspace(dev, nb, "solve" if engine == "resident" else "stream")
     yout = torch.empty((T,) + tuple(y0c.shape), dtype=torch.float32, device=y0c.device)
     st = _new_status()
     log, cap = _steplog()
-    fn = lib.phx_solve_forward if engine == "resident" else lib.phx_stream_solve_forward
-    rc = fn(_lib.ctx(dev), G, H, B, _ptr(packed), _ptr(y0c), _t_array(t_list), T, int(t_is_f32),
-            int(reversed_time), _lib.METHOD_IDS[method], float(rtol), float(atol), int(max_num_steps), _ptr(yout),
-            _ptr(ws), ws.numel(), _ptr(st), _ptr(log), cap, _stream_ptr(dev))
+    args = (_lib.ctx(dev), G, H, B, _ptr(packed), _ptr(y0c), _t_array(t_list), T, int(t_is_f32), int(reversed_time),
+            _lib.METHOD_IDS[method], float(rtol), float(atol), int(max_num_steps), _ptr(yout), _ptr(ws), ws.numel(),
+            _ptr(st), _ptr(log), cap)
+    if grid is None:
+        fn = lib.phx_solve_forward if engine == "resident" else lib.phx_stream_solve_forward
+        rc = fn(*args, _stream_ptr(dev))
+    else:
+        fn = lib.phx_solve_forward_grid if engine == "resident" else lib.phx_stream_solve_forward_grid
+        rc = fn(*args, *grid.args(), _stream_ptr(dev))
     _lib.check(rc, "solve_forward")
     _finish(st, "forward solve", dev)
     return yout
@@ -597,11 +694,12 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
 
 @_on_model_device
 def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
-                  param_mask=_lib.PARAMS_ALL):
+                  param_mask=_lib.PARAMS_ALL, step_size=None):
     """adj_y0 and the six parameter cotangents of one backward sweep.  ``param_mask`` (bit i = the i-th parameter in
     reference order): the adjoint parameters, the only ones integrated and put in the error norm; the cotangents of the
     others come back as zeros.  With ``_lib.NORM_SEMINORM`` also set, the dopri5 error norm leaves the parameter block
-    out altogether (the seminorm)."""
+    out altogether (the seminorm).  ``step_size`` (fixed-grid methods): every interval is integrated on its own grid of
+    that spacing (adjoint_grid); None: one step per interval."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -610,10 +708,14 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
         return gy[0].clone(), _zero_param_grads(net, G, H, ys.device)
     B = ys[0].numel() // G
     lib = _lib.load()
+    grids = _grids([t_list], t_is_f32, step_size, False)
     if _use_rows(lib, dev, G, H, B, True, single=True, T=T):
         return _adjoint_rows(lib, net, packed, G, H, dev, [t_list], t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[0].shape), param_mask)
+                             tuple(ys[0].shape), param_mask, grids)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
+    grid = _Grid(grids, False) if grids is not None else None
+    if grid is not None and engine == "resident":
+        nb += grid.nbytes(lib, 1, T)
     ws = _workspace(dev, nb, "solve" if engine == "resident" else "stream")
     adj_y0 = torch.empty_like(ys[0])
     P = 4 * G * H + 2 * H + G
@@ -624,7 +726,10 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     args = (_lib.ctx(dev), G, H, B, _ptr(packed), _t_array(t_list), T, int(t_is_f32), _lib.METHOD_IDS[method],
             float(rtol), float(atol), int(max_num_steps), _ptr(ys), _ptr(gy), _ptr(adj_y0), _ptr(grads), _ptr(ws),
             ws.numel(), _ptr(st), _ptr(log), cap)
-    if param_mask == _lib.PARAMS_ALL:
+    if grid is not None:
+        fn = lib.phx_solve_adjoint_grid if engine == "resident" else lib.phx_stream_solve_adjoint_grid
+        rc = fn(*args, param_mask, *grid.args(), _stream_ptr(dev))
+    elif param_mask == _lib.PARAMS_ALL:
         rc = fn(*args, _stream_ptr(dev))
     else:
         fn = lib.phx_solve_adjoint_masked if engine == "resident" else lib.phx_stream_solve_adjoint_masked
@@ -696,11 +801,11 @@ def _fan_in(dev, streams):
 
 
 @_on_model_device
-def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_steps):
+def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_steps, step_size=None):
     """y0 ``[N, *S, G]``: N independent problems, problem i integrated over its own times ``t_rows[i]`` (all of length
     T).  Every problem is one resident launch with its own step controller -- exactly the reference's per-sample call
     (train_insilico.py:128-130) -- but the weights are packed, the workspace fetched and the arguments marshalled once
-    for the whole set.  Returns ``[N, T, *S, G]``."""
+    for the whole set.  Returns ``[N, T, *S, G]``.  ``step_size``: as in solve_forward, every problem on its own grid."""
     packed, G, H, dev = packed_weights(net)
     if y0.shape[-1] != G:
         raise RuntimeError("last dimension of y0 (%d) must equal ndim (%d)" % (y0.shape[-1], G))
@@ -712,13 +817,20 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
         return y0c.unsqueeze(1).clone()
     B = y0c[0].numel() // G
     lib = _lib.load()
+    grids = _grids(t_rows, t_is_f32, step_size, True)
     if _use_rows(lib, dev, G, H, B, False):
         return _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, False, method, rtol, atol, max_num_steps,
-                             (N, T) + tuple(y0c.shape[1:]))
+                             (N, T) + tuple(y0c.shape[1:]), grids)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, False)
+    if grids is not None and engine == "resident":
+        nb += _Grid(grids, True).nbytes(lib, N, T)
     ws = _workspace(dev, nb, "solve" if engine == "resident" else "stream")
     yout = torch.empty((N, T) + tuple(y0c.shape[1:]), dtype=torch.float32, device=y0c.device)
     fn = lib.phx_solve_forward if engine == "resident" else lib.phx_stream_solve_forward
+    pg = [_Grid([g], True) for g in grids] if grids is not None else None   # (kept alive over the calls)
+    gx = (lambda i: pg[i].args()) if pg is not None else (lambda i: [])  # noqa: E731
+    if pg is not None:   # the grid of problem i goes right before the stream
+        fn = lib.phx_solve_forward_grid if engine == "resident" else lib.phx_stream_solve_forward_grid
     ctx, sp, mid = _lib.ctx(dev), _stream_ptr(dev), _lib.METHOD_IDS[method]
     pk, wsp, wsn = _ptr(packed), _ptr(ws), ws.numel()
     ybase, obase = y0c.data_ptr(), yout.data_ptr()
@@ -735,9 +847,14 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
             n = min(per, N - lo)
             stn = _new_status_block(n)
             flat_t = (ctypes.c_double * (n * T))(*[x for r in t_rows[lo:lo + n] for x in r])
-            rc = lib.phx_solve_forward_many(ctx, G, H, B, n, pk, ctypes.c_void_p(ybase + lo * ystride), flat_t, T,
-                                            int(t_is_f32), mid, float(rtol), float(atol), int(max_num_steps),
-                                            ctypes.c_void_p(obase + lo * ostride), wsp, wsn, _ptr(stn), sp)
+            args = (ctx, G, H, B, n, pk, ctypes.c_void_p(ybase + lo * ystride), flat_t, T, int(t_is_f32), mid,
+                    float(rtol), float(atol), int(max_num_steps), ctypes.c_void_p(obase + lo * ostride), wsp, wsn,
+                    _ptr(stn))
+            if grids is None:
+                rc = lib.phx_solve_forward_many(*args, sp)
+            else:
+                gm = _Grid(grids[lo:lo + n], True)
+                rc = lib.phx_solve_forward_many_grid(*args, *gm.args(), sp)
             _lib.check(rc, "solve_forward_many")
             for i in range(n):
                 _finish(stn[i], "forward solve %d" % (lo + i), dev)
@@ -751,13 +868,13 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
                     wsi = _workspace(dev, nb, "solve")
                     rc = fn(ctx, G, H, B, pk, ctypes.c_void_p(ybase + i * ystride), tarr[i], T, int(t_is_f32), 0, mid,
                             float(rtol), float(atol), int(max_num_steps), ctypes.c_void_p(obase + i * ostride),
-                            _ptr(wsi), wsi.numel(), _ptr(st), _ptr(log), cap, _stream_ptr(dev))
+                            _ptr(wsi), wsi.numel(), _ptr(st), _ptr(log), cap, *gx(i), _stream_ptr(dev))
                     _lib.check(rc, "solve_forward")
                     _finish(st, "forward solve %d" % i, dev)
                 continue
             rc = fn(ctx, G, H, B, pk, ctypes.c_void_p(ybase + i * ystride), tarr[i], T, int(t_is_f32), 0, mid,
                     float(rtol), float(atol), int(max_num_steps), ctypes.c_void_p(obase + i * ostride), wsp, wsn,
-                    _ptr(st), _ptr(log), cap, sp)
+                    _ptr(st), _ptr(log), cap, *gx(i), sp)
             _lib.check(rc, "solve_forward")
             _finish(st, "forward solve %d" % i, dev)
     finally:
@@ -768,10 +885,10 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
 
 @_on_model_device
 def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
-                       param_mask=_lib.PARAMS_ALL):
+                       param_mask=_lib.PARAMS_ALL, step_size=None):
     """Backward sweeps of N independent problems (``y_saved``, ``grad_y``: ``[N, T, *S, G]``): adj_y0 ``[N, *S, G]`` and
     the six parameter cotangents summed over the problems (what autograd accumulates into ``.grad``); zeros for the
-    parameters outside ``param_mask`` (see solve_adjoint)."""
+    parameters outside ``param_mask``; ``step_size``: see solve_adjoint)."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -780,10 +897,13 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
         return gy[:, 0].clone(), _zero_param_grads(net, G, H, ys.device)
     B = ys[0, 0].numel() // G
     lib = _lib.load()
+    grids = _grids(t_rows, t_is_f32, step_size, False)
     if _use_rows(lib, dev, G, H, B, True):
         return _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[:, 0].shape), param_mask)
+                             tuple(ys[:, 0].shape), param_mask, grids)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
+    if grids is not None and engine == "resident":
+        nb += _Grid(grids, False).nbytes(lib, N, T)
     ws = _workspace(dev, nb, "solve" if engine == "resident" else "stream")
     adj_y0 = torch.empty_like(ys[:, 0])
     P = 4 * G * H + 2 * H + G
@@ -791,7 +911,13 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     grads = torch.empty(chunk, P, dtype=torch.float32, device=ys.device)
     total = None
     full = param_mask == _lib.PARAMS_ALL
-    if full:
+    pg = [_Grid([g], False) for g in grids] if grids is not None else None   # (kept alive over the calls)
+    gx = (lambda i: pg[i].args()) if pg is not None else (lambda i: [])  # noqa: E731
+    if pg is not None:   # param_mask, then the grid, right before the stream
+        fn0 = lib.phx_solve_adjoint_grid if engine == "resident" else lib.phx_stream_solve_adjoint_grid
+        fn = lambda *a: fn0(*a[:-3], param_mask, *a[-3:])  # noqa: E731
+        many = None
+    elif full:
         fn = lib.phx_solve_adjoint if engine == "resident" else lib.phx_stream_solve_adjoint
         many = lib.phx_solve_adjoint_many
     else:   # the masked entry points take param_mask right before the stream
@@ -812,11 +938,15 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
                 n = min(per, hi - l2)
                 stn = _new_status_block(n)
                 flat_t = (ctypes.c_double * (n * T))(*[x for r in t_rows[l2:l2 + n] for x in r])
-                rc = many(
-                    ctx, G, H, B, n, pk, flat_t, T, int(t_is_f32), mid, float(rtol), float(atol), int(max_num_steps),
-                    ctypes.c_void_p(ys.data_ptr() + l2 * stride), ctypes.c_void_p(gy.data_ptr() + l2 * stride),
-                    ctypes.c_void_p(adj_y0.data_ptr() + l2 * astride),
-                    ctypes.c_void_p(grads.data_ptr() + (l2 - lo) * P * 4), wsp, wsn, _ptr(stn), sp)
+                args = (ctx, G, H, B, n, pk, flat_t, T, int(t_is_f32), mid, float(rtol), float(atol),
+                        int(max_num_steps), ctypes.c_void_p(ys.data_ptr() + l2 * stride),
+                        ctypes.c_void_p(gy.data_ptr() + l2 * stride), ctypes.c_void_p(adj_y0.data_ptr() + l2 * astride),
+                        ctypes.c_void_p(grads.data_ptr() + (l2 - lo) * P * 4), wsp, wsn, _ptr(stn))
+                if grids is None:
+                    rc = many(*args, sp)
+                else:
+                    gm = _Grid(grids[l2:l2 + n], False)
+                    rc = lib.phx_solve_adjoint_many_grid(*args, param_mask, *gm.args(), sp)
                 _lib.check(rc, "solve_adjoint_many")
                 for i in range(n):
                     _finish(stn[i], "adjoint solve %d" % (l2 + i), dev)
@@ -836,13 +966,13 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
                     with torch.cuda.stream(streams[i % len(streams)]):
                         wsi = _workspace(dev, nb, "solve")
                         rc = fn(ctx, G, H, B, pk, tarr[i], T, int(t_is_f32), mid, float(rtol), float(atol),
-                                int(max_num_steps), *args, _ptr(wsi), wsi.numel(), _ptr(st), _ptr(log), cap,
+                                int(max_num_steps), *args, _ptr(wsi), wsi.numel(), _ptr(st), _ptr(log), cap, *gx(i),
                                 _stream_ptr(dev))
                         _lib.check(rc, "solve_adjoint")
                         _finish(st, "adjoint solve %d" % i, dev)
                     continue
                 rc = fn(ctx, G, H, B, pk, tarr[i], T, int(t_is_f32), mid, float(rtol), float(atol), int(max_num_steps),
-                        *args, wsp, wsn, _ptr(st), _ptr(log), cap, sp)
+                        *args, wsp, wsn, _ptr(st), _ptr(log), cap, *gx(i), sp)
                 _lib.check(rc, "solve_adjoint")
                 _finish(st, "adjoint solve %d" % i, dev)
         finally:

@@ -18,8 +18,35 @@ _SUPPORTED = ('dopri5', 'euler', 'midpoint', 'rk4')
 _DEFAULT_MAX_STEPS = 2 ** 31 - 1
 
 
+_FIXED_GRID = ('euler', 'midpoint', 'rk4')
+
+
+def _step_size(method, options):
+    """The fixed-grid ``step_size`` option (solvers.py:48-50), or None when it is not given: a float, or for a tensor
+    ``(value, dtype)``.  A tensor keeps its dtype because the reference builds the grid under tensor type promotion (a
+    0-dim float64 step size makes the step count of a float32 t's grid a float64 division); the pair keeps the deferred
+    adjoint's group key hashable (_stepped turns it back into the tensor).  Only the three fixed-grid methods take it
+    (dopri5: the generic refusal of _normalise); ``grid_constructor`` is refused."""
+    if not options:
+        return None
+    if 'grid_constructor' in options:
+        raise NotImplementedError("options['grid_constructor'] is not supported on the B200 path: the backward would call "
+                                  "it with the augmented dynamics and state, which exist only on the device; use "
+                                  "step_size")
+    if 'step_size' not in options or (method or 'dopri5') not in _FIXED_GRID:
+        return None
+    h = options['step_size']
+    if torch.is_tensor(h) and h.dim() != 0:
+        raise NotImplementedError("a tensor step_size must be 0-dimensional (got shape {})".format(tuple(h.shape)))
+    v = float(h.item() if torch.is_tensor(h) else h)
+    if not (v > 0 and v != float('inf')):
+        raise ValueError("step_size must be a positive finite number (got {})".format(options['step_size']))
+    return (v, h.dtype) if torch.is_tensor(h) else v
+
+
 def _normalise(func, y0, t, rtol, atol, method, options):
-    """The checks of misc.py:165-241 that apply to a single-tensor state; returns the pieces the kernels need."""
+    """The checks of misc.py:165-241 that apply to a single-tensor state; returns the pieces the kernels need (the
+    fixed-grid ``step_size`` is checked here and read with _step_size)."""
     if not torch.is_tensor(y0):
         assert isinstance(y0, tuple), 'y0 must be either a torch.Tensor or a tuple'
         raise NotImplementedError("tuple-valued states are not part of the PHOENIX path (ODENet has a tensor state)")
@@ -36,6 +63,8 @@ def _normalise(func, y0, t, rtol, atol, method, options):
                                   'path implements {}'.format(method, _SUPPORTED))
     max_num_steps = int(options.pop('max_num_steps', _DEFAULT_MAX_STEPS))
     options.pop('dtype', None)
+    if _step_size(method, options) is not None:
+        options.pop('step_size')
     if options:
         raise NotImplementedError("solver options {} are not supported on the B200 path (the reference never passes "
                                   "options)".format(sorted(options)))
@@ -73,11 +102,12 @@ def odeint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None):
     (odeint.py:25-69).  Not differentiable — use ``odeint_adjoint`` (what every PHOENIX script imports as ``odeint``,
     train_insilico.py:15-18) when gradients are needed."""
     tl, t_is_f32, rev, rtol, atol, method, max_steps = _normalise(func, y0, t, rtol, atol, method, options)
+    step = _step_size(method, options)
     if torch.is_grad_enabled() and (y0.requires_grad or any(p.requires_grad for p in func.parameters())):
         warnings.warn("phoenix_b200.odeint does not record an autograd graph; use odeint_adjoint for gradients",
                       stacklevel=2)
     with torch.no_grad():
-        return engine.solve_forward(func, y0, tl, t_is_f32, rev, method, rtol, atol, max_steps)
+        return engine.solve_forward(func, y0, tl, t_is_f32, rev, method, rtol, atol, max_steps, **_stepped(step))
 
 
 # ---- the per-sample loop of training_step, backward side ----------------------------------------------------------------
@@ -112,8 +142,8 @@ def _register_node(ctx, func, y0, tl, t_is_f32, adj):
     with _defer_lock:
         _node_seq[0] += 1
         ctx.seq = _node_seq[0]
-        # adj[4], the adjoint parameter mask with the norm bit, is part of the key: only nodes with the same adjoint set
-        # and the same error norm share a sweep
+        # adj[4], the adjoint parameter mask with the norm bit, and adj[5], the backward step size, are part of the key:
+        # only nodes with the same adjoint set, error norm and step grid spacing share a sweep
         ctx.group = (len(tl), t_is_f32, adj, tuple(y0.shape), y0.device, tuple(ctx.needs_input_grad[9:]))
         nodes = _live_nodes.get(func)
         if nodes is None:
@@ -171,10 +201,11 @@ class OdeintAdjointMethod(torch.autograd.Function):
     augmented system per output interval (batched with the sibling nodes of the same backward pass, see above)."""
 
     @staticmethod
-    def forward(ctx, func, tl, t_is_f32, method, rtol, atol, max_steps, adj, y0, *adjoint_params):
+    def forward(ctx, func, tl, t_is_f32, fwd, rtol, atol, max_steps, adj, y0, *adjoint_params):
+        # fwd = (method, step_size); adj = (method, rtol, atol, max_num_steps, mask, step_size) of the backward
         ctx.func, ctx.tl, ctx.t_is_f32, ctx.adj = func, tl, t_is_f32, adj
         with torch.no_grad():
-            y = engine.solve_forward(func, y0, tl, t_is_f32, False, method, rtol, atol, max_steps)
+            y = engine.solve_forward(func, y0, tl, t_is_f32, False, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]))
         ctx.save_for_backward(y)
         _register_node(ctx, func, y0, tl, t_is_f32, adj)
         return y
@@ -182,20 +213,21 @@ class OdeintAdjointMethod(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
-        a_method, a_rtol, a_atol, a_max, mask = ctx.adj
+        a_method, a_rtol, a_atol, a_max, mask = ctx.adj[:5]
         if not mask & PARAMS_ALL and not ctx.needs_input_grad[8]:
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))   # only parameters outside adjoint_params want one
         batch = _defer(ctx, y, grad_y) if (ctx.group is not None and DEFER_ADJOINT) else _NOT_DEFERRED
         if batch is None:
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))
+        kw = dict(_masked(mask), **_stepped(ctx.adj[5]))
         with torch.no_grad():
             if batch is _NOT_DEFERRED:
                 adj_y0, grads = engine.solve_adjoint(ctx.func, ctx.tl, ctx.t_is_f32, a_method, a_rtol, a_atol, a_max,
-                                                     y, grad_y, **_masked(mask))
+                                                     y, grad_y, **kw)
             else:
                 t_rows, ys, gys = batch
                 adj_y0, grads = engine.solve_adjoint_many(ctx.func, t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
-                                                          a_max, ys, gys, **_masked(mask))
+                                                          a_max, ys, gys, **kw)
         return _grads_out(ctx, adj_y0, grads, mask)
 
 
@@ -203,6 +235,16 @@ def _masked(mask):
     """The engine's keyword for a proper subset of the parameters or the seminorm; with all six parameters and the
     default norm the engine is called as it always was."""
     return {} if mask == PARAMS_ALL else {"param_mask": mask}
+
+
+def _stepped(step_size):
+    """The engine's keyword for a fixed-grid step size (_step_size's form: a float, or (value, dtype) of a tensor);
+    without one the engine is called as it always was."""
+    if step_size is None:
+        return {}
+    if isinstance(step_size, tuple):
+        return {"step_size": torch.tensor(step_size[0], dtype=step_size[1])}
+    return {"step_size": step_size}
 
 
 def _grads_out(ctx, adj_y0, grads, mask):
@@ -275,38 +317,40 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
     same = (adjoint_rtol is rtol and adjoint_atol is atol and adjoint_method is method and not adjoint_options
             and not options)
     tl, t_is_f32, rev, rtol, atol, method, max_steps = _normalise(func, y0, t, rtol, atol, method, options)
+    step = _step_size(method, options)
     if same:
-        a_rtol, a_atol, a_method, a_max = rtol, atol, method, max_steps
+        a_rtol, a_atol, a_method, a_max, a_step = rtol, atol, method, max_steps, step
     else:
         _, _, _, a_rtol, a_atol, a_method, a_max = _normalise(func, y0, t, adjoint_rtol, adjoint_atol, adjoint_method,
                                                               adjoint_options)
+        a_step = _step_size(a_method, adjoint_options)
     if rev:
         raise NotImplementedError("odeint_adjoint with decreasing t is not part of the PHOENIX path")
     params, mask = _adjoint_mask(func, adjoint_params)
-    return OdeintAdjointMethod.apply(func, tl, t_is_f32, method, rtol, atol, max_steps,
-                                     (a_method, a_rtol, a_atol, a_max, mask | norm_bit), y0, *params)
+    return OdeintAdjointMethod.apply(func, tl, t_is_f32, (method, step), rtol, atol, max_steps,
+                                     (a_method, a_rtol, a_atol, a_max, mask | norm_bit, a_step), y0, *params)
 
 
 class OdeintAdjointManyMethod(torch.autograd.Function):
     """N independent ``OdeintAdjointMethod`` problems behind one autograd node (engine.solve_*_many)."""
 
     @staticmethod
-    def forward(ctx, func, t_rows, t_is_f32, method, rtol, atol, max_steps, adj, y0, *adjoint_params):
+    def forward(ctx, func, t_rows, t_is_f32, fwd, rtol, atol, max_steps, adj, y0, *adjoint_params):
         ctx.func, ctx.t_rows, ctx.t_is_f32, ctx.adj = func, t_rows, t_is_f32, adj
         with torch.no_grad():
-            y = engine.solve_forward_many(func, y0, t_rows, t_is_f32, method, rtol, atol, max_steps)
+            y = engine.solve_forward_many(func, y0, t_rows, t_is_f32, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]))
         ctx.save_for_backward(y)
         return y
 
     @staticmethod
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
-        a_method, a_rtol, a_atol, a_max, mask = ctx.adj
+        a_method, a_rtol, a_atol, a_max, mask = ctx.adj[:5]
         if not mask & PARAMS_ALL and not ctx.needs_input_grad[8]:
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))
         with torch.no_grad():
             adj_y0, grads = engine.solve_adjoint_many(ctx.func, ctx.t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
-                                                      a_max, y, grad_y, **_masked(mask))
+                                                      a_max, y, grad_y, **_masked(mask), **_stepped(ctx.adj[5]))
         return _grads_out(ctx, adj_y0, grads, mask)
 
 
@@ -331,10 +375,12 @@ def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=
         assert all(b > a for a, b in zip(r, r[1:])), 't must be strictly increasing for every sample'
     if rev:
         raise NotImplementedError("odeint_adjoint_many with decreasing t is not part of the PHOENIX path")
+    step = _step_size(method, options)
     adjoint_options, norm_bit = _adjoint_norm(adjoint_options)
-    a_max = max_steps
+    a_max, a_step = max_steps, step
     if adjoint_options is not None:
         a_max = _normalise(func, y0[0], t[0], rtol, atol, method, adjoint_options)[6]
+        a_step = _step_size(method, adjoint_options)
     params, mask = _adjoint_mask(func, adjoint_params)
-    return OdeintAdjointManyMethod.apply(func, rows, t_is_f32, method, rtol_f, atol_f, max_steps,
-                                         (method, rtol_f, atol_f, a_max, mask | norm_bit), y0, *params)
+    return OdeintAdjointManyMethod.apply(func, rows, t_is_f32, (method, step), rtol_f, atol_f, max_steps,
+                                         (method, rtol_f, atol_f, a_max, mask | norm_bit, a_step), y0, *params)
