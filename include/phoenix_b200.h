@@ -178,23 +178,18 @@ int phx_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, co
                       void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                       int steplog_cap, void* stream);
 /* ---- adjoint parameters (adjoint.py:185-193: the members of adjoint_params that require grad) -------------------------
- * The *_masked variants of the adjoint entry points take param_mask, a 6-bit set of parameters in reference order: bit
- * i = the i-th of (gene_multipliers, Wp, bp, Ws, bs, Wa), PHX_PARAMS_ALL = all six (what the unmasked entry points
- * pass).  Only the cotangents of the parameters in the mask are integrated, and only they make up the parameter block of
- * the error norm (count = their total size; with an empty mask the block is absent).  The blocks of grads_flat outside
- * the mask are written as zeros (phx_unpack_grads_masked with accumulate != 0 leaves them as they are).  A mask outside
- * 0 .. 0x3F returns PHX_ERR_INVALID.
- * PHX_NORM_SEMINORM may be OR-ed into the param_mask of the four adjoint solves (not phx_unpack_grads_masked): dopri5 then
+ * An adjoint phx_solve (below) takes param_mask, a 6-bit set of parameters in reference order: bit i = the i-th of
+ * (gene_multipliers, Wp, bp, Ws, bs, Wa), PHX_PARAMS_ALL = all six (what the other adjoint entry points pass).  Only the
+ * cotangents of the parameters in the mask are integrated, and only they make up the parameter block of the error norm
+ * (count = their total size; with an empty mask the block is absent).  The blocks of grads_flat outside the mask are
+ * written as zeros (phx_unpack_grads_masked with accumulate != 0 leaves them as they are).  A mask outside 0 .. 0x3F
+ * returns PHX_ERR_INVALID.
+ * PHX_NORM_SEMINORM may be OR-ed into the param_mask of an adjoint phx_solve (not phx_unpack_grads_masked): dopri5 then
  * measures the error with the seminorm of Kidger, Chen & Lyons (2021), the mixed norm without the parameter block, in
  * Hairer's initial step and in every error ratio, while the low six bits still choose the integrated cotangents.
  * Fixed grids use no norm and are unaffected.  With it the accepted range is 0 .. 0x7F. */
 #define PHX_PARAMS_ALL 0x3F
 #define PHX_NORM_SEMINORM 0x40
-int phx_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                             int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                             const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                             void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                             int steplog_cap, int param_mask, void* stream);
 
 /* ---- N independent problems per launch (the per-sample loop of training_step, train_insilico.py:128-130) -------- */
 /* Problem i: initial state y0 + i*B*G, its own T increasing times t_host[i*T .. i*T+T), outputs y_out + i*T*B*G, its own
@@ -210,11 +205,6 @@ int phx_solve_adjoint_many(phx_ctx* ctx, int G, int H, int B, int N, const float
                            int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                            void* workspace, size_t workspace_bytes, phx_status* status, void* stream);
-int phx_solve_adjoint_many_masked(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host,
-                                  int T, int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                  void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
-                                  void* stream);
 
 /* ---- the same two solves for ANY number of rows B (streaming engine) ---------------------------------------- */
 /* phx_solve_forward / phx_solve_adjoint keep the whole solve in one persistent cooperative launch and need the rows
@@ -242,11 +232,6 @@ int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* pac
                              const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                              void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                              int steplog_cap, void* stream);
-int phx_stream_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                                    int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                    const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                    void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                    int steplog_cap, int param_mask, void* stream);
 
 /* ---- the sample loop of training_step as rows of ONE launch (train_insilico.py:128-130) ------------------------------- */
 /* N independent ONE-ROW problems (y0 [N][G], each with its own T increasing times t_host[i*T .. i*T+T), its own dopri5 step
@@ -276,76 +261,59 @@ int phx_solve_adjoint_rows(phx_ctx* ctx, int G, int H, int N, const float* packe
                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
                            void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                            int steplog_cap, void* stream);
-int phx_solve_adjoint_rows_masked(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
-                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
-                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                  int steplog_cap, int param_mask, void* stream);
 size_t phx_packed_grad_bytes(int G, int H);
 int phx_rows_grad_parts(const phx_ctx* ctx, int G, int H, int N);
 
-/* ---- fixed-grid solves on a step grid (odeint options=dict(step_size=h), torchdiffeq solvers.py:48-50, 77-103) ----------
- * The *_grid variants take the same arguments as the entry point they are named after (the adjoint ones: as its *_masked
- * variant, param_mask included; PHX_NORM_SEMINORM is accepted and has no effect) plus the grid, host arrays, right before
- * the stream.  The method must be euler, midpoint or rk4; the caller builds the grid (the Python layer does it with the
- * reference's own tensor ops) and no kernel computes one:
+/* ---- every solve through one request (phx_solve) --------------------------------------------------------------------
+ * phx_solve runs one solve described by a phx_solve_desc; each entry point above is a phx_solve call with the options it
+ * does not take at their defaults.  `engine` picks the solver (PHX_ENGINE_RESIDENT: phx_solve_forward / _adjoint, and
+ * phx_solve_*_many when N > 1; PHX_ENGINE_ROWS: phx_solve_*_rows, B = 1; PHX_ENGINE_STREAM: phx_stream_solve_*, N = 1),
+ * `adjoint` the direction.  The fields mean what the arguments of the same names mean there, and the workspace is sized
+ * by the engine's own size function.  Forward solves read y0 and write y_out; adjoint solves read y_saved and grad_y and
+ * write adj_y0 and `grads` (flat [N][P] on the resident and streaming engines, the packed partial sums of
+ * phx_solve_adjoint_rows on the rows engine), with `param_mask` as described above (PHX_PARAMS_ALL for all six).
+ * The combinations no engine takes return PHX_ERR_INVALID: an unknown engine; `reversed` or `grid_out_*` on an adjoint
+ * solve; a nonzero param_mask on a forward solve; grid arrays without grid_dt; N != 1 on the streaming engine; B != 1 on
+ * the rows engine; `reversed` or a step log on the resident engine with N > 1.
+ *
+ * Fixed-grid solves on a step grid (odeint options=dict(step_size=h), torchdiffeq solvers.py:48-50, 77-103): with grid_dt
+ * set (NULL: one step per output interval) the method must be euler, midpoint or rk4, and PHX_NORM_SEMINORM is accepted
+ * and has no effect.  The caller builds the grid (the Python layer does it with the reference's own tensor ops) and no
+ * kernel computes one; its arrays are HOST arrays:
  *   grid_steps[q] >= 1 steps per segment and their float32 dt back to back in grid_dt (in segment order).  A forward
- *     segment is a problem (N of them; 1 for the one-problem calls); an adjoint segment is an output interval of a problem,
- *     [N][T-1] with the interval [t[i], t[i+1]] at index i, its steps in the order the backward takes them (from t[i+1]).
+ *     segment is a problem (N of them); an adjoint segment is an output interval of a problem, [N][T-1] with the interval
+ *     [t[i], t[i+1]] at index i, its steps in the order the backward takes them (from t[i+1]).
  *   forward only, [N][T-1]: grid_out_step[j-1] = the step (counted from 0 within the problem, non-decreasing in j) whose
  *     end is the first grid point >= t[j], and grid_out_slope[j-1] = (t[j] - t0) / (t1 - t0) of that step, rounded to
  *     float32; output j is then y0 + slope * (y1 - y0), or y1 itself when the slope is negative (t[j] == t1).
  * Between the steps the state is not restarted at the output times.  status.n_rhs = stages x steps.  The grid is copied
- * into the workspace (not for the streaming engine), which must then hold phx_grid_workspace_bytes(N, T, total steps)
- * more bytes than the entry point's own size function asks for.  An invalid grid (a step count < 1, a dt that is negative
- * or not finite, an output step out of range or decreasing, a NaN slope) returns PHX_ERR_INVALID. */
+ * into the workspace (not on the streaming engine), which must then hold phx_grid_workspace_bytes(N, T, total steps)
+ * more bytes than the engine's own size function asks for.  An invalid grid (a step count < 1, a dt that is negative or
+ * not finite, an output step out of range or decreasing, a NaN slope) returns PHX_ERR_INVALID. */
+enum { PHX_ENGINE_RESIDENT = 0, PHX_ENGINE_ROWS = 1, PHX_ENGINE_STREAM = 2 };
+typedef struct phx_solve_desc {
+    const float* packed;
+    const double* t_host;            /* [N][T] */
+    const float* y0;                 /* forward */
+    float* y_out;
+    const float* y_saved;            /* adjoint */
+    const float* grad_y;
+    float* adj_y0;
+    float* grads;
+    const float* grid_dt;            /* step grid (host arrays); NULL grid_dt: one step per output interval */
+    const int32_t* grid_steps;
+    const int32_t* grid_out_step;    /* forward grids only */
+    const float* grid_out_slope;
+    void* workspace;
+    size_t workspace_bytes;
+    phx_status* status;              /* [N] */
+    double* steplog;                 /* may be NULL */
+    double rtol, atol;
+    int64_t max_num_steps;
+    int32_t engine, adjoint, G, H, B, N, T, t_is_f32, reversed, method, param_mask, steplog_cap;
+} phx_solve_desc;
+int phx_solve(phx_ctx* ctx, const phx_solve_desc* desc, void* stream);
 size_t phx_grid_workspace_bytes(int N, int T, int64_t total_steps);
-int phx_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
-                           const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
-                           double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
-                           phx_status* status, double* steplog, int steplog_cap, const float* grid_dt,
-                           const int32_t* grid_steps, const int32_t* grid_out_step, const float* grid_out_slope,
-                           void* stream);
-int phx_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                           int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                           const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                           void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                           int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
-                           void* stream);
-int phx_solve_forward_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const float* y0,
-                                const double* t_host, int T, int t_is_f32, int method, double rtol, double atol,
-                                int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
-                                phx_status* status, const float* grid_dt, const int32_t* grid_steps,
-                                const int32_t* grid_out_step, const float* grid_out_slope, void* stream);
-int phx_solve_adjoint_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host,
-                                int T, int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
-                                const float* grid_dt, const int32_t* grid_steps, void* stream);
-int phx_solve_forward_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const float* y0,
-                                const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
-                                double atol, int64_t max_num_steps, float* y_out, void* workspace,
-                                size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
-                                const float* grid_dt, const int32_t* grid_steps, const int32_t* grid_out_step,
-                                const float* grid_out_slope, void* stream);
-int phx_solve_adjoint_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
-                                int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
-                                void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
-                                void* stream);
-int phx_stream_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
-                                  const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
-                                  double atol, int64_t max_num_steps, float* y_out, void* workspace,
-                                  size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
-                                  const float* grid_dt, const int32_t* grid_steps, const int32_t* grid_out_step,
-                                  const float* grid_out_slope, void* stream);
-int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                  int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
-                                  void* stream);
 int phx_unpack_grads(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
                      int accumulate, void* stream);
 int phx_unpack_grads_masked(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,

@@ -15,6 +15,7 @@ METHOD_IDS = {"euler": 0, "midpoint": 1, "rk4": 2, "dopri5": 3}
 PARAMS_ALL = 0x3F   # adjoint parameter mask: bit i = the i-th ODENet parameter in reference order
 NORM_SEMINORM = 0x40   # OR-ed into an adjoint solve's mask: the dopri5 error norm leaves out the parameter block
 PREC_FP32, PREC_TF32, PREC_3XTF32 = 0, 1, 3
+ENGINE_RESIDENT, ENGINE_ROWS, ENGINE_STREAM = 0, 1, 2
 ST_OK, ST_DT_UNDERFLOW, ST_NONFINITE, ST_MAX_STEPS, ST_RUNNING = 0, 1, 2, 3, 99
 
 EXPORTS = [
@@ -27,11 +28,7 @@ EXPORTS = [
     "phx_stream_workspace_bytes", "phx_stream_solve_forward", "phx_stream_solve_adjoint",
     "phx_rows_supported", "phx_rows_plan_describe", "phx_rows_workspace_bytes", "phx_solve_forward_rows",
     "phx_solve_adjoint_rows", "phx_unpack_grads", "phx_packed_grad_bytes", "phx_rows_grad_parts",
-    "phx_solve_adjoint_masked", "phx_solve_adjoint_many_masked", "phx_stream_solve_adjoint_masked",
-    "phx_solve_adjoint_rows_masked", "phx_unpack_grads_masked",
-    "phx_grid_workspace_bytes", "phx_solve_forward_grid", "phx_solve_adjoint_grid", "phx_solve_forward_many_grid",
-    "phx_solve_adjoint_many_grid", "phx_solve_forward_rows_grid", "phx_solve_adjoint_rows_grid",
-    "phx_stream_solve_forward_grid", "phx_stream_solve_adjoint_grid",
+    "phx_unpack_grads_masked", "phx_solve", "phx_grid_workspace_bytes",
     "phx_prior_loss", "phx_prior_setup", "phx_tc_set_pair", "phx_tc_prof_dump", "phx_ctx_set_global_norm", "phx_peer_allreduce", "phx_peer_allreduce_nvls", "phx_mse_grad", "phx_hill_planes", "phx_hill_cache_set",
 ]
 
@@ -40,6 +37,18 @@ class PhxStatus(ctypes.Structure):
     _fields_ = [("code", ctypes.c_int32), ("n_accepted", ctypes.c_int32), ("n_rejected", ctypes.c_int32),
                 ("n_rhs", ctypes.c_int32), ("n_logged", ctypes.c_int32), ("reserved", ctypes.c_int32),
                 ("t_fail", ctypes.c_double), ("dt_fail", ctypes.c_double)]
+
+
+class PhxSolveDesc(ctypes.Structure):
+    """phx_solve_desc: one solve request of phx_solve (the 8-byte fields first, so there is no padding)."""
+    _fields_ = ([(name, ctypes.c_void_p) for name in (
+                    "packed", "t_host", "y0", "y_out", "y_saved", "grad_y", "adj_y0", "grads", "grid_dt", "grid_steps",
+                    "grid_out_step", "grid_out_slope", "workspace")]
+                + [("workspace_bytes", ctypes.c_size_t), ("status", ctypes.c_void_p), ("steplog", ctypes.c_void_p),
+                   ("rtol", ctypes.c_double), ("atol", ctypes.c_double), ("max_num_steps", ctypes.c_int64)]
+                + [(name, ctypes.c_int32) for name in (
+                    "engine", "adjoint", "G", "H", "B", "N", "T", "t_is_f32", "reversed", "method", "param_mask",
+                    "steplog_cap")])
 
 
 class PhoenixLibraryError(RuntimeError):
@@ -139,24 +148,12 @@ def _declare(lib):
     lib.phx_rows_grad_parts.argtypes = [c_void_p, c_int, c_int, c_int]
     lib.phx_rows_grad_parts.restype = c_int
     lib.phx_unpack_grads.restype = c_int
-    # the *_masked variants: one int param_mask before the stream argument
-    for name in ("phx_solve_adjoint", "phx_solve_adjoint_many", "phx_stream_solve_adjoint", "phx_solve_adjoint_rows",
-                 "phx_unpack_grads"):
-        fn = getattr(lib, name + "_masked")
-        fn.argtypes = getattr(lib, name).argtypes[:-1] + [c_int, c_void_p]
-        fn.restype = c_int
-    # the *_grid variants (fixed-grid solves on a step grid): the forward ones take (grid_dt, grid_steps, grid_out_step,
-    # grid_out_slope), the adjoint ones -- which follow the *_masked argument lists -- (grid_dt, grid_steps) before the stream
+    lib.phx_unpack_grads_masked.argtypes = [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p]
+    lib.phx_unpack_grads_masked.restype = c_int
+    lib.phx_solve.argtypes = [c_void_p, ctypes.POINTER(PhxSolveDesc), c_void_p]
+    lib.phx_solve.restype = c_int
     lib.phx_grid_workspace_bytes.argtypes = [c_int, c_int, c_int64]
     lib.phx_grid_workspace_bytes.restype = c_size_t
-    for name in ("phx_solve_forward", "phx_solve_forward_many", "phx_solve_forward_rows", "phx_stream_solve_forward"):
-        fn = getattr(lib, name + "_grid")
-        fn.argtypes = getattr(lib, name).argtypes[:-1] + [c_void_p] * 4 + [c_void_p]
-        fn.restype = c_int
-    for name in ("phx_solve_adjoint", "phx_solve_adjoint_many", "phx_solve_adjoint_rows", "phx_stream_solve_adjoint"):
-        fn = getattr(lib, name + "_grid")
-        fn.argtypes = getattr(lib, name + "_masked").argtypes[:-1] + [c_void_p] * 2 + [c_void_p]
-        fn.restype = c_int
     lib.phx_prior_loss.argtypes = [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, ctypes.c_float, c_void_p,
                                    c_void_p, c_void_p, c_size_t, c_void_p]
     lib.phx_prior_loss.restype = c_int

@@ -161,7 +161,7 @@ bool check_dims(int G, int H, int B) {
     return true;
 }
 
-// ---- fixed-grid step grids (the *_grid entry points) -----------------------------------------------------------------
+// ---- fixed-grid step grids (phx_solve_desc.grid_*) ------------------------------------------------------------------
 // the grid goes to the workspace right after the solver's own part, 16-byte aligned
 size_t grid_room(size_t need) { return (need + 15) & ~(size_t)15; }
 
@@ -451,12 +451,35 @@ int phx_solve_workspace_init(void* workspace, size_t workspace_bytes, void* stre
     return PHX_OK;
 }
 
-static int solve_common(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                        int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps, int adjoint,
-                        void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                        int steplog_cap, cudaStream_t stream, ResParams* p, ResLaunchPlan* plan, int nprob = 1,
-                        const PhxGridHost* grid = nullptr) {
-    if (!ctx || !check_dims(G, H, B) || !packed || !t_host || !workspace) {
+}  // extern "C"
+
+/* ---- phx_solve: one request per solve, for every engine (include/phoenix_b200.h) ------------------------------------- */
+namespace {
+
+// the combinations of fields some engine takes
+bool check_request(const phx_solve_desc& d) {
+    if (d.engine < PHX_ENGINE_RESIDENT || d.engine > PHX_ENGINE_STREAM) {
+        phx_set_error("unknown engine id %d", d.engine);
+        return false;
+    }
+    const char* why = nullptr;
+    if (d.adjoint && d.reversed) why = "an adjoint solve takes no `reversed`";
+    else if (!d.adjoint && d.param_mask) why = "param_mask is for adjoint solves";
+    else if (d.adjoint && (d.grid_out_step || d.grid_out_slope)) why = "grid_out_step / grid_out_slope are for forward solves";
+    else if (!d.grid_dt && (d.grid_steps || d.grid_out_step || d.grid_out_slope)) why = "a step grid needs grid_dt";
+    else if (d.engine == PHX_ENGINE_STREAM && d.N != 1) why = "the streaming engine solves one problem per call (N = 1)";
+    else if (d.engine == PHX_ENGINE_ROWS && d.B != 1) why = "the rows engine solves one-row problems (B = 1)";
+    else if (d.engine == PHX_ENGINE_RESIDENT && d.N > 1 && (d.reversed || d.steplog))
+        why = "a resident solve of several problems takes no `reversed` and no step log";
+    if (why) phx_set_error("%s (engine %d, adjoint %d, N=%d, B=%d)", why, d.engine, d.adjoint, d.N, d.B);
+    return !why;
+}
+
+// the resident and rows engines: the whole solve in one persistent launch
+int solve_on_chip(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t stream) {
+    const bool rows = d.engine == PHX_ENGINE_ROWS;
+    const int G = d.G, H = d.H, B = d.B, N = d.N, T = d.T, adjoint = d.adjoint ? 1 : 0;
+    if (!ctx || !check_dims(G, H, B) || !d.packed || !d.t_host || !d.workspace || (rows && N < 1)) {
         if (g_err[0] == 0) phx_set_error("null argument");
         return PHX_ERR_INVALID;
     }
@@ -464,118 +487,182 @@ static int solve_common(phx_ctx* ctx, int G, int H, int B, const float* packed, 
         phx_set_error("t must hold at least two time points (got %d)", T);
         return PHX_ERR_INVALID;
     }
-    if (nprob < 1 || (nprob > 1 && nprob * T > PHX_T_INLINE)) {
-        phx_set_error("a multi-problem launch takes 1 <= N and N * T <= %d output times (got N=%d, T=%d)", PHX_T_INLINE,
-                      nprob, T);
+    if (!rows && (N < 1 || (N > 1 && N * T > PHX_T_INLINE))) {
+        phx_set_error("a multi-problem launch takes 1 <= N and N * T <= %d output times (got N=%d, T=%d)", PHX_T_INLINE, N,
+                      T);
         return PHX_ERR_INVALID;
     }
-    for (int q = 0; q < nprob; ++q)
-        for (int i = 1; i < T; ++i) {
-            if (!(t_host[q * T + i] > t_host[q * T + i - 1])) {
+    for (int q = 0; q < N; ++q)
+        for (int i = 1; i < T; ++i)
+            if (!(d.t_host[q * T + i] > d.t_host[q * T + i - 1])) {
                 phx_set_error("t must be strictly increasing at the C boundary (the Python shim negates decreasing t)");
                 return PHX_ERR_INVALID;
             }
-        }
-    if (method < PHX_EULER || method > PHX_DOPRI5) {
-        phx_set_error("unknown method id %d", method);
+    if (d.method < PHX_EULER || d.method > PHX_DOPRI5) {
+        phx_set_error("unknown method id %d", d.method);
         return PHX_ERR_INVALID;
     }
-    if (((uintptr_t)workspace & 15) || ((uintptr_t)packed & 15)) {
-        phx_set_error("workspace and packed weights must be 16-byte aligned");
+    if (((uintptr_t)d.workspace & (rows ? 127 : 15)) || ((uintptr_t)d.packed & 15)) {
+        phx_set_error(rows ? "workspace must be 128-byte and packed weights 16-byte aligned"
+                           : "workspace and packed weights must be 16-byte aligned");
         return PHX_ERR_INVALID;
     }
-    int rc = phx_resident_plan(ctx->num_sms, G, H, B, adjoint, plan);
+    ResLaunchPlan rplan;
+    RowsPlan wplan;
+    int rc = rows ? phx_rows_plan(ctx->num_sms, G, H, adjoint, &wplan)
+                  : phx_resident_plan(ctx->num_sms, G, H, B, adjoint, &rplan);
     if (rc != PHX_OK) return rc;
-    size_t o_t, o_th;
-    size_t need = phx_resident_workspace_floats(G, H, B, T, adjoint, &o_t, &o_th) * sizeof(float);
-    const size_t need_grid = grid ? grid_room(need) + phx_grid_workspace_bytes(nprob, T, grid_steps(*grid, nprob, T, adjoint)) : need;
-    if (workspace_bytes < need_grid) {
-        phx_set_error("solve workspace too small: %zu < %zu", workspace_bytes, need_grid);
+    size_t o_t, o_th;   // o_th: the rows kernels' per-row cotangent buffers, or the resident adjoint's scratch twin
+    const size_t need = (rows ? phx_rows_workspace_floats(G, H, N, T, wplan.rows, adjoint, &o_t, &o_th)
+                              : phx_resident_workspace_floats(G, H, B, T, adjoint, &o_t, &o_th)) * sizeof(float);
+    const PhxGridHost grid{d.grid_dt, d.grid_steps, d.grid_out_step, d.grid_out_slope};
+    const bool gridded = d.grid_dt != nullptr;
+    const size_t need_grid = gridded ? grid_room(need) + phx_grid_workspace_bytes(N, T, grid_steps(grid, N, T, adjoint))
+                                     : need;
+    if (d.workspace_bytes < need_grid) {
+        phx_set_error("%s workspace too small: %zu < %zu", rows ? "rows" : "solve", d.workspace_bytes, need_grid);
         return PHX_ERR_WORKSPACE;
     }
-    float* ws = (float*)workspace;
-    memset(p, 0, sizeof(*p));
-    p->G = G; p->H = H; p->Hp = phx_Hp(H); p->K2 = 2 * p->Hp; p->K2q = p->K2 / 4; p->B = B; p->T = T;
-    p->method = method; p->gpc = plan->gpc; p->t_is_f32 = t_is_f32; p->adjoint = adjoint;
-    p->ring_rows = plan->ring_rows; p->ring_stages = plan->ring_stages;
-    p->so = plan->so;
-    p->rtol_f = (float)rtol; p->atol_f = (float)atol; p->fsign = 1.f;
-    p->max_steps = (long long)max_num_steps;
-    p->w = phx_packed_view(packed, G, H);
-    p->ll = phx_ll_view(workspace);
-    p->t = (const double*)(ws + o_t);
-    p->theta1 = adjoint ? ws + o_th : nullptr;
-    p->status = status; p->steplog = steplog; p->steplog_cap = steplog ? steplog_cap : 0;
-    p->prof = ctx->prof;
-    p->nprob = nprob;
-    if (grid && (rc = phx_grid_stage(*grid, nprob, T, method, !adjoint, (char*)workspace + grid_room(need), stream, p,
-                                     nullptr)) != PHX_OK)
+    float* ws = (float*)d.workspace;
+    ResParams p;
+    memset(&p, 0, sizeof(p));
+    p.G = G; p.H = H; p.Hp = phx_Hp(H); p.K2 = 2 * p.Hp; p.K2q = p.K2 / 4; p.B = B; p.T = T;
+    p.method = d.method; p.t_is_f32 = d.t_is_f32; p.adjoint = adjoint;
+    p.gpc = rows ? wplan.gpc : rplan.gpc;
+    p.ring_rows = rows ? wplan.w1_stride_q : rplan.ring_rows;   // rows kernels: W1 row stride in shared memory (float4)
+    p.ring_stages = rows ? 0 : rplan.ring_stages;
+    p.so = rows ? wplan.so : rplan.so;
+    p.rtol_f = (float)d.rtol; p.atol_f = (float)d.atol; p.fsign = d.reversed ? -1.f : 1.f;
+    p.max_steps = (long long)d.max_num_steps;
+    p.w = phx_packed_view(d.packed, G, H);
+    p.ll = phx_ll_view(d.workspace);
+    p.t = (const double*)(ws + o_t);
+    p.status = d.status; p.steplog = d.steplog; p.steplog_cap = d.steplog ? d.steplog_cap : 0;
+    p.prof = ctx->prof;
+    // problem i reads and writes base + i * stride; the rows engine runs its N problems as the rows of one problem
+    p.nprob = rows ? 1 : N;
+    p.y0_stride = (long long)B * G; p.yout_stride = (long long)T * B * G; p.adj_stride = (long long)B * G;
+    if (rows) {
+        p.rows = wplan.rows; p.ntot = N; p.nqw = wplan.nqw; p.ngg = wplan.ngg; p.gpg = wplan.gpg;
+        p.tm_wa = wplan.tm_wa; p.tm_fac = wplan.tm_fac;
+        p.ppk = (long long)phx_packed_grad_offsets(G, H).total;
+    }
+    if (!adjoint) {
+        p.y0 = d.y0;
+        p.yout = d.y_out;
+    } else {
+        p.ysaved = d.y_saved;
+        p.grad_y = d.grad_y;
+        p.adj_y0 = d.adj_y0;
+        if (rows) {
+            p.theta_ws = ws + o_th;
+            p.gsum = d.grads;
+            p.gsum_acc = 0;
+            p.pmask = d.param_mask;
+        } else {
+            p.theta0 = d.grads;  // written once by the kernel (never read while still zero): no memset needed
+            p.theta1 = ws + o_th;
+            p.theta_stride = (long long)phx_grad_offsets(G, H).total;
+            // A resident grid solve drops PHX_NORM_SEMINORM (a fixed grid uses no norm) where the rows engine passes it
+            // on; both have always done so, and making them agree could change which kernel runs and its bits.
+            p.pmask = gridded ? d.param_mask & PHX_P_ALL : d.param_mask;
+        }
+    }
+    if (gridded && (rc = phx_grid_stage(grid, N, T, d.method, !adjoint, (char*)d.workspace + grid_room(need), stream, &p,
+                                        nullptr)) != PHX_OK)
         return rc;
-    if (T * nprob <= PHX_T_INLINE) {
-        for (int i = 0; i < T * nprob; ++i) p->t_small[i] = t_host[i];  // travels with the kernel parameters
-        return PHX_OK;
+    if ((size_t)T * N <= PHX_T_INLINE) {
+        for (int i = 0; i < T * N; ++i) p.t_small[i] = d.t_host[i];  // travels with the kernel parameters
+    } else {
+        cudaError_t e = cudaMemcpyAsync((void*)p.t, d.t_host, sizeof(double) * T * N, cudaMemcpyHostToDevice, stream);
+        if (e != cudaSuccess) {
+            phx_set_error("cudaMemcpyAsync(t): %s", cudaGetErrorString(e));
+            return PHX_ERR_CUDA;
+        }
     }
-    cudaError_t e = cudaMemcpyAsync((void*)p->t, t_host, sizeof(double) * T, cudaMemcpyHostToDevice, stream);
-    if (e != cudaSuccess) {
-        phx_set_error("cudaMemcpyAsync(t): %s", cudaGetErrorString(e));
-        return PHX_ERR_CUDA;
+    return rows ? phx_rows_launch(p, wplan, stream) : phx_resident_launch(p, rplan, stream);
+}
+
+// the request of one of the entry points that predate phx_solve: a forward solve, or an adjoint one of all six parameters
+phx_solve_desc forward_desc(int engine, int G, int H, int B, int N, const float* packed, const float* y0,
+                            const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol, double atol,
+                            int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
+                            phx_status* status, double* steplog, int steplog_cap) {
+    phx_solve_desc d;
+    memset(&d, 0, sizeof(d));
+    d.engine = engine; d.G = G; d.H = H; d.B = B; d.N = N; d.T = T;
+    d.packed = packed; d.t_host = t_host; d.t_is_f32 = t_is_f32; d.reversed = reversed; d.method = method;
+    d.rtol = rtol; d.atol = atol; d.max_num_steps = max_num_steps;
+    d.y0 = y0; d.y_out = y_out;
+    d.workspace = workspace; d.workspace_bytes = workspace_bytes; d.status = status;
+    d.steplog = steplog; d.steplog_cap = steplog_cap;
+    return d;
+}
+
+phx_solve_desc adjoint_desc(int engine, int G, int H, int B, int N, const float* packed, const double* t_host, int T,
+                            int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads, void* workspace,
+                            size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap) {
+    phx_solve_desc d = forward_desc(engine, G, H, B, N, packed, nullptr, t_host, T, t_is_f32, 0, method, rtol, atol,
+                                    max_num_steps, nullptr, workspace, workspace_bytes, status, steplog, steplog_cap);
+    d.adjoint = 1;
+    d.y_saved = y_saved; d.grad_y = grad_y; d.adj_y0 = adj_y0; d.grads = grads;
+    d.param_mask = PHX_P_ALL;
+    return d;
+}
+
+}  // namespace
+
+extern "C" {
+
+int phx_solve(phx_ctx* ctx, const phx_solve_desc* desc, void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    g_err[0] = 0;
+    if (!desc) {
+        phx_set_error("null solve request");
+        return PHX_ERR_INVALID;
     }
-    return PHX_OK;
+    const phx_solve_desc& d = *desc;
+    if (!check_request(d)) return PHX_ERR_INVALID;
+    const bool rows = d.engine == PHX_ENGINE_ROWS;
+    if (d.adjoint) {
+        if (!check_adjoint_mask(d.param_mask)) return PHX_ERR_INVALID;
+        if (!d.y_saved || !d.grad_y || !d.adj_y0 || !d.grads) {
+            phx_set_error(rows ? "null y_saved / grad_y / adj_y0 / grads_packed_parts"
+                               : "null y_saved / grad_y / adj_y0 / grads_flat");
+            return PHX_ERR_INVALID;
+        }
+        if (rows && ((uintptr_t)d.grads & 15)) {
+            phx_set_error("grads_packed_parts must be 16-byte aligned");
+            return PHX_ERR_INVALID;
+        }
+    } else if (!d.y0 || !d.y_out) {
+        phx_set_error("null y0 / y_out");
+        return PHX_ERR_INVALID;
+    }
+    if (d.engine == PHX_ENGINE_STREAM)
+        return d.adjoint ? phx_stream_adjoint(ctx, d, (cudaStream_t)stream) : phx_stream_forward(ctx, d, (cudaStream_t)stream);
+    return solve_on_chip(ctx, d, (cudaStream_t)stream);
 }
 
 int phx_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
                       const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol, double atol,
                       int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
                       phx_status* status, double* steplog, int steplog_cap, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!y0 || !y_out) {
-        phx_set_error("null y0 / y_out");
-        return PHX_ERR_INVALID;
-    }
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
-                          workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan);
-    if (rc != PHX_OK) return rc;
-    p.y0 = y0;
-    p.yout = y_out;
-    p.fsign = reversed ? -1.f : 1.f;
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+    const phx_solve_desc d = forward_desc(PHX_ENGINE_RESIDENT, G, H, B, 1, packed, y0, t_host, T, t_is_f32, reversed, method,
+                                          rtol, atol, max_num_steps, y_out, workspace, workspace_bytes, status, steplog,
+                                          steplog_cap);
+    return phx_solve(ctx, &d, stream);
 }
 
 int phx_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
                       int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                       const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat, void* workspace,
                       size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap, void* stream) {
-    return phx_solve_adjoint_masked(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, y_saved,
-                                    grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status, steplog, steplog_cap,
-                                    PHX_P_ALL, stream);
-}
-
-int phx_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                             int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                             const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat, void* workspace,
-                             size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
-                             int param_mask, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
-    if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
-        phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
-        return PHX_ERR_INVALID;
-    }
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
-                          workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan);
-    if (rc != PHX_OK) return rc;
-    p.ysaved = y_saved;
-    p.grad_y = grad_y;
-    p.adj_y0 = adj_y0;
-    p.theta0 = grads_flat;  // written once by the kernel (never read while still zero): no memset needed
-    p.pmask = param_mask;
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+    const phx_solve_desc d = adjoint_desc(PHX_ENGINE_RESIDENT, G, H, B, 1, packed, t_host, T, t_is_f32, method, rtol, atol,
+                                          max_num_steps, y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes,
+                                          status, steplog, steplog_cap);
+    return phx_solve(ctx, &d, stream);
 }
 
 /* ---- several independent problems per launch (SURVEY.md section 8 f1) -------------------------------------------- */
@@ -583,132 +670,44 @@ int phx_solve_forward_many(phx_ctx* ctx, int G, int H, int B, int N, const float
                            const double* t_host, int T, int t_is_f32, int method, double rtol, double atol,
                            int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
                            phx_status* status, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!y0 || !y_out) {
-        phx_set_error("null y0 / y_out");
-        return PHX_ERR_INVALID;
-    }
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
-                          workspace_bytes, status, nullptr, 0, (cudaStream_t)stream, &p, &plan, N);
-    if (rc != PHX_OK) return rc;
-    p.y0 = y0;
-    p.yout = y_out;
-    p.y0_stride = (long long)B * G;
-    p.yout_stride = (long long)T * B * G;
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+    const phx_solve_desc d = forward_desc(PHX_ENGINE_RESIDENT, G, H, B, N, packed, y0, t_host, T, t_is_f32, 0, method, rtol,
+                                          atol, max_num_steps, y_out, workspace, workspace_bytes, status, nullptr, 0);
+    return phx_solve(ctx, &d, stream);
 }
 
 int phx_solve_adjoint_many(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host, int T,
                            int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
                            const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
                            void* workspace, size_t workspace_bytes, phx_status* status, void* stream) {
-    return phx_solve_adjoint_many_masked(ctx, G, H, B, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
-                                         y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status, PHX_P_ALL,
-                                         stream);
+    const phx_solve_desc d = adjoint_desc(PHX_ENGINE_RESIDENT, G, H, B, N, packed, t_host, T, t_is_f32, method, rtol, atol,
+                                          max_num_steps, y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes,
+                                          status, nullptr, 0);
+    return phx_solve(ctx, &d, stream);
 }
 
-int phx_solve_adjoint_many_masked(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host,
-                                  int T, int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                  void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
-                                  void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
-    if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
-        phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
-        return PHX_ERR_INVALID;
-    }
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
-                          workspace_bytes, status, nullptr, 0, (cudaStream_t)stream, &p, &plan, N);
-    if (rc != PHX_OK) return rc;
-    p.ysaved = y_saved;
-    p.grad_y = grad_y;
-    p.adj_y0 = adj_y0;
-    p.theta0 = grads_flat;
-    p.yout_stride = (long long)T * B * G;
-    p.adj_stride = (long long)B * G;
-    p.theta_stride = (long long)phx_grad_offsets(G, H).total;
-    p.pmask = param_mask;
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
+/* ---- the streaming engine (phx_stream.cu) ------------------------------------------------------------------------- */
+int phx_stream_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
+                             const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
+                             double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
+                             phx_status* status, double* steplog, int steplog_cap, void* stream) {
+    const phx_solve_desc d = forward_desc(PHX_ENGINE_STREAM, G, H, B, 1, packed, y0, t_host, T, t_is_f32, reversed, method,
+                                          rtol, atol, max_num_steps, y_out, workspace, workspace_bytes, status, steplog,
+                                          steplog_cap);
+    return phx_solve(ctx, &d, stream);
 }
 
+int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
+                             int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                             const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
+                             void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                             int steplog_cap, void* stream) {
+    const phx_solve_desc d = adjoint_desc(PHX_ENGINE_STREAM, G, H, B, 1, packed, t_host, T, t_is_f32, method, rtol, atol,
+                                          max_num_steps, y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes,
+                                          status, steplog, steplog_cap);
+    return phx_solve(ctx, &d, stream);
+}
 
 /* ---- rows kernels: N independent one-row problems in lock-step (phx_rows.cuh) ------------------------------------------- */
-static int rows_common(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T, int t_is_f32,
-                       int method, double rtol, double atol, int64_t max_num_steps, int adjoint, void* workspace,
-                       size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap, cudaStream_t stream,
-                       ResParams* p, RowsPlan* plan, size_t* off_theta, const PhxGridHost* grid = nullptr) {
-    if (!ctx || !check_dims(G, H, 1) || !packed || !t_host || !workspace || N < 1) {
-        if (g_err[0] == 0) phx_set_error("null argument");
-        return PHX_ERR_INVALID;
-    }
-    if (T < 2) {
-        phx_set_error("t must hold at least two time points (got %d)", T);
-        return PHX_ERR_INVALID;
-    }
-    for (int q = 0; q < N; ++q)
-        for (int i = 1; i < T; ++i)
-            if (!(t_host[q * T + i] > t_host[q * T + i - 1])) {
-                phx_set_error("t must be strictly increasing at the C boundary (the Python shim negates decreasing t)");
-                return PHX_ERR_INVALID;
-            }
-    if (method < PHX_EULER || method > PHX_DOPRI5) {
-        phx_set_error("unknown method id %d", method);
-        return PHX_ERR_INVALID;
-    }
-    if (((uintptr_t)workspace & 127) || ((uintptr_t)packed & 15)) {
-        phx_set_error("workspace must be 128-byte and packed weights 16-byte aligned");
-        return PHX_ERR_INVALID;
-    }
-    int rc = phx_rows_plan(ctx->num_sms, G, H, adjoint, plan);
-    if (rc != PHX_OK) return rc;
-    size_t o_t;
-    const size_t need = phx_rows_workspace_floats(G, H, N, T, plan->rows, adjoint, &o_t, off_theta) * sizeof(float);
-    const size_t need_grid = grid ? grid_room(need) + phx_grid_workspace_bytes(N, T, grid_steps(*grid, N, T, adjoint)) : need;
-    if (workspace_bytes < need_grid) {
-        phx_set_error("rows workspace too small: %zu < %zu", workspace_bytes, need_grid);
-        return PHX_ERR_WORKSPACE;
-    }
-    float* ws = (float*)workspace;
-    memset(p, 0, sizeof(*p));
-    p->G = G; p->H = H; p->Hp = phx_Hp(H); p->K2 = 2 * p->Hp; p->K2q = p->K2 / 4; p->B = 1; p->T = T;
-    p->method = method; p->gpc = plan->gpc; p->t_is_f32 = t_is_f32; p->adjoint = adjoint;
-    p->ring_rows = plan->w1_stride_q;   // rows kernels: W1 row stride in shared memory (float4 units)
-    p->ring_stages = 0;
-    p->so = plan->so;
-    p->rtol_f = (float)rtol; p->atol_f = (float)atol; p->fsign = 1.f;
-    p->max_steps = (long long)max_num_steps;
-    p->w = phx_packed_view(packed, G, H);
-    p->ll = phx_ll_view(workspace);
-    p->t = (const double*)(ws + o_t);
-    p->status = status; p->steplog = steplog; p->steplog_cap = steplog ? steplog_cap : 0;
-    p->prof = ctx->prof;
-    p->nprob = 1;
-    p->rows = plan->rows; p->ntot = N; p->nqw = plan->nqw; p->ngg = plan->ngg; p->gpg = plan->gpg;
-    p->tm_wa = plan->tm_wa; p->tm_fac = plan->tm_fac;
-    p->y0_stride = G; p->yout_stride = (long long)T * G; p->adj_stride = G;
-    p->ppk = (long long)phx_packed_grad_offsets(G, H).total;
-    if (grid && (rc = phx_grid_stage(*grid, N, T, method, !adjoint, (char*)workspace + grid_room(need), stream, p,
-                                     nullptr)) != PHX_OK)
-        return rc;
-    if ((size_t)T * N <= PHX_T_INLINE) {
-        for (int i = 0; i < T * N; ++i) p->t_small[i] = t_host[i];
-        return PHX_OK;
-    }
-    cudaError_t e = cudaMemcpyAsync((void*)p->t, t_host, sizeof(double) * T * N, cudaMemcpyHostToDevice, stream);
-    if (e != cudaSuccess) {
-        phx_set_error("cudaMemcpyAsync(t): %s", cudaGetErrorString(e));
-        return PHX_ERR_CUDA;
-    }
-    return PHX_OK;
-}
-
 int phx_rows_supported(const phx_ctx* ctx, int G, int H, int adjoint) {
     if (!ctx) return 0;
     RowsPlan plan;
@@ -738,21 +737,21 @@ int phx_solve_forward_rows(phx_ctx* ctx, int G, int H, int N, const float* packe
                            int T, int t_is_f32, int reversed, int method, double rtol, double atol, int64_t max_num_steps,
                            float* y_out, void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
                            int steplog_cap, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!y0 || !y_out) {
-        phx_set_error("null y0 / y_out");
-        return PHX_ERR_INVALID;
-    }
-    ResParams p;
-    RowsPlan plan;
-    int rc = rows_common(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
-                         workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, nullptr);
-    if (rc != PHX_OK) return rc;
-    p.y0 = y0;
-    p.yout = y_out;
-    p.fsign = reversed ? -1.f : 1.f;
-    return phx_rows_launch(p, plan, (cudaStream_t)stream);
+    const phx_solve_desc d = forward_desc(PHX_ENGINE_ROWS, G, H, 1, N, packed, y0, t_host, T, t_is_f32, reversed, method,
+                                          rtol, atol, max_num_steps, y_out, workspace, workspace_bytes, status, steplog,
+                                          steplog_cap);
+    return phx_solve(ctx, &d, stream);
+}
+
+int phx_solve_adjoint_rows(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
+                           int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
+                           const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
+                           void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
+                           int steplog_cap, void* stream) {
+    const phx_solve_desc d = adjoint_desc(PHX_ENGINE_ROWS, G, H, 1, N, packed, t_host, T, t_is_f32, method, rtol, atol,
+                                          max_num_steps, y_saved, grad_y, adj_y0, grads_packed_parts, workspace,
+                                          workspace_bytes, status, steplog, steplog_cap);
+    return phx_solve(ctx, &d, stream);
 }
 
 int phx_rows_grad_parts(const phx_ctx* ctx, int G, int H, int N) {
@@ -811,214 +810,12 @@ int phx_mse_grad(phx_ctx* ctx, int rows, int G, const float* pred, size_t pred_s
     return PHX_OK;
 }
 
-int phx_solve_adjoint_rows(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
-                           int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                           const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
-                           void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                           int steplog_cap, void* stream) {
-    return phx_solve_adjoint_rows_masked(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
-                                         y_saved, grad_y, adj_y0, grads_packed_parts, workspace, workspace_bytes, status,
-                                         steplog, steplog_cap, PHX_P_ALL, stream);
-}
-
-int phx_solve_adjoint_rows_masked(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
-                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
-                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                  int steplog_cap, int param_mask, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
-    if (!y_saved || !grad_y || !adj_y0 || !grads_packed_parts) {
-        phx_set_error("null y_saved / grad_y / adj_y0 / grads_packed_parts");
-        return PHX_ERR_INVALID;
-    }
-    if ((uintptr_t)grads_packed_parts & 15) {
-        phx_set_error("grads_packed_parts must be 16-byte aligned");
-        return PHX_ERR_INVALID;
-    }
-    ResParams p;
-    RowsPlan plan;
-    size_t o_th = 0;
-    int rc = rows_common(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
-                         workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, &o_th);
-    if (rc != PHX_OK) return rc;
-    p.ysaved = y_saved;
-    p.grad_y = grad_y;
-    p.adj_y0 = adj_y0;
-    p.theta_ws = (float*)workspace + o_th;
-    p.gsum = grads_packed_parts;
-    p.gsum_acc = 0;
-    p.pmask = param_mask;
-    return phx_rows_launch(p, plan, (cudaStream_t)stream);
-}
-
 
 /* ---- fixed-grid solves on the caller's step grid (options=dict(step_size=...), solvers.py:48-50, 77-103) ---------------- */
 size_t phx_grid_workspace_bytes(int N, int T, int64_t total_steps) {
     if (N < 1 || T < 2 || total_steps < 0) return 0;
     const size_t nseg = (size_t)N * (T - 1);
     return 4 * (((size_t)total_steps + 3) / 4 * 4 + (nseg + 4) / 4 * 4 + 2 * ((nseg + 3) / 4 * 4)) + 16;
-}
-
-int phx_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0, const double* t_host,
-                           int T, int t_is_f32, int reversed, int method, double rtol, double atol, int64_t max_num_steps,
-                           float* y_out, void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                           int steplog_cap, const float* grid_dt, const int32_t* grid_steps_, const int32_t* grid_out_step,
-                           const float* grid_out_slope, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!y0 || !y_out) {
-        phx_set_error("null y0 / y_out");
-        return PHX_ERR_INVALID;
-    }
-    const PhxGridHost grid{grid_dt, grid_steps_, grid_out_step, grid_out_slope};
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
-                          workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, 1, &grid);
-    if (rc != PHX_OK) return rc;
-    p.y0 = y0;
-    p.yout = y_out;
-    p.fsign = reversed ? -1.f : 1.f;
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
-}
-
-int phx_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                           int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                           const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat, void* workspace,
-                           size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap, int param_mask,
-                           const float* grid_dt, const int32_t* grid_steps_, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
-    if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
-        phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
-        return PHX_ERR_INVALID;
-    }
-    const PhxGridHost grid{grid_dt, grid_steps_, nullptr, nullptr};
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
-                          workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, 1, &grid);
-    if (rc != PHX_OK) return rc;
-    p.ysaved = y_saved;
-    p.grad_y = grad_y;
-    p.adj_y0 = adj_y0;
-    p.theta0 = grads_flat;
-    p.pmask = param_mask & PHX_P_ALL;   // (a fixed grid uses no norm)
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
-}
-
-int phx_solve_forward_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const float* y0,
-                                const double* t_host, int T, int t_is_f32, int method, double rtol, double atol,
-                                int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
-                                phx_status* status, const float* grid_dt, const int32_t* grid_steps_,
-                                const int32_t* grid_out_step, const float* grid_out_slope, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!y0 || !y_out) {
-        phx_set_error("null y0 / y_out");
-        return PHX_ERR_INVALID;
-    }
-    const PhxGridHost grid{grid_dt, grid_steps_, grid_out_step, grid_out_slope};
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
-                          workspace_bytes, status, nullptr, 0, (cudaStream_t)stream, &p, &plan, N, &grid);
-    if (rc != PHX_OK) return rc;
-    p.y0 = y0;
-    p.yout = y_out;
-    p.y0_stride = (long long)B * G;
-    p.yout_stride = (long long)T * B * G;
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
-}
-
-int phx_solve_adjoint_many_grid(phx_ctx* ctx, int G, int H, int B, int N, const float* packed, const double* t_host, int T,
-                                int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                void* workspace, size_t workspace_bytes, phx_status* status, int param_mask,
-                                const float* grid_dt, const int32_t* grid_steps_, void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
-    if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
-        phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
-        return PHX_ERR_INVALID;
-    }
-    const PhxGridHost grid{grid_dt, grid_steps_, nullptr, nullptr};
-    ResParams p;
-    ResLaunchPlan plan;
-    int rc = solve_common(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
-                          workspace_bytes, status, nullptr, 0, (cudaStream_t)stream, &p, &plan, N, &grid);
-    if (rc != PHX_OK) return rc;
-    p.ysaved = y_saved;
-    p.grad_y = grad_y;
-    p.adj_y0 = adj_y0;
-    p.theta0 = grads_flat;
-    p.yout_stride = (long long)T * B * G;
-    p.adj_stride = (long long)B * G;
-    p.theta_stride = (long long)phx_grad_offsets(G, H).total;
-    p.pmask = param_mask & PHX_P_ALL;   // (a fixed grid uses no norm)
-    return phx_resident_launch(p, plan, (cudaStream_t)stream);
-}
-
-int phx_solve_forward_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const float* y0,
-                                const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
-                                double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
-                                phx_status* status, double* steplog, int steplog_cap, const float* grid_dt,
-                                const int32_t* grid_steps_, const int32_t* grid_out_step, const float* grid_out_slope,
-                                void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!y0 || !y_out) {
-        phx_set_error("null y0 / y_out");
-        return PHX_ERR_INVALID;
-    }
-    const PhxGridHost grid{grid_dt, grid_steps_, grid_out_step, grid_out_slope};
-    ResParams p;
-    RowsPlan plan;
-    int rc = rows_common(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
-                         workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, nullptr, &grid);
-    if (rc != PHX_OK) return rc;
-    p.y0 = y0;
-    p.yout = y_out;
-    p.fsign = reversed ? -1.f : 1.f;
-    return phx_rows_launch(p, plan, (cudaStream_t)stream);
-}
-
-int phx_solve_adjoint_rows_grid(phx_ctx* ctx, int G, int H, int N, const float* packed, const double* t_host, int T,
-                                int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                const float* y_saved, const float* grad_y, float* adj_y0, float* grads_packed_parts,
-                                void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps_,
-                                void* stream) {
-    PhxDevGuard dev_guard(ctx);
-    g_err[0] = 0;
-    if (!check_adjoint_mask(param_mask)) return PHX_ERR_INVALID;
-    if (!y_saved || !grad_y || !adj_y0 || !grads_packed_parts) {
-        phx_set_error("null y_saved / grad_y / adj_y0 / grads_packed_parts");
-        return PHX_ERR_INVALID;
-    }
-    if ((uintptr_t)grads_packed_parts & 15) {
-        phx_set_error("grads_packed_parts must be 16-byte aligned");
-        return PHX_ERR_INVALID;
-    }
-    const PhxGridHost grid{grid_dt, grid_steps_, nullptr, nullptr};
-    ResParams p;
-    RowsPlan plan;
-    size_t o_th = 0;
-    int rc = rows_common(ctx, G, H, N, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
-                         workspace_bytes, status, steplog, steplog_cap, (cudaStream_t)stream, &p, &plan, &o_th, &grid);
-    if (rc != PHX_OK) return rc;
-    p.ysaved = y_saved;
-    p.grad_y = grad_y;
-    p.adj_y0 = adj_y0;
-    p.theta_ws = (float*)workspace + o_th;
-    p.gsum = grads_packed_parts;
-    p.gsum_acc = 0;
-    p.pmask = param_mask;
-    return phx_rows_launch(p, plan, (cudaStream_t)stream);
 }
 
 }  // extern "C"

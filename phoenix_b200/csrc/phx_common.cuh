@@ -259,7 +259,7 @@ struct ResParams {
     float* adj_y0;         // [B][G]
     float* theta0;         // [P] caller's flat grads (result lands here)
     float* theta1;         // [P] scratch twin
-    // several independent problems per launch (phx_solve_*_many): problem i reads / writes base + i * stride (floats),
+    // several independent problems per launch (phx_solve with N > 1): problem i reads / writes base + i * stride (floats),
     // its output times are t_small[i*T .. i*T+T) and its status record is status[i]; nprob == 1 for the plain calls
     int nprob;
     long long y0_stride, yout_stride, adj_stride, theta_stride;
@@ -277,7 +277,7 @@ struct ResParams {
     int gsum_acc;          // != 0: add to gsum instead of overwriting it
     long long ppk;
     int pmask;             // adjoint: parameters whose cotangents are integrated (PHX_P_*)
-    // fixed-grid solves on the caller's step grid (the *_grid entry points, options=dict(step_size=...)); gdt == nullptr:
+    // fixed-grid solves on the caller's step grid (phx_solve_desc.grid_*, options=dict(step_size=...)); gdt == nullptr:
     // one step per output interval.  Segment q (forward: problem q; adjoint: interval iv of problem pi, q = pi*(T-1)+iv-1)
     // takes the steps gdt[goff[q] .. goff[q+1]).  Forward output j >= 1 of problem pi is written in step
     // gout[pi*(T-1)+j-1] of its problem, as y + gsl[...] * (y1 - y), or as y1 itself when gsl[...] < 0
@@ -371,7 +371,7 @@ int phx_resident_plan(int num_sms, int G, int H, int B, int adjoint, ResLaunchPl
 size_t phx_resident_workspace_floats(int G, int H, int B, int T, int adjoint, size_t* off_t, size_t* off_theta1);
 int phx_resident_launch(const ResParams& p, const ResLaunchPlan& plan, cudaStream_t stream);
 
-// A fixed-grid solve's step grid as the *_grid entry points take it (include/phoenix_b200.h): nseg segments (forward: the
+// A fixed-grid solve's step grid as phx_solve takes it (include/phoenix_b200.h): nseg segments (forward: the
 // N problems; adjoint: the N * (T-1) intervals, problem-major), steps[q] >= 1 steps each, their dt back to back; forward
 // only: out_step / out_slope [N][T-1], the step of each output time j >= 1 and its slope (< 0: exact hit, take y1).
 struct PhxGridHost {
@@ -385,6 +385,10 @@ struct PhxGridHost {
 // offsets into dt (nseg + 1 entries).
 int phx_grid_stage(const PhxGridHost& g, int N, int T, int method, int forward, void* room, cudaStream_t stream,
                    ResParams* p, std::vector<int>* off);
+// the streaming engine's solves (phx_stream.cu), called by phx_solve once it has checked the request's combination of
+// fields, its param_mask and its y0 / y_out or adjoint pointers
+int phx_stream_forward(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t stream);
+int phx_stream_adjoint(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t stream);
 
 // ---- RK stage algebra fused into the RHS (streaming solvers, forward solves on the tensor-core path) ------------------
 // With k = the stage derivative a forward RHS launch produces, the epilogue of the joint contraction also writes

@@ -670,25 +670,19 @@ size_t phx_stream_workspace_bytes(const phx_ctx* ctx, int G, int H, int B, int T
 
 }  // extern "C"
 
-namespace {
-
-int stream_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0, const double* t_host, int T,
-                   int t_is_f32, int reversed, int method, double rtol, double atol, int64_t max_num_steps, float* y_out,
-                   void* workspace, size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
-                   const PhxGridHost* grid, void* stream) {
-    PhxDevGuard dev_guard(ctx);
+int phx_stream_forward(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t st) {
+    const int G = d.G, H = d.H, B = d.B, T = d.T, method = d.method;
+    const double* t_host = d.t_host;
+    float* y_out = d.y_out;
     Stream S;
     float* base;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!y0 || !y_out) {
-        phx_set_error("null y0 / y_out");
-        return PHX_ERR_INVALID;
-    }
+    const PhxGridHost g{d.grid_dt, d.grid_steps, d.grid_out_step, d.grid_out_slope};
+    const PhxGridHost* grid = d.grid_dt ? &g : nullptr;
     if (grid && phx_grid_stage(*grid, 1, T, method, 1, nullptr, st, nullptr, nullptr) != PHX_OK) return PHX_ERR_INVALID;
-    int rc = setup(S, ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 0, workspace,
-                   workspace_bytes, steplog, steplog_cap, st, &base);
+    int rc = setup(S, ctx, G, H, B, d.packed, t_host, T, d.t_is_f32, method, d.rtol, d.atol, d.max_num_steps, 0,
+                   d.workspace, d.workspace_bytes, d.steplog, d.steplog_cap, st, &base);
     if (rc != PHX_OK) return rc;
-    S.fsign = reversed ? -1.f : 1.f;
+    S.fsign = d.reversed ? -1.f : 1.f;
     {
         // OFF unless PHX_STREAM_FUSE=1: measured slower at every shape (tools/stream_fuse_ab.py,
         // profiles/r04d_stream_fuse_ab.txt -- 60 rows x 11 165 genes rk4 0.40 ms fused / 0.34 ms not; 4 096 x 20 000:
@@ -706,7 +700,7 @@ int stream_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const
     y.x0 = base; y.x1 = base + BG; y.xs = base + 2 * BG;
     for (int i = 0; i < 7; ++i) y.k[i] = base + (3 + i) * BG;
     S.segs.push_back(y);
-    cudaMemcpyAsync(y_out, y0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
+    cudaMemcpyAsync(y_out, d.y0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
     if (method != PHX_DOPRI5 && grid) {
         // the caller's grid: a step that ends on an output time writes that output slice, the others a scratch slot
         // (x0 / x1, never the step's own input); output times inside the step are interpolated between the two
@@ -728,9 +722,9 @@ int stream_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const
     } else if (method != PHX_DOPRI5) {
         // fixed grid: the state of interval i is read from the output slice i and written to slice i + 1
         S.segs[0].x0 = y_out;
-        for (int i = 0; i + 1 < T && rc == PHX_OK; ++i) rc = S.fixed_step(fixed_dt(t_host, i, t_is_f32), y_out + (size_t)(i + 1) * BG);
+        for (int i = 0; i + 1 < T && rc == PHX_OK; ++i) rc = S.fixed_step(fixed_dt(t_host, i, d.t_is_f32), y_out + (size_t)(i + 1) * BG);
     } else {
-        cudaMemcpyAsync(y.x0, y0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
+        cudaMemcpyAsync(y.x0, d.y0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
         rc = S.dopri5(t_host[0], t_host + 1, T - 1,
                       [&](int j, const float* xs, const int* sl, float dtf, const float* cmid) {
                           S.interp_seg(0, y_out + (size_t)(j + 1) * BG, xs, sl, dtf, cmid);
@@ -742,78 +736,22 @@ int stream_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const
         phx_set_error("stream forward: %s", cudaGetErrorString(e));
         return PHX_ERR_CUDA;
     }
-    write_back(S, status);
+    write_back(S, d.status);
     return PHX_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int phx_stream_solve_forward(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
-                             const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
-                             double atol, int64_t max_num_steps, float* y_out, void* workspace, size_t workspace_bytes,
-                             phx_status* status, double* steplog, int steplog_cap, void* stream) {
-    return stream_forward(ctx, G, H, B, packed, y0, t_host, T, t_is_f32, reversed, method, rtol, atol, max_num_steps,
-                          y_out, workspace, workspace_bytes, status, steplog, steplog_cap, nullptr, stream);
-}
-
-int phx_stream_solve_forward_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const float* y0,
-                                  const double* t_host, int T, int t_is_f32, int reversed, int method, double rtol,
-                                  double atol, int64_t max_num_steps, float* y_out, void* workspace,
-                                  size_t workspace_bytes, phx_status* status, double* steplog, int steplog_cap,
-                                  const float* grid_dt, const int32_t* grid_steps, const int32_t* grid_out_step,
-                                  const float* grid_out_slope, void* stream) {
-    const PhxGridHost grid{grid_dt, grid_steps, grid_out_step, grid_out_slope};
-    return stream_forward(ctx, G, H, B, packed, y0, t_host, T, t_is_f32, reversed, method, rtol, atol, max_num_steps,
-                          y_out, workspace, workspace_bytes, status, steplog, steplog_cap, &grid, stream);
-}
-
-int phx_stream_solve_adjoint(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                             int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                             const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                             void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                             int steplog_cap, void* stream) {
-    return phx_stream_solve_adjoint_masked(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
-                                           y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status,
-                                           steplog, steplog_cap, PHX_P_ALL, stream);
-}
-
-int phx_stream_solve_adjoint_masked(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                                    int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                    const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                    void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                    int steplog_cap, int param_mask, void* stream) {
-    return phx_stream_solve_adjoint_grid(ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps,
-                                         y_saved, grad_y, adj_y0, grads_flat, workspace, workspace_bytes, status, steplog,
-                                         steplog_cap, param_mask, nullptr, nullptr, stream);
-}
-
-// grid_dt == nullptr: one step per interval (the entry points above)
-int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float* packed, const double* t_host, int T,
-                                  int t_is_f32, int method, double rtol, double atol, int64_t max_num_steps,
-                                  const float* y_saved, const float* grad_y, float* adj_y0, float* grads_flat,
-                                  void* workspace, size_t workspace_bytes, phx_status* status, double* steplog,
-                                  int steplog_cap, int param_mask, const float* grid_dt, const int32_t* grid_steps,
-                                  void* stream) {
-    PhxDevGuard dev_guard(ctx);
+int phx_stream_adjoint(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t st) {
+    const int G = d.G, H = d.H, B = d.B, T = d.T, method = d.method, param_mask = d.param_mask;
+    const double* t_host = d.t_host;
+    const float *y_saved = d.y_saved, *grad_y = d.grad_y, *grid_dt = d.grid_dt;
+    float* grads_flat = d.grads;
     Stream S;
     float* base;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (param_mask < 0 || param_mask > (PHX_P_ALL | PHX_NORM_SEMINORM)) {
-        phx_set_error("param_mask must be a 6-bit mask, optionally with PHX_NORM_SEMINORM (0 .. 0x7F), got %d",
-                      param_mask);
-        return PHX_ERR_INVALID;
-    }
-    if (!y_saved || !grad_y || !adj_y0 || !grads_flat) {
-        phx_set_error("null y_saved / grad_y / adj_y0 / grads_flat");
-        return PHX_ERR_INVALID;
-    }
     std::vector<int> goff;   // the grid's interval offsets into grid_dt
-    const PhxGridHost grid{grid_dt, grid_steps, nullptr, nullptr};
+    const PhxGridHost grid{grid_dt, d.grid_steps, nullptr, nullptr};
     if (grid_dt && phx_grid_stage(grid, 1, T, method, 0, nullptr, st, nullptr, &goff) != PHX_OK) return PHX_ERR_INVALID;
-    int rc = setup(S, ctx, G, H, B, packed, t_host, T, t_is_f32, method, rtol, atol, max_num_steps, 1, workspace,
-                   workspace_bytes, steplog, steplog_cap, st, &base);
+    int rc = setup(S, ctx, G, H, B, d.packed, t_host, T, d.t_is_f32, method, d.rtol, d.atol, d.max_num_steps, 1,
+                   d.workspace, d.workspace_bytes, d.steplog, d.steplog_cap, st, &base);
     if (rc != PHX_OK) return rc;
     const size_t BG = (size_t)B * G, P = phx_grad_offsets(G, H).total;
     // the theta segment holds the adjoint parameters' cotangents only, back to back in reference order (all six: the
@@ -831,7 +769,7 @@ int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float
     a.x0 = ab; a.x1 = ab + BG; a.xs = ab + 2 * BG;
     for (int i = 0; i < 7; ++i) a.k[i] = ab + (3 + i) * BG;
     float* tb = ab + 10 * BG;
-    tb += (4 - ((size_t)(tb - (float*)workspace) & 3)) & 3;
+    tb += (4 - ((size_t)(tb - (float*)d.workspace) & 3)) & 3;
     th.n = PS; th.count = (double)PS;
     th.in_norm = !(param_mask & PHX_NORM_SEMINORM);
     th.x0 = grads_flat; th.x1 = tb; th.xs = nullptr;
@@ -846,7 +784,7 @@ int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float
         if (method != PHX_DOPRI5 && grid_dt) {
             for (int k = goff[iv - 1]; k < goff[iv] && rc == PHX_OK; ++k) rc = S.fixed_step(grid_dt[k]);
         } else if (method != PHX_DOPRI5) {
-            rc = S.fixed_step(fixed_dt(t_host, iv - 1, t_is_f32));
+            rc = S.fixed_step(fixed_dt(t_host, iv - 1, d.t_is_f32));
         } else {
             double t_end = -t_host[iv - 1];
             rc = S.dopri5(-t_host[iv], &t_end, 1,
@@ -863,7 +801,7 @@ int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float
         add_kernel<<<nblk(BG), EB, 0, st>>>(as.x0, grad_y + (size_t)(iv - 1) * BG, BG);
     }
     if (rc != PHX_OK) return rc;
-    cudaMemcpyAsync(adj_y0, S.segs[1].x0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
+    cudaMemcpyAsync(d.adj_y0, S.segs[1].x0, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
     if (pm == PHX_P_ALL) {
         if (S.segs[2].x0 != grads_flat)
             cudaMemcpyAsync(grads_flat, S.segs[2].x0, P * sizeof(float), cudaMemcpyDeviceToDevice, st);
@@ -891,8 +829,6 @@ int phx_stream_solve_adjoint_grid(phx_ctx* ctx, int G, int H, int B, const float
         phx_set_error("stream adjoint: %s", cudaGetErrorString(e));
         return PHX_ERR_CUDA;
     }
-    write_back(S, status);
+    write_back(S, d.status);
     return PHX_OK;
 }
-
-}  // extern "C"

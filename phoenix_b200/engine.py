@@ -503,7 +503,7 @@ def adjoint_grid(t_list, t_is_f32, step_size):
 
 
 class _Grid:
-    """Step grids of consecutive problems as the *_grid entry points take them (host arrays, kept alive here)."""
+    """Step grids of consecutive problems as phx_solve takes them (host arrays, kept alive here)."""
 
     def __init__(self, parts, forward):
         self.forward = forward
@@ -515,11 +515,11 @@ class _Grid:
         else:
             self.steps = torch.tensor([n for q in parts for n in q[1]], dtype=torch.int32)
 
-    def args(self):
-        a = [ctypes.c_void_p(self.dt.data_ptr()), ctypes.c_void_p(self.steps.data_ptr())]
+    def put(self, d):
+        """Point the grid fields of the request ``d`` at these arrays."""
+        d.grid_dt, d.grid_steps = self.dt.data_ptr(), self.steps.data_ptr()
         if self.forward:
-            a += [ctypes.c_void_p(self.out_step.data_ptr()), ctypes.c_void_p(self.out_slope.data_ptr())]
-        return a
+            d.grid_out_step, d.grid_out_slope = self.out_step.data_ptr(), self.out_slope.data_ptr()
 
     def nbytes(self, lib, N, T):
         """Workspace room for the grid behind the solver's own part (16-byte alignment included)."""
@@ -532,6 +532,28 @@ def _grids(t_rows, t_is_f32, step_size, forward):
         return None
     build = forward_grid if forward else adjoint_grid
     return [build(r, t_is_f32, step_size) for r in t_rows]
+
+
+_ENGINE_IDS = {"resident": _lib.ENGINE_RESIDENT, "rows": _lib.ENGINE_ROWS, "stream": _lib.ENGINE_STREAM}
+
+
+def _solve_desc(engine, adjoint, packed, G, H, B, N, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask=0,
+                reversed_time=False):
+    """The phx_solve request of a solve on ``engine`` ('resident' | 'rows' | 'stream'), with the fields all its launches
+    share; each launch points it at its own times, state, workspace and status (_launch)."""
+    d = _lib.PhxSolveDesc()
+    d.engine, d.adjoint, d.G, d.H, d.B, d.N, d.T = _ENGINE_IDS[engine], int(adjoint), G, H, B, N, T
+    d.packed, d.t_is_f32, d.reversed, d.method = packed.data_ptr(), int(t_is_f32), int(reversed_time), _lib.METHOD_IDS[method]
+    d.rtol, d.atol, d.max_num_steps, d.param_mask = float(rtol), float(atol), int(max_num_steps), param_mask
+    return d
+
+
+def _launch(lib, dev, d, t, ws, status, log, cap, what, stream=None):
+    """phx_solve of ``d`` with the times ``t`` (a ctypes double array), workspace, status record(s) and step log given."""
+    d.t_host = ctypes.addressof(t)
+    d.workspace, d.workspace_bytes, d.status = ws.data_ptr(), ws.numel(), status.data_ptr()
+    d.steplog, d.steplog_cap = (log.data_ptr(), cap) if log is not None else (None, 0)
+    _lib.check(lib.phx_solve(_lib.ctx(dev), ctypes.byref(d), stream if stream is not None else _stream_ptr(dev)), what)
 
 
 def _pick_engine(lib, dev, G, H, B, T, adjoint):
@@ -595,14 +617,12 @@ def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_t
     stn = _new_status_block(N)
     log, cap = _steplog_rows(N)
     flat_t = (ctypes.c_double * (N * T))(*[x for r in t_rows for x in r])
-    args = (_lib.ctx(dev), G, H, N, _ptr(packed), _ptr(y0c), flat_t, T, int(t_is_f32), int(reversed_time),
-            _lib.METHOD_IDS[method], float(rtol), float(atol), int(max_num_steps), _ptr(yout), _ptr(ws), ws.numel(),
-            _ptr(stn), _ptr(log), cap)
-    if grid is None:
-        rc = lib.phx_solve_forward_rows(*args, _stream_ptr(dev))
-    else:
-        rc = lib.phx_solve_forward_rows_grid(*args, *grid.args(), _stream_ptr(dev))
-    _lib.check(rc, "solve_forward_rows")
+    d = _solve_desc("rows", False, packed, G, H, 1, N, T, t_is_f32, method, rtol, atol, max_num_steps,
+                    reversed_time=reversed_time)
+    d.y0, d.y_out = y0c.data_ptr(), yout.data_ptr()
+    if grid is not None:
+        grid.put(d)
+    _launch(lib, dev, d, flat_t, ws, stn, log, cap, "solve_forward_rows")
     _tls().last_status_block = stn
     for i in range(N):
         _finish(stn[i], "forward solve %d" % i if N > 1 else "forward solve", dev)
@@ -630,21 +650,13 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
     log, cap = _steplog_rows(N)
     flat_t = (ctypes.c_double * (N * T))(*[x for r in t_rows for x in r])
     sp = _stream_ptr(dev)
-    args = (ctx, G, H, N, _ptr(packed), flat_t, T, int(t_is_f32), _lib.METHOD_IDS[method], float(rtol), float(atol),
-            int(max_num_steps), _ptr(ys), _ptr(gy), _ptr(adj_y0), _ptr(gpk), _ptr(ws), ws.numel(), _ptr(stn), _ptr(log), cap)
+    d = _solve_desc("rows", True, packed, G, H, 1, N, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask)
+    d.y_saved, d.grad_y, d.adj_y0, d.grads = ys.data_ptr(), gy.data_ptr(), adj_y0.data_ptr(), gpk.data_ptr()
     if grid is not None:
-        _lib.check(lib.phx_solve_adjoint_rows_grid(*args, param_mask, *grid.args(), sp), "solve_adjoint_rows")
-        _lib.check(lib.phx_unpack_grads_masked(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0,
-                                               param_mask & _lib.PARAMS_ALL, sp),
-                   "unpack_grads")
-    elif param_mask == _lib.PARAMS_ALL:
-        _lib.check(lib.phx_solve_adjoint_rows(*args, sp), "solve_adjoint_rows")
-        _lib.check(lib.phx_unpack_grads(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, sp), "unpack_grads")
-    else:
-        _lib.check(lib.phx_solve_adjoint_rows_masked(*args, param_mask, sp), "solve_adjoint_rows")
-        _lib.check(lib.phx_unpack_grads_masked(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0,
-                                               param_mask & _lib.PARAMS_ALL, sp),
-                   "unpack_grads")
+        grid.put(d)
+    _launch(lib, dev, d, flat_t, ws, stn, log, cap, "solve_adjoint_rows", sp)
+    _lib.check(lib.phx_unpack_grads_masked(ctx, G, H, _ptr(gpk), parts, _ptr(flat), 0, param_mask & _lib.PARAMS_ALL,
+                                           sp), "unpack_grads")
     _tls().last_status_block = stn
     for i in range(N):
         _finish(stn[i], "adjoint solve %d" % i if N > 1 else "adjoint solve", dev)
@@ -678,16 +690,12 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
     yout = torch.empty((T,) + tuple(y0c.shape), dtype=torch.float32, device=y0c.device)
     st = _new_status()
     log, cap = _steplog()
-    args = (_lib.ctx(dev), G, H, B, _ptr(packed), _ptr(y0c), _t_array(t_list), T, int(t_is_f32), int(reversed_time),
-            _lib.METHOD_IDS[method], float(rtol), float(atol), int(max_num_steps), _ptr(yout), _ptr(ws), ws.numel(),
-            _ptr(st), _ptr(log), cap)
-    if grid is None:
-        fn = lib.phx_solve_forward if engine == "resident" else lib.phx_stream_solve_forward
-        rc = fn(*args, _stream_ptr(dev))
-    else:
-        fn = lib.phx_solve_forward_grid if engine == "resident" else lib.phx_stream_solve_forward_grid
-        rc = fn(*args, *grid.args(), _stream_ptr(dev))
-    _lib.check(rc, "solve_forward")
+    d = _solve_desc(engine, False, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps,
+                    reversed_time=reversed_time)
+    d.y0, d.y_out = y0c.data_ptr(), yout.data_ptr()
+    if grid is not None:
+        grid.put(d)
+    _launch(lib, dev, d, _t_array(t_list), ws, st, log, cap, "solve_forward")
     _finish(st, "forward solve", dev)
     return yout
 
@@ -722,19 +730,11 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     grads = new_flat_grads(net, P, ys.device)
     st = _new_status()
     log, cap = _steplog()
-    fn = lib.phx_solve_adjoint if engine == "resident" else lib.phx_stream_solve_adjoint
-    args = (_lib.ctx(dev), G, H, B, _ptr(packed), _t_array(t_list), T, int(t_is_f32), _lib.METHOD_IDS[method],
-            float(rtol), float(atol), int(max_num_steps), _ptr(ys), _ptr(gy), _ptr(adj_y0), _ptr(grads), _ptr(ws),
-            ws.numel(), _ptr(st), _ptr(log), cap)
+    d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask)
+    d.y_saved, d.grad_y, d.adj_y0, d.grads = ys.data_ptr(), gy.data_ptr(), adj_y0.data_ptr(), grads.data_ptr()
     if grid is not None:
-        fn = lib.phx_solve_adjoint_grid if engine == "resident" else lib.phx_stream_solve_adjoint_grid
-        rc = fn(*args, param_mask, *grid.args(), _stream_ptr(dev))
-    elif param_mask == _lib.PARAMS_ALL:
-        rc = fn(*args, _stream_ptr(dev))
-    else:
-        fn = lib.phx_solve_adjoint_masked if engine == "resident" else lib.phx_stream_solve_adjoint_masked
-        rc = fn(*args, param_mask, _stream_ptr(dev))
-    _lib.check(rc, "solve_adjoint")
+        grid.put(d)
+    _launch(lib, dev, d, _t_array(t_list), ws, st, log, cap, "solve_adjoint")
     _finish(st, "adjoint solve", dev)
     return adj_y0, split_flat_grads(grads, G, H)
 
@@ -826,13 +826,7 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
         nb += _Grid(grids, True).nbytes(lib, N, T)
     ws = _workspace(dev, nb, "solve" if engine == "resident" else "stream")
     yout = torch.empty((N, T) + tuple(y0c.shape[1:]), dtype=torch.float32, device=y0c.device)
-    fn = lib.phx_solve_forward if engine == "resident" else lib.phx_stream_solve_forward
-    pg = [_Grid([g], True) for g in grids] if grids is not None else None   # (kept alive over the calls)
-    gx = (lambda i: pg[i].args()) if pg is not None else (lambda i: [])  # noqa: E731
-    if pg is not None:   # the grid of problem i goes right before the stream
-        fn = lib.phx_solve_forward_grid if engine == "resident" else lib.phx_stream_solve_forward_grid
-    ctx, sp, mid = _lib.ctx(dev), _stream_ptr(dev), _lib.METHOD_IDS[method]
-    pk, wsp, wsn = _ptr(packed), _ptr(ws), ws.numel()
+    sp = _stream_ptr(dev)
     ybase, obase = y0c.data_ptr(), yout.data_ptr()
     ystride, ostride = y0c[0].numel() * 4, yout[0].numel() * 4
     tarr = _t_rows(t_rows)
@@ -840,6 +834,7 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
     if streams:
         _fan_out(dev, streams)
     per = _problems_per_launch(T) if (engine == "resident" and not streams and not STEP_LOGGING) else 1
+    d = _solve_desc(engine, False, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps)
     if per > 1:
         # genome-scale model: a solve fills the GPU, so the problems go through ONE persistent launch a few at a time
         # and the weights are staged on chip once per launch instead of once per problem
@@ -847,35 +842,28 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
             n = min(per, N - lo)
             stn = _new_status_block(n)
             flat_t = (ctypes.c_double * (n * T))(*[x for r in t_rows[lo:lo + n] for x in r])
-            args = (ctx, G, H, B, n, pk, ctypes.c_void_p(ybase + lo * ystride), flat_t, T, int(t_is_f32), mid,
-                    float(rtol), float(atol), int(max_num_steps), ctypes.c_void_p(obase + lo * ostride), wsp, wsn,
-                    _ptr(stn))
-            if grids is None:
-                rc = lib.phx_solve_forward_many(*args, sp)
-            else:
+            d.N, d.y0, d.y_out = n, ybase + lo * ystride, obase + lo * ostride
+            if grids is not None:
                 gm = _Grid(grids[lo:lo + n], True)
-                rc = lib.phx_solve_forward_many_grid(*args, *gm.args(), sp)
-            _lib.check(rc, "solve_forward_many")
+                gm.put(d)
+            _launch(lib, dev, d, flat_t, ws, stn, None, 0, "solve_forward_many", sp)
             for i in range(n):
                 _finish(stn[i], "forward solve %d" % (lo + i), dev)
         return yout
+    pg = [_Grid([g], True) for g in grids] if grids is not None else None   # (kept alive over the calls)
     try:   # an error raised for one problem must not leave the caller's stream un-ordered after the side streams
         for i in range(N):
             st = _new_status()
             log, cap = _steplog()
+            d.y0, d.y_out = ybase + i * ystride, obase + i * ostride
+            if pg is not None:
+                pg[i].put(d)
             if streams:
                 with torch.cuda.stream(streams[i % len(streams)]):
-                    wsi = _workspace(dev, nb, "solve")
-                    rc = fn(ctx, G, H, B, pk, ctypes.c_void_p(ybase + i * ystride), tarr[i], T, int(t_is_f32), 0, mid,
-                            float(rtol), float(atol), int(max_num_steps), ctypes.c_void_p(obase + i * ostride),
-                            _ptr(wsi), wsi.numel(), _ptr(st), _ptr(log), cap, *gx(i), _stream_ptr(dev))
-                    _lib.check(rc, "solve_forward")
+                    _launch(lib, dev, d, tarr[i], _workspace(dev, nb, "solve"), st, log, cap, "solve_forward")
                     _finish(st, "forward solve %d" % i, dev)
                 continue
-            rc = fn(ctx, G, H, B, pk, ctypes.c_void_p(ybase + i * ystride), tarr[i], T, int(t_is_f32), 0, mid,
-                    float(rtol), float(atol), int(max_num_steps), ctypes.c_void_p(obase + i * ostride), wsp, wsn,
-                    _ptr(st), _ptr(log), cap, *gx(i), sp)
-            _lib.check(rc, "solve_forward")
+            _launch(lib, dev, d, tarr[i], ws, st, log, cap, "solve_forward", sp)
             _finish(st, "forward solve %d" % i, dev)
     finally:
         if streams:
@@ -910,27 +898,15 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     chunk = min(N, _MANY_CHUNK)
     grads = torch.empty(chunk, P, dtype=torch.float32, device=ys.device)
     total = None
-    full = param_mask == _lib.PARAMS_ALL
     pg = [_Grid([g], False) for g in grids] if grids is not None else None   # (kept alive over the calls)
-    gx = (lambda i: pg[i].args()) if pg is not None else (lambda i: [])  # noqa: E731
-    if pg is not None:   # param_mask, then the grid, right before the stream
-        fn0 = lib.phx_solve_adjoint_grid if engine == "resident" else lib.phx_stream_solve_adjoint_grid
-        fn = lambda *a: fn0(*a[:-3], param_mask, *a[-3:])  # noqa: E731
-        many = None
-    elif full:
-        fn = lib.phx_solve_adjoint if engine == "resident" else lib.phx_stream_solve_adjoint
-        many = lib.phx_solve_adjoint_many
-    else:   # the masked entry points take param_mask right before the stream
-        fn0 = lib.phx_solve_adjoint_masked if engine == "resident" else lib.phx_stream_solve_adjoint_masked
-        fn = lambda *a: fn0(*a[:-1], param_mask, a[-1])  # noqa: E731
-        many = lambda *a: lib.phx_solve_adjoint_many_masked(*a[:-1], param_mask, a[-1])  # noqa: E731
-    ctx, sp, mid = _lib.ctx(dev), _stream_ptr(dev), _lib.METHOD_IDS[method]
-    pk, wsp, wsn = _ptr(packed), _ptr(ws), ws.numel()
+    sp = _stream_ptr(dev)
+    ybase, gbase, abase, tbase = ys.data_ptr(), gy.data_ptr(), adj_y0.data_ptr(), grads.data_ptr()
     stride = ys[0].numel() * 4
     astride = adj_y0[0].numel() * 4
     tarr = _t_rows(t_rows)
     streams = _concurrency(lib, dev, G, H, B, True, engine, N)
     per = _problems_per_launch(T) if (engine == "resident" and not streams and not STEP_LOGGING) else 1
+    d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask)
     for lo in range(0, N, chunk):
         hi = min(N, lo + chunk)
         if per > 1:
@@ -938,16 +914,12 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
                 n = min(per, hi - l2)
                 stn = _new_status_block(n)
                 flat_t = (ctypes.c_double * (n * T))(*[x for r in t_rows[l2:l2 + n] for x in r])
-                args = (ctx, G, H, B, n, pk, flat_t, T, int(t_is_f32), mid, float(rtol), float(atol),
-                        int(max_num_steps), ctypes.c_void_p(ys.data_ptr() + l2 * stride),
-                        ctypes.c_void_p(gy.data_ptr() + l2 * stride), ctypes.c_void_p(adj_y0.data_ptr() + l2 * astride),
-                        ctypes.c_void_p(grads.data_ptr() + (l2 - lo) * P * 4), wsp, wsn, _ptr(stn))
-                if grids is None:
-                    rc = many(*args, sp)
-                else:
+                d.N, d.y_saved, d.grad_y = n, ybase + l2 * stride, gbase + l2 * stride
+                d.adj_y0, d.grads = abase + l2 * astride, tbase + (l2 - lo) * P * 4
+                if grids is not None:
                     gm = _Grid(grids[l2:l2 + n], False)
-                    rc = lib.phx_solve_adjoint_many_grid(*args, param_mask, *gm.args(), sp)
-                _lib.check(rc, "solve_adjoint_many")
+                    gm.put(d)
+                _launch(lib, dev, d, flat_t, ws, stn, None, 0, "solve_adjoint_many", sp)
                 for i in range(n):
                     _finish(stn[i], "adjoint solve %d" % (l2 + i), dev)
             part = grads[:hi - lo].sum(dim=0)
@@ -959,21 +931,16 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
             for i in range(lo, hi):
                 st = _new_status()
                 log, cap = _steplog()
-                args = (ctypes.c_void_p(ys.data_ptr() + i * stride), ctypes.c_void_p(gy.data_ptr() + i * stride),
-                        ctypes.c_void_p(adj_y0.data_ptr() + i * astride),
-                        ctypes.c_void_p(grads.data_ptr() + (i - lo) * P * 4))
+                d.y_saved, d.grad_y = ybase + i * stride, gbase + i * stride
+                d.adj_y0, d.grads = abase + i * astride, tbase + (i - lo) * P * 4
+                if pg is not None:
+                    pg[i].put(d)
                 if streams:
                     with torch.cuda.stream(streams[i % len(streams)]):
-                        wsi = _workspace(dev, nb, "solve")
-                        rc = fn(ctx, G, H, B, pk, tarr[i], T, int(t_is_f32), mid, float(rtol), float(atol),
-                                int(max_num_steps), *args, _ptr(wsi), wsi.numel(), _ptr(st), _ptr(log), cap, *gx(i),
-                                _stream_ptr(dev))
-                        _lib.check(rc, "solve_adjoint")
+                        _launch(lib, dev, d, tarr[i], _workspace(dev, nb, "solve"), st, log, cap, "solve_adjoint")
                         _finish(st, "adjoint solve %d" % i, dev)
                     continue
-                rc = fn(ctx, G, H, B, pk, tarr[i], T, int(t_is_f32), mid, float(rtol), float(atol), int(max_num_steps),
-                        *args, wsp, wsn, _ptr(st), _ptr(log), cap, *gx(i), sp)
-                _lib.check(rc, "solve_adjoint")
+                _launch(lib, dev, d, tarr[i], ws, st, log, cap, "solve_adjoint", sp)
                 _finish(st, "adjoint solve %d" % i, dev)
         finally:
             if streams:

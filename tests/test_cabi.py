@@ -65,3 +65,22 @@ def test_rows_plans_for_the_baseline_shapes():
 
 def test_status_struct_matches_header():
     assert ctypes.sizeof(_lib.PhxStatus) == 40
+
+
+def test_solve_desc_matches_header(tmp_path):
+    """The ctypes PhxSolveDesc has the size and field offsets of phx_solve_desc as a C compiler lays it out."""
+    import shutil
+    import subprocess
+    cc = shutil.which("cc")
+    if not cc:
+        return
+    fields = [f[0] for f in _lib.PhxSolveDesc._fields_]
+    src = tmp_path / "layout.c"
+    src.write_text("#include <stdio.h>\n#include <stddef.h>\n#include \"phoenix_b200.h\"\nint main(void) {\n"
+                   "    printf(\"%zu\\n\", sizeof(phx_solve_desc));\n"
+                   + "".join("    printf(\"%%zu\\n\", offsetof(phx_solve_desc, %s));\n" % f for f in fields)
+                   + "    return 0;\n}\n")
+    exe = tmp_path / "layout"
+    subprocess.run([cc, "-I", os.path.join(REPO, "include"), str(src), "-o", str(exe)], check=True)
+    got = [int(x) for x in subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout.split()]
+    assert got == [ctypes.sizeof(_lib.PhxSolveDesc)] + [getattr(_lib.PhxSolveDesc, f).offset for f in fields]

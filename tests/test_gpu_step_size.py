@@ -611,27 +611,63 @@ def test_float64_tensor_step_on_float32_t(pb, e, method):
         assert rel_l2(grads[i], g_ref[i]) <= 1e-5, (NAMES[i], rel_l2(grads[i], g_ref[i]))
 
 
+class _Requests:
+    """phx_solve requests of one-problem solves of a 350 x 40 model at T = 3 on each engine, with the buffers they need."""
+
+    def __init__(self, pb):
+        import ctypes
+        from phoenix_b200 import _lib
+        self.lib, self.ctypes, self._lib = _lib.load(), ctypes, _lib
+        G, H, T = self.G, self.H, self.T = 350, 40, 3
+        net = make_net(pb, _weights(G, H, 91))
+        self.packed, _, _, dev = pb.engine.packed_weights(net)
+        self.ctx, self.sp = _lib.ctx(dev), pb.engine._stream_ptr(dev)
+        self.y0 = torch.rand(2, 2, G, device="cuda")   # room for N = 2 problems of B = 2 rows
+        self.yout = torch.empty(2, T, 2, G, device="cuda")
+        self.gy = torch.rand(2, T, 2, G, device="cuda")
+        self.adj = torch.empty(2, 2, G, device="cuda")
+        self.flat = torch.empty(2, 4 * G * H + 2 * H + G, device="cuda")
+        self.gparts = torch.empty(self.lib.phx_packed_grad_bytes(G, H) // 4, device="cuda")
+        self.tarr = (ctypes.c_double * (2 * T))(0.0, 0.05, 0.1, 0.0, 0.05, 0.1)
+        self.log = torch.zeros(16, 3, dtype=torch.float64).pin_memory()
+        self.st = pb.engine._new_status_block(2)
+        room = 16 + self.lib.phx_grid_workspace_bytes(1, T, 4)
+        self.ws = {}
+        for engine in ("resident", "rows", "stream"):
+            size = {"resident": self.lib.phx_solve_workspace_bytes, "rows": self.lib.phx_rows_workspace_bytes,
+                    "stream": self.lib.phx_stream_workspace_bytes}[engine]
+            nb = max(size(self.ctx, G, H, 2, T, a) for a in (0, 1))   # B = 2 rows, or N = 2 rows problems
+            self.ws[engine] = pb.engine._workspace(dev, nb + room, "solve" if engine != "stream" else "stream")
+
+    def solve(self, which, adjoint, grid=(), method=2, **fields):
+        """phx_solve of a one-problem, one-row rk4 solve on engine ``which`` (grid: the grid arrays in field order), with
+        ``fields`` of the request overridden."""
+        _lib = self._lib
+        ws = self.ws[which]
+        d = _lib.PhxSolveDesc(engine={"resident": 0, "rows": 1, "stream": 2}[which], adjoint=adjoint, G=self.G, H=self.H,
+                              B=1, N=1, T=self.T, method=method, rtol=1e-7, atol=1e-9, max_num_steps=2 ** 31 - 1,
+                              packed=self.packed.data_ptr(), t_host=self.ctypes.addressof(self.tarr),
+                              workspace=ws.data_ptr(), workspace_bytes=ws.numel(), status=self.st.data_ptr())
+        if adjoint:
+            d.y_saved, d.grad_y, d.adj_y0 = self.yout.data_ptr(), self.gy.data_ptr(), self.adj.data_ptr()
+            d.grads = (self.gparts if which == "rows" else self.flat).data_ptr()
+            d.param_mask = _lib.PARAMS_ALL
+        else:
+            d.y0, d.y_out = self.y0.data_ptr(), self.yout.data_ptr()
+        for name, x in zip(("grid_dt", "grid_steps", "grid_out_step", "grid_out_slope"), grid):
+            setattr(d, name, x.data_ptr())
+        for name, v in fields.items():
+            setattr(d, name, v)
+        return self.lib.phx_solve(self.ctx, self.ctypes.byref(d), self.sp)
+
+
 @pytest.mark.gpu
-def test_invalid_grids_are_refused_at_the_c_abi(pb):
-    """Every refusal of a *_grid entry point: PHX_ERR_INVALID before anything is enqueued -- a step count < 1, a negative
-    or non-finite dt, an output step out of range or decreasing, a NaN slope, dopri5 -- for the resident, rows and
-    streaming forward and adjoint solves; the valid grid next to them runs."""
-    import ctypes
+def test_invalid_grids_are_refused_by_phx_solve(pb):
+    """Every refusal of a step grid by phx_solve: PHX_ERR_INVALID before anything is enqueued -- a step count < 1, a
+    negative or non-finite dt, an output step out of range or decreasing, a NaN slope, dopri5 -- for the resident, rows
+    and streaming forward and adjoint solves; the valid grid next to them runs."""
     from phoenix_b200 import _lib
-    lib = _lib.load()
-    G, H, T = 350, 40, 3
-    w = _weights(G, H, 91)
-    net = make_net(pb, w)
-    packed, _, _, dev = pb.engine.packed_weights(net)
-    ctx, sp = _lib.ctx(dev), pb.engine._stream_ptr(dev)
-    y0 = torch.rand(1, G, device="cuda")
-    yout = torch.empty(T, 1, G, device="cuda")
-    gy = torch.rand(T, 1, G, device="cuda")
-    adj = torch.empty(1, G, device="cuda")
-    flat = torch.empty(4 * G * H + 2 * H + G, device="cuda")
-    tarr = (ctypes.c_double * T)(0.0, 0.05, 0.1)
-    P = ctypes.c_void_p
-    ptr = lambda x: P(x.data_ptr())   # noqa: E731
+    rq = _Requests(pb)
     I32 = lambda *v: torch.tensor(v, dtype=torch.int32)   # noqa: E731
     F32 = lambda *v: torch.tensor(v, dtype=torch.float32)   # noqa: E731
     good_f = (F32(0.03, 0.02, 0.03, 0.02), I32(4), I32(1, 3), F32(-1.0, -1.0))
@@ -647,41 +683,40 @@ def test_invalid_grids_are_refused_at_the_c_abi(pb):
     bad_a = [(F32(0.03, 0.02, 0.03), I32(2, 0)), (F32(0.03, -0.02, 0.03, 0.02), I32(2, 2)),
              (F32(0.03, float("inf"), 0.03, 0.02), I32(2, 2))]
     for engine in ("resident", "rows", "stream"):
-        if engine == "resident":
-            nb_f = lib.phx_solve_workspace_bytes(ctx, G, H, 1, T, 0)
-            nb_a = lib.phx_solve_workspace_bytes(ctx, G, H, 1, T, 1)
-        elif engine == "rows":
-            nb_f = lib.phx_rows_workspace_bytes(ctx, G, H, 1, T, 0)
-            nb_a = lib.phx_rows_workspace_bytes(ctx, G, H, 1, T, 1)
-        else:
-            nb_f = lib.phx_stream_workspace_bytes(ctx, G, H, 1, T, 0)
-            nb_a = lib.phx_stream_workspace_bytes(ctx, G, H, 1, T, 1)
-        room = 16 + lib.phx_grid_workspace_bytes(1, T, 4)
-        ws = pb.engine._workspace(dev, max(nb_f, nb_a) + room, "solve" if engine != "stream" else "stream")
-        gparts = torch.empty(lib.phx_packed_grad_bytes(G, H) // 4, device="cuda")
-        st = pb.engine._new_status()
-
-        def fwd(g, method=2):
-            args = [ctx, G, H, 1, ptr(packed), ptr(y0), tarr, T, 0, 0, method, 1e-7, 1e-9, 2 ** 31 - 1, ptr(yout),
-                    ptr(ws), ws.numel(), ptr(st), None, 0] + [ptr(x) for x in g] + [sp]
-            fn = {"resident": lib.phx_solve_forward_grid, "rows": lib.phx_solve_forward_rows_grid,
-                  "stream": lib.phx_stream_solve_forward_grid}[engine]
-            return fn(*args)
-
-        def bwd(g, method=2):
-            out = ptr(gparts) if engine == "rows" else ptr(flat)
-            args = [ctx, G, H, 1, ptr(packed), tarr, T, 0, method, 1e-7, 1e-9, 2 ** 31 - 1, ptr(yout), ptr(gy), ptr(adj),
-                    out, ptr(ws), ws.numel(), ptr(st), None, 0, 0x3F] + [ptr(x) for x in g] + [sp]
-            fn = {"resident": lib.phx_solve_adjoint_grid, "rows": lib.phx_solve_adjoint_rows_grid,
-                  "stream": lib.phx_stream_solve_adjoint_grid}[engine]
-            return fn(*args)
-
         for g in bad_f:
-            assert fwd(g) == -1, (engine, g)   # PHX_ERR_INVALID
+            assert rq.solve(engine, 0, g) == -1, (engine, g)   # PHX_ERR_INVALID
         for g in bad_a:
-            assert bwd(g) == -1, (engine, g)
-        assert fwd(good_f, method=3) == -1 and bwd(good_a, method=3) == -1, engine   # dopri5 takes no grid
-        assert fwd(good_f) == 0, (engine, _lib.last_error())
+            assert rq.solve(engine, 1, g) == -1, (engine, g)
+        assert rq.solve(engine, 0, good_f, method=3) == -1 and rq.solve(engine, 1, good_a, method=3) == -1, engine  # dopri5
+        assert rq.solve(engine, 0, good_f) == 0, (engine, _lib.last_error())
         torch.cuda.synchronize()
-        assert bwd(good_a) == 0, (engine, _lib.last_error())
+        assert rq.solve(engine, 1, good_a) == 0, (engine, _lib.last_error())
+        torch.cuda.synchronize()
+
+
+@pytest.mark.gpu
+def test_phx_solve_refuses_the_combinations_no_engine_takes(pb):
+    """phx_solve refuses, with PHX_ERR_INVALID and a message, what none of the engines takes: an unknown engine,
+    `reversed` or forward-grid outputs on an adjoint solve, a param_mask on a forward solve, grid arrays without grid_dt,
+    N != 1 on the streaming engine, B != 1 on the rows engine, `reversed` or a step log with N > 1 on the resident
+    engine; the plain requests next to them run."""
+    from phoenix_b200 import _lib
+    rq = _Requests(pb)
+    steps, out_step, slope = (torch.tensor(v, dtype=t) for v, t in
+                              (((4,), torch.int32), ((1, 3), torch.int32), ((-1.0, -1.0), torch.float32)))
+    refused = [("resident", 0, dict(engine=3)), ("stream", 1, dict(engine=-1)),
+               ("resident", 1, dict(reversed=1)), ("rows", 1, dict(reversed=1)), ("stream", 1, dict(reversed=1)),
+               ("resident", 0, dict(param_mask=_lib.PARAMS_ALL)), ("rows", 0, dict(param_mask=1)),
+               ("stream", 0, dict(param_mask=_lib.NORM_SEMINORM)),
+               ("resident", 1, dict(grid_out_step=out_step.data_ptr())), ("rows", 1, dict(grid_out_slope=slope.data_ptr())),
+               ("resident", 0, dict(grid_steps=steps.data_ptr())), ("stream", 1, dict(grid_steps=steps.data_ptr())),
+               ("stream", 0, dict(N=2)), ("stream", 1, dict(N=2)), ("rows", 0, dict(B=2)), ("rows", 1, dict(B=2)),
+               ("resident", 0, dict(N=2, reversed=1)), ("resident", 0, dict(N=2, steplog=rq.log.data_ptr(), steplog_cap=16))]
+    for engine, adjoint, fields in refused:
+        assert rq.solve(engine, adjoint, **fields) == -1, (engine, adjoint, fields)
+        assert _lib.last_error(), (engine, adjoint, fields)
+    for engine, adjoint, fields in [("resident", 0, dict(reversed=1, steplog=rq.log.data_ptr(), steplog_cap=16)),
+                                    ("resident", 0, dict(N=2, B=2)), ("resident", 1, dict(N=2, B=2)),
+                                    ("rows", 0, dict(N=2)), ("stream", 0, dict(B=2, reversed=1))]:
+        assert rq.solve(engine, adjoint, **fields) == 0, (engine, adjoint, fields, _lib.last_error())
         torch.cuda.synchronize()
