@@ -289,7 +289,20 @@ int phx_rows_grad_parts(const phx_ctx* ctx, int G, int H, int N);
  * Between the steps the state is not restarted at the output times.  status.n_rhs = stages x steps.  The grid is copied
  * into the workspace (not on the streaming engine), which must then hold phx_grid_workspace_bytes(N, T, total steps)
  * more bytes than the engine's own size function asks for.  An invalid grid (a step count < 1, a dt that is negative or
- * not finite, an output step out of range or decreasing, a NaN slope) returns PHX_ERR_INVALID. */
+ * not finite, an output step out of range or decreasing, a NaN slope) returns PHX_ERR_INVALID.
+ *
+ * dopri5 step control (odeint options first_step, safety, ifactor, dfactor; rk_common.py:111-228, misc.py:94-103):
+ * 0 in a field means its default -- Hairer's initial-step estimate (misc.py:47-86), 0.9, 10 and 0.2 -- so a
+ * zero-initialised request and every entry point above keep the reference's default controller.
+ *   first_step > 0: the first attempted dt of the solve, and of every output interval of an adjoint solve (each is its
+ *     own odeint call in the reference's backward), in the increasing time the solve runs in.  f0 is still evaluated
+ *     (it counts in status.n_rhs and gives the non-finite check of the initial state); Hairer's second evaluation and
+ *     its norms (in the adjoint also those of the parameter cotangents) are skipped.  A first step beyond the next
+ *     output time is legal: steps are never clipped to output times.
+ *   safety, ifactor, dfactor: with the error ratio r, the next dt is dt * ifactor when r == 0, else
+ *     dt * min(ifactor, max(safety / r^(1/5), r < 1 ? 1 : dfactor)).
+ * A negative, NaN or infinite value in any of the four, or a nonzero one with a method other than dopri5, returns
+ * PHX_ERR_INVALID. */
 enum { PHX_ENGINE_RESIDENT = 0, PHX_ENGINE_ROWS = 1, PHX_ENGINE_STREAM = 2 };
 typedef struct phx_solve_desc {
     const float* packed;
@@ -310,6 +323,7 @@ typedef struct phx_solve_desc {
     double* steplog;                 /* may be NULL */
     double rtol, atol;
     int64_t max_num_steps;
+    double first_step, safety, ifactor, dfactor;   /* dopri5 step control; 0: the default */
     int32_t engine, adjoint, G, H, B, N, T, t_is_f32, reversed, method, param_mask, steplog_cap;
 } phx_solve_desc;
 int phx_solve(phx_ctx* ctx, const phx_solve_desc* desc, void* stream);

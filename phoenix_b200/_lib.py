@@ -45,7 +45,9 @@ class PhxSolveDesc(ctypes.Structure):
                     "packed", "t_host", "y0", "y_out", "y_saved", "grad_y", "adj_y0", "grads", "grid_dt", "grid_steps",
                     "grid_out_step", "grid_out_slope", "workspace")]
                 + [("workspace_bytes", ctypes.c_size_t), ("status", ctypes.c_void_p), ("steplog", ctypes.c_void_p),
-                   ("rtol", ctypes.c_double), ("atol", ctypes.c_double), ("max_num_steps", ctypes.c_int64)]
+                   ("rtol", ctypes.c_double), ("atol", ctypes.c_double), ("max_num_steps", ctypes.c_int64),
+                   ("first_step", ctypes.c_double), ("safety", ctypes.c_double), ("ifactor", ctypes.c_double),
+                   ("dfactor", ctypes.c_double)]
                 + [(name, ctypes.c_int32) for name in (
                     "engine", "adjoint", "G", "H", "B", "N", "T", "t_is_f32", "reversed", "method", "param_mask",
                     "steplog_cap")])

@@ -475,6 +475,23 @@ bool check_request(const phx_solve_desc& d) {
     return !why;
 }
 
+// the dopri5 step-control fields: 0 (the default) or a positive finite number, and only with dopri5
+bool check_step_control(const phx_solve_desc& d) {
+    const char* names[4] = {"first_step", "safety", "ifactor", "dfactor"};
+    const double v[4] = {d.first_step, d.safety, d.ifactor, d.dfactor};
+    for (int i = 0; i < 4; ++i) {
+        if (!(v[i] >= 0.0 && v[i] < INFINITY)) {
+            phx_set_error("%s must be 0 (the default) or a positive finite number (got %g)", names[i], v[i]);
+            return false;
+        }
+        if (v[i] != 0.0 && d.method != PHX_DOPRI5) {
+            phx_set_error("%s is a dopri5 option (method %d)", names[i], d.method);
+            return false;
+        }
+    }
+    return true;
+}
+
 // the resident and rows engines: the whole solve in one persistent launch
 int solve_on_chip(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t stream) {
     const bool rows = d.engine == PHX_ENGINE_ROWS;
@@ -534,6 +551,10 @@ int solve_on_chip(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t stream) {
     p.so = rows ? wplan.so : rplan.so;
     p.rtol_f = (float)d.rtol; p.atol_f = (float)d.atol; p.fsign = d.reversed ? -1.f : 1.f;
     p.max_steps = (long long)d.max_num_steps;
+    p.first_step = d.first_step;
+    p.safety = d.safety > 0 ? d.safety : 0.9;
+    p.ifactor = d.ifactor > 0 ? d.ifactor : 10.0;
+    p.dfactor = d.dfactor > 0 ? d.dfactor : 0.2;
     p.w = phx_packed_view(d.packed, G, H);
     p.ll = phx_ll_view(d.workspace);
     p.t = (const double*)(ws + o_t);
@@ -623,7 +644,7 @@ int phx_solve(phx_ctx* ctx, const phx_solve_desc* desc, void* stream) {
         return PHX_ERR_INVALID;
     }
     const phx_solve_desc& d = *desc;
-    if (!check_request(d)) return PHX_ERR_INVALID;
+    if (!check_request(d) || !check_step_control(d)) return PHX_ERR_INVALID;
     const bool rows = d.engine == PHX_ENGINE_ROWS;
     if (d.adjoint) {
         if (!check_adjoint_mask(d.param_mask)) return PHX_ERR_INVALID;

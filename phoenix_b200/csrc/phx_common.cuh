@@ -247,6 +247,9 @@ struct ResParams {
     float rtol_f, atol_f;
     float fsign;           // +1, or -1 when the caller's t was decreasing (f -> -f(-t, y), misc.py:159-162)
     long long max_steps;
+    // dopri5 step control (phx_solve_desc): first_step > 0 replaces Hairer's initial-step estimate (of every output
+    // interval in the adjoint); the controller constants of next_dt, defaults filled in by the host
+    double first_step, safety, ifactor, dfactor;
     PhxPacked w;
     const double* t;       // [T] device copy of the output times (only used when T > PHX_T_INLINE)
     double t_small[64];    // the output times themselves when nprob * T <= PHX_T_INLINE (no host->device copy per call)

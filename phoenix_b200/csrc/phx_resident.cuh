@@ -1215,17 +1215,23 @@ __device__ void set_step_coeffs(Ctrl* c) {
     }
 }
 
-// misc.py:94-103 with safety 0.9, ifactor 10, dfactor 0.2, order 5
-__device__ double next_dt(double dt, float ratio) {
-    if (ratio == 0.f) return dt * 10.0;
-    double dfactor = (ratio < 1.f) ? 1.0 : 0.2;
+// misc.py:94-103 with order 5 and the request's safety, ifactor, dfactor (defaults 0.9, 10, 0.2)
+__device__ double next_dt(const ResParams& p, double dt, float ratio) {
+    if (ratio == 0.f) return dt * p.ifactor;
+    double dfactor = (ratio < 1.f) ? 1.0 : p.dfactor;
     double r = (double)ratio;
     if (isnan(r)) return nan("");
-    double f = 0.9 / pow(r, 0.2);
+    double f = p.safety / pow(r, 0.2);
     f = fmax(f, dfactor);
-    f = fmin(10.0, f);
+    f = fmin(p.ifactor, f);
     return dt * f;
 }
+
+// the caller gives the first step of a dopri5 solve (phx_solve_desc.first_step; never with a step grid, which is
+// fixed-grid only).  Read at each use rather than held in a variable: the default instantiations then keep their
+// register allocation
+template <bool GRID>
+__device__ __forceinline__ bool given_step(const ResParams& p) { return !GRID && p.first_step > 0; }
 
 // misc.py:47-86 tail: h0 from d0, d1
 __device__ float init_h0(float d0, float d1) {
@@ -1455,7 +1461,8 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_fwd_kernel(const __grid_co
     }
 
     // ---- dopri5 (rk_common.py:111-228) ----
-    // f0 and the initial step (misc.py:47-86): two evaluations through one call site
+    // f0 and the initial step (misc.py:47-86): two evaluations through one call site, or f0 alone when the caller gives
+    // the first step
     for (int which = 0; which < 2; ++which) {
         double acc[3] = {0, 0, 0};
         eval_A<NV, BT>(p, s);
@@ -1486,8 +1493,15 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_fwd_kernel(const __grid_co
                 c->d1 = d1;
                 c->h0 = init_h0(d0, d1);
                 c->nonfinite_prev = c->dsum[2] > 0.0;
+                if (given_step<GRID>(p)) {
+                    c->dt = p.first_step;
+                    c->tprev = c->tcur;
+                    c->n_rhs = 1;
+                    c->n_steps_interval = 0;
+                }
             }
             __syncthreads();
+            if (given_step<GRID>(p)) break;   // the caller's first step: no second evaluation
             const float h0 = c->h0;
             for_local(p, g_lo, n_loc, [&](int b, int j, int g, size_t gi, int li) {
                 set_stage_input(li, Y[li] + h0 * K(0)[li]);
@@ -1575,7 +1589,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_fwd_kernel(const __grid_co
             } else {
                 c->n_rej++;
             }
-            c->dt = next_dt(c->dt, ratio);
+            c->dt = next_dt(p, c->dt, ratio);
             c->accept = accept;
             c->n_rhs += 6;
             c->n_steps_interval++;
@@ -2198,7 +2212,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
             }
             __syncthreads();
             // f0 and Hairer's initial step under the mixed norm max(RMS_y, RMS_a, RMS_theta): two evaluations through
-            // one call site
+            // one call site, or f0 alone when the caller gives the first step
             for (int which = 0; which < 2; ++which) {
                 double acc[7] = {0, 0, 0, 0, 0, 0, 0};
                 adj_eval<NV, BT>(p, s, which, false, false, no_y, [&](int b, int j, int li, float ka, bool lead) {
@@ -2229,7 +2243,8 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 __syncthreads();
                 pf.tick(PT_COMBINE);
                 if (which == 0) {
-                    if (!SEMI) {   // (the seminorm has no theta block)
+                    if (!SEMI && !given_step<GRID>(p)) {   // (the seminorm has no theta block; a given first step
+                                                          // needs no norm)
                         if (theta_zero) {
                             acc[5] += theta_zero_norm<BT>(p, n_loc, 0, -1);
                         } else {
@@ -2250,8 +2265,13 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                         c->d1 = d1;
                         c->h0 = init_h0(d0, d1);
                         c->nonfinite_prev = c->dsum[6] > 0.0;
+                        if (given_step<GRID>(p)) {
+                            c->dt = p.first_step;
+                            c->n_rhs += 1;
+                        }
                     }
                     __syncthreads();
+                    if (given_step<GRID>(p)) break;   // the caller's first step: no second evaluation
                     const float h0 = c->h0;
                     for_local(p, g_lo, n_loc, [&](int b, int j, int g, size_t gi, int li) {
                         set_y_input(s.ysb(), s.acts(), s.actl(), li, Y[li] + h0 * KY(0)[li]);
@@ -2390,7 +2410,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                     } else {
                         c->n_rej++;
                     }
-                    c->dt = next_dt(c->dt, ratio);
+                    c->dt = next_dt(p, c->dt, ratio);
                     c->accept = accept;
                     c->n_rhs += 6;
                     c->n_steps_interval++;

@@ -645,6 +645,12 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_fwd_kernel(const __gr
                     c.d1 = d1;
                     c.h0 = init_h0(d0, d1);
                     c.nonfinite_prev = d[2] > 0.0;
+                    if (p.first_step > 0) {
+                        c.dt = p.first_step;
+                        c.tprev = c.tcur;
+                        c.n_rhs = 1;
+                        c.n_steps_interval = 0;
+                    }
                 } else {
                     const float d2 = sqrtf((float)(d[0] / Nel)) / c.h0;
                     c.dt = init_dt(c.h0, c.d1, d2);
@@ -654,6 +660,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_fwd_kernel(const __gr
                 }
             }
             __syncthreads();
+            if (p.first_step > 0) break;   // the caller's first step (every row's): no second evaluation
             if (which == 0) {
                 for (int e = threadIdx.x; e < tot; e += THREADS) set_input(e, Y[e] + rc->r[e & 3].h0 * K(0)[e]);
                 __syncthreads();
@@ -724,7 +731,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_fwd_kernel(const __gr
                     } else {
                         c.n_rej++;
                     }
-                    c.dt = next_dt(c.dt, ratio);
+                    c.dt = next_dt(p, c.dt, ratio);
                     c.accept = accept;
                     c.n_rhs += 6;
                     c.n_steps_interval++;
@@ -1614,9 +1621,11 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         a.active = !c.done && !c.theta_zero;
                     }
                     __syncthreads();
+                    // (a given first step needs no norm)
+                    const bool thn = !semi && !(p.first_step > 0);
                     const double zn =
-                        semi ? 0.0 : rows_theta_zero_norm(p, n_loc, s.tmem, which == 0 ? 0 : 6, which == 0 ? -1 : 0);
-                    if (any_nz && !semi) {
+                        thn ? rows_theta_zero_norm(p, n_loc, s.tmem, which == 0 ? 0 : 6, which == 0 ? -1 : 0) : 0.0;
+                    if (any_nz && thn) {
                         if (which == 0) rows_theta_pass<TP_D01, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
                         else rows_theta_pass<TP_D2, SEMI>(p, g_lo, n_loc, s.tmem, tsum);
                     }
@@ -1625,8 +1634,8 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                     if (threadIdx.x < RM) {
                         const RowCtl& c = rc->r[threadIdx.x];
                         double* d = dsum + threadIdx.x * 7;
-                        if (semi) {
-                            // (the seminorm has no theta block)
+                        if (!thn) {
+                            // (the seminorm has no theta block; a given first step needs none)
                         } else if (c.theta_zero) {
                             d[which == 0 ? 5 : 2] += zn;
                         } else if (which == 0) {
@@ -1650,6 +1659,10 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                             c.d1 = d1;
                             c.h0 = init_h0(d0, d1);
                             c.nonfinite_prev = d[6] > 0.0;
+                            if (p.first_step > 0) {
+                                c.dt = p.first_step;
+                                if (!c.done) c.n_rhs += 1;
+                            }
                         } else {
                             const float d2 = fmaxf(fmaxf(sqrtf((float)(d[0] / Nel)), sqrtf((float)(d[1] / Nel))),
                                                    th_rms(d[2])) / c.h0;
@@ -1658,6 +1671,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         }
                     }
                     __syncthreads();
+                    if (p.first_step > 0) break;   // the caller's first step (every row's): no second evaluation
                     if (which == 0) {
                         for (int e = threadIdx.x; e < tot; e += THREADS) {
                             const RowCtl& c = rc->r[e & 3];
@@ -1784,7 +1798,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                             } else {
                                 c.n_rej++;
                             }
-                            c.dt = next_dt(c.dt, ratio);
+                            c.dt = next_dt(p, c.dt, ratio);
                             c.accept = accept;
                             c.n_rhs += 6;
                             c.n_steps_interval++;

@@ -248,14 +248,15 @@ struct Seg {
     bool in_norm = true;   // false: the seminorm's parameter segment -- no norm sums, no error kernel
 };
 
-double next_dt_host(double dt, float ratio) {
-    if (ratio == 0.f) return dt * 10.0;
-    double dfactor = (ratio < 1.f) ? 1.0 : 0.2;
+// misc.py:94-103 with order 5 (next_dt of the resident kernels)
+double next_dt_host(double dt, float ratio, double safety, double ifactor, double dfactor_ge1) {
+    if (ratio == 0.f) return dt * ifactor;
+    double dfactor = (ratio < 1.f) ? 1.0 : dfactor_ge1;
     double r = (double)ratio;
     if (isnan(r)) return nan("");
-    double f = 0.9 / pow(r, 0.2);
+    double f = safety / pow(r, 0.2);
     f = fmax(f, dfactor);
-    f = fmin(10.0, f);
+    f = fmin(ifactor, f);
     return dt * f;
 }
 
@@ -279,6 +280,8 @@ struct Stream {
     void* sum_user = nullptr;
     int sum_world = 1;
     bool fuse = false;                 // stage algebra in the RHS epilogue (forward solves on the tensor-core path)
+    // dopri5 step control (phx_solve_desc): first_step > 0 replaces Hairer's estimate; the controller constants
+    double first_step = 0, safety = 0.9, ifactor = 10.0, dfactor = 0.2;
     int pmask = PHX_P_ALL;             // adjoint: parameters whose cotangents make up the theta segment
     PhxGradOff goff{};                 // adjoint: their offsets in the theta segment (back to back, reference order)
 
@@ -444,29 +447,35 @@ struct Stream {
             finish_sums((int)si);
         }
         if ((rc = fetch_sums()) != PHX_OK) return rc;
-        float d0 = block_norm(0), d1 = block_norm(1);
         bool nonfinite = false;
         for (size_t si = 0; si < ns; ++si) nonfinite = nonfinite || (segs[si].in_norm && sums_host[3 * si + 2] > 0.0);
-        float h0 = (d0 < 1e-5f || d1 < 1e-5f) ? 1e-6f : 0.01f * d0 / d1;
-        {
-            std::vector<KSet> ks(ns);
-            int s0[1] = {0};
-            float c0[1] = {h0};
-            for (size_t si = 0; si < ns; ++si) ks[si] = kset((int)si, s0, c0, 1);
-            set_inputs(ks.data());
+        double dt = first_step;
+        if (first_step > 0) {
+            // the caller's first step: the fetch above was for the non-finite count only
+            status.n_rhs += 1;
+        } else {
+            float d0 = block_norm(0), d1 = block_norm(1);
+            float h0 = (d0 < 1e-5f || d1 < 1e-5f) ? 1e-6f : 0.01f * d0 / d1;
+            {
+                std::vector<KSet> ks(ns);
+                int s0[1] = {0};
+                float c0[1] = {h0};
+                for (size_t si = 0; si < ns; ++si) ks[si] = kset((int)si, s0, c0, 1);
+                set_inputs(ks.data());
+            }
+            if ((rc = eval(1)) != PHX_OK) return rc;
+            for (size_t si = 0; si < ns; ++si) {
+                Seg& s = segs[si];
+                if (!s.in_norm) continue;
+                initd2_kernel<<<nblk(s.n), EB, 0, st>>>(s.x0, s.k[0], s.k[1], rtol_f, atol_f, s.n, partial);
+                finish_sums((int)si);
+            }
+            if ((rc = fetch_sums()) != PHX_OK) return rc;
+            float d2 = block_norm(0) / h0;
+            float h1 = (d1 <= 1e-15f && d2 <= 1e-15f) ? fmaxf(1e-6f, h0 * 1e-3f) : powf(0.01f / fmaxf(d1, d2), 0.2f);
+            dt = (double)fminf(100.f * h0, h1);
+            status.n_rhs += 2;
         }
-        if ((rc = eval(1)) != PHX_OK) return rc;
-        for (size_t si = 0; si < ns; ++si) {
-            Seg& s = segs[si];
-            if (!s.in_norm) continue;
-            initd2_kernel<<<nblk(s.n), EB, 0, st>>>(s.x0, s.k[0], s.k[1], rtol_f, atol_f, s.n, partial);
-            finish_sums((int)si);
-        }
-        if ((rc = fetch_sums()) != PHX_OK) return rc;
-        float d2 = block_norm(0) / h0;
-        float h1 = (d1 <= 1e-15f && d2 <= 1e-15f) ? fmaxf(1e-6f, h0 * 1e-3f) : powf(0.01f / fmaxf(d1, d2), 0.2f);
-        double dt = (double)fminf(100.f * h0, h1);
-        status.n_rhs += 2;
         double tcur = t_start, tprev = t_start;
         int next_out = 0;
         long long nsteps = 0;
@@ -531,7 +540,7 @@ struct Stream {
             tprev = tcur;
             ++nsteps;
             double dt_used = dt;
-            dt = next_dt_host(dt, ratio);
+            dt = next_dt_host(dt, ratio, safety, ifactor, dfactor);
             if (!accept) {
                 status.n_rejected++;
                 continue;
@@ -655,6 +664,14 @@ int setup(Stream& S, phx_ctx* ctx, int G, int H, int B, const float* packed, con
     return PHX_OK;
 }
 
+// the request's dopri5 step control (0: the default)
+void set_step_control(Stream& S, const phx_solve_desc& d) {
+    S.first_step = d.first_step;
+    if (d.safety > 0) S.safety = d.safety;
+    if (d.ifactor > 0) S.ifactor = d.ifactor;
+    if (d.dfactor > 0) S.dfactor = d.dfactor;
+}
+
 float fixed_dt(const double* t, int i, int t_is_f32) {
     return t_is_f32 ? ((float)t[i + 1] - (float)t[i]) : (float)(t[i + 1] - t[i]);
 }
@@ -683,6 +700,7 @@ int phx_stream_forward(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t st) {
                    d.workspace, d.workspace_bytes, d.steplog, d.steplog_cap, st, &base);
     if (rc != PHX_OK) return rc;
     S.fsign = d.reversed ? -1.f : 1.f;
+    set_step_control(S, d);
     {
         // OFF unless PHX_STREAM_FUSE=1: measured slower at every shape (tools/stream_fuse_ab.py,
         // profiles/r04d_stream_fuse_ab.txt -- 60 rows x 11 165 genes rk4 0.40 ms fused / 0.34 ms not; 4 096 x 20 000:
@@ -753,6 +771,7 @@ int phx_stream_adjoint(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t st) {
     int rc = setup(S, ctx, G, H, B, d.packed, t_host, T, d.t_is_f32, method, d.rtol, d.atol, d.max_num_steps, 1,
                    d.workspace, d.workspace_bytes, d.steplog, d.steplog_cap, st, &base);
     if (rc != PHX_OK) return rc;
+    set_step_control(S, d);
     const size_t BG = (size_t)B * G, P = phx_grad_offsets(G, H).total;
     // the theta segment holds the adjoint parameters' cotangents only, back to back in reference order (all six: the
     // flat layout itself), at the start of grads_flat; it is absent when there are none

@@ -538,13 +538,16 @@ _ENGINE_IDS = {"resident": _lib.ENGINE_RESIDENT, "rows": _lib.ENGINE_ROWS, "stre
 
 
 def _solve_desc(engine, adjoint, packed, G, H, B, N, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask=0,
-                reversed_time=False):
+                reversed_time=False, step_control=None):
     """The phx_solve request of a solve on ``engine`` ('resident' | 'rows' | 'stream'), with the fields all its launches
-    share; each launch points it at its own times, state, workspace and status (_launch)."""
+    share; each launch points it at its own times, state, workspace and status (_launch).  ``step_control``: dopri5's
+    (first_step, safety, ifactor, dfactor), 0 for a default, or None for all four defaults."""
     d = _lib.PhxSolveDesc()
     d.engine, d.adjoint, d.G, d.H, d.B, d.N, d.T = _ENGINE_IDS[engine], int(adjoint), G, H, B, N, T
     d.packed, d.t_is_f32, d.reversed, d.method = packed.data_ptr(), int(t_is_f32), int(reversed_time), _lib.METHOD_IDS[method]
     d.rtol, d.atol, d.max_num_steps, d.param_mask = float(rtol), float(atol), int(max_num_steps), param_mask
+    if step_control is not None:
+        d.first_step, d.safety, d.ifactor, d.dfactor = (float(v) for v in step_control)
     return d
 
 
@@ -604,9 +607,9 @@ def _steplog_rows(n):
 
 
 def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_time, method, rtol, atol, max_num_steps,
-                  out_shape, grids=None):
+                  out_shape, grids=None, step_control=None):
     """N one-row problems (y0c [N, G]) in lock-step; returns yout of shape out_shape (= [N, T, ..., G] memory order).
-    ``grids``: the problems' forward step grids (forward_grid), or None."""
+    ``grids``: the problems' forward step grids (forward_grid), or None; ``step_control``: see _solve_desc."""
     N, T = len(t_rows), len(t_rows[0])
     nb = lib.phx_rows_workspace_bytes(_lib.ctx(dev), G, H, N, T, 0)
     grid = _Grid(grids, True) if grids is not None else None
@@ -618,7 +621,7 @@ def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_t
     log, cap = _steplog_rows(N)
     flat_t = (ctypes.c_double * (N * T))(*[x for r in t_rows for x in r])
     d = _solve_desc("rows", False, packed, G, H, 1, N, T, t_is_f32, method, rtol, atol, max_num_steps,
-                    reversed_time=reversed_time)
+                    reversed_time=reversed_time, step_control=step_control)
     d.y0, d.y_out = y0c.data_ptr(), yout.data_ptr()
     if grid is not None:
         grid.put(d)
@@ -630,10 +633,10 @@ def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_t
 
 
 def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy, adj_shape,
-                  param_mask=_lib.PARAMS_ALL, grids=None):
+                  param_mask=_lib.PARAMS_ALL, grids=None, step_control=None):
     """Backward sweeps of N one-row problems (ys, gy: [N, T, ..., G] memory order): adj_y0 and the SUM over the problems of
     the six parameter cotangents (flat, reference order; zeros for the parameters outside ``param_mask``).  ``grids``:
-    the problems' backward step grids (adjoint_grid), or None."""
+    the problems' backward step grids (adjoint_grid), or None; ``step_control``: see _solve_desc."""
     N, T = len(t_rows), len(t_rows[0])
     nb = lib.phx_rows_workspace_bytes(_lib.ctx(dev), G, H, N, T, 1)
     grid = _Grid(grids, False) if grids is not None else None
@@ -650,7 +653,8 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
     log, cap = _steplog_rows(N)
     flat_t = (ctypes.c_double * (N * T))(*[x for r in t_rows for x in r])
     sp = _stream_ptr(dev)
-    d = _solve_desc("rows", True, packed, G, H, 1, N, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask)
+    d = _solve_desc("rows", True, packed, G, H, 1, N, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask,
+                    step_control=step_control)
     d.y_saved, d.grad_y, d.adj_y0, d.grads = ys.data_ptr(), gy.data_ptr(), adj_y0.data_ptr(), gpk.data_ptr()
     if grid is not None:
         grid.put(d)
@@ -664,9 +668,11 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
 
 
 @_on_model_device
-def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, max_num_steps, step_size=None):
+def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, max_num_steps, step_size=None,
+                  step_control=None):
     """``step_size`` (fixed-grid methods): integrate on the reference's grid of that spacing and interpolate the output
-    times inside a step (solvers.py:48-50, 77-103); None: one step per output interval."""
+    times inside a step (solvers.py:48-50, 77-103); None: one step per output interval.  ``step_control`` (dopri5):
+    (first_step, safety, ifactor, dfactor), 0 for a default (include/phoenix_b200.h, phx_solve), or None."""
     packed, G, H, dev = packed_weights(net)
     if y0.shape[-1] != G:
         raise RuntimeError("last dimension of y0 (%d) must equal ndim (%d)" % (y0.shape[-1], G))
@@ -681,7 +687,7 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
     grids = _grids([t_list], t_is_f32, step_size, True)
     if _use_rows(lib, dev, G, H, B, False, single=True, T=T):
         return _forward_rows(lib, net, packed, G, H, dev, y0c, [t_list], t_is_f32, reversed_time, method, rtol, atol,
-                             max_num_steps, (T,) + tuple(y0c.shape), grids)
+                             max_num_steps, (T,) + tuple(y0c.shape), grids, step_control)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, False)
     grid = _Grid(grids, True) if grids is not None else None
     if grid is not None and engine == "resident":
@@ -691,7 +697,7 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
     st = _new_status()
     log, cap = _steplog()
     d = _solve_desc(engine, False, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps,
-                    reversed_time=reversed_time)
+                    reversed_time=reversed_time, step_control=step_control)
     d.y0, d.y_out = y0c.data_ptr(), yout.data_ptr()
     if grid is not None:
         grid.put(d)
@@ -702,12 +708,13 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
 
 @_on_model_device
 def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
-                  param_mask=_lib.PARAMS_ALL, step_size=None):
+                  param_mask=_lib.PARAMS_ALL, step_size=None, step_control=None):
     """adj_y0 and the six parameter cotangents of one backward sweep.  ``param_mask`` (bit i = the i-th parameter in
     reference order): the adjoint parameters, the only ones integrated and put in the error norm; the cotangents of the
     others come back as zeros.  With ``_lib.NORM_SEMINORM`` also set, the dopri5 error norm leaves the parameter block
     out altogether (the seminorm).  ``step_size`` (fixed-grid methods): every interval is integrated on its own grid of
-    that spacing (adjoint_grid); None: one step per interval."""
+    that spacing (adjoint_grid); None: one step per interval.  ``step_control``: as in solve_forward, with first_step the
+    first dt of every interval."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -719,7 +726,7 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     grids = _grids([t_list], t_is_f32, step_size, False)
     if _use_rows(lib, dev, G, H, B, True, single=True, T=T):
         return _adjoint_rows(lib, net, packed, G, H, dev, [t_list], t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[0].shape), param_mask, grids)
+                             tuple(ys[0].shape), param_mask, grids, step_control)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
     grid = _Grid(grids, False) if grids is not None else None
     if grid is not None and engine == "resident":
@@ -730,7 +737,8 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     grads = new_flat_grads(net, P, ys.device)
     st = _new_status()
     log, cap = _steplog()
-    d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask)
+    d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask,
+                    step_control=step_control)
     d.y_saved, d.grad_y, d.adj_y0, d.grads = ys.data_ptr(), gy.data_ptr(), adj_y0.data_ptr(), grads.data_ptr()
     if grid is not None:
         grid.put(d)
@@ -801,11 +809,12 @@ def _fan_in(dev, streams):
 
 
 @_on_model_device
-def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_steps, step_size=None):
+def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_steps, step_size=None, step_control=None):
     """y0 ``[N, *S, G]``: N independent problems, problem i integrated over its own times ``t_rows[i]`` (all of length
     T).  Every problem is one resident launch with its own step controller -- exactly the reference's per-sample call
     (train_insilico.py:128-130) -- but the weights are packed, the workspace fetched and the arguments marshalled once
-    for the whole set.  Returns ``[N, T, *S, G]``.  ``step_size``: as in solve_forward, every problem on its own grid."""
+    for the whole set.  Returns ``[N, T, *S, G]``.  ``step_size``: as in solve_forward, every problem on its own grid;
+    ``step_control``: as in solve_forward."""
     packed, G, H, dev = packed_weights(net)
     if y0.shape[-1] != G:
         raise RuntimeError("last dimension of y0 (%d) must equal ndim (%d)" % (y0.shape[-1], G))
@@ -820,7 +829,7 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
     grids = _grids(t_rows, t_is_f32, step_size, True)
     if _use_rows(lib, dev, G, H, B, False):
         return _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, False, method, rtol, atol, max_num_steps,
-                             (N, T) + tuple(y0c.shape[1:]), grids)
+                             (N, T) + tuple(y0c.shape[1:]), grids, step_control)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, False)
     if grids is not None and engine == "resident":
         nb += _Grid(grids, True).nbytes(lib, N, T)
@@ -834,7 +843,8 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
     if streams:
         _fan_out(dev, streams)
     per = _problems_per_launch(T) if (engine == "resident" and not streams and not STEP_LOGGING) else 1
-    d = _solve_desc(engine, False, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps)
+    d = _solve_desc(engine, False, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps,
+                    step_control=step_control)
     if per > 1:
         # genome-scale model: a solve fills the GPU, so the problems go through ONE persistent launch a few at a time
         # and the weights are staged on chip once per launch instead of once per problem
@@ -873,10 +883,10 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
 
 @_on_model_device
 def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
-                       param_mask=_lib.PARAMS_ALL, step_size=None):
+                       param_mask=_lib.PARAMS_ALL, step_size=None, step_control=None):
     """Backward sweeps of N independent problems (``y_saved``, ``grad_y``: ``[N, T, *S, G]``): adj_y0 ``[N, *S, G]`` and
     the six parameter cotangents summed over the problems (what autograd accumulates into ``.grad``); zeros for the
-    parameters outside ``param_mask``; ``step_size``: see solve_adjoint)."""
+    parameters outside ``param_mask``; ``step_size``, ``step_control``: see solve_adjoint)."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -888,7 +898,7 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     grids = _grids(t_rows, t_is_f32, step_size, False)
     if _use_rows(lib, dev, G, H, B, True):
         return _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[:, 0].shape), param_mask, grids)
+                             tuple(ys[:, 0].shape), param_mask, grids, step_control)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
     if grids is not None and engine == "resident":
         nb += _Grid(grids, False).nbytes(lib, N, T)
@@ -906,7 +916,8 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     tarr = _t_rows(t_rows)
     streams = _concurrency(lib, dev, G, H, B, True, engine, N)
     per = _problems_per_launch(T) if (engine == "resident" and not streams and not STEP_LOGGING) else 1
-    d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask)
+    d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask,
+                    step_control=step_control)
     for lo in range(0, N, chunk):
         hi = min(N, lo + chunk)
         if per > 1:

@@ -44,9 +44,35 @@ def _step_size(method, options):
     return (v, h.dtype) if torch.is_tensor(h) else v
 
 
+_STEP_CONTROL = ('first_step', 'safety', 'ifactor', 'dfactor')
+
+
+def _step_control(method, options):
+    """The dopri5 step-control options (rk_common.py:111-228, misc.py:94-103) as a tuple of floats (first_step, safety,
+    ifactor, dfactor), 0.0 for one not given (the engine's default: Hairer's initial-step estimate, 0.9, 10, 0.2), or
+    None when none of them is given.  Only dopri5 takes them (the fixed-grid methods: the generic refusal of
+    _normalise).  Non-positive or non-finite values are refused: the reference would loop or hit its underflow
+    assertion."""
+    if not options or (method or 'dopri5') != 'dopri5' or not any(k in options for k in _STEP_CONTROL):
+        return None
+    out = []
+    for k in _STEP_CONTROL:
+        if k not in options:
+            out.append(0.0)
+            continue
+        v = options[k]
+        if torch.is_tensor(v) and v.dim() != 0:
+            raise NotImplementedError("a tensor {} must be 0-dimensional (got shape {})".format(k, tuple(v.shape)))
+        f = float(v)
+        if not (f > 0 and f != float('inf')):
+            raise ValueError("{} must be a positive finite number (got {})".format(k, v))
+        out.append(f)
+    return tuple(out)
+
+
 def _normalise(func, y0, t, rtol, atol, method, options):
     """The checks of misc.py:165-241 that apply to a single-tensor state; returns the pieces the kernels need (the
-    fixed-grid ``step_size`` is checked here and read with _step_size)."""
+    fixed-grid ``step_size`` and the dopri5 step control are checked here and read with _step_size / _step_control)."""
     if not torch.is_tensor(y0):
         assert isinstance(y0, tuple), 'y0 must be either a torch.Tensor or a tuple'
         raise NotImplementedError("tuple-valued states are not part of the PHOENIX path (ODENet has a tensor state)")
@@ -65,9 +91,13 @@ def _normalise(func, y0, t, rtol, atol, method, options):
     options.pop('dtype', None)
     if _step_size(method, options) is not None:
         options.pop('step_size')
+    if _step_control(method, options) is not None:
+        for k in _STEP_CONTROL:
+            options.pop(k, None)
     if options:
-        raise NotImplementedError("solver options {} are not supported on the B200 path (the reference never passes "
-                                  "options)".format(sorted(options)))
+        raise NotImplementedError("solver options {} are not supported on the B200 path with method {!r} (it takes "
+                                  "max_num_steps and dtype; dopri5 also first_step, safety, ifactor and dfactor; "
+                                  "euler, midpoint and rk4 also step_size)".format(sorted(options), method))
     assert torch.is_tensor(t), 't must be a torch.Tensor'
     assert t.ndimension() == 1, "{} must be one dimensional".format('t')
     if not torch.is_floating_point(t):
@@ -102,12 +132,13 @@ def odeint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None):
     (odeint.py:25-69).  Not differentiable — use ``odeint_adjoint`` (what every PHOENIX script imports as ``odeint``,
     train_insilico.py:15-18) when gradients are needed."""
     tl, t_is_f32, rev, rtol, atol, method, max_steps = _normalise(func, y0, t, rtol, atol, method, options)
-    step = _step_size(method, options)
+    step, ctl = _step_size(method, options), _step_control(method, options)
     if torch.is_grad_enabled() and (y0.requires_grad or any(p.requires_grad for p in func.parameters())):
         warnings.warn("phoenix_b200.odeint does not record an autograd graph; use odeint_adjoint for gradients",
                       stacklevel=2)
     with torch.no_grad():
-        return engine.solve_forward(func, y0, tl, t_is_f32, rev, method, rtol, atol, max_steps, **_stepped(step))
+        return engine.solve_forward(func, y0, tl, t_is_f32, rev, method, rtol, atol, max_steps, **_stepped(step),
+                                    **_controlled((ctl,), 0))
 
 
 # ---- the per-sample loop of training_step, backward side ----------------------------------------------------------------
@@ -142,8 +173,9 @@ def _register_node(ctx, func, y0, tl, t_is_f32, adj):
     with _defer_lock:
         _node_seq[0] += 1
         ctx.seq = _node_seq[0]
-        # adj[4], the adjoint parameter mask with the norm bit, and adj[5], the backward step size, are part of the key:
-        # only nodes with the same adjoint set, error norm and step grid spacing share a sweep
+        # adj[4], the adjoint parameter mask with the norm bit, adj[5], the backward step size, and adj[6], its dopri5
+        # step control when given, are part of the key: only nodes with the same adjoint set, error norm, step grid spacing and
+        # controller share a sweep
         ctx.group = (len(tl), t_is_f32, adj, tuple(y0.shape), y0.device, tuple(ctx.needs_input_grad[9:]))
         nodes = _live_nodes.get(func)
         if nodes is None:
@@ -202,10 +234,12 @@ class OdeintAdjointMethod(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, func, tl, t_is_f32, fwd, rtol, atol, max_steps, adj, y0, *adjoint_params):
-        # fwd = (method, step_size); adj = (method, rtol, atol, max_num_steps, mask, step_size) of the backward
+        # fwd = (method, step_size); adj = (method, rtol, atol, max_num_steps, mask, step_size) of the backward; each
+        # with the dopri5 step control appended when it is given (_with_control)
         ctx.func, ctx.tl, ctx.t_is_f32, ctx.adj = func, tl, t_is_f32, adj
         with torch.no_grad():
-            y = engine.solve_forward(func, y0, tl, t_is_f32, False, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]))
+            y = engine.solve_forward(func, y0, tl, t_is_f32, False, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]),
+                                     **_controlled(fwd, 2))
         ctx.save_for_backward(y)
         _register_node(ctx, func, y0, tl, t_is_f32, adj)
         return y
@@ -219,7 +253,7 @@ class OdeintAdjointMethod(torch.autograd.Function):
         batch = _defer(ctx, y, grad_y) if (ctx.group is not None and DEFER_ADJOINT) else _NOT_DEFERRED
         if batch is None:
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))
-        kw = dict(_masked(mask), **_stepped(ctx.adj[5]))
+        kw = dict(_masked(mask), **_stepped(ctx.adj[5]), **_controlled(ctx.adj, 6))
         with torch.no_grad():
             if batch is _NOT_DEFERRED:
                 adj_y0, grads = engine.solve_adjoint(ctx.func, ctx.tl, ctx.t_is_f32, a_method, a_rtol, a_atol, a_max,
@@ -245,6 +279,18 @@ def _stepped(step_size):
     if isinstance(step_size, tuple):
         return {"step_size": torch.tensor(step_size[0], dtype=step_size[1])}
     return {"step_size": step_size}
+
+
+def _with_control(tup, step_control):
+    """The fwd / adj tuple of an adjoint node with the dopri5 step control (_step_control's tuple) appended; without one
+    the tuple is what it always was."""
+    return tup if step_control is None else tup + (step_control,)
+
+
+def _controlled(tup, i):
+    """The engine's keyword for the step control at tup[i] (_with_control); without one the engine is called as it always
+    was."""
+    return {} if len(tup) <= i or tup[i] is None else {"step_control": tup[i]}
 
 
 def _grads_out(ctx, adj_y0, grads, mask):
@@ -317,18 +363,19 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
     same = (adjoint_rtol is rtol and adjoint_atol is atol and adjoint_method is method and not adjoint_options
             and not options)
     tl, t_is_f32, rev, rtol, atol, method, max_steps = _normalise(func, y0, t, rtol, atol, method, options)
-    step = _step_size(method, options)
+    step, ctl = _step_size(method, options), _step_control(method, options)
     if same:
-        a_rtol, a_atol, a_method, a_max, a_step = rtol, atol, method, max_steps, step
+        a_rtol, a_atol, a_method, a_max, a_step, a_ctl = rtol, atol, method, max_steps, step, ctl
     else:
         _, _, _, a_rtol, a_atol, a_method, a_max = _normalise(func, y0, t, adjoint_rtol, adjoint_atol, adjoint_method,
                                                               adjoint_options)
-        a_step = _step_size(a_method, adjoint_options)
+        a_step, a_ctl = _step_size(a_method, adjoint_options), _step_control(a_method, adjoint_options)
     if rev:
         raise NotImplementedError("odeint_adjoint with decreasing t is not part of the PHOENIX path")
     params, mask = _adjoint_mask(func, adjoint_params)
-    return OdeintAdjointMethod.apply(func, tl, t_is_f32, (method, step), rtol, atol, max_steps,
-                                     (a_method, a_rtol, a_atol, a_max, mask | norm_bit, a_step), y0, *params)
+    return OdeintAdjointMethod.apply(func, tl, t_is_f32, _with_control((method, step), ctl), rtol, atol, max_steps,
+                                     _with_control((a_method, a_rtol, a_atol, a_max, mask | norm_bit, a_step), a_ctl),
+                                     y0, *params)
 
 
 class OdeintAdjointManyMethod(torch.autograd.Function):
@@ -338,7 +385,8 @@ class OdeintAdjointManyMethod(torch.autograd.Function):
     def forward(ctx, func, t_rows, t_is_f32, fwd, rtol, atol, max_steps, adj, y0, *adjoint_params):
         ctx.func, ctx.t_rows, ctx.t_is_f32, ctx.adj = func, t_rows, t_is_f32, adj
         with torch.no_grad():
-            y = engine.solve_forward_many(func, y0, t_rows, t_is_f32, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]))
+            y = engine.solve_forward_many(func, y0, t_rows, t_is_f32, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]),
+                                          **_controlled(fwd, 2))
         ctx.save_for_backward(y)
         return y
 
@@ -350,7 +398,8 @@ class OdeintAdjointManyMethod(torch.autograd.Function):
             return (None,) * (9 + len(ctx.needs_input_grad[9:]))
         with torch.no_grad():
             adj_y0, grads = engine.solve_adjoint_many(ctx.func, ctx.t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
-                                                      a_max, y, grad_y, **_masked(mask), **_stepped(ctx.adj[5]))
+                                                      a_max, y, grad_y, **_masked(mask), **_stepped(ctx.adj[5]),
+                                                      **_controlled(ctx.adj, 6))
         return _grads_out(ctx, adj_y0, grads, mask)
 
 
@@ -375,12 +424,14 @@ def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=
         assert all(b > a for a, b in zip(r, r[1:])), 't must be strictly increasing for every sample'
     if rev:
         raise NotImplementedError("odeint_adjoint_many with decreasing t is not part of the PHOENIX path")
-    step = _step_size(method, options)
+    step, ctl = _step_size(method, options), _step_control(method, options)
     adjoint_options, norm_bit = _adjoint_norm(adjoint_options)
-    a_max, a_step = max_steps, step
+    a_max, a_step, a_ctl = max_steps, step, ctl
     if adjoint_options is not None:
         a_max = _normalise(func, y0[0], t[0], rtol, atol, method, adjoint_options)[6]
-        a_step = _step_size(method, adjoint_options)
+        a_step, a_ctl = _step_size(method, adjoint_options), _step_control(method, adjoint_options)
     params, mask = _adjoint_mask(func, adjoint_params)
-    return OdeintAdjointManyMethod.apply(func, rows, t_is_f32, (method, step), rtol_f, atol_f, max_steps,
-                                         (method, rtol_f, atol_f, a_max, mask | norm_bit, a_step), y0, *params)
+    return OdeintAdjointManyMethod.apply(func, rows, t_is_f32, _with_control((method, step), ctl), rtol_f, atol_f,
+                                         max_steps,
+                                         _with_control((method, rtol_f, atol_f, a_max, mask | norm_bit, a_step), a_ctl),
+                                         y0, *params)
