@@ -302,7 +302,15 @@ int phx_rows_grad_parts(const phx_ctx* ctx, int G, int H, int N);
  *   safety, ifactor, dfactor: with the error ratio r, the next dt is dt * ifactor when r == 0, else
  *     dt * min(ifactor, max(safety / r^(1/5), r < 1 ? 1 : dfactor)).
  * A negative, NaN or infinite value in any of the four, or a nonzero one with a method other than dopri5, returns
- * PHX_ERR_INVALID. */
+ * PHX_ERR_INVALID.
+ *
+ * Gradients with respect to t (adjoint.py, backward with t requiring grad): t_vjp (a DEVICE array, [N][T-1], e.g. the
+ * one phx_time_vjp writes; NULL: all zero) is the time cotangent v carried through each output interval, the interval
+ * [t[i], t[i+1]] at index i.  The RHS is autonomous, so v is constant over the interval and the adjoint solve only
+ * reads it: in dopri5's initial-step estimate of the interval, where it is the one-element block of the mixed norm
+ * (d0 = max(d0, |v| / (atol + |v| * rtol)), also under the seminorm; it is computed but unused with first_step), and
+ * in the non-finite check of the initial state (a non-finite v gives PHX_ST_NONFINITE).  Fixed grids use no norm and
+ * are unaffected.  A non-NULL t_vjp on a forward solve returns PHX_ERR_INVALID. */
 enum { PHX_ENGINE_RESIDENT = 0, PHX_ENGINE_ROWS = 1, PHX_ENGINE_STREAM = 2 };
 typedef struct phx_solve_desc {
     const float* packed;
@@ -324,12 +332,26 @@ typedef struct phx_solve_desc {
     double rtol, atol;
     int64_t max_num_steps;
     double first_step, safety, ifactor, dfactor;   /* dopri5 step control; 0: the default */
+    const float* t_vjp;              /* adjoint, [N][T-1] device array; NULL: v = 0 */
     int32_t engine, adjoint, G, H, B, N, T, t_is_f32, reversed, method, param_mask, steplog_cap;
 } phx_solve_desc;
 int phx_solve(phx_ctx* ctx, const phx_solve_desc* desc, void* stream);
 size_t phx_grid_workspace_bytes(int N, int T, int64_t total_steps);
 int phx_unpack_grads(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
                      int accumulate, void* stream);
+/* ---- time cotangents of the adjoint backward (adjoint.py, backward with t requiring grad) ----------------------------
+ * For N problems with saved outputs y_saved and their cotangents grad_y ([N][T][B][G]), the reference's backward
+ * forms, before integrating interval i = T-1 .. 1, dLd_i = f(y_saved[i]) . grad_y[i] (f = ODENet.forward, summed over
+ * the B rows and G genes) and subtracts it from the time cotangent vjp_t, which the autonomous RHS then carries
+ * through the interval unchanged.  phx_time_vjp writes t_grad[N][T] (t_grad[i] = dLd_i for i >= 1, t_grad[0] = the
+ * final vjp_t, i.e. -(dLd_{T-1} + ... + dLd_1) accumulated in fp32 in that order) and t_vjp[N][T-1] (the vjp_t each
+ * interval starts from, the interval [t[i], t[i+1]] at index i: what phx_solve_desc.t_vjp takes).  f comes from the
+ * contraction of phx_rhs_forward; the dot products are summed in float64 in a fixed order, so results are identical
+ * from run to run.  Nothing synchronises the stream.  T = 1 gives t_grad = 0 and no t_vjp. */
+size_t phx_time_vjp_workspace_bytes(int G, int H, int B, int N, int T);
+int phx_time_vjp(phx_ctx* ctx, int G, int H, int B, int N, int T, const float* packed, const float* y_saved,
+                 const float* grad_y, float* t_grad, float* t_vjp, void* workspace, size_t workspace_bytes,
+                 void* stream);
 int phx_unpack_grads_masked(phx_ctx* ctx, int G, int H, const float* packed_grads, int nparts, float* grads_flat,
                             int accumulate, int param_mask, void* stream);
 /* Cotangent of the data loss of training_step, loss = torch.mean((predictions - targets)**2) (train_insilico.py:132):

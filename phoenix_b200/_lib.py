@@ -28,7 +28,7 @@ EXPORTS = [
     "phx_stream_workspace_bytes", "phx_stream_solve_forward", "phx_stream_solve_adjoint",
     "phx_rows_supported", "phx_rows_plan_describe", "phx_rows_workspace_bytes", "phx_solve_forward_rows",
     "phx_solve_adjoint_rows", "phx_unpack_grads", "phx_packed_grad_bytes", "phx_rows_grad_parts",
-    "phx_unpack_grads_masked", "phx_solve", "phx_grid_workspace_bytes",
+    "phx_unpack_grads_masked", "phx_solve", "phx_grid_workspace_bytes", "phx_time_vjp", "phx_time_vjp_workspace_bytes",
     "phx_prior_loss", "phx_prior_setup", "phx_tc_set_pair", "phx_tc_prof_dump", "phx_ctx_set_global_norm", "phx_peer_allreduce", "phx_peer_allreduce_nvls", "phx_mse_grad", "phx_hill_planes", "phx_hill_cache_set",
 ]
 
@@ -47,7 +47,7 @@ class PhxSolveDesc(ctypes.Structure):
                 + [("workspace_bytes", ctypes.c_size_t), ("status", ctypes.c_void_p), ("steplog", ctypes.c_void_p),
                    ("rtol", ctypes.c_double), ("atol", ctypes.c_double), ("max_num_steps", ctypes.c_int64),
                    ("first_step", ctypes.c_double), ("safety", ctypes.c_double), ("ifactor", ctypes.c_double),
-                   ("dfactor", ctypes.c_double)]
+                   ("dfactor", ctypes.c_double), ("t_vjp", ctypes.c_void_p)]
                 + [(name, ctypes.c_int32) for name in (
                     "engine", "adjoint", "G", "H", "B", "N", "T", "t_is_f32", "reversed", "method", "param_mask",
                     "steplog_cap")])
@@ -156,6 +156,10 @@ def _declare(lib):
     lib.phx_solve.restype = c_int
     lib.phx_grid_workspace_bytes.argtypes = [c_int, c_int, c_int64]
     lib.phx_grid_workspace_bytes.restype = c_size_t
+    lib.phx_time_vjp_workspace_bytes.argtypes = [c_int] * 5
+    lib.phx_time_vjp_workspace_bytes.restype = c_size_t
+    lib.phx_time_vjp.argtypes = [c_void_p] + [c_int] * 5 + [c_void_p] * 6 + [c_size_t, c_void_p]
+    lib.phx_time_vjp.restype = c_int
     lib.phx_prior_loss.argtypes = [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, ctypes.c_float, c_void_p,
                                    c_void_p, c_void_p, c_size_t, c_void_p]
     lib.phx_prior_loss.restype = c_int

@@ -104,6 +104,53 @@ __global__ void mse_grad_kernel(int rows, int G, const float* __restrict__ pred,
         grad[r * grad_stride + g] = scale * (pred[r * pred_stride + g] - target[i]);
     }
 }
+// time cotangents (phx_time_vjp).  Block q = (problem n, output i >= 1, chunk c), c fastest, sums f * grad_y over the
+// elements [c * chunk, (c + 1) * chunk) of output i in float64 (products of two floats are exact there) with a fixed
+// thread stride and a fixed tree, and writes its partial sum to part[q].  Problem n's f starts at f + n * fstride
+constexpr int TV_THREADS = 256;
+__global__ void __launch_bounds__(TV_THREADS) time_dot_kernel(size_t BG, int T, int nch, size_t chunk, size_t fstride,
+                                                              const float* __restrict__ f, const float* __restrict__ g,
+                                                              double* __restrict__ part) {
+    __shared__ double red[TV_THREADS];
+    const size_t q = blockIdx.x;
+    const int c = (int)(q % nch);
+    const size_t iv = q / nch;                     // n * (T-1) + i-1
+    const size_t n = iv / (T - 1), i = iv % (T - 1) + 1;
+    const size_t fb = n * fstride + i * BG, gb = (n * T + i) * BG;
+    const size_t lo = (size_t)c * chunk, hi = lo + chunk < BG ? lo + chunk : BG;
+    double acc = 0.0;
+    for (size_t k = lo + threadIdx.x; k < hi; k += TV_THREADS) acc += (double)f[fb + k] * (double)g[gb + k];
+    red[threadIdx.x] = acc;
+    __syncthreads();
+    for (int s = TV_THREADS / 2; s > 0; s >>= 1) {
+        if (threadIdx.x < s) red[threadIdx.x] += red[threadIdx.x + s];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) part[q] = red[0];
+}
+// one thread per problem: dLd_i = the chunk sums of output i in chunk order, rounded to fp32, then the reference's running
+// fp32 subtraction vjp_t -= dLd_i for i = T-1 .. 1
+__global__ void time_scan_kernel(int N, int T, int nch, const double* __restrict__ part, float* __restrict__ t_grad,
+                                 float* __restrict__ t_vjp) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    float v = 0.f;
+    for (int i = T - 1; i >= 1; --i) {
+        const double* pq = part + ((size_t)n * (T - 1) + i - 1) * nch;
+        double s = 0.0;
+        for (int c = 0; c < nch; ++c) s += pq[c];
+        const float d = (float)s;
+        t_grad[(size_t)n * T + i] = d;
+        v = v - d;
+        t_vjp[(size_t)n * (T - 1) + i - 1] = v;
+    }
+    t_grad[(size_t)n * T] = v;
+}
+// elements of one output per time_dot_kernel block, and the number of such chunks
+constexpr size_t TV_CHUNK = 16 * TV_THREADS;
+int time_vjp_chunks(size_t BG) { return (int)((BG + TV_CHUNK - 1) / TV_CHUNK); }
+size_t round256(size_t n) { return (n + 255) & ~(size_t)255; }
+
 __global__ void unpack_rest_kernel(int G, int H, int Hp, int K2, const float* __restrict__ wabar,
                                    const float* __restrict__ biasbar, const float* __restrict__ mbar, int nparts,
                                    size_t pstride, float* __restrict__ Wa, float* __restrict__ bs,
@@ -465,6 +512,7 @@ bool check_request(const phx_solve_desc& d) {
     const char* why = nullptr;
     if (d.adjoint && d.reversed) why = "an adjoint solve takes no `reversed`";
     else if (!d.adjoint && d.param_mask) why = "param_mask is for adjoint solves";
+    else if (!d.adjoint && d.t_vjp) why = "t_vjp is for adjoint solves";
     else if (d.adjoint && (d.grid_out_step || d.grid_out_slope)) why = "grid_out_step / grid_out_slope are for forward solves";
     else if (!d.grid_dt && (d.grid_steps || d.grid_out_step || d.grid_out_slope)) why = "a step grid needs grid_dt";
     else if (d.engine == PHX_ENGINE_STREAM && d.N != 1) why = "the streaming engine solves one problem per call (N = 1)";
@@ -575,6 +623,7 @@ int solve_on_chip(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t stream) {
         p.ysaved = d.y_saved;
         p.grad_y = d.grad_y;
         p.adj_y0 = d.adj_y0;
+        p.t_vjp = d.t_vjp;
         if (rows) {
             p.theta_ws = ws + o_th;
             p.gsum = d.grads;
@@ -837,6 +886,106 @@ size_t phx_grid_workspace_bytes(int N, int T, int64_t total_steps) {
     if (N < 1 || T < 2 || total_steps < 0) return 0;
     const size_t nseg = (size_t)N * (T - 1);
     return 4 * (((size_t)total_steps + 3) / 4 * 4 + (nseg + 4) / 4 * 4 + 2 * ((nseg + 3) / 4 * 4)) + 16;
+}
+
+/* ---- time cotangents of the adjoint backward (adjoint.py, backward with t requiring grad) ------------------------------ */
+}  // extern "C"
+namespace {
+// rows of one problem's RHS launch: its T * B saved rows, padded to the tensor-core minimum (the CUDA-core contraction of a
+// handful of rows runs its whole K = G loop in a few CTAs; the padding rows are zeros, and every output row depends on its
+// own input row only)
+int time_vjp_rows(int H, int B, int T, bool tc) {
+    const int rows = T * B, padded = rows > phx_tc_min_rows_rt() ? rows : phx_tc_min_rows_rt();
+    return tc && phx_tc_shape_ok(H, padded) ? padded : rows;
+}
+// workspace: the RHS workspace of one problem's launch | the padded input rows | f of all N problems | the partial dot
+// products, each part 256-byte aligned
+struct TimeVjpWs {
+    size_t ypad, f, part, total;
+};
+TimeVjpWs time_vjp_ws(int G, int H, int B, int N, int T, int rp) {
+    TimeVjpWs o;
+    o.ypad = round256(phx_rhs_workspace_bytes(G, H, rp));
+    o.f = o.ypad + (rp > T * B ? round256(sizeof(float) * (size_t)rp * G) : 0);
+    o.part = o.f + round256(sizeof(float) * (size_t)N * rp * G);
+    o.total = o.part + round256(sizeof(double) * (size_t)N * (T - 1) * time_vjp_chunks((size_t)B * G));
+    return o;
+}
+}  // namespace
+extern "C" {
+
+size_t phx_time_vjp_workspace_bytes(int G, int H, int B, int N, int T) {
+    if (G < 1 || H < 1 || B < 1 || N < 1 || T < 1) return 0;
+    if (T == 1) return 256;
+    return time_vjp_ws(G, H, B, N, T, time_vjp_rows(H, B, T, true)).total;
+}
+
+int phx_time_vjp(phx_ctx* ctx, int G, int H, int B, int N, int T, const float* packed, const float* y_saved,
+                 const float* grad_y, float* t_grad, float* t_vjp, void* workspace, size_t workspace_bytes,
+                 void* stream) {
+    PhxDevGuard dev_guard(ctx);
+    if (!ctx || !check_dims(G, H, B)) return PHX_ERR_INVALID;
+    if (N < 1 || T < 1 || !t_grad || (T > 1 && (!packed || !y_saved || !grad_y || !t_vjp || !workspace))) {
+        phx_set_error("time_vjp: N=%d and T=%d must be >= 1, and the arrays non-null", N, T);
+        return PHX_ERR_INVALID;
+    }
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (T > 1) {
+        const int rows = T * B, rp = time_vjp_rows(H, B, T, ctx->precision != PHX_PREC_FP32);
+        const TimeVjpWs o = time_vjp_ws(G, H, B, N, T, rp);
+        const size_t need = o.total;
+        if (workspace_bytes < need) {
+            phx_set_error("time_vjp workspace too small: %zu < %zu", workspace_bytes, need);
+            return PHX_ERR_WORKSPACE;
+        }
+        if ((uintptr_t)workspace & 255) {
+            phx_set_error("time_vjp workspace must be 256-byte aligned");
+            return PHX_ERR_INVALID;
+        }
+        // f at every saved output of a problem (the unused t[0] one too: the rows stay contiguous), one problem per
+        // launch: the contraction (CUDA or tensor cores, its blocking) depends on the number of rows, and a problem must
+        // get the same f -- and so the same dopri5 steps -- alone or beside others
+        const size_t BG = (size_t)B * G, fstride = (size_t)rp * G;
+        char* ws = (char*)workspace;
+        float* ypad = (float*)(ws + o.ypad);
+        float* f = (float*)(ws + o.f);
+        double* part = (double*)(ws + o.part);
+        PhxPacked w;
+        int rc = phx_tc_prepare(ctx, G, H, rp, packed, &w, st);
+        if (rc != PHX_OK) return rc;
+        cudaError_t e = cudaSuccess;
+        if (rp > rows)
+            e = cudaMemsetAsync(ypad + (size_t)rows * G, 0, sizeof(float) * (size_t)(rp - rows) * G, st);
+        for (int n = 0; n < N && rc == PHX_OK && e == cudaSuccess; ++n) {
+            const float* yn = y_saved + (size_t)n * rows * G;
+            if (rp > rows) {
+                e = cudaMemcpyAsync(ypad, yn, sizeof(float) * (size_t)rows * G, cudaMemcpyDeviceToDevice, st);
+                yn = ypad;
+            }
+            if (e == cudaSuccess) rc = phx_rhs_forward_launch(G, H, rp, w, yn, f + n * fstride, 1, 1.f, (float*)ws, st);
+        }
+        if (e != cudaSuccess) {
+            phx_set_error("time_vjp copy: %s", cudaGetErrorString(e));
+            return PHX_ERR_CUDA;
+        }
+        if (rc != PHX_OK) return rc;
+        const int nch = time_vjp_chunks(BG);
+        time_dot_kernel<<<(unsigned)((size_t)N * (T - 1) * nch), TV_THREADS, 0, st>>>(BG, T, nch, TV_CHUNK, fstride, f,
+                                                                                       grad_y, part);
+        time_scan_kernel<<<(N + 127) / 128, 128, 0, st>>>(N, T, nch, part, t_grad, t_vjp);
+    } else {
+        cudaError_t e = cudaMemsetAsync(t_grad, 0, sizeof(float) * N, st);
+        if (e != cudaSuccess) {
+            phx_set_error("cudaMemsetAsync(t_grad): %s", cudaGetErrorString(e));
+            return PHX_ERR_CUDA;
+        }
+    }
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        phx_set_error("time_vjp launch: %s", cudaGetErrorString(e));
+        return PHX_ERR_CUDA;
+    }
+    return PHX_OK;
 }
 
 }  // extern "C"

@@ -288,6 +288,9 @@ struct ResParams {
     const int* goff;
     const int* gout;
     const float* gsl;
+    // adjoint: the time cotangent v of every output interval (phx_solve_desc.t_vjp, [N][T-1], interval [t[i-1], t[i]] of
+    // problem pi at pi*(T-1) + i-1), or nullptr for v = 0.  dopri5 folds it into d0 of the interval's initial step
+    const float* t_vjp;
 };
 #define PHX_PROF_SLOTS 32
 #define PHX_T_INLINE 64

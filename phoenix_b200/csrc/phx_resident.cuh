@@ -66,6 +66,7 @@ struct Ctrl {
     int accept, stop, nonfinite_prev, last;
     int n_acc, n_rej, n_rhs, n_log, n_steps_interval;
     int slot[7];
+    float vjp_t;  // adjoint: the time cotangent of the current interval (fold_t_vjp)
 };
 
 // Optional in-kernel phase timer (diagnostics; phx_ctx_set_profile): thread 0 of CTA 0 accumulates SM-clock deltas
@@ -1233,6 +1234,18 @@ __device__ double next_dt(const ResParams& p, double dt, float ratio) {
 template <bool GRID>
 __device__ __forceinline__ bool given_step(const ResParams& p) { return !GRID && p.first_step > 0; }
 
+// whether the adjoint has time cotangents (phx_solve_desc.t_vjp; never in the step-grid instantiations, which are
+// fixed-grid only).  Read at each use, like given_step
+template <bool GRID>
+__device__ __forceinline__ bool has_t_vjp(const ResParams& p) { return !GRID && p.t_vjp != nullptr; }
+// the time cotangent v of an adjoint interval (Ctrl.vjp_t) as the one-element block of the mixed norm in d0 of Hairer's
+// estimate; returns whether v is non-finite (the reference asserts a finite augmented state)
+__device__ __forceinline__ bool fold_t_vjp(const ResParams& p, float v, float& d0) {
+    const float r = v / (p.atol_f + fabsf(v) * p.rtol_f);
+    d0 = fmaxf(d0, sqrtf(r * r));
+    return !isfinite(v);
+}
+
 // misc.py:47-86 tail: h0 from d0, d1
 __device__ float init_h0(float d0, float d1) {
     if (d0 < 1e-5f || d1 < 1e-5f) return 1e-6f;
@@ -2209,6 +2222,7 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                 c->t_end = t_end;
                 c->n_steps_interval = 0;
                 for (int i = 0; i < 7; ++i) c->slot[i] = i;
+                if (has_t_vjp<GRID>(p)) c->vjp_t = p.t_vjp[(size_t)pi * (p.T - 1) + iv - 1];
             }
             __syncthreads();
             // f0 and Hairer's initial step under the mixed norm max(RMS_y, RMS_a, RMS_theta): two evaluations through
@@ -2263,8 +2277,9 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_adj_kernel(const __grid_co
                         float d1 = fmaxf(fmaxf(sqrtf((float)(c->dsum[3] / Nel)), sqrtf((float)(c->dsum[4] / Nel))),
                                          th_rms(c->dsum[5]));
                         c->d1 = d1;
-                        c->h0 = init_h0(d0, d1);
                         c->nonfinite_prev = c->dsum[6] > 0.0;
+                        if (has_t_vjp<GRID>(p) && fold_t_vjp(p, c->vjp_t, d0)) c->nonfinite_prev = 1;
+                        c->h0 = init_h0(d0, d1);
                         if (given_step<GRID>(p)) {
                             c->dt = p.first_step;
                             c->n_rhs += 1;

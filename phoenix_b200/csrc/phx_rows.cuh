@@ -1652,13 +1652,16 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                         RowCtl& c = rc->r[threadIdx.x];
                         const double* d = dsum + threadIdx.x * 7;
                         if (which == 0) {
-                            const float d0 = fmaxf(fmaxf(sqrtf((float)(d[0] / Nel)), sqrtf((float)(d[1] / Nel))),
-                                                   th_rms(d[2]));
+                            float d0 = fmaxf(fmaxf(sqrtf((float)(d[0] / Nel)), sqrtf((float)(d[1] / Nel))),
+                                             th_rms(d[2]));
+                            const bool bad_v =
+                                c.valid && p.t_vjp &&
+                                fold_t_vjp(p, p.t_vjp[(size_t)(q0 + threadIdx.x) * (p.T - 1) + iv - 1], d0);
                             const float d1 = fmaxf(fmaxf(sqrtf((float)(d[3] / Nel)), sqrtf((float)(d[4] / Nel))),
                                                    th_rms(d[5]));
                             c.d1 = d1;
                             c.h0 = init_h0(d0, d1);
-                            c.nonfinite_prev = d[6] > 0.0;
+                            c.nonfinite_prev = d[6] > 0.0 || bad_v;
                             if (p.first_step > 0) {
                                 c.dt = p.first_step;
                                 if (!c.done) c.n_rhs += 1;

@@ -282,7 +282,10 @@ struct Stream {
     bool fuse = false;                 // stage algebra in the RHS epilogue (forward solves on the tensor-core path)
     // dopri5 step control (phx_solve_desc): first_step > 0 replaces Hairer's estimate; the controller constants
     double first_step = 0, safety = 0.9, ifactor = 10.0, dfactor = 0.2;
-    int pmask = PHX_P_ALL;             // adjoint: parameters whose cotangents make up the theta segment
+    // adjoint: the time cotangent v of the interval being solved (phx_solve_desc.t_vjp), in pinned host memory that is
+    // filled on the stream before the first synchronisation of the solve; nullptr: v = 0
+    const float* vjp_t = nullptr;
+    int pmask = PHX_P_ALL;            // adjoint: parameters whose cotangents make up the theta segment
     PhxGradOff goff{};                 // adjoint: their offsets in the theta segment (back to back, reference order)
 
     // stage derivative `slot` of every segment at the current stage inputs (at_x0: at the step's start values themselves,
@@ -449,12 +452,20 @@ struct Stream {
         if ((rc = fetch_sums()) != PHX_OK) return rc;
         bool nonfinite = false;
         for (size_t si = 0; si < ns; ++si) nonfinite = nonfinite || (segs[si].in_norm && sums_host[3 * si + 2] > 0.0);
+        // v as the one-element block of the mixed norm (read after the fetch: its copy was enqueued before it)
+        float d0v = 0.f;
+        if (vjp_t) {
+            const float v = *vjp_t, r = v / (atol_f + fabsf(v) * rtol_f);
+            d0v = sqrtf(r * r);
+            nonfinite = nonfinite || !isfinite(v);
+        }
         double dt = first_step;
         if (first_step > 0) {
             // the caller's first step: the fetch above was for the non-finite count only
             status.n_rhs += 1;
         } else {
             float d0 = block_norm(0), d1 = block_norm(1);
+            if (vjp_t) d0 = fmaxf(d0, d0v);
             float h0 = (d0 < 1e-5f || d1 < 1e-5f) ? 1e-6f : 0.01f * d0 / d1;
             {
                 std::vector<KSet> ks(ns);
@@ -798,7 +809,30 @@ int phx_stream_adjoint(phx_ctx* ctx, const phx_solve_desc& d, cudaStream_t st) {
     if (PS > 0) S.segs.push_back(th);
     cudaMemsetAsync(grads_flat, 0, P * sizeof(float), st);
     cudaMemcpyAsync(S.segs[1].x0, grad_y + (size_t)(T - 1) * BG, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
+    // the time cotangents of the T-1 intervals, fetched once: dopri5 reads interval iv's after its first synchronisation
+    float* tv = nullptr;
+    if (d.t_vjp && method == PHX_DOPRI5) {
+        static thread_local float* pinned_tv = nullptr;
+        static thread_local int pinned_cap = 0;
+        if (pinned_cap < T - 1) {
+            if (pinned_tv) cudaFreeHost(pinned_tv);
+            pinned_cap = 0;
+            if (cudaMallocHost((void**)&pinned_tv, sizeof(float) * (T - 1)) != cudaSuccess) {
+                pinned_tv = nullptr;
+                phx_set_error("cudaMallocHost failed");
+                return PHX_ERR_CUDA;
+            }
+            pinned_cap = T - 1;
+        }
+        tv = pinned_tv;
+        cudaError_t e = cudaMemcpyAsync(tv, d.t_vjp, sizeof(float) * (T - 1), cudaMemcpyDeviceToHost, st);
+        if (e != cudaSuccess) {
+            phx_set_error("cudaMemcpyAsync(t_vjp): %s", cudaGetErrorString(e));
+            return PHX_ERR_CUDA;
+        }
+    }
     for (int iv = T - 1; iv >= 1 && rc == PHX_OK && S.status.code == PHX_ST_OK; --iv) {
+        S.vjp_t = tv ? tv + iv - 1 : nullptr;
         cudaMemcpyAsync(S.segs[0].x0, y_saved + (size_t)iv * BG, BG * sizeof(float), cudaMemcpyDeviceToDevice, st);
         if (method != PHX_DOPRI5 && grid_dt) {
             for (int k = goff[iv - 1]; k < goff[iv] && rc == PHX_OK; ++k) rc = S.fixed_step(grid_dt[k]);

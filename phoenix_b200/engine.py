@@ -538,16 +538,19 @@ _ENGINE_IDS = {"resident": _lib.ENGINE_RESIDENT, "rows": _lib.ENGINE_ROWS, "stre
 
 
 def _solve_desc(engine, adjoint, packed, G, H, B, N, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask=0,
-                reversed_time=False, step_control=None):
+                reversed_time=False, step_control=None, t_vjp=None):
     """The phx_solve request of a solve on ``engine`` ('resident' | 'rows' | 'stream'), with the fields all its launches
     share; each launch points it at its own times, state, workspace and status (_launch).  ``step_control``: dopri5's
-    (first_step, safety, ifactor, dfactor), 0 for a default, or None for all four defaults."""
+    (first_step, safety, ifactor, dfactor), 0 for a default, or None for all four defaults.  ``t_vjp``: the adjoint's
+    time cotangents [N, T-1] (time_vjp), or None for zero; a launch of a later problem points the request at its row."""
     d = _lib.PhxSolveDesc()
     d.engine, d.adjoint, d.G, d.H, d.B, d.N, d.T = _ENGINE_IDS[engine], int(adjoint), G, H, B, N, T
     d.packed, d.t_is_f32, d.reversed, d.method = packed.data_ptr(), int(t_is_f32), int(reversed_time), _lib.METHOD_IDS[method]
     d.rtol, d.atol, d.max_num_steps, d.param_mask = float(rtol), float(atol), int(max_num_steps), param_mask
     if step_control is not None:
         d.first_step, d.safety, d.ifactor, d.dfactor = (float(v) for v in step_control)
+    if t_vjp is not None:
+        d.t_vjp = t_vjp.data_ptr()
     return d
 
 
@@ -633,10 +636,10 @@ def _forward_rows(lib, net, packed, G, H, dev, y0c, t_rows, t_is_f32, reversed_t
 
 
 def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy, adj_shape,
-                  param_mask=_lib.PARAMS_ALL, grids=None, step_control=None):
+                  param_mask=_lib.PARAMS_ALL, grids=None, step_control=None, t_vjp=None):
     """Backward sweeps of N one-row problems (ys, gy: [N, T, ..., G] memory order): adj_y0 and the SUM over the problems of
     the six parameter cotangents (flat, reference order; zeros for the parameters outside ``param_mask``).  ``grids``:
-    the problems' backward step grids (adjoint_grid), or None; ``step_control``: see _solve_desc."""
+    the problems' backward step grids (adjoint_grid), or None; ``step_control``, ``t_vjp`` ([N, T-1]): see _solve_desc."""
     N, T = len(t_rows), len(t_rows[0])
     nb = lib.phx_rows_workspace_bytes(_lib.ctx(dev), G, H, N, T, 1)
     grid = _Grid(grids, False) if grids is not None else None
@@ -654,7 +657,7 @@ def _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, a
     flat_t = (ctypes.c_double * (N * T))(*[x for r in t_rows for x in r])
     sp = _stream_ptr(dev)
     d = _solve_desc("rows", True, packed, G, H, 1, N, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask,
-                    step_control=step_control)
+                    step_control=step_control, t_vjp=t_vjp)
     d.y_saved, d.grad_y, d.adj_y0, d.grads = ys.data_ptr(), gy.data_ptr(), adj_y0.data_ptr(), gpk.data_ptr()
     if grid is not None:
         grid.put(d)
@@ -708,13 +711,14 @@ def solve_forward(net, y0, t_list, t_is_f32, reversed_time, method, rtol, atol, 
 
 @_on_model_device
 def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
-                  param_mask=_lib.PARAMS_ALL, step_size=None, step_control=None):
+                  param_mask=_lib.PARAMS_ALL, step_size=None, step_control=None, t_vjp=None):
     """adj_y0 and the six parameter cotangents of one backward sweep.  ``param_mask`` (bit i = the i-th parameter in
     reference order): the adjoint parameters, the only ones integrated and put in the error norm; the cotangents of the
     others come back as zeros.  With ``_lib.NORM_SEMINORM`` also set, the dopri5 error norm leaves the parameter block
     out altogether (the seminorm).  ``step_size`` (fixed-grid methods): every interval is integrated on its own grid of
     that spacing (adjoint_grid); None: one step per interval.  ``step_control``: as in solve_forward, with first_step the
-    first dt of every interval."""
+    first dt of every interval.  ``t_vjp``: the time cotangent entering each interval, [1, T-1] float32 on the device
+    (time_vjp), when t needs a gradient; None: zero."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -726,7 +730,7 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     grids = _grids([t_list], t_is_f32, step_size, False)
     if _use_rows(lib, dev, G, H, B, True, single=True, T=T):
         return _adjoint_rows(lib, net, packed, G, H, dev, [t_list], t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[0].shape), param_mask, grids, step_control)
+                             tuple(ys[0].shape), param_mask, grids, step_control, t_vjp)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
     grid = _Grid(grids, False) if grids is not None else None
     if grid is not None and engine == "resident":
@@ -738,13 +742,35 @@ def solve_adjoint(net, t_list, t_is_f32, method, rtol, atol, max_num_steps, y_sa
     st = _new_status()
     log, cap = _steplog()
     d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask,
-                    step_control=step_control)
+                    step_control=step_control, t_vjp=t_vjp)
     d.y_saved, d.grad_y, d.adj_y0, d.grads = ys.data_ptr(), gy.data_ptr(), adj_y0.data_ptr(), grads.data_ptr()
     if grid is not None:
         grid.put(d)
     _launch(lib, dev, d, _t_array(t_list), ws, st, log, cap, "solve_adjoint")
     _finish(st, "adjoint solve", dev)
     return adj_y0, split_flat_grads(grads, G, H)
+
+
+@_on_model_device
+def time_vjp(net, y_saved, grad_y):
+    """The time cotangents of N adjoint backwards (adjoint.py, backward with t requiring grad) from the saved outputs and
+    their cotangents ``[N, T, *S, G]``: ``(t_grad [N, T], t_vjp [N, T-1])``, float32 on the device.  t_grad is the
+    gradient with respect to each problem's t; t_vjp[:, i] is the time cotangent the reference carries through the
+    interval [t[i], t[i+1]], what solve_adjoint / solve_adjoint_many take to start dopri5 there as the reference does.
+    No sweep is needed for them: the RHS is autonomous (include/phoenix_b200.h, phx_time_vjp)."""
+    packed, G, H, dev = packed_weights(net)
+    ys = y_saved.detach().contiguous()
+    gy = grad_y.detach().to(torch.float32).contiguous()
+    N, T = ys.shape[0], ys.shape[1]
+    B = ys[0, 0].numel() // G
+    t_grad = torch.empty(N, T, dtype=torch.float32, device=ys.device)
+    t_vjp = torch.empty(N, T - 1, dtype=torch.float32, device=ys.device)
+    lib = _lib.load()
+    nb = lib.phx_time_vjp_workspace_bytes(G, H, B, N, T)
+    ws = _workspace(dev, nb, "tvjp")   # (not the "rhs" one: that may still hold [S|P] for a pending rhs_vjp)
+    _lib.check(lib.phx_time_vjp(_lib.ctx(dev), G, H, B, N, T, _ptr(packed), _ptr(ys), _ptr(gy), _ptr(t_grad),
+                                _ptr(t_vjp), _ptr(ws), ws.numel(), _stream_ptr(dev)), "time_vjp")
+    return t_grad, t_vjp
 
 
 # ---- many independent problems per call (SURVEY.md section 8 f1: the per-sample loop of training_step) -----------------
@@ -883,10 +909,11 @@ def solve_forward_many(net, y0, t_rows, t_is_f32, method, rtol, atol, max_num_st
 
 @_on_model_device
 def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps, y_saved, grad_y,
-                       param_mask=_lib.PARAMS_ALL, step_size=None, step_control=None):
+                       param_mask=_lib.PARAMS_ALL, step_size=None, step_control=None, t_vjp=None):
     """Backward sweeps of N independent problems (``y_saved``, ``grad_y``: ``[N, T, *S, G]``): adj_y0 ``[N, *S, G]`` and
     the six parameter cotangents summed over the problems (what autograd accumulates into ``.grad``); zeros for the
-    parameters outside ``param_mask``; ``step_size``, ``step_control``: see solve_adjoint)."""
+    parameters outside ``param_mask``; ``step_size``, ``step_control``: see solve_adjoint; ``t_vjp``: [N, T-1], row i
+    for problem i, see solve_adjoint)."""
     packed, G, H, dev = packed_weights(net)
     ys = y_saved.detach().contiguous()
     gy = grad_y.detach().to(torch.float32).contiguous()
@@ -898,7 +925,7 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     grids = _grids(t_rows, t_is_f32, step_size, False)
     if _use_rows(lib, dev, G, H, B, True):
         return _adjoint_rows(lib, net, packed, G, H, dev, t_rows, t_is_f32, method, rtol, atol, max_num_steps, ys, gy,
-                             tuple(ys[:, 0].shape), param_mask, grids, step_control)
+                             tuple(ys[:, 0].shape), param_mask, grids, step_control, t_vjp)
     engine, nb = _pick_engine(lib, dev, G, H, B, T, True)
     if grids is not None and engine == "resident":
         nb += _Grid(grids, False).nbytes(lib, N, T)
@@ -917,7 +944,8 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
     streams = _concurrency(lib, dev, G, H, B, True, engine, N)
     per = _problems_per_launch(T) if (engine == "resident" and not streams and not STEP_LOGGING) else 1
     d = _solve_desc(engine, True, packed, G, H, B, 1, T, t_is_f32, method, rtol, atol, max_num_steps, param_mask,
-                    step_control=step_control)
+                    step_control=step_control, t_vjp=t_vjp)
+    tv_row = 4 * (T - 1)   # bytes between the t_vjp rows of consecutive problems
     for lo in range(0, N, chunk):
         hi = min(N, lo + chunk)
         if per > 1:
@@ -927,6 +955,8 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
                 flat_t = (ctypes.c_double * (n * T))(*[x for r in t_rows[l2:l2 + n] for x in r])
                 d.N, d.y_saved, d.grad_y = n, ybase + l2 * stride, gbase + l2 * stride
                 d.adj_y0, d.grads = abase + l2 * astride, tbase + (l2 - lo) * P * 4
+                if t_vjp is not None:
+                    d.t_vjp = t_vjp.data_ptr() + l2 * tv_row
                 if grids is not None:
                     gm = _Grid(grids[l2:l2 + n], False)
                     gm.put(d)
@@ -944,6 +974,8 @@ def solve_adjoint_many(net, t_rows, t_is_f32, method, rtol, atol, max_num_steps,
                 log, cap = _steplog()
                 d.y_saved, d.grad_y = ybase + i * stride, gbase + i * stride
                 d.adj_y0, d.grads = abase + i * astride, tbase + (i - lo) * P * 4
+                if t_vjp is not None:
+                    d.t_vjp = t_vjp.data_ptr() + i * tv_row
                 if pg is not None:
                     pg[i].put(d)
                 if streams:

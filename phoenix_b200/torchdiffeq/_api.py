@@ -70,9 +70,10 @@ def _step_control(method, options):
     return tuple(out)
 
 
-def _normalise(func, y0, t, rtol, atol, method, options):
+def _normalise(func, y0, t, rtol, atol, method, options, t_grad=False):
     """The checks of misc.py:165-241 that apply to a single-tensor state; returns the pieces the kernels need (the
-    fixed-grid ``step_size`` and the dopri5 step control are checked here and read with _step_size / _step_control)."""
+    fixed-grid ``step_size`` and the dopri5 step control are checked here and read with _step_size / _step_control).
+    ``t_grad``: the caller differentiates with respect to t (the adjoint entry points), so t may require grad."""
     if not torch.is_tensor(y0):
         assert isinstance(y0, tuple), 'y0 must be either a torch.Tensor or a tuple'
         raise NotImplementedError("tuple-valued states are not part of the PHOENIX path (ODENet has a tensor state)")
@@ -102,8 +103,9 @@ def _normalise(func, y0, t, rtol, atol, method, options):
     assert t.ndimension() == 1, "{} must be one dimensional".format('t')
     if not torch.is_floating_point(t):
         raise TypeError('`{}` must be a floating point Tensor but is a {}'.format('t', t.type()))
-    if t.requires_grad:
-        raise NotImplementedError("gradients with respect to t are not computed on the B200 path")
+    if t.requires_grad and not t_grad:
+        raise NotImplementedError("odeint records no autograd graph, so it computes no gradient with respect to t; use "
+                                  "odeint_adjoint")
     # the times are consumed on the host (float32 values are promoted exactly, like solvers.py:26); plain Python from
     # here on: this runs once per sample of every training step
     t_is_f32 = t.dtype != torch.float64
@@ -167,7 +169,7 @@ def _register_node(ctx, func, y0, tl, t_is_f32, adj):
     """Forward side: note the node if its backward may be batched with its siblings' (a one-row state that needs no
     gradient itself -- the training loop's case)."""
     ctx.group = None
-    if (not DEFER_ADJOINT or ctx.needs_input_grad[8] or not any(ctx.needs_input_grad[9:]) or not adj[4] & PARAMS_ALL
+    if (not DEFER_ADJOINT or ctx.needs_input_grad[8] or not any(ctx.needs_input_grad[9:15]) or not adj[4] & PARAMS_ALL
             or y0.numel() != y0.shape[-1]):
         return   # (nothing to differentiate -- e.g. a validation pass under no_grad -- is not a node at all)
     with _defer_lock:
@@ -175,8 +177,10 @@ def _register_node(ctx, func, y0, tl, t_is_f32, adj):
         ctx.seq = _node_seq[0]
         # adj[4], the adjoint parameter mask with the norm bit, adj[5], the backward step size, and adj[6], its dopri5
         # step control when given, are part of the key: only nodes with the same adjoint set, error norm, step grid spacing and
-        # controller share a sweep
-        ctx.group = (len(tl), t_is_f32, adj, tuple(y0.shape), y0.device, tuple(ctx.needs_input_grad[9:]))
+        # controller share a sweep; so is a t that needs a gradient (its time cotangents start dopri5's intervals)
+        ctx.group = (len(tl), t_is_f32, adj, tuple(y0.shape), y0.device, tuple(ctx.needs_input_grad[9:15]))
+        if _t_needs_grad(ctx):
+            ctx.group += ("t",)
         nodes = _live_nodes.get(func)
         if nodes is None:
             nodes = _live_nodes[func] = weakref.WeakSet()
@@ -195,9 +199,11 @@ def _unresolved(key):
     return check
 
 
-def _defer(ctx, y, grad_y):
+def _defer(ctx, y, grad_y, t_vjp=None):
     """Backward side.  Returns _NOT_DEFERRED (the caller solves its own sweep), the all-None tuple (the cotangent waits for
-    the last sibling) or, in the last sibling, (t_rows, ys, gys) of every waiting node in creation order."""
+    the last sibling) or, in the last sibling, (t_rows, ys, gys, t_vjps) of every waiting node in creation order.  Each
+    node of a group whose t needs a gradient leaves its ``t_vjp`` row ([1, T-1]) here, and t_vjps is their stack
+    ([N, T-1]; None for the other groups)."""
     try:
         gid = torch._C._current_graph_task_id()
         will_run = torch._C._will_engine_execute_node
@@ -220,12 +226,13 @@ def _defer(ctx, y, grad_y):
                 del _deferred[k]
             ent = _deferred[key] = [len(peers), []]
             queue_callback(_unresolved(key))   # runs when this backward pass ends: loud if a counted sibling never came
-        ent[1].append((ctx.seq, y, grad_y, ctx.tl))
+        ent[1].append((ctx.seq, y, grad_y, ctx.tl, t_vjp))
         if len(ent[1]) < ent[0]:
             return None
         del _deferred[key]
     items = sorted(ent[1], key=lambda it: it[0])
-    return [it[3] for it in items], torch.stack([it[1] for it in items]), torch.stack([it[2] for it in items])
+    t_vjps = torch.cat([it[4] for it in items]) if items[0][4] is not None else None
+    return [it[3] for it in items], torch.stack([it[1] for it in items]), torch.stack([it[2] for it in items]), t_vjps
 
 
 class OdeintAdjointMethod(torch.autograd.Function):
@@ -235,8 +242,10 @@ class OdeintAdjointMethod(torch.autograd.Function):
     @staticmethod
     def forward(ctx, func, tl, t_is_f32, fwd, rtol, atol, max_steps, adj, y0, *adjoint_params):
         # fwd = (method, step_size); adj = (method, rtol, atol, max_num_steps, mask, step_size) of the backward; each
-        # with the dopri5 step control appended when it is given (_with_control)
+        # with the dopri5 step control appended when it is given (_with_control).  adjoint_params: the six parameters,
+        # then t when it needs a gradient (_with_t)
         ctx.func, ctx.tl, ctx.t_is_f32, ctx.adj = func, tl, t_is_f32, adj
+        _note_t(ctx, adjoint_params)
         with torch.no_grad():
             y = engine.solve_forward(func, y0, tl, t_is_f32, False, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]),
                                      **_controlled(fwd, 2))
@@ -248,21 +257,23 @@ class OdeintAdjointMethod(torch.autograd.Function):
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
         a_method, a_rtol, a_atol, a_max, mask = ctx.adj[:5]
+        t_out, t_vjp = _time_grads(ctx, y.unsqueeze(0), grad_y.unsqueeze(0), True)
         if not mask & PARAMS_ALL and not ctx.needs_input_grad[8]:
-            return (None,) * (9 + len(ctx.needs_input_grad[9:]))   # only parameters outside adjoint_params want one
-        batch = _defer(ctx, y, grad_y) if (ctx.group is not None and DEFER_ADJOINT) else _NOT_DEFERRED
+            # only parameters outside adjoint_params want one, or only t: its cotangents need no sweep
+            return (None,) * (9 + len(ctx.needs_input_grad[9:15])) + t_out
+        batch = _defer(ctx, y, grad_y, t_vjp) if (ctx.group is not None and DEFER_ADJOINT) else _NOT_DEFERRED
         if batch is None:
-            return (None,) * (9 + len(ctx.needs_input_grad[9:]))
+            return (None,) * (9 + len(ctx.needs_input_grad[9:15])) + t_out
         kw = dict(_masked(mask), **_stepped(ctx.adj[5]), **_controlled(ctx.adj, 6))
         with torch.no_grad():
             if batch is _NOT_DEFERRED:
                 adj_y0, grads = engine.solve_adjoint(ctx.func, ctx.tl, ctx.t_is_f32, a_method, a_rtol, a_atol, a_max,
-                                                     y, grad_y, **kw)
+                                                     y, grad_y, **kw, **_t_vjp_kw(t_vjp))
             else:
-                t_rows, ys, gys = batch
+                t_rows, ys, gys, t_vjps = batch
                 adj_y0, grads = engine.solve_adjoint_many(ctx.func, t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
-                                                          a_max, ys, gys, **kw)
-        return _grads_out(ctx, adj_y0, grads, mask)
+                                                          a_max, ys, gys, **kw, **_t_vjp_kw(t_vjps))
+        return _grads_out(ctx, adj_y0, grads, mask) + t_out
 
 
 def _masked(mask):
@@ -294,13 +305,50 @@ def _controlled(tup, i):
 
 
 def _grads_out(ctx, adj_y0, grads, mask):
-    """backward's result: adj_y0 for y0, and a cotangent only for the parameters in the adjoint set (None for the others
-    even when they require grad: the reference's adjoint node does not take them as inputs).  Only the six parameter bits
-    of ``mask`` are read, never the norm bit."""
+    """backward's result for the first 15 inputs: adj_y0 for y0, and a cotangent only for the parameters in the adjoint
+    set (None for the others even when they require grad: the reference's adjoint node does not take them as inputs).
+    Only the six parameter bits of ``mask`` are read, never the norm bit."""
     out = [None] * 8 + [adj_y0 if ctx.needs_input_grad[8] else None]
-    for i, need in enumerate(ctx.needs_input_grad[9:]):
+    for i, need in enumerate(ctx.needs_input_grad[9:15]):
         out.append(grads[i] if (need and mask >> i & 1) else None)
     return tuple(out)
+
+
+# ---- gradients with respect to t (adjoint.py, backward with t requiring grad) -------------------------------------------------
+# ODENet is autonomous, so the time cotangents need no sweep: f(y_i) . grad_y_i for every output i >= 1 and minus their sum
+# for t[0] (engine.time_vjp).  The reference also carries the running time cotangent vjp_t through each interval's solve,
+# where it is a block of dopri5's mixed norm and so moves the initial step: the engine takes it as t_vjp.  t is an extra
+# trailing input of the autograd node only when it requires grad, so without it the node is what it always was.
+def _with_t(t):
+    """The trailing node input for t: (t,) when its gradient is wanted, else ()."""
+    return (t,) if t.requires_grad and torch.is_grad_enabled() else ()
+
+
+def _note_t(ctx, adjoint_params):
+    """Forward side: keep the dtype and device of t (the 7th trailing input, when given) for its gradient."""
+    if len(adjoint_params) > 6:
+        ctx.t_meta = (adjoint_params[6].dtype, adjoint_params[6].device)
+
+
+def _t_needs_grad(ctx):
+    """Whether the node has t as its 16th input and autograd wants its gradient (hand-built contexts have 15 flags)."""
+    return len(ctx.needs_input_grad) > 15 and ctx.needs_input_grad[15]
+
+
+def _time_grads(ctx, y, grad_y, single):
+    """((t.grad,), t_vjp) when t needs a gradient, else ((), None).  y, grad_y: [N, T, *S, G]; t.grad has t's shape
+    ([T] when ``single``, else [N, T]), dtype and device; t_vjp is [N, T-1] on the model's device."""
+    if not _t_needs_grad(ctx):
+        return (), None
+    with torch.no_grad():
+        t_grad, t_vjp = engine.time_vjp(ctx.func, y, grad_y)
+    dtype, device = ctx.t_meta
+    return ((t_grad[0] if single else t_grad).to(device=device, dtype=dtype),), t_vjp
+
+
+def _t_vjp_kw(t_vjp):
+    """The engine's keyword for the time cotangents; without them the engine is called as it always was."""
+    return {} if t_vjp is None else {"t_vjp": t_vjp}
 
 
 def _adjoint_mask(func, adjoint_params):
@@ -346,7 +394,8 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
     """adjoint.py:165-204: same as ``odeint`` but differentiable w.r.t. y0 and the ODENet parameters through the
     continuous adjoint, solved backwards with the forward method / tolerances unless overridden.
     ``adjoint_options=dict(norm="seminorm")`` measures the dopri5 backward's error without the parameter cotangents
-    (Kidger, Chen & Lyons, 2021), in the initial step and in every error ratio."""
+    (Kidger, Chen & Lyons, 2021), in the initial step and in every error ratio.  A ``t`` that requires grad gets the
+    reference's ``time_vjps`` as its gradient (increasing t only); when nothing else needs a gradient no sweep runs."""
     if adjoint_params is None and not isinstance(func, nn.Module):
         raise ValueError('func must be an instance of nn.Module to specify the adjoint parameters; alternatively they '
                          'can be specified explicitly via the `adjoint_params` argument. If there are no parameters '
@@ -362,20 +411,20 @@ def odeint_adjoint(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None,
         adjoint_options = {k: v for k, v in options.items() if k != "norm"} if options is not None else {}
     same = (adjoint_rtol is rtol and adjoint_atol is atol and adjoint_method is method and not adjoint_options
             and not options)
-    tl, t_is_f32, rev, rtol, atol, method, max_steps = _normalise(func, y0, t, rtol, atol, method, options)
+    tl, t_is_f32, rev, rtol, atol, method, max_steps = _normalise(func, y0, t, rtol, atol, method, options, True)
     step, ctl = _step_size(method, options), _step_control(method, options)
     if same:
         a_rtol, a_atol, a_method, a_max, a_step, a_ctl = rtol, atol, method, max_steps, step, ctl
     else:
         _, _, _, a_rtol, a_atol, a_method, a_max = _normalise(func, y0, t, adjoint_rtol, adjoint_atol, adjoint_method,
-                                                              adjoint_options)
+                                                              adjoint_options, True)
         a_step, a_ctl = _step_size(a_method, adjoint_options), _step_control(a_method, adjoint_options)
     if rev:
         raise NotImplementedError("odeint_adjoint with decreasing t is not part of the PHOENIX path")
     params, mask = _adjoint_mask(func, adjoint_params)
     return OdeintAdjointMethod.apply(func, tl, t_is_f32, _with_control((method, step), ctl), rtol, atol, max_steps,
                                      _with_control((a_method, a_rtol, a_atol, a_max, mask | norm_bit, a_step), a_ctl),
-                                     y0, *params)
+                                     y0, *params, *_with_t(t))
 
 
 class OdeintAdjointManyMethod(torch.autograd.Function):
@@ -384,6 +433,7 @@ class OdeintAdjointManyMethod(torch.autograd.Function):
     @staticmethod
     def forward(ctx, func, t_rows, t_is_f32, fwd, rtol, atol, max_steps, adj, y0, *adjoint_params):
         ctx.func, ctx.t_rows, ctx.t_is_f32, ctx.adj = func, t_rows, t_is_f32, adj
+        _note_t(ctx, adjoint_params)
         with torch.no_grad():
             y = engine.solve_forward_many(func, y0, t_rows, t_is_f32, fwd[0], rtol, atol, max_steps, **_stepped(fwd[1]),
                                           **_controlled(fwd, 2))
@@ -394,13 +444,14 @@ class OdeintAdjointManyMethod(torch.autograd.Function):
     def backward(ctx, grad_y):
         (y,) = ctx.saved_tensors
         a_method, a_rtol, a_atol, a_max, mask = ctx.adj[:5]
+        t_out, t_vjp = _time_grads(ctx, y, grad_y, False)
         if not mask & PARAMS_ALL and not ctx.needs_input_grad[8]:
-            return (None,) * (9 + len(ctx.needs_input_grad[9:]))
+            return (None,) * (9 + len(ctx.needs_input_grad[9:15])) + t_out
         with torch.no_grad():
             adj_y0, grads = engine.solve_adjoint_many(ctx.func, ctx.t_rows, ctx.t_is_f32, a_method, a_rtol, a_atol,
                                                       a_max, y, grad_y, **_masked(mask), **_stepped(ctx.adj[5]),
-                                                      **_controlled(ctx.adj, 6))
-        return _grads_out(ctx, adj_y0, grads, mask)
+                                                      **_controlled(ctx.adj, 6), **_t_vjp_kw(t_vjp))
+        return _grads_out(ctx, adj_y0, grads, mask) + t_out
 
 
 def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=None, adjoint_params=None,
@@ -411,15 +462,16 @@ def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=
     ``[N, T, *S, G]`` with ``result[i] == odeint_adjoint(func, y0[i], t[i], ...)`` bit for bit: every sample is still
     its own solve with its own step controller (NOT the global-norm batched call).  Gradients flow to ``y0`` and to the
     ODENet parameters of ``adjoint_params`` that require grad (default: all six; summed over the samples) through one
-    autograd node.  ``adjoint_options`` as in ``odeint_adjoint`` (default: the forward options without ``norm``).  No
-    reference counterpart: opt-in."""
+    autograd node, and to ``t`` when it requires grad (row i: what ``odeint_adjoint`` gives ``t[i]``).
+    ``adjoint_options`` as in ``odeint_adjoint`` (default: the forward options without ``norm``).  No reference
+    counterpart: opt-in."""
     assert torch.is_tensor(t) and t.ndimension() == 2, "t must be a [N, T] tensor of per-sample times"
     assert torch.is_tensor(y0) and y0.shape[0] == t.shape[0], "y0 and t must hold the same number of samples"
     if y0.shape[0] == 0:
         raise ValueError("odeint_adjoint_many needs at least one sample")
     t_is_f32 = t.dtype != torch.float64
     rows = t.tolist()
-    tl0, _, rev, rtol_f, atol_f, method, max_steps = _normalise(func, y0[0], t[0], rtol, atol, method, options)
+    tl0, _, rev, rtol_f, atol_f, method, max_steps = _normalise(func, y0[0], t[0], rtol, atol, method, options, True)
     for r in rows:
         assert all(b > a for a, b in zip(r, r[1:])), 't must be strictly increasing for every sample'
     if rev:
@@ -428,10 +480,10 @@ def odeint_adjoint_many(func, y0, t, rtol=1e-7, atol=1e-9, method=None, options=
     adjoint_options, norm_bit = _adjoint_norm(adjoint_options)
     a_max, a_step, a_ctl = max_steps, step, ctl
     if adjoint_options is not None:
-        a_max = _normalise(func, y0[0], t[0], rtol, atol, method, adjoint_options)[6]
+        a_max = _normalise(func, y0[0], t[0], rtol, atol, method, adjoint_options, True)[6]
         a_step, a_ctl = _step_size(method, adjoint_options), _step_control(method, adjoint_options)
     params, mask = _adjoint_mask(func, adjoint_params)
     return OdeintAdjointManyMethod.apply(func, rows, t_is_f32, _with_control((method, step), ctl), rtol_f, atol_f,
                                          max_steps,
                                          _with_control((method, rtol_f, atol_f, a_max, mask | norm_bit, a_step), a_ctl),
-                                         y0, *params)
+                                         y0, *params, *_with_t(t))
