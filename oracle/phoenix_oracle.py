@@ -26,7 +26,7 @@ Parameter order everywhere is the reference's ``ODENet.parameters()`` order (SUR
 from __future__ import annotations
 
 import math
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 from typing import Callable, List, Optional, Sequence, Tuple
 
 import torch
@@ -202,10 +202,36 @@ def block_max_rms(sizes: Sequence[int]) -> Callable[[torch.Tensor], torch.Tensor
 
 @dataclass
 class StepLog:
-    """(t0, dt, accepted) per attempted adaptive step, plus RHS-evaluation count."""
+    """(t0, dt, accepted) per attempted adaptive step, plus RHS-evaluation count.  dopri5 also records the error ratio
+    it computes for each attempt and, per solve, (index of its first attempt, Hairer's initial step estimate)."""
 
     steps: List[Tuple[float, float, bool]]
     nfe: int = 0
+    ratios: List[float] = field(default_factory=list)
+    starts: List[Tuple[int, float]] = field(default_factory=list)
+
+
+class Replay:
+    """A step schedule ``(t0, dt, accepted)`` per attempt -- the rows of ``engine.last_step_log()`` -- that dopri5 solves
+    consume in order in place of their step-size controller (``_solve_dopri5``).  ``finish()`` checks that every attempt
+    was used."""
+
+    def __init__(self, steps):
+        self.steps = [(float(a), float(b), bool(c)) for a, b, c in steps]
+        self.pos = 0
+
+    def take(self, t1: float) -> Tuple[float, bool]:
+        assert self.pos < len(self.steps), "replay: the schedule ends at attempt %d, before the solve does" % self.pos
+        t0, dt, acc = self.steps[self.pos]
+        assert abs(t0 - t1) <= 1e-12 * (abs(t1) + abs(dt)), \
+            "replay: attempt %d starts at %r, the last accepted step ended at %r" % (self.pos, t0, t1)
+        assert dt != 0 and math.isfinite(dt), "replay: attempt %d has dt %r" % (self.pos, dt)
+        self.pos += 1
+        return dt, acc
+
+    def finish(self):
+        assert self.pos == len(self.steps), "replay: %d of %d attempts left over" % (len(self.steps) - self.pos,
+                                                                                 len(self.steps))
 
 
 def _initial_step(func, t0, y0, f0, rtol, atol, norm) -> torch.Tensor:
@@ -243,11 +269,16 @@ def _next_dt(dt: torch.Tensor, ratio: torch.Tensor) -> torch.Tensor:
 
 
 def _solve_dopri5(func, y0: torch.Tensor, t: torch.Tensor, rtol: float, atol: float, norm, log: StepLog,
-                  max_num_steps: int = 2 ** 31 - 1) -> torch.Tensor:
+                  max_num_steps: int = 2 ** 31 - 1, replay: Optional[Replay] = None) -> torch.Tensor:
     """Adaptive Dormand-Prince solve returning y at every t (rk_common.py:140-228, solvers.py:23-30).
 
     State dtype = y0.dtype (fp32); every time-like scalar is a 0-dim float64 tensor; the stage matrix ``k`` has the
-    stage index innermost and stage combinations are ``k[..., :i+1] @ (beta_i * dt)`` as in rk_common.py:62-76."""
+    stage index innermost and stage combinations are ``k[..., :i+1] @ (beta_i * dt)`` as in rk_common.py:62-76.
+
+    ``replay``: take each attempt's dt and accept decision from the schedule instead of Hairer's estimate, the
+    controller and ``ratio <= 1``; everything else runs as without it (the estimate and the ratios are still computed
+    and logged).  The schedule must be one a solve of these output times can take: each attempt starts where the last
+    accepted step ended, so the first one at t[0], and no attempt follows the step that covers the last output time."""
     dtype = y0.dtype
     t = t.to(torch.float64)
     rt = torch.as_tensor(rtol, dtype=torch.float64)
@@ -264,12 +295,16 @@ def _solve_dopri5(func, y0: torch.Tensor, t: torch.Tensor, rtol: float, atol: fl
     out[0] = y0
     f0 = f(t[0], y0)
     dt = _initial_step(f, t[0], y0, f0, rt, at, norm)
+    log.starts.append((len(log.steps), float(dt)))
     y, t0, t1 = y0, t[0], t[0]
     coeff = [y0] * 5
     for i in range(1, len(t)):
         n = 0
         while t[i] > t1:
             assert n < max_num_steps, "max_num_steps exceeded ({}>={})".format(n, max_num_steps)
+            if replay is not None:
+                dt_r, accept_r = replay.take(float(t1))
+                dt = torch.tensor(dt_r, dtype=torch.float64)
             assert t1 + dt > t1, "underflow in dt {}".format(dt.item())
             assert torch.isfinite(y).all(), "non-finite values in state `y`: {}".format(y)
             ts, dts = t1.to(dtype), dt.to(dtype)
@@ -282,8 +317,9 @@ def _solve_dopri5(func, y0: torch.Tensor, t: torch.Tensor, rtol: float, atol: fl
             err = k.matmul(dts * c_err)
             tol = at + rt * torch.max(y.abs(), y1.abs())
             ratio = norm(err / tol)
-            accept = bool(ratio <= 1)
+            accept = bool(ratio <= 1) if replay is None else accept_r
             log.steps.append((float(t1), float(dt), accept))
+            log.ratios.append(float(ratio))
             if accept:
                 ymid = y + k.matmul(dts * c_mid).view_as(y)
                 ka, kb = k[..., 0], k[..., 6]
@@ -340,38 +376,45 @@ def _solve_fixed(func, y0: torch.Tensor, t: torch.Tensor, method: str, log: Step
     return out
 
 
-def _solve(func, y0, t, method, rtol, atol, norm, log):
+def _solve(func, y0, t, method, rtol, atol, norm, log, replay=None):
     if method is None:
         method = "dopri5"
     assert t.ndim == 1 and bool((t[1:] > t[:-1]).all()), "t must be strictly increasing here"
     if method == "dopri5":
-        return _solve_dopri5(func, y0, t, rtol, atol, norm, log)
+        return _solve_dopri5(func, y0, t, rtol, atol, norm, log, replay=replay)
+    assert replay is None, "a step schedule is for dopri5"
     return _solve_fixed(func, y0, t, method, log)
 
 
 def odeint(w: Weights, y0: torch.Tensor, t: torch.Tensor, method: Optional[str] = None, rtol: float = 1e-7,
-           atol: float = 1e-9) -> Tuple[torch.Tensor, StepLog]:
+           atol: float = 1e-9, replay=None) -> Tuple[torch.Tensor, StepLog]:
     """Forward solve ``[len(t), *y0.shape]`` with the reference defaults (odeint.py:25; norm = RMS over the whole
-    state, misc.py:198-201).  Decreasing ``t`` is handled by time negation as misc.py:210-218."""
+    state, misc.py:198-201).  Decreasing ``t`` is handled by time negation as misc.py:210-218.  ``replay``: a dopri5
+    step log to take instead of the controller's steps (``Replay``)."""
     log = StepLog([])
     sign = 1.0
     if bool((t[1:] < t[:-1]).all()):
         sign, t = -1.0, -t
     func = (lambda tt, yy: rhs(w, yy)) if sign > 0 else (lambda tt, yy: -rhs(w, yy))
+    rp = None if replay is None else Replay(replay)
     with torch.no_grad():
-        y = _solve(func, y0, t, method, rtol, atol, rms, log)
+        y = _solve(func, y0, t, method, rtol, atol, rms, log, rp)
+    if rp is not None:
+        rp.finish()
     return y, log
 
 
 def adjoint_backward(w: Weights, t: torch.Tensor, y: torch.Tensor, grad_y: torch.Tensor,
-                     method: Optional[str] = None, rtol: float = 1e-7, atol: float = 1e-9):
+                     method: Optional[str] = None, rtol: float = 1e-7, atol: float = 1e-9, replay=None):
     """The backward sweep of ``OdeintAdjointMethod`` (adjoint.py:32-162) for increasing ``t``.
 
     For each output interval, from the last to the first, the flat augmented vector
     ``[vjp_t(1), y(N), adj_y(N), adj_params(P)]`` is integrated from t[i] to t[i-1] in negated time
     (misc.py:210-212) with the forward method and tolerances, under the norm
     ``max(RMS(vjp_t), RMS(y), RMS(adj_y), RMS(adj_params))`` (adjoint.py:72-78 / 198-200).  ``vjp_t`` stays 0
-    because t does not require grad.  Returns (adj_y0, [6 grads], StepLog over all intervals)."""
+    because t does not require grad.  ``replay``: a dopri5 backward step log, the attempts of all intervals in the
+    order they run (T-1 .. 1, negated time), taken instead of the controller's steps (``Replay``).  Returns (adj_y0,
+    [6 grads], StepLog over all intervals)."""
     log = StepLog([])
     shape = y.shape[1:]
     N = y[0].numel()
@@ -388,6 +431,7 @@ def adjoint_backward(w: Weights, t: torch.Tensor, y: torch.Tensor, grad_y: torch
                          + [p.reshape(-1) for p in pbar])
         return -full
 
+    rp = None if replay is None else Replay(replay)
     with torch.no_grad():
         adj_y = grad_y[-1].clone()
         adj_p = torch.zeros(P, dtype=y.dtype)
@@ -395,10 +439,12 @@ def adjoint_backward(w: Weights, t: torch.Tensor, y: torch.Tensor, grad_y: torch
         for i in range(len(t) - 1, 0, -1):
             z0 = torch.cat([torch.zeros(1, dtype=y.dtype), cur_y.reshape(-1), adj_y.reshape(-1), adj_p])
             tt = -t[i - 1:i + 1].flip(0)
-            z = _solve(aug_reversed, z0, tt, method, rtol, atol, norm, log)[1]
+            z = _solve(aug_reversed, z0, tt, method, rtol, atol, norm, log, rp)[1]
             adj_p = z[1 + 2 * N:]
             cur_y = y[i - 1]
             adj_y = z[1 + N:1 + 2 * N].reshape(shape) + grad_y[i - 1]
+        if rp is not None:
+            rp.finish()
         grads, lo = [], 0
         for p, n in zip(params, psz):
             grads.append(adj_p[lo:lo + n].reshape(p.shape))

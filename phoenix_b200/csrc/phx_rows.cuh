@@ -1454,6 +1454,19 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
 
         for (int iv = p.T - 1; iv >= 1; --iv) {
             const bool first_iv = iv == p.T - 1;
+            if (dop) {
+                // dopri5 restarts every interval from the identity slot maps.  This comes before the loads: they store
+                // the stage-0 input record into factor slot fslot[0], which the last interval's accepted steps may have
+                // swapped to slot 5 (FSAL), where stage 0 of this interval would not read it.
+                if (threadIdx.x < RM) {
+                    RowCtl& c = rc->r[threadIdx.x];
+                    for (int i = 0; i < 7; ++i) c.slot[i] = i;
+                    c.fslot[0] = 0;
+                    c.fslot[1] = -1;
+                    for (int i = 2; i < 7; ++i) c.fslot[i] = i - 1;
+                }
+                __syncthreads();
+            }
             for (int e = threadIdx.x; e < p.gpc * RM; e += THREADS) {
                 const int j = e >> 2, b = e & 3;
                 float y = 0.5f, av = 0.f;
@@ -1577,16 +1590,8 @@ __global__ void __launch_bounds__(PHX_THREADS, 1) phx_rows_adj_kernel(const __gr
                 }
             } else {
                 // ------------------------------ dopri5 on the augmented state, one controller per row -----------------
-                if (threadIdx.x < RM) {
-                    RowCtl& c = rc->r[threadIdx.x];
-                    for (int i = 0; i < 7; ++i) c.slot[i] = i;
-                    c.fslot[0] = 0;
-                    c.fslot[1] = -1;
-                    for (int i = 2; i < 7; ++i) c.fslot[i] = i - 1;
-                }
-                __syncthreads();
-                // (the stage-0 input record was stored in factor slot fslot[0] == 0 by set_input above: the mapping is
-                // reset to the identity at every interval start, before the loads)
+                // (the slot maps were reset to the identity at the interval start: the loads above stored the stage-0
+                // input record into factor slot 0)
                 for (int which = 0; which < 2; ++which) {
                     const int sid = which == 0 ? 0 : 6;
                     double acc[7] = {0, 0, 0, 0, 0, 0, 0};

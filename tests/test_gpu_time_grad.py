@@ -26,22 +26,32 @@ NAMES = O.PARAM_ORDER
 
 # ---- oracle extension (CPU) -----------------------------------------------------------------------------------------------
 def adjoint_backward_t(w, t, y, grad_y, method="dopri5", rtol=1e-7, atol=1e-9, t_requires_grad=False, semi=False,
-                       first_step=None, step_size=None):
+                       first_step=None, step_size=None, params=None, replay=None):
     """O.adjoint_backward with the augmented state's vjp_t carried from interval to interval, as the reference carries
     ``aug_state[0]``; with ``t_requires_grad`` it also forms the reference's time_vjps.  ``semi``: the seminorm (the
     norm of the first 1 + 2N entries); ``first_step`` (dopri5) starts every interval; ``step_size`` (fixed grids) steps
-    every interval on its own grid.  Returns (adj_y0, [6 grads], StepLog, time_vjps in t's dtype or None)."""
+    every interval on its own grid.  ``params``: the adjoint set S as indices (None: all six) -- the default norm's
+    parameter block holds only S (``adjoint_backward_s``), while all six cotangents are still integrated (the y / adj_y
+    algebra never reads them); ``replay``: a dopri5 backward step log to take instead of the controller's steps
+    (``O.Replay``; ``first_step`` is then only in the log).  Returns (adj_y0, [6 grads], StepLog, time_vjps in t's dtype
+    or None)."""
     log = O.StepLog([])
     shape = y.shape[1:]
     N = y[0].numel()
-    params = w.as_list()
-    psz = [p.numel() for p in params]
+    params_all = w.as_list()
+    psz = [p.numel() for p in params_all]
     P = sum(psz)
     if semi:
         head = O.block_max_rms([1, N, N])
         norm = lambda x: head(x[:1 + 2 * N])   # noqa: E731
-    else:
+    elif params is None or sorted(set(params)) == list(range(6)):
         norm = O.block_max_rms([1, N, N, P])
+    else:
+        keep = torch.cat([torch.full((n,), i in set(params), dtype=torch.bool) for i, n in enumerate(psz)])
+        ps = int(keep.sum())
+        blocks = O.block_max_rms([1, N, N, ps] if ps else [1, N, N])
+        norm = lambda x: blocks(torch.cat([x[:1 + 2 * N], x[1 + 2 * N:][keep]]))   # noqa: E731
+    rp = None if replay is None else O.Replay(replay)
 
     def aug_reversed(tt, z):
         f, ybar, pbar = O.rhs_vjp(w, z[1:1 + N].reshape(shape), -z[1 + N:1 + 2 * N].reshape(shape))
@@ -51,8 +61,8 @@ def adjoint_backward_t(w, t, y, grad_y, method="dopri5", rtol=1e-7, atol=1e-9, t
     def solve(z0, tt):
         if method != "dopri5":
             return solve_fixed_grid(aug_reversed, z0, tt, method, log, step_size)
-        if first_step is None:
-            return O._solve(aug_reversed, z0, tt, method, rtol, atol, norm, log)
+        if first_step is None or rp is not None:
+            return O._solve(aug_reversed, z0, tt, method, rtol, atol, norm, log, rp)
         return solve_dopri5_x(aug_reversed, z0, tt, rtol, atol, norm, log, first_step=first_step)
 
     with torch.no_grad():
@@ -72,10 +82,12 @@ def adjoint_backward_t(w, t, y, grad_y, method="dopri5", rtol=1e-7, atol=1e-9, t
             adj_p = z[1 + 2 * N:]
             cur_y = y[i - 1]
             adj_y = z[1 + N:1 + 2 * N].reshape(shape) + grad_y[i - 1]
+        if rp is not None:
+            rp.finish()
         if t_requires_grad:
             time_vjps[0] = vjp_t[0]
         grads, lo = [], 0
-        for p, n in zip(params, psz):
+        for p, n in zip(params_all, psz):
             grads.append(adj_p[lo:lo + n].reshape(p.shape))
             lo += n
     return adj_y, grads, log, time_vjps
@@ -317,10 +329,7 @@ def _sq_loss(target, many):
 @pytest.mark.parametrize("e", ENGINES, ids=[_eid(e) for e in ENGINES])
 def test_t_grad_against_oracle(pb, e, variant):
     """t.grad (rel-L2 <= 1e-5), y, adj_y0 and the gradients (the tolerances of test_dopri5_seminorm_against_oracle)
-    against the oracle extension, for T = 2 and 4 and a float32 and a float64 t; dopri5 backward logs to the oracle's.
-    Rows engine, dopri5, several intervals (the known defect of DESIGN.md section 8: its step sequence leaves the
-    oracle's from the second interval on, and Ws / Wp are off): Ws and Wp and the logs are not compared, adj_y0 is
-    compared at the gradients' tolerance; t.grad needs no sweep and keeps its bound."""
+    against the oracle extension, for T = 2 and 4 and a float32 and a float64 t; dopri5 backward logs to the oracle's."""
     engine, G, H, shape, many, _ = e
     name, method, aopts, okw = variant
     rtol, atol = 1e-5, 1e-7
@@ -337,13 +346,10 @@ def test_t_grad_against_oracle(pb, e, variant):
             assert tgrad.shape == tt.shape and tgrad.dtype == dtype and tgrad.device == tt.device, what
             assert rel_l2(tgrad, tv_r) <= 1e-5, (what, tgrad, tv_r)
             assert rel_l2(y, y_r) < 1e-5, what
-            defect = engine == "rows" and method == "dopri5" and T > 2
-            assert rel_l2(ady, ady_r) < (5e-5 if defect else 1e-5), (what, rel_l2(ady, ady_r))
-            skip = {1, 3} if defect else set()
+            assert rel_l2(ady, ady_r) < 1e-5, (what, rel_l2(ady, ady_r))
             for i in range(6):
-                if i not in skip:
-                    assert rel_l2(grads[i], g_r[i]) < 5e-5, (what, NAMES[i], rel_l2(grads[i], g_r[i]))
-            if logs is not None and not defect:
+                assert rel_l2(grads[i], g_r[i]) < 5e-5, (what, NAMES[i], rel_l2(grads[i], g_r[i]))
+            if logs is not None:
                 for i, (mine, r) in enumerate(zip(logs, logs_r)):
                     assert_logs_close(mine, r, 0.25, "%s bwd %d" % (what, i))
 
