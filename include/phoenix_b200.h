@@ -96,6 +96,13 @@ int phx_tc_min_rows(void);
  * cotangents) and M rows is split over CTAs.  out = {128-row tiles, K-splits of the prods half, k-blocks per split,
  * K-splits of the sums half, k-blocks per split, partial-sum slots}; a k-block is 16 k-elements. */
 int phx_tc_plan_describe(int K, int M, int32_t out[6]);
+/* Host-only: the launch configuration of one branch-type tensor-core contraction of a (G genes, H hidden, B rows) call,
+ * as the library would launch it now (environment overrides and phx_tc_set_pair included).  contraction: 0 forward
+ * [S|P], 1 gSP, 2 Ws_bar | Wp_bar, 3 Wa_bar (2 and 3: K = B); + 4 on 0 or 2 when the activation operand is a pair of
+ * cached Hill planes (phx_hill_cache_set).  out = {128-row tiles, K-splits of the prods half, k-blocks per split,
+ * K-splits of the sums half, k-blocks per split, partial-sum slots, depth of the A-operand ring in tensor memory
+ * (0: A in shared memory), shared-memory pipeline stages}. */
+int phx_tc_launch_describe(int contraction, int G, int H, int B, int32_t out[8]);
 /* Diagnostics (no reference counterpart).  phx_tc_set_pair(1): run the branch-type tensor-core contractions as CTA pairs
  * (tcgen05 cta_group::2) -- bit-identical results, measured slower on B200, off by default (tests compare the two).
  * phx_tc_prof_dump: print and reset the device counters collected when the process runs with PHX_TC_PROF=1. */

@@ -22,6 +22,7 @@ EXPORTS = [
     "phx_ctx_create", "phx_ctx_destroy", "phx_last_error", "phx_ctx_num_sms", "phx_resident_max_rows",
     "phx_ctx_set_profile", "phx_profile_slots", "phx_plan_describe",
     "phx_ctx_set_precision", "phx_ctx_get_precision", "phx_tc_min_rows", "phx_tc_plan_describe",
+    "phx_tc_launch_describe",
     "phx_packed_bytes", "phx_pack_weights", "phx_rhs_forward", "phx_rhs_vjp", "phx_rhs_workspace_bytes",
     "phx_solve_workspace_bytes", "phx_solve_workspace_init_bytes", "phx_solve_workspace_init", "phx_solve_forward",
     "phx_solve_adjoint", "phx_solve_forward_many", "phx_solve_adjoint_many",
@@ -87,6 +88,8 @@ def _declare(lib):
     lib.phx_ctx_get_precision.restype = c_int
     lib.phx_tc_plan_describe.argtypes = [c_int, c_int, ctypes.POINTER(ctypes.c_int32)]
     lib.phx_tc_plan_describe.restype = c_int
+    lib.phx_tc_launch_describe.argtypes = [c_int] * 4 + [ctypes.POINTER(ctypes.c_int32)]
+    lib.phx_tc_launch_describe.restype = c_int
     lib.phx_tc_min_rows.argtypes = []
     lib.phx_tc_min_rows.restype = c_int
     lib.phx_packed_bytes.argtypes = [c_int, c_int]

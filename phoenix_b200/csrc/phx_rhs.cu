@@ -10,6 +10,7 @@
 //   ybar[B][G]  = (GS_s Ws + (GS_p Wp)/(1+s)) / (1+|y-.5|)^2 - g relu(m)                 soft-sign / log1p backward
 //   Wa_bar = gJ^T SP,  Ws_bar = GS_s^T s,  Wp_bar = GS_p^T l,  biases / multipliers: column sums
 // The tcgen05 (3xTF32) variant of the same decomposition replaces sgemm_kernel for large B in a later round.
+#include <float.h>
 #include <math.h>
 #include "phx_common.cuh"
 
@@ -238,23 +239,40 @@ __global__ void decay_kernel(const float* J, const float* y, const float* relum,
 }
 // m_bar[g] = mask[g] * sum_b g[b][g] * (J - y)[b][g].  from_f != 0: `f_nodecay` is the finished RHS value
 // f = fscale * relu(m) * (J - y) instead of J, and (J - y) is recovered per gene after the column sum
-// (mask[g] != 0  <=>  relu(m)[g] > 0).
+// (mask[g] != 0  <=>  relu(m)[g] > 0).  That division holds only while fscale * relu(m) and f are normal numbers: for a
+// tiny multiplier (1e-30, a subnormal) the product underflows and the cotangent would be lost, so such elements take
+// (J - y) from J recomputed as the fp32 dot product of the plain [S|P] row SP[b] with the WA row of the gene.
 __global__ void colsum_mult_kernel(const float* g, const float* f_nodecay, const float* y, const float* maskm, int B,
                                    int G, float* m_bar, int accumulate, int decay, int from_f, const float* relum,
-                                   float fscale) {
+                                   float fscale, const float* SP, const float* WA, int K2, int Hp, int H) {
     __shared__ float sh[CS][CS + 1];
     const int gg = blockIdx.x * CS + threadIdx.x;
-    const bool ok = gg < G;
-    float t = 0.f;
-    if (ok && decay)
+    const bool ok = gg < G && decay && maskm[gg] != 0.f;
+    const float den = ok && from_f ? fscale * relum[gg] : 0.f;
+    const bool den_normal = fabsf(den) >= FLT_MIN;
+    float t = 0.f, tj = 0.f;
+    if (ok)
         for (int b = threadIdx.y; b < B; b += CS) {
             size_t i = (size_t)b * G + gg;
-            t += from_f ? g[i] * f_nodecay[i] : g[i] * (f_nodecay[i] - y[i]);
+            if (!from_f) {
+                t += g[i] * (f_nodecay[i] - y[i]);
+            } else if (den_normal && !(fabsf(f_nodecay[i]) < FLT_MIN)) {
+                t += g[i] * f_nodecay[i];
+            } else {
+                float J = 0.f;
+                for (int k = 0; k < K2; ++k)
+                    if (k % Hp < H) J = fmaf(SP[(size_t)b * K2 + k], WA[(size_t)gg * K2 + k], J);
+                tj += g[i] * (J - y[i]);
+            }
         }
     t = colsum_fold(t, sh);
-    if (ok && threadIdx.y == 0) {
-        if (!decay || maskm[gg] == 0.f) t = 0.f;
-        else if (from_f) t = t / (fscale * relum[gg]);
+    if (from_f) {   // (uniform over the block)
+        __syncthreads();
+        tj = colsum_fold(tj, sh);
+    }
+    if (gg < G && threadIdx.y == 0) {
+        if (!ok) t = 0.f;
+        else if (from_f) t = (den_normal ? t / den : 0.f) + tj;
         m_bar[gg] = accumulate ? m_bar[gg] + t : t;
     }
 }
@@ -324,7 +342,7 @@ int phx_rhs_vjp_launch(int G, int H, int B, const PhxPacked& w, const float* y, 
     bool direct_f = false;
     if (tc) {
         // tensor cores: [S|P], gSP, the state cotangent and the un-decayed joint (phx_tc.cu); the K = B parameter
-        // contractions below stay on the fp32 path
+        // contractions below run there too (phx_tc_vjp_params_launch), the bias and multiplier column sums do not
         float* tcws = ws + rhs_base_floats(G, H, B);
         int rc = PHX_OK;
         if (!(accumulate_flags & 2))   // bit 1: the workspace still holds [S|P] (+ images) of this (weights, y)
@@ -409,7 +427,7 @@ int phx_rhs_vjp_launch(int G, int H, int B, const PhxPacked& w, const float* y, 
         if (pmask & PHX_P_M)
             colsum_mult_kernel<<<(G + CS - 1) / CS, dim3(CS, CS), 0, st>>>(g, direct_f ? f_out : J, y, w.maskm, B, G,
                                                                            grads + off.m, accumulate, decay, direct_f,
-                                                                           w.relum, fscale);
+                                                                           w.relum, fscale, SP, WA, K2, Hp, H);
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {

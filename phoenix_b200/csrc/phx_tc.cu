@@ -280,16 +280,23 @@ __device__ __forceinline__ void split_tf32_finite(float x, float& hi, float& lo)
     hi = __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u);
     lo = __uint_as_float((__float_as_uint(x - hi) + 0x1000u) & 0xffffe000u);
 }
-__device__ __forceinline__ float rcp_fast(float x) {   // MUFU.RCP, 1 ulp; callers pass x >= 1
+__device__ __forceinline__ float rcp_fast(float x) {   // MUFU.RCP, 1 ulp; callers pass 1 <= x <= 1 + HILL_RCP_MAX
     float r;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
+// rcp.approx.ftz flushes 1/x to 0 once it is subnormal (x > 2^126 ~ 8.5e37), which would give s = 0 for huge finite z.
+// Beyond this |z| the exactly rounded z / (1 + |z|) of the fp32 path (phx_rhs.cu::hill) is +-1 (1 / (1 + |z|) is far
+// below half an ulp of 1), and NaN for an infinite z: copysign(1, z) + (z - z) gives exactly that.
+constexpr float HILL_RCP_MAX = 1e30f;
 // soft-sign s = z / (1 + |z|), z = y - 0.5 (odenet.py:21-27): the denominator is >= 1, so the range handling of a generic
 // fast division is dead weight in the producers, which are instruction-bound
+__device__ __forceinline__ float softsign_z(float z, float az) {
+    return az <= HILL_RCP_MAX ? z * rcp_fast(1.0f + az) : copysignf(1.0f, z) + (z - z);
+}
 __device__ __forceinline__ float hill_s(float y) {
     const float z = y - 0.5f;
-    return z * rcp_fast(1.0f + fabsf(z));
+    return softsign_z(z, fabsf(z));
 }
 // l = log1p(s) (odenet.py:29-35).  With s = z / (1 + |z|):  log1p(s) = 2 atanh(u), u = s / (2 + s) = z / (2 + 2|z| + z),
 // so l needs ONE reciprocal and an odd series in u.  For |z| <= 0.65 (y in [-0.15, 1.15]: expression data live in [0, 1])
@@ -309,7 +316,7 @@ __device__ __forceinline__ float hill_l_series(float z, float az) {   // valid f
 __device__ __forceinline__ float hill_l(float y) {
     const float z = y - 0.5f, az = fabsf(z);
     if (az <= HILL_L_SERIES_MAX) return hill_l_series(z, az);
-    return log1pf(z * rcp_fast(1.0f + az));   // NaN lands here too
+    return log1pf(softsign_z(z, az));   // NaN lands here too
 }
 // The producers' conversion of four source values into hi / lo A-operand values.  The common case -- every value of the
 // WARP finite and, for the log1p branch, inside the series range -- is decided with ONE vote and runs as straight-line
@@ -325,7 +332,7 @@ __device__ __forceinline__ void convert4(const float (&x)[4], const float (&sc)[
         m = fmaxf(m, fabsf(v[j]));   // fmaxf drops a NaN operand: tested separately below
     }
     const bool fin = (v[0] - v[0]) + (v[1] - v[1]) + (v[2] - v[2]) + (v[3] - v[3]) == 0.f;   // false with any NaN / inf
-    const float lim = (!MODE && br) ? HILL_L_SERIES_MAX : 1e38f;
+    const float lim = MODE ? 1e38f : (br ? HILL_L_SERIES_MAX : HILL_RCP_MAX);
     if (__all_sync(0xffffffffu, fin && m <= lim)) {
         if (MODE) {
 #pragma unroll
@@ -1515,11 +1522,19 @@ void set_attrs() {
     done = true;
 }
 
-// partial[B x 2Hn] = A(src) x image^T, then the finishing pass (mode 0: bias/exp -> [S|P]; mode 1: * Pr -> gSP)
-// the branch-type contraction itself: part[slot][Mpad][2*Hn] = A(src) x image^T.  trans = 0: M = batch rows, K = genes;
-// trans = 1: M = genes, K = batch rows.  Returns the plan used (slot counts per half) through *plan.
-int launch_branch_mma(int mode, int trans, int G, int H, int B, int nterms, const float* src, const float* ascale,
-                      const float* bimg, float* spart, PhxTcBranchPlan* plan, cudaStream_t st) {
+// Launch configuration of one branch-type contraction, decided on the host: the K split (with the equal-cost split of
+// mode 1), the substitution of cached Hill planes, where the A operand lives (a ring of `a_stages` stages in tensor memory,
+// 0: shared-memory tiles) and the depth S1 of the shared-memory pipeline.  launch_branch_mma and phx_tc_launch_describe
+// both take it from here, so what the library reports is what it launches.
+struct BranchConfig {
+    PhxTcBranchPlan pl;
+    int mode;                   // after the cached-Hill substitution (mode 0 over cached planes runs as mode 1)
+    bool hill_cached;
+    int pair, a_stages, a_hi_col[4], a_lo_col[4];
+    size_t stage1, staging, running;
+    int S1;
+};
+int branch_config(int mode, int trans, int G, int H, int B, bool hill_cached, BranchConfig& c) {
     const int Hn = phx_tc_Hn(H);
     const int Kdim = trans ? B : G, Mdim = trans ? G : B;
     PhxTcBranchPlan pl = phx_tc_branch_plan(Kdim, Mdim);
@@ -1527,21 +1542,73 @@ int launch_branch_mma(int mode, int trans, int G, int H, int B, int nterms, cons
         pl.per_p = pl.per_s = pl.per_e;
         pl.ks_p = pl.ks_s = pl.ks_e;
     }
+    c.hill_cached = mode == 0 && hill_cached;
+    if (c.hill_cached) {   // cached Hill activations: a mode-1 launch over the two planes
+        mode = 1;
+        pl.per_p = pl.per_s = pl.per_e;
+        pl.ks_p = pl.ks_s = pl.ks_e;
+    }
+    c.pl = pl;
+    c.mode = mode;
+    c.pair = pair_mode();
+    for (int i = 0; i < 4; ++i) c.a_hi_col[i] = c.a_lo_col[i] = 0;
+    const int chunk = phx_tc_chunk();
+    const int Hb = c.pair ? Hn / 2 : Hn;   // B rows staged per CTA
+    c.a_stages = (!c.pair && ts_mode()) ? ts_plan(Hn, c.a_hi_col, c.a_lo_col) : 0;
+    int ts = c.a_stages > 0;
+    size_t stage1 = (size_t)2 * Hb * BK * 4;
+    // TS: single-buffered staging (4 lane quarters x 32 rows) and the running sum [Hn / 4][128] float4 behind it
+    size_t staging = trans ? 0 : (size_t)4 * 32 * (K1_PF * BK + 4) * sizeof(float);
+    size_t running = (size_t)Hn * 128 * sizeof(float);
+    if (ts && (PHX_SMEM_LIMIT - 256 - staging - running) / stage1 < 2) ts = 0;   // no room for a B ring: shared-memory A
+    // the tensor-memory form pays off through the overlapped chunk folds: a CTA needs at least two chunks of K (measured:
+    // 3 551 x 120 x 1 024, one chunk per CTA, is 3-15 % slower with it; 20 000 x 200 x 4 096 is 8 % faster)
+    if (ts && (pl.per_p > pl.per_s ? pl.per_p : pl.per_s) < 2 * chunk && !getenv("PHX_TC_TS_FORCE")) ts = 0;
+    if (!ts) {
+        c.a_stages = 0;
+        stage1 += K1_A_BYTES;
+        staging = trans ? 0 : (size_t)K1_PWARPS * 2 * 8 * (K1_PF * BK + 4) * sizeof(float);
+        running = 0;
+    }
+    int S1 = (int)((PHX_SMEM_LIMIT - 256 - staging - running) / stage1);
+    if (S1 > 6) S1 = 6;
+    if (const char* e = getenv("PHX_TC_STAGES")) {   // experiment
+        int v = atoi(e);
+        if (v >= 1 && v < S1) S1 = v;
+    }
+    c.stage1 = stage1; c.staging = staging; c.running = running; c.S1 = S1;
+    if (S1 < 1) {
+        phx_set_error("tc branch kernel: stage of %zu bytes does not fit", stage1);
+        return PHX_ERR_UNSUPPORTED;
+    }
+    return PHX_OK;
+}
+
+// the branch-type contraction itself: part[slot][Mpad][2*Hn] = A(src) x image^T.  trans = 0: M = batch rows, K = genes;
+// trans = 1: M = genes, K = batch rows.  Returns the plan used (slot counts per half) through *plan.
+int launch_branch_mma(int mode, int trans, int G, int H, int B, int nterms, const float* src, const float* ascale,
+                      const float* bimg, float* spart, PhxTcBranchPlan* plan, cudaStream_t st) {
+    const int Hn = phx_tc_Hn(H);
+    const int Kdim = trans ? B : G, Mdim = trans ? G : B;
     const float* src2 = nullptr;
-    if (mode == 0) {   // cached Hill activations of this very matrix: a mode-1 launch over the two planes
+    bool hill_cached = false;
+    if (mode == 0) {   // cached Hill activations of this very matrix
         std::lock_guard<std::mutex> lk(g_hill_mu);
         if (g_hill.x == src && g_hill.n == (size_t)G * B && g_hill.s && g_hill.l) {
-            mode = 1;
+            hill_cached = true;
             src = g_hill.s;
             src2 = g_hill.l;
             ascale = nullptr;
-            pl.per_p = pl.per_s = pl.per_e;
-            pl.ks_p = pl.ks_s = pl.ks_e;
         }
     }
+    BranchConfig cf;
+    const int rc = branch_config(mode, trans, G, H, B, hill_cached, cf);
+    const PhxTcBranchPlan& pl = cf.pl;
     *plan = pl;
+    if (rc != PHX_OK) return rc;
+    mode = cf.mode;
     BranchParams bp;
-    const int pair = pair_mode();
+    const int pair = cf.pair;
     bp.G = Kdim; bp.B = Mdim; bp.Bpad = phx_round_up(pl.mtiles, 2) * 128; bp.Hn = Hn; bp.KB1 = phx_tc_KB1(Kdim); bp.chunk = phx_tc_chunk();
     bp.ld = G;
     bp.nterms = nterms; bp.mode = mode; bp.ascale = ascale;
@@ -1556,33 +1623,15 @@ int launch_branch_mma(int mode, int trans, int G, int H, int B, int nterms, cons
 #endif
     bp.y = src; bp.y2 = src2; bp.w1img = bimg; bp.spart = spart;
     bp.prof = phx_tc_prof_buffer();
-    bp.a_stages = (!pair && ts_mode()) ? ts_plan(Hn, bp.a_hi_col, bp.a_lo_col) : 0;
-    int ts = bp.a_stages > 0;
-    size_t stage1 = (size_t)2 * Hb * BK * 4;
-    // TS: single-buffered staging (4 lane quarters x 32 rows) and the running sum [Hn / 4][128] float4 behind it
-    size_t staging = trans ? 0 : (size_t)4 * 32 * (K1_PF * BK + 4) * sizeof(float);
-    size_t running = (size_t)Hn * 128 * sizeof(float);
-    if (ts && (PHX_SMEM_LIMIT - 256 - staging - running) / stage1 < 2) ts = 0;   // no room for a B ring: shared-memory A
-    // the tensor-memory form pays off through the overlapped chunk folds: a CTA needs at least two chunks of K (measured:
-    // 3 551 x 120 x 1 024, one chunk per CTA, is 3-15 % slower with it; 20 000 x 200 x 4 096 is 8 % faster)
-    if (ts && (pl.per_p > pl.per_s ? pl.per_p : pl.per_s) < 2 * bp.chunk && !getenv("PHX_TC_TS_FORCE")) ts = 0;
-    if (!ts) {
-        bp.a_stages = 0;
-        stage1 += K1_A_BYTES;
-        staging = trans ? 0 : (size_t)K1_PWARPS * 2 * 8 * (K1_PF * BK + 4) * sizeof(float);
-        running = 0;
+    bp.a_stages = cf.a_stages;
+    for (int i = 0; i < 4; ++i) {
+        bp.a_hi_col[i] = cf.a_hi_col[i];
+        bp.a_lo_col[i] = cf.a_lo_col[i];
     }
+    const int ts = cf.a_stages > 0;
+    const size_t stage1 = cf.stage1, staging = cf.staging, running = cf.running;
     bp.stg_bytes = (unsigned)staging;
-    int S1 = (int)((PHX_SMEM_LIMIT - 256 - staging - running) / stage1);
-    if (S1 > 6) S1 = 6;
-    if (const char* e = getenv("PHX_TC_STAGES")) {   // experiment
-        int v = atoi(e);
-        if (v >= 1 && v < S1) S1 = v;
-    }
-    if (S1 < 1) {
-        phx_set_error("tc branch kernel: stage of %zu bytes does not fit", stage1);
-        return PHX_ERR_UNSUPPORTED;
-    }
+    const int S1 = cf.S1;
     bp.stages = S1;
     set_attrs();
     const size_t smem1 = (size_t)S1 * stage1 + 256 + staging + running;
@@ -1788,6 +1837,24 @@ int phx_tc_prior_loss_launch(int G, int H, int B, const PhxPacked& w, const floa
 }
 
 extern "C" void phx_tc_set_pair(int on) { g_pair = on ? 1 : 0; }
+
+// contraction (bits 0-1): 0 forward [S|P], 1 gSP, 2 Ws_bar | Wp_bar, 3 Wa_bar; bit 2: the activation operand is a pair of
+// cached Hill planes (contractions 0 and 2 only).  Same decision as the launch, under the same environment and pair mode.
+extern "C" int phx_tc_launch_describe(int contraction, int G, int H, int B, int32_t out[8]) {
+    const int c = contraction & 3;
+    const bool cached = (contraction & 4) != 0;
+    if (!out || contraction < 0 || contraction > 7 || (cached && (c & 1)) || G < 1 || H < 1 || B < 1 ||
+        phx_tc_Hn(H) > PHX_TC_MAX_HN) {
+        phx_set_error("tc_launch_describe: invalid argument");
+        return PHX_ERR_INVALID;
+    }
+    BranchConfig cf;
+    const int rc = branch_config(c & 1, c >> 1, G, H, B, cached, cf);
+    if (rc != PHX_OK) return rc;
+    out[0] = cf.pl.mtiles; out[1] = cf.pl.ks_p; out[2] = cf.pl.per_p; out[3] = cf.pl.ks_s; out[4] = cf.pl.per_s;
+    out[5] = cf.pl.slots; out[6] = cf.a_stages; out[7] = cf.S1;
+    return PHX_OK;
+}
 
 extern "C" void phx_tc_prof_dump(void) {
     if (!g_prof) return;
